@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm (CUDA, libwofdm.so)
     python bench.py --impl reference [--steps K] [--warmup W]      # CPU arm: port of the reference's loop
     torchrun --nproc-per-node N ... bench.py --gpus N ...          # N > 1: one rank per GPU
+    python bench.py ... --dump-outputs DIR                         # + the last timed step's counters as DIR/*.npy
 
 A step = one pass of the BER chain over one batch of BASELINE.json configs[1] -- wtx-OFDM, N=256, cp=16, tail_tx=8,
 16-QAM, optimised-Tx-window stand-in, the full channel set (250 Vehicular-A realisations, 21 taps), 30 SNR points
@@ -23,6 +24,7 @@ import math
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -30,6 +32,7 @@ import numpy as np
 
 REPO = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REPO)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 METRIC = "w-OFDM BER Monte Carlo OFDM symbols/s"
 UNIT = "OFDM symbols/s"
@@ -131,8 +134,15 @@ class ClockSampler:
                 "power_w_median": float(np.median(pw)), "power_w_max": max(pw)}
 
 
+_NUMBA_CACHE = None
+
+
 def cpu_port_throughput(budget_s, workers):
     """The CPU port of the reference's loop (oracle/wofdm_cpu_port.py) on a bounded sample of the workload."""
+    global _NUMBA_CACHE
+    if "NUMBA_CACHE_DIR" not in os.environ:              # numba would cache the port next to its source, in the tree
+        _NUMBA_CACHE = tempfile.TemporaryDirectory(prefix="wofdm_numba_")
+        os.environ["NUMBA_CACHE_DIR"] = _NUMBA_CACHE.name
     from oracle import wofdm_cpu_port as P
     c = CFG
     chan, snr = workload_inputs(c)
@@ -348,7 +358,14 @@ def main():
                     help="weak (default): per-GPU work fixed; strong: the one-GPU batch sharded over the GPUs")
     ap.add_argument("--workload", default="configs1", choices=["configs1", "configs4"],
                     help="configs1 = BASELINE's headline configuration (default); configs4 = the N=1024 stress case")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the counters of the last timed step (bit_err, bit_tot, sym_err, sym_tot per SNR point) "
+                         "as DIR/<name>.npy, float64, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the CPU arm times a sample of the workload, not the timed GPU path")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -398,6 +415,10 @@ def main():
     be, se = job.plan.read()
     bt, st_ = job.plan.totals(job.ens_total, job.shard if world == 1 else (0, 1))
     # (N > 1: the in-place all-reduce left the job-wide counters in every rank's device buffer)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in (("bit_err", be), ("bit_tot", bt), ("sym_err", se), ("sym_tot", st_)):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.asarray(a, dtype=np.float64))   # exact below 2**53
 
     # ---------------- end-to-end arm: C-ABI call with HOST buffers, copies inside the timed region ----------------
     pin = lambda a: torch.from_numpy(np.ascontiguousarray(a)).pin_memory().numpy()

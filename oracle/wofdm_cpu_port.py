@@ -1,7 +1,7 @@
 """CPU port of the reference's Monte-Carlo loop for TIMING  --  TEST/BENCH INFRASTRUCTURE ONLY.
 
 ``bench.py``'s ``cpu_baseline`` leg and ``bench.py --impl reference`` time this module on the GPU
-box's host cores (the reference itself is Python under /root/reference and does not travel).  It
+box's host cores (the reference itself is not part of this repository).  It
 restates python/ofdm_utils/wofdm_simulation.py:171-240 with the reference's own cost profile:
 numba-jitted, single-threaded per task, dense ``tx_mat @ X`` / ``rx_mat @ frame`` products
 (:187, :221), ``np.convolve`` (:206), exact-SNR AWGN (:135-138), and the 16-way ``argmin |sym - x|``

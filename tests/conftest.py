@@ -12,7 +12,6 @@ GOLDEN = os.path.join(REPO, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (builder container only)")
 
 
 @pytest.fixture(scope="session")

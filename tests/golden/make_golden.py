@@ -1,8 +1,7 @@
-"""Generate tests/golden/*.npz by executing the REFERENCE itself (this container only).
+"""Generate tests/golden/*.npz by executing the REFERENCE itself.
 
-Run:  python -B tests/golden/make_golden.py
-Needs /root/reference (read-only; imported with bytecode writing disabled).  The GPU box
-has no /root/reference: tests read only the committed .npz files.
+Run:  WOFDM_REFERENCE=<checkout of felipescoelho/w-ofdm-optimization> python -B tests/golden/make_golden.py
+The reference is imported read-only (bytecode writing disabled); tests read only the committed .npz files.
 
 What is stored
 * ser_<sys>.npz     -- inputs + the SER vectors returned by the reference's own Monte-Carlo
@@ -20,7 +19,7 @@ import tempfile
 sys.dont_write_bytecode = True
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
-sys.path.insert(0, "/root/reference/python")
+sys.path.insert(0, os.path.join(os.environ["WOFDM_REFERENCE"], "python"))
 sys.path.insert(0, REPO)
 
 import numpy as np  # noqa: E402

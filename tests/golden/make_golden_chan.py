@@ -2,13 +2,13 @@
 channel_model.gen_chan (python/channel_model/itur_channels.py:33-94) under np.random.seed; the phases it drew are
 recovered by replaying the same seed (np.random.randn(1) per oscillator part, rayleigh_fading.py:95-98).
 
-Run:  python -B tests/golden/make_golden_chan.py      (this container only; needs /root/reference)"""
+Run:  WOFDM_REFERENCE=<checkout of felipescoelho/w-ofdm-optimization> python -B tests/golden/make_golden_chan.py"""
 import os
 import sys
 
 sys.dont_write_bytecode = True
 HERE = os.path.dirname(os.path.abspath(__file__))
-sys.path.insert(0, "/root/reference/python")
+sys.path.insert(0, os.path.join(os.environ["WOFDM_REFERENCE"], "python"))
 import numpy as np  # noqa: E402
 from channel_model.itur_channels import gen_chan, CHANNEL_ITUR  # noqa: E402
 

@@ -2,13 +2,13 @@
 OptimizerTx / OptimizerRx / OptimizerTxRx .gen_hessian (python/optimization_tools/optimizers.py) on a small system
 (N = 64) so that the reference's O(n^2 N^2) loops finish in seconds.
 
-Run:  python -B tests/golden/make_golden_hessian.py      (this container only; needs /root/reference)"""
+Run:  WOFDM_REFERENCE=<checkout of felipescoelho/w-ofdm-optimization> python -B tests/golden/make_golden_hessian.py"""
 import os
 import sys
 
 sys.dont_write_bytecode = True
 HERE = os.path.dirname(os.path.abspath(__file__))
-sys.path.insert(0, "/root/reference/python")
+sys.path.insert(0, os.path.join(os.environ["WOFDM_REFERENCE"], "python"))
 import numpy as np  # noqa: E402
 from optimization_tools.optimizers import OptimizerTx, OptimizerRx, OptimizerTxRx  # noqa: E402
 

@@ -2,13 +2,13 @@
 wOFDMSystem.estimate_obr (python/ofdm_utils/timefreq_simulation.py:216-296) under np.random.seed; the symbols it drew
 are recovered by replaying the same seed (its first and only RNG call is np.random.choice(symbols, (N - 96, 256))).
 
-Run:  python -B tests/golden/make_golden_psd.py      (this container only; needs /root/reference)"""
+Run:  WOFDM_REFERENCE=<checkout of felipescoelho/w-ofdm-optimization> python -B tests/golden/make_golden_psd.py"""
 import os
 import sys
 
 sys.dont_write_bytecode = True
 HERE = os.path.dirname(os.path.abspath(__file__))
-sys.path.insert(0, "/root/reference/python")
+sys.path.insert(0, os.path.join(os.environ["WOFDM_REFERENCE"], "python"))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 import numpy as np  # noqa: E402
 from ofdm_utils.timefreq_simulation import wOFDMSystem  # noqa: E402

@@ -4,14 +4,14 @@ enough frames that a production run of the device kernel (its own Philox draws) 
 the reference's confidence interval at every SNR point (north star: "BER must fall within the 95 % CI of the
 reference").  Stores the inputs, the reference's SER (optimised and RC windows) and the number of frames behind it.
 
-Run:  python -B tests/golden/make_golden_stat.py      (this container only; needs /root/reference; ~2 min)"""
+Run:  WOFDM_REFERENCE=<checkout of felipescoelho/w-ofdm-optimization> python -B tests/golden/make_golden_stat.py   (~2 min)"""
 import os
 import sys
 
 sys.dont_write_bytecode = True
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
-sys.path.insert(0, "/root/reference/python")
+sys.path.insert(0, os.path.join(os.environ["WOFDM_REFERENCE"], "python"))
 sys.path.insert(0, REPO)
 sys.path.insert(0, HERE)
 import numpy as np  # noqa: E402

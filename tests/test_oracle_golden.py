@@ -34,6 +34,23 @@ def test_single_frames_match_reference_counts(name):
                 assert res.sym_err == int(round(want)), (name, snr, w, chain.__name__)
 
 
+@pytest.mark.parametrize("name", ["WOLA", "CPwtx", "wrx"])
+def test_replay_at_cp22_matches_stored_vectors(name):
+    """np.random replayed at cp = 22, S = 3 (tests/golden/make_golden_replay.py): the dense AND the structured form must
+    give the stored SER vectors bit for bit.  The stored file names its source: as committed it is the oracle's dense
+    replay (the reference could not be run when it was made), so this pins the oracle against drift and the structured
+    form against the dense one; regenerated from the reference it checks both against the reference."""
+    g = np.load(f"{GOLDEN}/ser_replay.npz")
+    ttx = 8 if name in ("CPW", "WOLA", "CPwtx", "wtx") else 0
+    trx = 10 if name in ("CPW", "WOLA", "CPwrx", "wrx") else 0
+    p = O.system_params(name, int(g["N"]), int(g["cp"]), ttx, trx, S=int(g["S"]))
+    wins = [(g[f"{name}_v_tx"], g[f"{name}_v_rx"]), (O.rc_window_tx(p), O.rc_window_rx(p))]
+    for dense in (True, False):
+        np.random.seed(int(g[f"{name}_seed"]))
+        ser = O.ser_sweep_replay(p, wins, g[f"{name}_channels"], int(g["ensemble"]), g["snr"], dense=dense)
+        assert np.array_equal(ser, g[f"{name}_ser"]), (name, dense, str(g["source"]))
+
+
 @pytest.mark.parametrize("name", O.SYSTEMS)
 def test_structured_equals_dense(name):
     g = load_ser_golden(name)
