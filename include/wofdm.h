@@ -223,6 +223,25 @@ WOFDM_API int wofdm_window_hessian(wofdm_handle h, const wofdm_sys_t* sys, const
  *   HTx (or HRx) = alpha * H_ici + (1 - alpha) * diag(row sums of H_isi)       (H2 = real(diag(diag(B2' B2 C C'))), :628-631). */
 WOFDM_API int wofdm_window_hessian_parts(wofdm_handle h, const wofdm_sys_t* sys, const double* chan, int L,
                                const double* basis_tx, int n_tb, const double* basis_rx, int n_rb, double* H_ici, double* H_isi);
+/* Mean over a channel set of wofdm_window_hessian: H = (1/C) sum_c H(h_c), the quadratic form of the EXPECTED interference
+ * power over the set (the reference optimises against the mean impulse response, one random channel of covariance R/C).
+ * chan: complex L x C column-major (channels/vehicularA.npy layout).  Same variable order, same n_var.
+ * H(h) is a linear function of h h^H, so the mean equals sum_j H(g_j) for any factor sum_j g_j g_j^H of the sample tap
+ * covariance R = (1/C) sum_c h_c h_c^H.  C <= L: the channels themselves (C passes, weight 1/C; C = 1 gives exactly
+ * wofdm_window_hessian).  C > L: R is formed in fp64 on the host and factored by a pivoted Cholesky decomposition into
+ * r = rank(R) <= L virtual channels; directions whose remaining variance is at most 1e-14 of the largest diagonal entry of
+ * R are dropped.  One pass of the device pipeline per virtual channel, the Gram products summed on the device, one download.
+ * Runs on device slot 0 of the handle only (a multi-device handle gives the single-device result).
+ * WOFDM_EINVAL: C < 1, NULL buffers, non-finite taps, or what wofdm_window_hessian rejects; N % 64 != 0: WOFDM_EUNSUPPORTED. */
+WOFDM_API int wofdm_window_hessian_set(wofdm_handle h, const wofdm_sys_t* sys, const double* chan, int L, int C, double* H, int* n_var);
+/* Mean over the set of the two parts of wofdm_window_hessian_parts (arbitrary bases, MATLAB quad_objective semantics): same
+ * factor and passes as wofdm_window_hessian_set, H_ici and H_isi each the mean of the per-channel parts. */
+WOFDM_API int wofdm_window_hessian_parts_set(wofdm_handle h, const wofdm_sys_t* sys, const double* chan, int L, int C,
+                                             const double* basis_tx, int n_tb, const double* basis_rx, int n_rb, double* H_ici, double* H_isi);
+/* Of the handle's last wofdm_window_hessian* call: device time from the first upload to the end of the download (CUDA events
+ * on its stream, ms; -1 = not taken), host time of the channel-set factorisation (ms; 0 for a single channel) and the passes
+ * of the device pipeline (virtual channels).  Any may be NULL. */
+WOFDM_API int wofdm_window_hessian_last_timing(wofdm_handle h, double* device_ms, double* factor_ms, int* passes);
 
 /* ---- Channel generation (next-row 8f-4) ------------------------------------------------------------------
  * ITU-R tapped-delay-line channels with GMEDS_1 Rayleigh fading on the device: channel_model.gen_chan

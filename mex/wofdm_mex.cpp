@@ -15,6 +15,8 @@
 //   berSNR = wofdm_mex('run_simulation_sweep_multi', ...)   every window variant of a (system, CP) on the same bits, one job
 //   [berMasked, ber] = wofdm_mex('run_sim_mc', ...)          run_sim_mc of matlab/main_channel_mask.m:334-337
 //   H = wofdm_mex('window_hessian', ...)                     quad_objective_tx / _rx of matlab/window_optimization.m:596-680
+//   H = wofdm_mex('window_hessian_expected', ...), 'quad_objective_tx_expected', 'quad_objective_rx_expected'
+//       -- the same, averaged over a channel set (C x L, rows = realisations) instead of built from one impulse response
 //   channels = wofdm_mex('gen_channels', ...)                the stored channel sets' generator
 //       (argument lists at the functions below)
 // Windows arrive as dense diagonal matrices (or vectors); channels as rows = realisations.
@@ -73,6 +75,19 @@ static std::vector<double> interleave(const mxArray* a, size_t count, size_t str
         z[2 * i + 1] = im ? im[offset + i * stride] : 0.0;
     }
     return z;
+}
+
+// channels(channelIndex, :) (C x L, rows = realisations) -> column-major L x C complex
+static std::vector<double> channel_rows(const mxArray* a, int* L, int* C) {
+    const size_t c_n = mxGetM(a), l_n = mxGetN(a);
+    std::vector<double> chan(2 * l_n * c_n);
+    for (size_t c = 0; c < c_n; ++c) {
+        const std::vector<double> row = interleave(a, l_n, c_n, c);
+        memcpy(chan.data() + 2 * l_n * c, row.data(), 2 * l_n * sizeof(double));
+    }
+    *L = (int)l_n;
+    *C = (int)c_n;
+    return chan;
 }
 
 // sweep = false: one channel (vector), one SNR -> scalar; sweep = true: C x L channel matrix, SNR vector -> n_snr x 1
@@ -216,7 +231,9 @@ static void do_run_sim_mc(int nlhs, mxArray* plhs[], int nrhs, const mxArray* pr
 //      python's OptimizerTx/Rx/TxRx.gen_hessian builds it.  channel: ONE impulse response.  (quad_objective_tx / _rx of
 //      matlab/window_optimization.m:596-680 work in the full window variable with the other window fixed, weight the
 //      two terms with alpha and keep only the diagonal of the ISI term: 'quad_objective_tx' / 'quad_objective_rx' below.)
-static void do_window_hessian(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
+// H = wofdm_mex('window_hessian_expected', typeOFDM, numSubcar, cpLength, tailTx, tailRx, channels)
+//   -- the same averaged over the channel set (C x L, rows = realisations): the expected interference over the set.
+static void do_window_hessian(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[], bool expected) {
     if (nrhs < 6) mexErrMsgIdAndTxt("wofdm:nargin", "window_hessian needs 6 arguments");
     (void)nlhs;
     char name[16];
@@ -227,11 +244,17 @@ static void do_window_hessian(int nlhs, mxArray* plhs[], int nrhs, const mxArray
     if (wofdm_params_from_name(name, (int)mxGetScalar(prhs[1]), (int)mxGetScalar(prhs[2]), (int)mxGetScalar(prhs[3]),
                                (int)mxGetScalar(prhs[4]), &s) != WOFDM_OK)
         mexErrMsgIdAndTxt("wofdm:type", "unknown typeOFDM '%s'", name);
-    const int L = (int)mxGetNumberOfElements(prhs[5]);
-    const std::vector<double> chan = interleave(prhs[5], (size_t)L, 1, 0);
     const int n_var = (s.tail_rx / 2 + 1) * (s.tail_tx + 1);
     plhs[0] = mxCreateDoubleMatrix((mwSize)n_var, (mwSize)n_var, mxREAL);
     int nv = 0;
+    if (expected) {
+        int L = 0, C = 0;
+        const std::vector<double> chan = channel_rows(prhs[5], &L, &C);
+        check(wofdm_window_hessian_set(handle(), &s, chan.data(), L, C, mxGetPr(plhs[0]), &nv), "wofdm_window_hessian_set");
+        return;
+    }
+    const int L = (int)mxGetNumberOfElements(prhs[5]);
+    const std::vector<double> chan = interleave(prhs[5], (size_t)L, 1, 0);
     check(wofdm_window_hessian(handle(), &s, chan.data(), L, mxGetPr(plhs[0]), &nv), "wofdm_window_hessian");
 }
 
@@ -241,7 +264,9 @@ static void do_window_hessian(int nlhs, mxArray* plhs[], int nrhs, const mxArray
 //      (n_tx, or N + tailRx, entries), the other side's window (diagonal matrix or vector) is fixed:
 //      H = 2 (alpha H1 + (1 - alpha) H2), H1 the off-diagonal ICI term, H2 = real(diag(diag(.))) of the ISI term (:628-631).
 //      channel: ONE impulse response (the script passes array_ici_isi of the mean channel; the device builds those matrices).
-static void do_quad_objective(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[], bool tx_side) {
+// HTx = wofdm_mex('quad_objective_tx_expected', <the same arguments with channels C x L, rows = realisations>), and _rx:
+//      the mean over the set of quad_objective_tx / _rx (the formula is linear in the two parts, so their means suffice).
+static void do_quad_objective(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[], bool tx_side, bool expected) {
     if (nrhs < 8) mexErrMsgIdAndTxt("wofdm:nargin", "quad_objective_tx / _rx need 8 arguments");
     (void)nlhs;
     char name[16];
@@ -255,14 +280,23 @@ static void do_quad_objective(int nlhs, mxArray* plhs[], int nrhs, const mxArray
     const size_t n_tx = (size_t)(s.N + s.cp + s.cs), n_w = (size_t)(s.N + s.tail_rx);
     const size_t n = tx_side ? n_tx : n_w;                       // variables: the full window of this side
     const std::vector<double> fixed = diag_of(prhs[5], tx_side ? n_w : n_tx);
-    const int L = (int)mxGetNumberOfElements(prhs[6]);
-    const std::vector<double> chan = interleave(prhs[6], (size_t)L, 1, 0);
     const double alpha = mxGetScalar(prhs[7]);
     std::vector<double> eye(n * n, 0.0), hc(n * n), hs(n * n);
     for (size_t i = 0; i < n; ++i) eye[i * n + i] = 1.0;
-    check(wofdm_window_hessian_parts(handle(), &s, chan.data(), L, tx_side ? eye.data() : fixed.data(), tx_side ? (int)n : 1,
-                                     tx_side ? fixed.data() : eye.data(), tx_side ? 1 : (int)n, hc.data(), hs.data()),
-          "wofdm_window_hessian_parts");
+    const double* bt = tx_side ? eye.data() : fixed.data();
+    const double* br = tx_side ? fixed.data() : eye.data();
+    const int n_tb = tx_side ? (int)n : 1, n_rb = tx_side ? 1 : (int)n;
+    if (expected) {
+        int L = 0, C = 0;
+        const std::vector<double> chan = channel_rows(prhs[6], &L, &C);
+        check(wofdm_window_hessian_parts_set(handle(), &s, chan.data(), L, C, bt, n_tb, br, n_rb, hc.data(), hs.data()),
+              "wofdm_window_hessian_parts_set");
+    } else {
+        const int L = (int)mxGetNumberOfElements(prhs[6]);
+        const std::vector<double> chan = interleave(prhs[6], (size_t)L, 1, 0);
+        check(wofdm_window_hessian_parts(handle(), &s, chan.data(), L, bt, n_tb, br, n_rb, hc.data(), hs.data()),
+              "wofdm_window_hessian_parts");
+    }
     plhs[0] = mxCreateDoubleMatrix((mwSize)n, (mwSize)n, mxREAL);
     double* H = mxGetPr(plhs[0]);
     for (size_t i = 0; i < n; ++i) {
@@ -324,14 +358,17 @@ static void do_calculate_interference(int nlhs, mxArray* plhs[], int nrhs, const
 extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     char cmd[32];
     if (nrhs < 1 || !mxIsChar(prhs[0]) || mxGetString(prhs[0], cmd, sizeof(cmd)))
-        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_sim_mc', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx' or 'gen_channels'");
+        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_sim_mc', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
     if (!strcmp(cmd, "run_simulation")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_simulation_sweep")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, true);
     else if (!strcmp(cmd, "run_simulation_sweep_multi")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1);
     else if (!strcmp(cmd, "run_sim_mc")) do_run_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1);
-    else if (!strcmp(cmd, "window_hessian")) do_window_hessian(nlhs, plhs, nrhs - 1, prhs + 1);
-    else if (!strcmp(cmd, "quad_objective_tx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, true);
-    else if (!strcmp(cmd, "quad_objective_rx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, false);
+    else if (!strcmp(cmd, "window_hessian")) do_window_hessian(nlhs, plhs, nrhs - 1, prhs + 1, false);
+    else if (!strcmp(cmd, "quad_objective_tx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, true, false);
+    else if (!strcmp(cmd, "quad_objective_rx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, false, false);
+    else if (!strcmp(cmd, "window_hessian_expected")) do_window_hessian(nlhs, plhs, nrhs - 1, prhs + 1, true);
+    else if (!strcmp(cmd, "quad_objective_tx_expected")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, true, true);
+    else if (!strcmp(cmd, "quad_objective_rx_expected")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, false, true);
     else if (!strcmp(cmd, "gen_channels")) do_gen_channels(nlhs, plhs, nrhs - 1, prhs + 1);
     else if (!strcmp(cmd, "calculate_interference")) do_calculate_interference(nlhs, plhs, nrhs - 1, prhs + 1);
     else mexErrMsgIdAndTxt("wofdm:usage", "unknown command '%s'", cmd);

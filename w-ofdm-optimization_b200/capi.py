@@ -98,6 +98,10 @@ SIGNATURES = {
                                        C.c_uint32, C.c_int, _i64p, _i64p, _i64p, _i64p]),
     "wofdm_window_hessian": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, _dp, _P(C.c_int)]),
     "wofdm_window_hessian_parts": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, _dp, C.c_int, _dp, C.c_int, _dp, _dp]),
+    "wofdm_window_hessian_set": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, C.c_int, _dp, _P(C.c_int)]),
+    "wofdm_window_hessian_parts_set": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, C.c_int, _dp, C.c_int, _dp, C.c_int,
+                                                 _dp, _dp]),
+    "wofdm_window_hessian_last_timing": (C.c_int, [C.c_void_p, _dp, _dp, _P(C.c_int)]),
     "wofdm_channel_profile": (C.c_int, [C.c_char_p]),
     "wofdm_gen_channels": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_double, C.c_double, C.c_double, C.c_int, C.c_int,
                                      C.c_uint64, _dp, _dp]),
@@ -387,6 +391,48 @@ class Handle:
                                                _ptr(br, _dp), br.shape[0], _ptr(Hc, _dp), _ptr(Hs, _dp))
         self._check(rc)
         return Hc, Hs
+
+    @staticmethod
+    def _chan_set(chans):
+        """(L, C) channel set (a 1-D array is one channel) -> contiguous (C, L) complex128 == L x C column-major, L, C"""
+        ch = np.asarray(chans)
+        if ch.ndim == 1:
+            ch = ch[:, None]
+        if ch.ndim != 2:
+            raise WofdmError(EINVAL, "channel set must be an (L, C) array")
+        return _cplx(ch.T), ch.shape[0], ch.shape[1]
+
+    def window_hessian_set(self, s, chans):
+        """Mean over the channel set chans (L, C) of window_hessian (wofdm_window_hessian_set): the quadratic form of the
+        expected interference power over the set, (n_var, n_var), same variable order as window_hessian."""
+        chf, L, Cn = self._chan_set(chans)
+        n_var = (s.tail_rx // 2 + 1) * (s.tail_tx + 1)
+        H = np.empty((n_var, n_var))
+        nv = C.c_int(0)
+        rc = load().wofdm_window_hessian_set(self._h, C.byref(s), _ptr(chf, _dp), L, Cn, _ptr(H, _dp), C.byref(nv))
+        self._check(rc)
+        assert nv.value == n_var
+        return H
+
+    def window_hessian_parts_set(self, s, chans, basis_tx, basis_rx):
+        """Mean over the channel set chans (L, C) of window_hessian_parts (wofdm_window_hessian_parts_set) -> (H_ici, H_isi)."""
+        chf, L, Cn = self._chan_set(chans)
+        bt = np.ascontiguousarray(np.atleast_2d(basis_tx), dtype=np.float64)
+        br = np.ascontiguousarray(np.atleast_2d(basis_rx), dtype=np.float64)
+        if bt.shape[1] != s.n_tx or br.shape[1] != s.N + s.tail_rx:
+            raise WofdmError(EINVAL, f"basis windows must have {s.n_tx} (Tx) and {s.N + s.tail_rx} (Rx) samples")
+        n_var = bt.shape[0] * br.shape[0]
+        Hc, Hs = np.empty((n_var, n_var)), np.empty((n_var, n_var))
+        rc = load().wofdm_window_hessian_parts_set(self._h, C.byref(s), _ptr(chf, _dp), L, Cn, _ptr(bt, _dp), bt.shape[0],
+                                                   _ptr(br, _dp), br.shape[0], _ptr(Hc, _dp), _ptr(Hs, _dp))
+        self._check(rc)
+        return Hc, Hs
+
+    def window_hessian_last_timing(self):
+        """dict(device_ms, factor_ms, passes) of the last window_hessian* call (wofdm_window_hessian_last_timing)."""
+        t, f, n = C.c_double(), C.c_double(), C.c_int()
+        self._check(load().wofdm_window_hessian_last_timing(self._h, C.byref(t), C.byref(f), C.byref(n)))
+        return dict(device_ms=t.value, factor_ms=f.value, passes=n.value)
 
     def gen_channels(self, standard, L, doppler_freq, sampling_rate, frame_duration, no_frames=1, n_sets=1, seed=0,
                      phases=None):

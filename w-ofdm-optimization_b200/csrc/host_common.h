@@ -36,6 +36,11 @@ struct wofdm_ctx {
     cudaEvent_t interf_ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     double interf_ms[3] = {-1.0, -1.0, -1.0};
     double interf_k_isi = 0.0, interf_kp = 0.0;      // K rows contracted per ISI slice / per slice 0
+    // last wofdm_window_hessian* call: device time (uploads to download, CUDA events), host time of the channel-set
+    // factorisation, passes of the device pipeline (virtual channels); -1 / 0 = not taken
+    cudaEvent_t hess_ev[2] = {nullptr, nullptr};
+    double hess_ms = -1.0, hess_factor_ms = 0.0;
+    int hess_passes = 0;
 };
 
 namespace wofdm {

@@ -15,6 +15,7 @@
 //       dimension, with the off-diagonal mask and the row-wise sum of |.|^2 fused into the epilogue.
 // The TF32-split tensor path (mode 1) lives in interf_tf32.cu.
 #include <algorithm>
+#include <chrono>
 #include <cstdlib>
 #include <type_traits>
 
@@ -493,8 +494,9 @@ __global__ void __launch_bounds__(256) quad_w_kernel(const double2* __restrict__
 // P[c][k] = sum_f wf[c][f] qf[k][f]: a TS x TS tile per CTA (64, or 32 when 64 would leave most SMs idle), RT x RT outputs
 // per thread, F in tiles of 16 (plain FP64 FMAs: the product is C x L(L+1) x N, 0.06 GFLOP for the 250 channels of
 // configs[3]).  scalar: the row sum over k instead.
-// (also the Gram product of the window Hessian's parts: ldw / ldq = row pitches, F = features contracted, scale on the way out)
-template <int TS>
+// (also the Gram product of the window Hessian's parts: ldw / ldq = row pitches, F = features contracted, scale on the way out;
+// ACC: P += scale * product instead of P = ..., for the channel-set Hessian's passes after the first -- non-scalar only)
+template <int TS, bool ACC = false>
 __global__ void __launch_bounds__(256) quad_eval_kernel(const double* __restrict__ wf, const double* __restrict__ qf,
                                                         double* __restrict__ P, int N, int C, int F, int scalar,
                                                         size_t ldw, size_t ldq, double scale) {
@@ -543,7 +545,11 @@ __global__ void __launch_bounds__(256) quad_eval_kernel(const double* __restrict
             atomicAdd(&P[c], scale * sum);
         } else {
 #pragma unroll
-            for (int j = 0; j < RT; ++j) if (k0 + RT * tx + j < N) P[(size_t)c * N + k0 + RT * tx + j] = scale * acc[i][j];
+            for (int j = 0; j < RT; ++j) {
+                if (k0 + RT * tx + j >= N) continue;
+                double* const o = P + (size_t)c * N + k0 + RT * tx + j;
+                *o = ACC ? *o + scale * acc[i][j] : scale * acc[i][j];
+            }
         }
     }
 }
@@ -648,6 +654,9 @@ static int interf_run_quad(wofdm_handle h, const wofdm_sys_t* sys, const double*
 // pair u = (Rx basis a, Tx basis b) on slice 0 / on the sum of the ISI slices.  Replaces the O(n^2 N^2) loops of
 // OptimizerTx/Rx/TxRx.gen_hessian (python/optimization_tools/optimizers.py:132-175, 232-257, 427-507, 808-833) and
 // quad_objective_tx/_rx (matlab/window_optimization.m:596-680).  X[u][ms][2N][N] holds [Re A; Im A].
+// ACC: H += the Gram entries (passes after the first of a channel set); otherwise H = them, so that whatever H held before
+// never enters the sum.
+template <bool ACC>
 __global__ void __launch_bounds__(256) gram_offdiag(const double* __restrict__ X, double* __restrict__ H, int n_var, int N,
                                                     int n_tb) {
     __shared__ double red[256];
@@ -673,7 +682,16 @@ __global__ void __launch_bounds__(256) gram_offdiag(const double* __restrict__ X
         if (threadIdx.x < st) red[threadIdx.x] += red[threadIdx.x + st];
         __syncthreads();
     }
-    if (threadIdx.x == 0) { H[(size_t)u * n_var + up] = 2.0 * red[0]; H[(size_t)up * n_var + u] = 2.0 * red[0]; }
+    if (threadIdx.x == 0) {
+        const double g = 2.0 * red[0];
+        if (ACC) {
+            H[(size_t)u * n_var + up] += g;
+            if (up != u) H[(size_t)up * n_var + u] += g;          // (a diagonal entry is one element: add once)
+        } else {
+            H[(size_t)u * n_var + up] = g;
+            H[(size_t)up * n_var + u] = g;
+        }
+    }
     (void)n_tb;
 }
 
@@ -686,10 +704,16 @@ __global__ void zero_diag_kernel(double* __restrict__ X, int n_var, int N) {
 
 // bt: n_tb Tx windows (n_tx each), br: n_rb Rx windows (N + tail_rx each), host.  H_out (sum of the parts, gram_offdiag) or
 // the parts H_ici / H_isi (Gram products through quad_eval_kernel); n_var = n_rb * n_tb, u = a * n_tb + b.
-static int window_hessian_core(wofdm_handle h, const wofdm_sys_t* sys, const double* chan, int L, const double* bt_h, int n_tb,
-                               const double* br_h, int n_rb, double* H_out, double* H_ici, double* H_isi) {
+// chan: r impulse responses of L taps back to back; the result is the SUM over them of each one's Hessian: one pass of the
+// band product and the contraction per response, the first pass storing the Gram products and every later one adding to
+// them on the device.  The basis operands Tx_mat(t_b) / Rbig(r_a) do not depend on the channel and are built once.
+static int window_hessian_core(wofdm_handle h, const wofdm_sys_t* sys, const double* chan, int L, int r, const double* bt_h,
+                               int n_tb, const double* br_h, int n_rb, double* H_out, double* H_ici, double* H_isi) {
     DeviceCtx& d = h->devs[0];
     WOFDM_CUDA(h, cudaSetDevice(d.dev));
+    for (auto& e : h->hess_ev)
+        if (!e) WOFDM_CUDA(h, cudaEventCreate(&e));
+    WOFDM_CUDA(h, cudaEventRecord(h->hess_ev[0], d.stream));
     const int N = sys->N, n_tx = N + sys->cp + sys->cs, n_rx = n_tx - sys->tail_tx, n_w = N + sys->tail_rx;
     const int n_var = n_tb * n_rb;
     const int Kp = ((2 * n_rx + 63) / 64) * 64;
@@ -697,94 +721,199 @@ static int window_hessian_core(wofdm_handle h, const wofdm_sys_t* sys, const dou
     const int Ms = 2;                                          // slice 0 and the sum of the ISI slices
     const int k_isi = interf_isi_k(L, sys->tail_tx, n_rx, Kp);
     const size_t matb = (size_t)2 * N * N * 8;
-    const size_t need = (size_t)n_tb * n_tx * 8 + (size_t)n_rb * n_w * 8 + (size_t)L * 16 + (size_t)n_tx * N * 16 + (size_t)2 * N * Kp * 8 +
-                        (size_t)n_tb * Ms * Kp * N * 8 + (size_t)n_var * Ms * matb + (size_t)2 * n_var * n_var * 8;
+    const size_t t_one = (size_t)n_tx * N, r_one = (size_t)2 * N * Kp;     // elements of one Tx_mat (double2) / one Rbig
+    const size_t need = (size_t)n_tb * n_tx * 8 + (size_t)n_rb * n_w * 8 + (size_t)r * L * 16 + (size_t)n_tb * t_one * 16 +
+                        (size_t)n_rb * r_one * 8 + (size_t)n_tb * Ms * Kp * N * 8 + (size_t)n_var * Ms * matb + (size_t)2 * n_var * n_var * 8;
     int rc = arena_reserve(h, d, need);
     if (rc) return rc;
     double* d_bt = static_cast<double*>(arena_take(d, (size_t)n_tb * n_tx * 8));
     double* d_br = static_cast<double*>(arena_take(d, (size_t)n_rb * n_w * 8));
-    double2* d_chan = static_cast<double2*>(arena_take(d, (size_t)L * 16));
-    double2* d_T = static_cast<double2*>(arena_take(d, (size_t)n_tx * N * 16));
-    double* d_R = static_cast<double*>(arena_take(d, (size_t)2 * N * Kp * 8));
+    double2* d_chan = static_cast<double2*>(arena_take(d, (size_t)r * L * 16));
+    double2* d_T = static_cast<double2*>(arena_take(d, (size_t)n_tb * t_one * 16));
+    double* d_R = static_cast<double*>(arena_take(d, (size_t)n_rb * r_one * 8));
     double* d_B = static_cast<double*>(arena_take(d, (size_t)n_tb * Ms * Kp * N * 8));
     double* d_X = static_cast<double*>(arena_take(d, (size_t)n_var * Ms * matb));
     double* d_H = static_cast<double*>(arena_take(d, (size_t)2 * n_var * n_var * 8));
     if (!d_bt || !d_br || !d_chan || !d_T || !d_R || !d_B || !d_X || !d_H) return fail(h, WOFDM_ENOMEM, "arena exhausted");
     WOFDM_CUDA(h, cudaMemcpyAsync(d_bt, bt_h, (size_t)n_tb * n_tx * 8, cudaMemcpyHostToDevice, d.stream));
     WOFDM_CUDA(h, cudaMemcpyAsync(d_br, br_h, (size_t)n_rb * n_w * 8, cudaMemcpyHostToDevice, d.stream));
-    WOFDM_CUDA(h, cudaMemcpyAsync(d_chan, chan, (size_t)L * 16, cudaMemcpyHostToDevice, d.stream));
-    // B_{b,ms} = H_ms . Tx_mat(t_b) for every Tx basis window
-    for (int b = 0; b < n_tb; ++b) {
-        build_tx_matrix<<<n_tx, 256, 0, d.stream>>>(d_T, d_bt + (size_t)b * n_tx, N, sys->cp, n_tx);
-        build_b<false><<<dim3((N + 255) / 256, (Kp / 2 + BB - 1) / BB, Ms), 256, (size_t)(L + 2 * BB) * sizeof(double2), d.stream>>>(
-            d_B + (size_t)b * Ms * Kp * N, d_T, d_chan, L, N, n_tx, n_rx, n_rx, Kp, Ms, M, 0, 1, k_isi);
-    }
+    WOFDM_CUDA(h, cudaMemcpyAsync(d_chan, chan, (size_t)r * L * 16, cudaMemcpyHostToDevice, d.stream));
+    for (int b = 0; b < n_tb; ++b)
+        build_tx_matrix<<<n_tx, 256, 0, d.stream>>>(d_T + (size_t)b * t_one, d_bt + (size_t)b * n_tx, N, sys->cp, n_tx);
+    for (int a = 0; a < n_rb; ++a)
+        build_rx_matrix<<<N, 256, 0, d.stream>>>(d_R + (size_t)a * r_one, d_br + (size_t)a * n_w, N, sys->tail_rx, sys->rm, sys->shift, n_rx, Kp);
     WOFDM_CUDA(h, cudaGetLastError());
-    // X[a][b][ms] = Rbig(r_a) . B_{b,ms}: one stored contraction per Rx basis window over all Tx slices
     constexpr size_t smem = (size_t)(2 * BM * AS + 2 * BK * BS) * sizeof(double);
     WOFDM_CUDA(h, cudaFuncSetAttribute(gemm_power_f64<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    for (int a = 0; a < n_rb; ++a) {
-        build_rx_matrix<<<N, 256, 0, d.stream>>>(d_R, d_br + (size_t)a * n_w, N, sys->tail_rx, sys->rm, sys->shift, n_rx, Kp);
-        gemm_power_f64<true><<<dim3(N / BN, 2 * N / BM, n_tb * Ms), 256, smem, d.stream>>>(
-            d_R, d_B, d_X + (size_t)a * n_tb * Ms * 2 * N * N, N, Kp, Ms, 0, 0, k_isi);
-    }
-    WOFDM_CUDA(h, cudaGetLastError());
-    h->launches += 2 * n_tb + 2 * n_rb + 1;
-    if (H_out) {
-        gram_offdiag<<<n_var * (n_var + 1) / 2, 256, 0, d.stream>>>(d_X, d_H, n_var, N, n_tb);
+    const size_t mat = (size_t)2 * N * N;
+    const dim3 g((n_var + 63) / 64, (n_var + 63) / 64);
+    for (int v = 0; v < r; ++v) {
+        // B_{b,ms} = H_ms(g_v) . Tx_mat(t_b) for every Tx basis window (channel v of d_chan: c0 = v)
+        for (int b = 0; b < n_tb; ++b)
+            build_b<false><<<dim3((N + 255) / 256, (Kp / 2 + BB - 1) / BB, Ms), 256, (size_t)(L + 2 * BB) * sizeof(double2), d.stream>>>(
+                d_B + (size_t)b * Ms * Kp * N, d_T + (size_t)b * t_one, d_chan, L, N, n_tx, n_rx, n_rx, Kp, Ms, M, v, 1, k_isi);
+        // X[a][b][ms] = Rbig(r_a) . B_{b,ms}: one stored contraction per Rx basis window over all Tx slices
+        for (int a = 0; a < n_rb; ++a)
+            gemm_power_f64<true><<<dim3(N / BN, 2 * N / BM, n_tb * Ms), 256, smem, d.stream>>>(
+                d_R + (size_t)a * r_one, d_B, d_X + (size_t)a * n_tb * Ms * 2 * N * N, N, Kp, Ms, 0, 0, k_isi);
         WOFDM_CUDA(h, cudaGetLastError());
+        h->launches += n_tb + n_rb + 1;
+        if (H_out) {
+            if (v == 0) gram_offdiag<false><<<n_var * (n_var + 1) / 2, 256, 0, d.stream>>>(d_X, d_H, n_var, N, n_tb);
+            else gram_offdiag<true><<<n_var * (n_var + 1) / 2, 256, 0, d.stream>>>(d_X, d_H, n_var, N, n_tb);
+        } else {
+            // the parts, each one Gram product of the stored matrices (rows of pitch 2 mat: [slice 0 | ISI sum])
+            zero_diag_kernel<<<n_var, 256, 0, d.stream>>>(d_X, n_var, N);
+            for (int part = 0; part < 2; ++part) {
+                double* const x = d_X + part * mat;
+                double* const o = d_H + (size_t)part * n_var * n_var;
+                if (v == 0) quad_eval_kernel<64, false><<<g, 256, 0, d.stream>>>(x, x, o, n_var, n_var, (int)mat, 0, 2 * mat, 2 * mat, 2.0);
+                else quad_eval_kernel<64, true><<<g, 256, 0, d.stream>>>(x, x, o, n_var, n_var, (int)mat, 0, 2 * mat, 2 * mat, 2.0);
+            }
+            h->launches += 2;
+        }
+        WOFDM_CUDA(h, cudaGetLastError());
+    }
+    h->launches += n_tb + n_rb;
+    if (H_out) {
         WOFDM_CUDA(h, cudaMemcpyAsync(H_out, d_H, (size_t)n_var * n_var * 8, cudaMemcpyDeviceToHost, d.stream));
     } else {
-        // the parts, each one Gram product of the stored matrices (rows of pitch 2 mat: [slice 0 | ISI sum])
-        const size_t mat = (size_t)2 * N * N;
-        zero_diag_kernel<<<n_var, 256, 0, d.stream>>>(d_X, n_var, N);
-        const dim3 g((n_var + 63) / 64, (n_var + 63) / 64);
-        quad_eval_kernel<64><<<g, 256, 0, d.stream>>>(d_X, d_X, d_H, n_var, n_var, (int)mat, 0, 2 * mat, 2 * mat, 2.0);
-        quad_eval_kernel<64><<<g, 256, 0, d.stream>>>(d_X + mat, d_X + mat, d_H + (size_t)n_var * n_var, n_var, n_var, (int)mat, 0, 2 * mat, 2 * mat, 2.0);
-        WOFDM_CUDA(h, cudaGetLastError());
-        h->launches += 2;
         WOFDM_CUDA(h, cudaMemcpyAsync(H_ici, d_H, (size_t)n_var * n_var * 8, cudaMemcpyDeviceToHost, d.stream));
         WOFDM_CUDA(h, cudaMemcpyAsync(H_isi, d_H + (size_t)n_var * n_var, (size_t)n_var * n_var * 8, cudaMemcpyDeviceToHost, d.stream));
     }
+    WOFDM_CUDA(h, cudaEventRecord(h->hess_ev[1], d.stream));
     WOFDM_CUDA(h, cudaStreamSynchronize(d.stream));
+    float ms = 0.f;
+    h->hess_ms = cudaEventElapsedTime(&ms, h->hess_ev[0], h->hess_ev[1]) == cudaSuccess ? ms : -1.0;
+    h->hess_passes = r;
     return WOFDM_OK;
 }
 
-static int window_hessian_run(wofdm_handle h, const wofdm_sys_t* sys, const double* chan, int L, double* H_out, int* n_var_out) {
-    NvtxRange nvtx_("wofdm_window_hessian");
-    if (!h) return WOFDM_EINVAL;
-    int rc = validate_sys(h, sys, L);
-    if (rc) return rc;
-    if (!chan || !H_out) return fail(h, WOFDM_EINVAL, "bad buffer");
-    if (sys->N % 64) return fail(h, WOFDM_EUNSUPPORTED, "interference path needs N to be a multiple of 64");
-    const int N = sys->N, n_tx = N + sys->cp + sys->cs, n_w = N + sys->tail_rx;
+// ---- the channel set as a few virtual channels --------------------------------------------------------------------------
+// The Hessian is a Hermitian form in the taps: A0_u(h), AS_u(h) are linear in h, so H(h) = F(h h^H) with F linear, and
+//     (1/C) sum_c H(h_c) = F(R) = sum_j H(g_j)   for R = (1/C) sum_c h_c h_c^H and ANY factor R = sum_j g_j g_j^H.
+// C <= L: the channels themselves are that factor (weight 1/C on the result).  C > L: R (O(C L^2)) is factored by a
+// pivoted Cholesky decomposition into r = rank(R) <= L columns g_j (weight 1): a set of 250 channels costs at most L passes.
+// The decomposition stops when the largest remaining pivot (the variance left in the best unexplained tap) is at most
+// kSetFactorTol times the largest diagonal entry of R, so the dropped remainder is a PSD matrix of trace at most
+// L * kSetFactorTol * max_l R[l][l] -- below the fp64 rounding of the Gram sums for L <= 88.  Taps that are exact linear
+// combinations of others (a rank-deficient set: repeated channels, a few propagation paths sinc-interpolated onto many
+// taps) leave pivots at the rounding level and cost no pass.
+constexpr double kSetFactorTol = 1e-14;
+
+// chan: complex L x C column-major.  On return *virt points at r complex impulse responses of L taps (chan itself or fac)
+// and *w is the weight of their summed Hessian.
+static int channel_set_factor(wofdm_handle h, const double* chan, int L, int C, std::vector<double>& fac, const double** virt,
+                              int* r, double* w) {
+    for (size_t i = 0; i < (size_t)2 * L * C; ++i)
+        if (!std::isfinite(chan[i])) return fail(h, WOFDM_EINVAL, "channel set: non-finite tap");
+    if (C <= L) {
+        *virt = chan; *r = C; *w = 1.0 / (double)C;
+        return WOFDM_OK;
+    }
+    // R[i][j] = (1/C) sum_c h_c[i] conj(h_c[j]), row-major complex
+    std::vector<double> R((size_t)2 * L * L, 0.0);
+    for (int c = 0; c < C; ++c) {
+        const double* hc = chan + (size_t)2 * L * c;
+        for (int i = 0; i < L; ++i)
+            for (int j = 0; j < L; ++j) {
+                R[2 * ((size_t)i * L + j)] += hc[2 * i] * hc[2 * j] + hc[2 * i + 1] * hc[2 * j + 1];
+                R[2 * ((size_t)i * L + j) + 1] += hc[2 * i + 1] * hc[2 * j] - hc[2 * i] * hc[2 * j + 1];
+            }
+    }
+    for (double& x : R) x /= (double)C;
+    // pivoted Cholesky: column k = (R[:, p] - sum_{j<k} g_j conj(g_j[p])) / sqrt(d_p), p the largest remaining diagonal
+    std::vector<double> dg(L);
+    std::vector<char> used(L, 0);
+    double dmax = 0.0;
+    for (int i = 0; i < L; ++i) { dg[i] = R[2 * ((size_t)i * L + i)]; dmax = std::max(dmax, dg[i]); }
+    fac.assign((size_t)2 * L * L, 0.0);
+    int k = 0;
+    for (; k < L; ++k) {
+        int p = -1;
+        for (int i = 0; i < L; ++i)
+            if (!used[i] && (p < 0 || dg[i] > dg[p])) p = i;
+        if (!(dg[p] > kSetFactorTol * dmax)) break;
+        const double s = std::sqrt(dg[p]);
+        used[p] = 1;
+        double* gk = fac.data() + (size_t)2 * L * k;
+        for (int i = 0; i < L; ++i) {
+            if (used[i]) continue;                          // pivots already taken (and p itself, set below)
+            double re = R[2 * ((size_t)i * L + p)], im = R[2 * ((size_t)i * L + p) + 1];
+            for (int j = 0; j < k; ++j) {                   // - g_j[i] conj(g_j[p])
+                const double* gj = fac.data() + (size_t)2 * L * j;
+                re -= gj[2 * i] * gj[2 * p] + gj[2 * i + 1] * gj[2 * p + 1];
+                im -= gj[2 * i + 1] * gj[2 * p] - gj[2 * i] * gj[2 * p + 1];
+            }
+            gk[2 * i] = re / s; gk[2 * i + 1] = im / s;
+            dg[i] -= gk[2 * i] * gk[2 * i] + gk[2 * i + 1] * gk[2 * i + 1];
+        }
+        gk[2 * p] = s;
+    }
+    *virt = fac.data(); *r = std::max(k, 1); *w = 1.0;         // (R = 0: one all-zero channel, H = 0)
+    return WOFDM_OK;
+}
+
+// the reduced bases: columns of reduce_variable_tx / _rx (optimization_tools/utils.py:13-73) as full windows
+static int reduced_bases(wofdm_handle h, const wofdm_sys_t* sys, std::vector<double>& bt, std::vector<double>& br) {
+    const int n_tx = sys->N + sys->cp + sys->cs, n_w = sys->N + sys->tail_rx;
     const int n_tb = sys->tail_tx + 1, n_rb = sys->tail_rx / 2 + 1;
-    if (n_var_out) *n_var_out = n_tb * n_rb;
-    // basis windows = columns of reduce_variable_tx / _rx (optimization_tools/utils.py:13-73)
-    std::vector<double> bt((size_t)n_tb * n_tx), br((size_t)n_rb * n_w), e(std::max(n_tb, n_rb));
+    bt.assign((size_t)n_tb * n_tx, 0.0);
+    br.assign((size_t)n_rb * n_w, 0.0);
+    std::vector<double> e(std::max(n_tb, n_rb));
     for (int b = 0; b < n_tb; ++b) {
         std::fill(e.begin(), e.end(), 0.0); e[b] = 1.0;
-        rc = wofdm_expand_window_tx(sys, e.data(), bt.data() + (size_t)b * n_tx);
+        int rc = wofdm_expand_window_tx(sys, e.data(), bt.data() + (size_t)b * n_tx);
         if (rc) return fail(h, rc, "expand_window_tx");
     }
     for (int a = 0; a < n_rb; ++a) {
         std::fill(e.begin(), e.end(), 0.0); e[a] = 1.0;
-        rc = wofdm_expand_window_rx(sys, e.data(), br.data() + (size_t)a * n_w);
+        int rc = wofdm_expand_window_rx(sys, e.data(), br.data() + (size_t)a * n_w);
         if (rc) return fail(h, rc, "expand_window_rx");
     }
-    return window_hessian_core(h, sys, chan, L, bt.data(), n_tb, br.data(), n_rb, H_out, nullptr, nullptr);
+    return WOFDM_OK;
 }
 
-static int window_hessian_parts_run(wofdm_handle h, const wofdm_sys_t* sys, const double* chan, int L, const double* basis_tx,
-                                    int n_tb, const double* basis_rx, int n_rb, double* H_ici, double* H_isi) {
-    NvtxRange nvtx_("wofdm_window_hessian_parts");
+// set = false: ONE impulse response (C = 1, no further checks); set = true: the mean over a set of C channels.
+// H_out (the reduced-basis Hessian) or, with basis_tx / basis_rx given, the parts H_ici / H_isi.
+static int window_hessian_run(wofdm_handle h, const wofdm_sys_t* sys, const double* chan, int L, int C, bool set,
+                              const double* basis_tx, int n_tb, const double* basis_rx, int n_rb,
+                              double* H_out, int* n_var_out, double* H_ici, double* H_isi) {
     if (!h) return WOFDM_EINVAL;
     int rc = validate_sys(h, sys, L);
     if (rc) return rc;
-    if (!chan || !basis_tx || !basis_rx || !H_ici || !H_isi || n_tb < 1 || n_rb < 1) return fail(h, WOFDM_EINVAL, "bad buffer");
+    const bool parts = H_out == nullptr;
+    if (!parts && (!chan || !H_out)) return fail(h, WOFDM_EINVAL, "bad buffer");
+    if (parts && (!chan || !basis_tx || !basis_rx || !H_ici || !H_isi || n_tb < 1 || n_rb < 1)) return fail(h, WOFDM_EINVAL, "bad buffer");
+    if (set && C < 1) return fail(h, WOFDM_EINVAL, "channel set: C must be >= 1");
     if (sys->N % 64) return fail(h, WOFDM_EUNSUPPORTED, "interference path needs N to be a multiple of 64");
-    if ((size_t)2 * sys->N * sys->N % 16) return fail(h, WOFDM_EUNSUPPORTED, "N");
-    return window_hessian_core(h, sys, chan, L, basis_tx, n_tb, basis_rx, n_rb, nullptr, H_ici, H_isi);
+    if (parts && (size_t)2 * sys->N * sys->N % 16) return fail(h, WOFDM_EUNSUPPORTED, "N");
+    std::vector<double> bt, br;
+    if (!parts) {
+        n_tb = sys->tail_tx + 1; n_rb = sys->tail_rx / 2 + 1;
+        if (n_var_out) *n_var_out = n_tb * n_rb;
+        rc = reduced_bases(h, sys, bt, br);
+        if (rc) return rc;
+        basis_tx = bt.data(); basis_rx = br.data();
+    }
+    const double* virt = chan;
+    int r = 1;
+    double w = 1.0;
+    std::vector<double> fac;
+    h->hess_factor_ms = 0.0;
+    if (set) {
+        const auto t0 = std::chrono::steady_clock::now();
+        rc = channel_set_factor(h, chan, L, C, fac, &virt, &r, &w);
+        if (rc) return rc;
+        h->hess_factor_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    }
+    rc = window_hessian_core(h, sys, virt, L, r, basis_tx, n_tb, basis_rx, n_rb, H_out, H_ici, H_isi);
+    if (rc || w == 1.0) return rc;
+    const size_t nn = (size_t)n_tb * n_rb * n_tb * n_rb;
+    for (double* H : {H_out, H_ici, H_isi})
+        if (H)
+            for (size_t i = 0; i < nn; ++i) H[i] *= w;
+    return WOFDM_OK;
 }
 
 }  // namespace wofdm
@@ -814,12 +943,33 @@ int wofdm_interf_last_timing(wofdm_handle h, double* total_ms, double* band_ms, 
 }
 
 int wofdm_window_hessian(wofdm_handle h, const wofdm_sys_t* sys, const double* chan, int L, double* H, int* n_var) {
-    return window_hessian_run(h, sys, chan, L, H, n_var);
+    NvtxRange nvtx_("wofdm_window_hessian");
+    return window_hessian_run(h, sys, chan, L, 1, false, nullptr, 0, nullptr, 0, H, n_var, nullptr, nullptr);
 }
 
 int wofdm_window_hessian_parts(wofdm_handle h, const wofdm_sys_t* sys, const double* chan, int L, const double* basis_tx, int n_tb,
                                const double* basis_rx, int n_rb, double* H_ici, double* H_isi) {
-    return window_hessian_parts_run(h, sys, chan, L, basis_tx, n_tb, basis_rx, n_rb, H_ici, H_isi);
+    NvtxRange nvtx_("wofdm_window_hessian_parts");
+    return window_hessian_run(h, sys, chan, L, 1, false, basis_tx, n_tb, basis_rx, n_rb, nullptr, nullptr, H_ici, H_isi);
+}
+
+int wofdm_window_hessian_set(wofdm_handle h, const wofdm_sys_t* sys, const double* chan, int L, int C, double* H, int* n_var) {
+    NvtxRange nvtx_("wofdm_window_hessian_set");
+    return window_hessian_run(h, sys, chan, L, C, true, nullptr, 0, nullptr, 0, H, n_var, nullptr, nullptr);
+}
+
+int wofdm_window_hessian_parts_set(wofdm_handle h, const wofdm_sys_t* sys, const double* chan, int L, int C, const double* basis_tx,
+                                   int n_tb, const double* basis_rx, int n_rb, double* H_ici, double* H_isi) {
+    NvtxRange nvtx_("wofdm_window_hessian_parts_set");
+    return window_hessian_run(h, sys, chan, L, C, true, basis_tx, n_tb, basis_rx, n_rb, nullptr, nullptr, H_ici, H_isi);
+}
+
+int wofdm_window_hessian_last_timing(wofdm_handle h, double* device_ms, double* factor_ms, int* passes) {
+    if (!h) return WOFDM_EINVAL;
+    if (device_ms) *device_ms = h->hess_ms;
+    if (factor_ms) *factor_ms = h->hess_factor_ms;
+    if (passes) *passes = h->hess_passes;
+    return WOFDM_OK;
 }
 
 }  // extern "C"

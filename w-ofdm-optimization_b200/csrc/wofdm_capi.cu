@@ -171,6 +171,8 @@ int wofdm_destroy(wofdm_handle h) {
     if (!h->devs.empty()) cudaSetDevice(h->devs[0].dev);
     for (auto& e : h->interf_ev)
         if (e) cudaEventDestroy(e);
+    for (auto& e : h->hess_ev)
+        if (e) cudaEventDestroy(e);
     delete h;
     return WOFDM_OK;
 }

@@ -191,14 +191,18 @@ def calculate_interference(cpLength, typeOFDM, windowTx, windowRx, numSubcar, ta
     return float(h.interf_power(s, _diag(windowTx), _diag(windowRx), mean_ir[:, None], mode=mode, scalar=True)[0])
 
 
-def _quad_objective(side, typeOFDM, window_fixed, numSubcar, cpLength, tailTx, tailRx, channel, alpha, handle=None):
+def _quad_objective(side, typeOFDM, window_fixed, numSubcar, cpLength, tailTx, tailRx, channel, alpha, handle=None,
+                    channel_set=False):
+    """channel_set: `channel` is an (L, C) set and the parts are its means (wofdm_window_hessian_parts_set); the result is
+    linear in the parts, so it is the mean of the per-channel quad_objective."""
     h = handle or default_handle()
     s = capi.params_from_name(typeOFDM, int(numSubcar), int(cpLength), int(tailTx), int(tailRx))
     fixed = _diag(window_fixed)
+    parts = h.window_hessian_parts_set if channel_set else h.window_hessian_parts
     if side == "tx":
-        Hc, Hs = h.window_hessian_parts(s, channel, np.eye(s.n_tx), fixed[None, :])
+        Hc, Hs = parts(s, channel, np.eye(s.n_tx), fixed[None, :])
     else:
-        Hc, Hs = h.window_hessian_parts(s, channel, fixed[None, :], np.eye(s.N + s.tail_rx))
+        Hc, Hs = parts(s, channel, fixed[None, :], np.eye(s.N + s.tail_rx))
     return float(alpha) * Hc + (1.0 - float(alpha)) * np.diag(Hs.sum(axis=1))
 
 
@@ -215,3 +219,17 @@ def quad_objective_rx(windowTx, numSubcar, tailRx, cpLength, typeOFDM, tailTx, c
     """HRx of quad_objective_rx (matlab/window_optimization.m:637-680): the full Rx window (N + tailRx entries) is the
     variable, windowTx is fixed."""
     return _quad_objective("rx", typeOFDM, windowTx, numSubcar, cpLength, tailTx, tailRx, channel, alpha, handle)
+
+
+def quad_objective_tx_expected(windowRx, numSubcar, tailRx, cpLength, typeOFDM, tailTx, channels, alpha, handle=None):
+    """quad_objective_tx averaged over a channel set: `channels` is C x L, rows = realisations (as vehA200channel2 is
+    stored), and the result is the mean over the rows of quad_objective_tx -- the expected interference instead of the
+    interference of the mean channel."""
+    ch = np.atleast_2d(np.asarray(channels)).T
+    return _quad_objective("tx", typeOFDM, windowRx, numSubcar, cpLength, tailTx, tailRx, ch, alpha, handle, channel_set=True)
+
+
+def quad_objective_rx_expected(windowTx, numSubcar, tailRx, cpLength, typeOFDM, tailTx, channels, alpha, handle=None):
+    """quad_objective_rx averaged over a channel set (`channels` C x L, rows = realisations)."""
+    ch = np.atleast_2d(np.asarray(channels)).T
+    return _quad_objective("rx", typeOFDM, windowTx, numSubcar, cpLength, tailTx, tailRx, ch, alpha, handle, channel_set=True)

@@ -7,6 +7,7 @@ reference's ``optimization_fun`` calls before the QP / trust-region solve
 
     chann = opt.calculate_chann_matrices(channel_ir)      # here: just the impulse response (the device builds H_m)
     H = opt.gen_hessian(chann)                            # one device call instead of the O(n^2 N^2) loops
+    H = opt.gen_hessian_expected(channels)                # or: the expected interference over the whole (L, C) set
 
 The solvers themselves (quadratic_solver, scipy trust-constr) are the reference's and stay on the CPU: they are
 sequential 9- to 54-variable problems (SURVEY section 2, out of scope).  No CPU fallback for the Hessian."""
@@ -30,6 +31,13 @@ class _Base:
     def gen_hessian(self, channel_tensor):
         h = self._h or ofdm_utils.default_handle()
         return h.window_hessian(self._sys, channel_tensor)
+
+    def gen_hessian_expected(self, channels):
+        """Hessian of the interference power averaged over every realisation of the stored set: channels (L, C) as the
+        reference stores them (channels/<standard>.npy), instead of gen_hessian on their mean impulse response.  The
+        mean of C zero-mean Rayleigh channels is one random channel of covariance R / C, not a typical one."""
+        h = self._h or ofdm_utils.default_handle()
+        return h.window_hessian_set(self._sys, channels)
 
 
 class OptimizerTx(_Base):
