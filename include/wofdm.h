@@ -128,6 +128,27 @@ WOFDM_API int wofdm_ber_run_multi(wofdm_handle h, const wofdm_sys_t* sys, const 
                         uint64_t seed, uint32_t variant, int shard_index, int shard_count,
                         int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot);
 
+/* The counters of wofdm_ber_run_multi resolved by sub-carrier and / or by channel realisation: where the errors come from
+ * (guard-band edges, the bins a window protects, the deep-faded realisations that set the error floor).
+ *   resolve: a non-empty combination of the flags below.  Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1,
+ *            Nr = (resolve & WOFDM_BY_SUBCARRIER) ? N : 1 (FFT bin order, as wofdm_interf_power's sub-carrier axis).
+ *   bit_err / sym_err: int64[n_var][n_snr][Cr][Nr]; sym_tot: int64[n_snr][Cr][Nr] (the same for every pair): this shard's
+ *            frames of the cell times S-1 on active bins, 0 on guard bins; bit totals are sym_tot * bits.
+ * Draws, noise numbering, window pairs (variant + v), sharding and the split over the handle's devices are those of
+ * wofdm_ber_run_multi.  The call runs the resolved twin of the kernel wofdm_ber_run_multi picks for the same arguments (same
+ * arithmetic): summed over the channel and bin axes, the counters equal that function's, bit for bit.  Where the twin's
+ * per-sub-carrier accumulators do not fit the device's shared memory, the staged kernel runs instead with the same draws;
+ * in fp32 its sums then agree up to decisions within rounding of a boundary (fp64 is staged on both sides: exact).  The
+ * arrays are int64 and additive, so shards of several processes add up as the unresolved ones do.
+ * WOFDM_EINVAL: resolve 0 or unknown bits, NULL buffers, a counter array whose size overflows, and what
+ * wofdm_ber_run_multi rejects; WOFDM_ENOMEM: the device counter buffer cannot be allocated. */
+#define WOFDM_BY_SUBCARRIER 1
+#define WOFDM_BY_CHANNEL    2
+WOFDM_API int wofdm_ber_run_resolved(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
+                       const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                       uint64_t seed, uint32_t variant, int shard_index, int shard_count, int resolve,
+                       int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot);
+
 /* Device-resident form: inputs are uploaded once, launches are asynchronous. */
 WOFDM_API int wofdm_ber_plan_create(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
                           const double* chan, int L, int C, const double* snr_db, int n_snr,

@@ -7,6 +7,7 @@
 typedef struct mxArray_tag mxArray;
 typedef size_t mwSize;
 typedef enum { mxREAL = 0, mxCOMPLEX = 1 } mxComplexity;
+typedef enum { mxDOUBLE_CLASS = 6 } mxClassID;
 extern "C" {
 double* mxGetPr(const mxArray*);
 double* mxGetPi(const mxArray*);
@@ -21,6 +22,7 @@ bool mxIsComplex(const mxArray*);
 int mxGetString(const mxArray*, char*, mwSize);
 mxArray* mxCreateDoubleMatrix(mwSize, mwSize, mxComplexity);
 mxArray* mxCreateDoubleScalar(double);
+mxArray* mxCreateNumericArray(mwSize, const mwSize*, mxClassID, mxComplexity);
 void mexErrMsgIdAndTxt(const char*, const char*, ...);
 int mexAtExit(void (*)(void));
 }

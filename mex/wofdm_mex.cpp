@@ -13,6 +13,7 @@
 //       -- calculate_interference, matlab/main_interference_calculation.m:177-180; the values the reference
 //          reads from settingsData.mat / the channel file inside the function are passed explicitly.
 //   berSNR = wofdm_mex('run_simulation_sweep_multi', ...)   every window variant of a (system, CP) on the same bits, one job
+//   berK = wofdm_mex('run_simulation_per_subcarrier', ...)  the same, BER per sub-carrier: n_snr x N x n_var
 //   [berMasked, ber] = wofdm_mex('run_sim_mc', ...)          run_sim_mc of matlab/main_channel_mask.m:334-337
 //   H = wofdm_mex('window_hessian', ...)                     quad_objective_tx / _rx of matlab/window_optimization.m:596-680
 //   H = wofdm_mex('window_hessian_expected', ...), 'quad_objective_tx_expected', 'quad_objective_rx_expected'
@@ -159,8 +160,10 @@ static std::vector<double> windows_of(const mxArray* a, size_t want, size_t* n_v
 // windowRx CELL ARRAYS of n_var windows (a single window is repeated): every window pair on the same bits, one device job
 // -- the {optimised, RC} pairs of matlab/main_BER_calculation.m:66-117 and the RC + CaseA/CaseB steps 1-3 of :118-198.
 // Returns n_snr x n_var; column v = run_simulation_sweep with pair v (its noise stream: variant v).
-static void do_run_simulation_multi(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
-    if (nrhs < 14) mexErrMsgIdAndTxt("wofdm:nargin", "run_simulation_sweep_multi needs 14 arguments");
+// per_subcarrier = true ('run_simulation_per_subcarrier', the same arguments): BER of every sub-carrier,
+// n_snr x N x n_var (FFT bin order; guard bins 0), from wofdm_ber_run_resolved on the same draws.
+static void do_run_simulation_multi(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[], bool per_subcarrier) {
+    if (nrhs < 14) mexErrMsgIdAndTxt("wofdm:nargin", "%s needs 14 arguments", per_subcarrier ? "run_simulation_per_subcarrier" : "run_simulation_sweep_multi");
     (void)nlhs;
     wofdm_sys_t s;
     memset(&s, 0, sizeof(s));
@@ -186,6 +189,24 @@ static void do_run_simulation_multi(int nlhs, mxArray* plhs[], int nrhs, const m
         memcpy(chan.data() + 2 * L * c, row.data(), 2 * L * sizeof(double));
     }
     const size_t n_snr = mxGetNumberOfElements(prhs[8]);
+    if (per_subcarrier) {
+        const size_t N = (size_t)s.N;
+        std::vector<long long> be(n_var * n_snr * N), se(n_var * n_snr * N), st(n_snr * N);
+        check(wofdm_ber_run_resolved(handle(), &s, wtx.data(), wrx.data(), (int)n_var, chan.data(), (int)L, (int)C, mxGetPr(prhs[8]),
+                                     (int)n_snr, ensemble, seed, 0, 0, 1, WOFDM_BY_SUBCARRIER, (int64_t*)be.data(), (int64_t*)se.data(),
+                                     (int64_t*)st.data()),
+              "wofdm_ber_run_resolved");
+        const mwSize dims[3] = {(mwSize)n_snr, (mwSize)N, (mwSize)n_var};
+        plhs[0] = mxCreateNumericArray(3, dims, mxDOUBLE_CLASS, mxREAL);
+        double* out = mxGetPr(plhs[0]);
+        for (size_t v = 0; v < n_var; ++v)          // column-major: out(i, k, v)
+            for (size_t k = 0; k < N; ++k)
+                for (size_t i = 0; i < n_snr; ++i) {
+                    const long long bt = st[i * N + k] * s.bits;
+                    out[(v * N + k) * n_snr + i] = bt ? (double)be[(v * n_snr + i) * N + k] / (double)bt : 0.0;
+                }
+        return;
+    }
     std::vector<long long> be(n_var * n_snr), se(n_var * n_snr), bt(n_snr), st(n_snr);
     check(wofdm_ber_run_multi(handle(), &s, wtx.data(), wrx.data(), (int)n_var, chan.data(), (int)L, (int)C, mxGetPr(prhs[8]), (int)n_snr,
                               ensemble, seed, 0, 0, 1, (int64_t*)be.data(), (int64_t*)bt.data(), (int64_t*)se.data(), (int64_t*)st.data()),
@@ -358,10 +379,11 @@ static void do_calculate_interference(int nlhs, mxArray* plhs[], int nrhs, const
 extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     char cmd[32];
     if (nrhs < 1 || !mxIsChar(prhs[0]) || mxGetString(prhs[0], cmd, sizeof(cmd)))
-        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_sim_mc', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
+        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_sim_mc', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
     if (!strcmp(cmd, "run_simulation")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_simulation_sweep")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, true);
-    else if (!strcmp(cmd, "run_simulation_sweep_multi")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1);
+    else if (!strcmp(cmd, "run_simulation_sweep_multi")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, false);
+    else if (!strcmp(cmd, "run_simulation_per_subcarrier")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, true);
     else if (!strcmp(cmd, "run_sim_mc")) do_run_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1);
     else if (!strcmp(cmd, "window_hessian")) do_window_hessian(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "quad_objective_tx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, true, false);

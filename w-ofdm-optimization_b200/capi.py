@@ -16,6 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libwofdm.so")
 
 OK, EINVAL, ECUDA, ENOMEM, ENODEV, EUNSUPPORTED = 0, -1, -2, -3, -4, -5
+WOFDM_BY_SUBCARRIER, WOFDM_BY_CHANNEL = 1, 2         # wofdm_ber_run_resolved: resolve flags
 _ERRNAME = {EINVAL: "WOFDM_EINVAL", ECUDA: "WOFDM_ECUDA", ENOMEM: "WOFDM_ENOMEM", ENODEV: "WOFDM_ENODEV",
             EUNSUPPORTED: "WOFDM_EUNSUPPORTED"}
 
@@ -78,6 +79,8 @@ SIGNATURES = {
                                       C.c_uint64, C.c_uint32, C.c_int, C.c_int, _i64p, _i64p, _i64p, _i64p]),
     "wofdm_ber_run_multi": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, C.c_int, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
                                       C.c_uint64, C.c_uint32, C.c_int, C.c_int, _i64p, _i64p, _i64p, _i64p]),
+    "wofdm_ber_run_resolved": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, C.c_int, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
+                                         C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_int, _i64p, _i64p, _i64p]),
     "wofdm_ber_plan_create_multi": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, C.c_int, _dp, C.c_int, C.c_int, _dp, C.c_int,
                                               _P(C.c_void_p)]),
     "wofdm_ber_plan_variants": (C.c_int, [C.c_void_p, _P(C.c_int)]),
@@ -277,6 +280,25 @@ class Handle:
                                         _ptr(be, _i64p), _ptr(bt, _i64p), _ptr(se, _i64p), _ptr(st, _i64p))
         self._check(rc)
         return dict(bit_err=be, bit_tot=bt, sym_err=se, sym_tot=st)
+
+    def ber_run_resolved(self, s, wins_tx, wins_rx, chan, snr_db, ensemble, seed=0, variant=0, shard=(0, 1),
+                         by_subcarrier=True, by_channel=False):
+        """ber_run_multi with the counters resolved by sub-carrier and / or channel (wofdm_ber_run_resolved).
+        bit_err / sym_err: (n_var, n_snr, Cr, Nr), sym_tot / bit_tot: (n_snr, Cr, Nr), Cr = C if by_channel else 1,
+        Nr = N (FFT bin order) if by_subcarrier else 1.  Summed over the last two axes: ber_run_multi's counters."""
+        wt, wr = self._win_multi(s, wins_tx, wins_rx)
+        _, _, chf, L, Cn = self._win_chan(s, wt[0], wr[0], chan)
+        snr = _f64(np.ravel(snr_db))
+        n, nv = snr.size, wt.shape[0]
+        resolve = (WOFDM_BY_SUBCARRIER if by_subcarrier else 0) | (WOFDM_BY_CHANNEL if by_channel else 0)
+        cr, nr = (Cn if by_channel else 1), (s.N if by_subcarrier else 1)
+        be, se = np.zeros((nv, n, cr, nr), dtype=np.int64), np.zeros((nv, n, cr, nr), dtype=np.int64)
+        st = np.zeros((n, cr, nr), dtype=np.int64)
+        rc = load().wofdm_ber_run_resolved(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), nv, _ptr(chf, _dp), L, Cn,
+                                           _ptr(snr, _dp), n, int(ensemble), int(seed), int(variant), int(shard[0]),
+                                           int(shard[1]), int(resolve), _ptr(be, _i64p), _ptr(se, _i64p), _ptr(st, _i64p))
+        self._check(rc)
+        return dict(bit_err=be, sym_err=se, sym_tot=st, bit_tot=st * int(s.bits))
 
     def ber_run_masked(self, s, win_tx, win_rx, chan, snr_db, ensemble, seed=0, variant=0, roll_off=10):
         """Channel-mask variant (wofdm_ber_run_masked): counters of the MASKED signal; ber_run with the same `s`

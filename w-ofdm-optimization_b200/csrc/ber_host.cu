@@ -34,6 +34,11 @@ struct wofdm_ber_plan_s {
     int n_var = 1;                 // window pairs of the plan
     bool fused = false;            // all of them in ONE launch (second-generation tensor-core kernel); else one launch each
     bool transient = false;    // buffers live in the devices' arenas (one-shot plan of wofdm_ber_run*): nothing to free
+    // resolved counters (wofdm_ber_run_resolved): WOFDM_BY_* flags, 0 for the plans of the public plan API.  The kernel that
+    // production picks for the same arguments fixes the noise numbering (chunk, split, n48): noise_var; else noise_var == var
+    int resolve = 0;
+    const BerVariant* noise_var = nullptr;
+    size_t cnt_per_var = 0;        // u64 counters of one window pair: [cells][bins][2] (unresolved: [n_snr][2])
     std::vector<PlanDev> devs;
 };
 
@@ -72,7 +77,7 @@ void fill_split(BerParams& prm, const BerVariant& v) {
 // win_tx (may be NULL): the circular-interior kernels need it flat between the tails; no_circ excludes them
 int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, bool verify, bool force_staged, size_t smem_cap,
                    Choice* out, const double* win_tx = nullptr, bool no_circ = false, bool want_txs = false,
-                   bool no_tconv = false, int nvar = 1, bool want_txy = false) {
+                   bool no_tconv = false, int nvar = 1, bool want_txy = false, bool want_resolved = false) {
     const int stride = s.N + s.cp + s.cs - s.tail_tx;
     const int sec = s.S * stride;
     const bool fp64 = s.precision == 1;
@@ -88,6 +93,7 @@ int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, bool verify, bool 
     if (!fp64 && !force_staged) {
         for (const auto& v : h->variants) {
             if (v.TC == 0 || v.fp64 || v.verify != verify || v.N != s.N) continue;
+            if (v.res != want_resolved) continue;                // (the resolved-counter twins serve wofdm_ber_run_resolved only)
             if (want && !strstr(v.name, want)) continue;
             if (v.ntile > 0) {
                 // channel convolution on the tensor cores (ber_tconv.cuh): first choice wherever it applies -- one Tx pass,
@@ -141,6 +147,7 @@ int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, bool verify, bool 
     if (!best.var) {
         for (const auto& v : h->variants) {
             if (v.TC != 0 || v.fp64 != fp64 || v.verify != verify || v.N != s.N) continue;
+            if (v.res != want_resolved) continue;
             best.var = &v;
             best.chunk = ((sec + 255) / 256) | 1;   // noise block B of the staged policy (any odd number)
             best.lay = v.layout(s.S, stride, s.tail_tx, s.tail_rx, L, 0, 0);
@@ -156,6 +163,56 @@ int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, bool verify, bool 
     if (!best.var) return fail(h, WOFDM_EUNSUPPORTED, "no compiled kernel variant for this N / precision");
     *out = best;
     return WOFDM_OK;
+}
+
+// Resolved counters: the twin (BerVariant::res) of the kernel `prod` that wofdm_ber_run_multi picks, where one is compiled
+// and its accumulators fit (nvar: pairs per launch, 1 = one launch per pair); else the staged twin, which numbers its noise
+// like `prod` through noise_at (BerParams::chunk / split / n48).  *fused_out: the twin evaluates all pairs in one launch.
+int choose_resolved(wofdm_ctx* h, const wofdm_sys_t& s, int L, size_t smem_cap, const Choice& prod, bool fused, int n_var,
+                    Choice* out, bool* fused_out) {
+    const BerVariant& p = *prod.var;
+    const int stride = s.N + s.cp + s.cs - s.tail_tx;
+    const bool staged_only = getenv("WOFDM_RESOLVED_STAGED") != nullptr;   // test aid: the staged twin with production's numbering
+    if (p.gen == 0 && p.TC > 0 && !staged_only) {
+        // register policies: the twin of the same instantiation (same arithmetic, same noise blocks)
+        for (const auto& v : h->variants) {
+            if (!v.res || v.gen != 0 || v.TC != p.TC || v.N != p.N || v.NT != p.NT || v.LB != p.LB || v.MINB != p.MINB || v.CL != p.CL ||
+                v.circ != p.circ || v.full != p.full || v.verify) continue;
+            const BerSmem lay = v.layout(s.S / v.CL, stride, s.tail_tx, s.tail_rx, L, prod.chunk, 0);
+            if (lay.bytes > smem_cap) break;
+            out->var = &v; out->lay = lay; out->chunk = prod.chunk; out->use_global = 0;
+            *fused_out = false;
+            return WOFDM_OK;
+        }
+    }
+    if (p.gen == 2 && !staged_only) {
+        for (const auto& v : h->variants) {
+            if (!v.res || v.gen != 2 || v.verify || v.N != p.N || v.NT != p.NT || v.ntile != p.ntile || v.LB != p.LB || v.CL != p.CL) continue;
+            // all pairs in one launch where the accumulators of all of them fit, else one launch per pair (same counters)
+            for (int nv : {fused ? n_var : 1, 1}) {
+                const BerSmem lay = v.layout(s.S / v.CL, stride, s.tail_tx, s.tail_rx, L, nv, 0);
+                if (lay.bytes > smem_cap) continue;
+                out->var = &v; out->lay = lay; out->chunk = 0; out->use_global = 0;
+                *fused_out = fused && nv == n_var;
+                return WOFDM_OK;
+            }
+        }
+    }
+    for (const auto& v : h->variants) {
+        if (!v.res || v.TC != 0 || v.fp64 != (s.precision == 1) || v.verify || v.N != s.N) continue;
+        out->var = &v;
+        out->chunk = prod.chunk;
+        out->use_global = 0;
+        out->lay = v.layout(s.S, stride, s.tail_tx, s.tail_rx, L, 0, 0);
+        if (out->lay.bytes > smem_cap) {
+            out->use_global = 1;
+            out->lay = v.layout(s.S, stride, s.tail_tx, s.tail_rx, L, 0, 1);
+            if (out->lay.bytes > smem_cap) return fail(h, WOFDM_EUNSUPPORTED, "frame does not fit the staged kernel's shared memory");
+        }
+        *fused_out = false;
+        return WOFDM_OK;
+    }
+    return fail(h, WOFDM_EUNSUPPORTED, "no compiled resolved-counter kernel for this N / precision");
 }
 
 template <typename T> void cast_vec(const std::vector<double>& src, std::vector<unsigned char>& dst) {
@@ -270,9 +327,10 @@ size_t elem_bytes(const wofdm_sys_t& s) { return s.precision == 1 ? sizeof(doubl
 
 // transient = true: device buffers come out of the per-device arena (no cudaMalloc / cudaFree per call); such a plan
 // must be destroyed before the arena is used again (wofdm_ber_run_shard does exactly that)
+// resolve != 0 (WOFDM_BY_* flags): counters [n_var][n_snr * Cr][Nr][2] in a buffer of their own (wofdm_ber_run_resolved)
 static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
                             const double* chan, int L, int C, const double* snr_db, int n_snr,
-                            wofdm_ber_plan* out, bool transient) {
+                            wofdm_ber_plan* out, bool transient, int resolve = 0) {
     NvtxRange nvtx_("wofdm_ber_plan_create");
     if (!h) return WOFDM_EINVAL;
     if (!out) return fail(h, WOFDM_EINVAL, "plan out pointer is NULL");
@@ -296,6 +354,18 @@ static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double
     p->fused = rc == WOFDM_OK && n_var > 1 && ch.var->gen == 2;
     if (n_var > 1 && !p->fused) rc = choose_variant(h, *sys, L, false, false, cap, &ch, win_tx, /*no_circ=*/true);
     if (rc) { delete p; return rc; }
+    p->noise_var = ch.var;
+    p->cnt_per_var = (size_t)n_snr * 2;
+    if (resolve) {
+        Choice rch;
+        bool rfused = false;
+        rc = choose_resolved(h, *sys, L, cap, ch, p->fused, n_var, &rch, &rfused);
+        if (rc) { delete p; return rc; }
+        ch.var = rch.var; ch.lay = rch.lay; ch.use_global = rch.use_global;     // (ch.chunk: the noise block of production)
+        p->fused = rfused;
+        p->resolve = resolve;
+        p->cnt_per_var = (size_t)n_snr * ((resolve & WOFDM_BY_CHANNEL) ? C : 1) * ((resolve & WOFDM_BY_SUBCARRIER) ? sys->N : 1) * 2;
+    }
     p->var = ch.var; p->lay = ch.lay; p->chunk = ch.chunk; p->use_global = ch.use_global;
     {
         BerParams fp;
@@ -343,7 +413,7 @@ static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double
         pd.scratch_bytes = p->use_global ? (size_t)pd.blocks_per_sm * d.sm_count * 2 * scratch_elems * elem_bytes(*sys) : 0;
         if (e == cudaSuccess && transient) {
             rc = arena_reserve(h, d, t.wtx.size() + t.wrx.size() + t.tw.size() + hchan.size() + hsnr.size() +
-                                         (size_t)n_var * n_snr * 16 + pd.scratch_bytes);
+                                         (resolve ? 0 : (size_t)n_var * n_snr * 16) + pd.scratch_bytes);
             if (rc) { const std::string msg = h->err; wofdm_ber_plan_destroy(p); h->err = msg; return rc; }
         }
         if (e == cudaSuccess) e = up(&pd.d_wtx, t.wtx);
@@ -351,7 +421,9 @@ static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double
         if (e == cudaSuccess) e = up(&pd.d_tw, t.tw);
         if (e == cudaSuccess) e = up(&pd.d_chan, hchan);
         if (e == cudaSuccess) e = up(&pd.d_snr, hsnr);
-        if (e == cudaSuccess) e = dev_alloc(reinterpret_cast<void**>(&pd.d_cnt), (size_t)n_var * n_snr * 2 * sizeof(unsigned long long));
+        // (resolved counters: a buffer of their own, outside the arena -- it can be large, and failing to get it is WOFDM_ENOMEM)
+        if (e == cudaSuccess && resolve) e = cudaMalloc(reinterpret_cast<void**>(&pd.d_cnt), n_var * p->cnt_per_var * sizeof(unsigned long long));
+        else if (e == cudaSuccess) e = dev_alloc(reinterpret_cast<void**>(&pd.d_cnt), (size_t)n_var * n_snr * 2 * sizeof(unsigned long long));
         if (e == cudaSuccess) e = cudaStreamSynchronize(d.stream);   // host vectors go out of scope
         if (e == cudaSuccess && p->use_global) e = dev_alloc(&pd.d_scratch, pd.scratch_bytes);
         if (e != cudaSuccess) {
@@ -403,7 +475,9 @@ int wofdm_ber_plan_launch(wofdm_ber_plan p, int slot, int64_t ensemble, uint64_t
     fill_sys(prm, p->sys, p->L);
     prm.chunk = p->chunk; prm.use_global = p->use_global;
     prm.flat_tx = p->flat_tx; prm.flat_rx = p->flat_rx;
-    fill_split(prm, *p->var);
+    fill_split(prm, *p->noise_var);
+    prm.res_chan = (p->resolve & WOFDM_BY_CHANNEL) ? 1 : 0;
+    prm.res_bins = (p->resolve & WOFDM_BY_SUBCARRIER) ? 1 : 0;
     prm.win_tx = pd.d_wtx; prm.win_rx = pd.d_wrx; prm.tw = pd.d_tw; prm.chan = pd.d_chan; prm.snr_lin = pd.d_snr;
     prm.C = p->C; prm.n_snr = p->n_snr; prm.ensemble = ensemble;
     prm.seed = seed; prm.variant = variant;
@@ -415,7 +489,7 @@ int wofdm_ber_plan_launch(wofdm_ber_plan p, int slot, int64_t ensemble, uint64_t
 
     // a launch owns its slot's counters: one that is still pending on ANOTHER stream must finish before they are zeroed
     if (pd.pending && pd.last_stream != st) WOFDM_CUDA(h, cudaStreamSynchronize(pd.last_stream));
-    WOFDM_CUDA(h, cudaMemsetAsync(pd.d_cnt, 0, (size_t)p->n_var * p->n_snr * 2 * sizeof(unsigned long long), st));
+    WOFDM_CUDA(h, cudaMemsetAsync(pd.d_cnt, 0, (size_t)p->n_var * p->cnt_per_var * sizeof(unsigned long long), st));
     if (mine > 0) {
         long long cap = pd.max_ctas;
         if (const char* lim = getenv("WOFDM_MAX_CTAS_PER_SM"))            // tuning aid: occupancy sensitivity
@@ -437,7 +511,7 @@ int wofdm_ber_plan_launch(wofdm_ber_plan p, int slot, int64_t ensemble, uint64_t
                 pv.win_rx = static_cast<const char*>(pd.d_wrx) + (size_t)v * n_wr * eb;
                 pv.flat_tx = (p->flat_tx >> v) & 1; pv.flat_rx = (p->flat_rx >> v) & 1;
                 pv.variant = variant + (uint32_t)v;
-                pv.counters = pd.d_cnt + (size_t)v * p->n_snr * 2;
+                pv.counters = pd.d_cnt + (size_t)v * p->cnt_per_var;
                 WOFDM_CUDA(h, p->var->launch(pv, grid, p->lay.bytes, st));
                 h->launches += 1;
             }
@@ -477,9 +551,11 @@ int wofdm_ber_plan_destroy(wofdm_ber_plan p) {
         PlanDev& pd = p->devs[s];
         cudaSetDevice(p->ctx->devs[s].dev);
         if (pd.pending && pd.last_stream) cudaStreamSynchronize(pd.last_stream);
+        if (p->resolve) cudaFree(pd.d_cnt);     // (its own buffer, also in a transient plan)
         if (p->transient) continue;             // arena memory
         cudaFree(pd.d_wtx); cudaFree(pd.d_wrx); cudaFree(pd.d_tw); cudaFree(pd.d_chan); cudaFree(pd.d_snr);
-        cudaFree(pd.d_cnt); cudaFree(pd.d_scratch);
+        if (!p->resolve) cudaFree(pd.d_cnt);
+        cudaFree(pd.d_scratch);
     }
     cudaGetLastError();
     delete p;
@@ -526,6 +602,71 @@ int wofdm_ber_run_multi(wofdm_handle h, const wofdm_sys_t* sys, const double* wi
         sym_tot[i] = frames * (long long)(sys->N - 2 * sys->guard) * (sys->S - 1);   // active sub-carriers only
         bit_tot[i] = sym_tot[i] * sys->bits;
     }
+    return WOFDM_OK;
+}
+
+int wofdm_ber_run_resolved(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
+                           const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                           uint64_t seed, uint32_t variant, int shard_index, int shard_count, int resolve,
+                           int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot) {
+    NvtxRange nvtx_("wofdm_ber_run_resolved");
+    if (!h) return WOFDM_EINVAL;
+    if (resolve == 0 || (resolve & ~(WOFDM_BY_SUBCARRIER | WOFDM_BY_CHANNEL)))
+        return fail(h, WOFDM_EINVAL, "resolve must be a non-empty combination of WOFDM_BY_SUBCARRIER and WOFDM_BY_CHANNEL");
+    if (!bit_err || !sym_err || !sym_tot) return fail(h, WOFDM_EINVAL, "NULL output buffer");
+    if (shard_count < 1 || shard_index < 0 || shard_index >= shard_count) return fail(h, WOFDM_EINVAL, "bad shard");
+    if (ensemble < 1) return fail(h, WOFDM_EINVAL, "ensemble must be >= 1");
+    int rc = validate_sys(h, sys, L);
+    if (rc) return rc;
+    if (C < 1 || n_snr < 1) return fail(h, WOFDM_EINVAL, "C and n_snr must be >= 1");
+    if (n_var < 1 || n_var > WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "n_var must be in [1, WOFDM_MAX_VARIANTS]");
+    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? sys->N : 1;
+    // n_var * n_snr * Cr * Nr counters (x 2 on the device, x 8 bytes): all of it must be representable
+    size_t cells = 0, n_out = 0, dev_bytes = 0;
+    if (__builtin_mul_overflow((size_t)n_snr, (size_t)Cr, &cells) || __builtin_mul_overflow(cells, (size_t)Nr, &cells) ||
+        __builtin_mul_overflow(cells, (size_t)n_var, &n_out) || __builtin_mul_overflow(n_out, (size_t)16, &dev_bytes) ||
+        n_out > (size_t)INT64_MAX / 16)
+        return fail(h, WOFDM_EINVAL, "resolved counter array too large");
+    wofdm_ber_plan p = nullptr;
+    rc = plan_create_impl(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, &p, true, resolve);
+    if (rc) return rc;
+    // the handle's devices split this shard's frames as in wofdm_ber_run_multi; their counter arrays are summed here
+    const int nd = (int)h->devs.size();
+    for (int i = 0; i < nd && rc == WOFDM_OK; ++i)
+        rc = wofdm_ber_plan_launch(p, i, ensemble, seed, variant, shard_index + shard_count * i, shard_count * nd,
+                                   nullptr, nullptr);
+    std::vector<unsigned long long> tmp;
+    if (rc == WOFDM_OK) {
+        for (size_t i = 0; i < n_out; ++i) { bit_err[i] = 0; sym_err[i] = 0; }
+        try { tmp.resize(n_out * 2); } catch (const std::bad_alloc&) { rc = fail(h, WOFDM_ENOMEM, "host allocation failed"); }
+    }
+    for (int i = 0; i < nd && rc == WOFDM_OK; ++i) {
+        PlanDev& pd = p->devs[i];
+        if (!pd.pending) continue;
+        cudaError_t e = cudaSetDevice(h->devs[i].dev);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(tmp.data(), pd.d_cnt, dev_bytes, cudaMemcpyDeviceToHost, pd.last_stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(pd.last_stream);
+        if (e != cudaSuccess) { rc = fail(h, WOFDM_ECUDA, std::string("resolved counters: ") + cudaGetErrorString(e)); break; }
+        for (size_t k = 0; k < n_out; ++k) { bit_err[k] += (int64_t)tmp[2 * k]; sym_err[k] += (int64_t)tmp[2 * k + 1]; }
+        pd.pending = false;
+    }
+    wofdm_ber_plan_destroy(p);
+    if (rc) return rc;
+    // frames of this shard per cell (si, c): f in [(si*C + c)*ensemble, +ensemble), f = shard_index (mod shard_count);
+    // guard bins never carry data and count nothing
+    auto count_upto = [&](long long x) -> long long { return x > shard_index ? (x - shard_index + shard_count - 1) / shard_count : 0; };
+    const long long active = sys->N - 2 * sys->guard;
+    for (int si = 0; si < n_snr; ++si)
+        for (int c = 0; c < Cr; ++c) {
+            const long long lo = ((long long)si * C + (Cr > 1 ? c : 0)) * ensemble, hi = lo + (Cr > 1 ? 1 : (long long)C) * ensemble;
+            const long long frames = count_upto(hi) - count_upto(lo);
+            int64_t* out = sym_tot + ((size_t)si * Cr + c) * Nr;
+            if (Nr == 1) { out[0] = frames * active * (sys->S - 1); continue; }
+            for (int k = 0; k < Nr; ++k) {
+                const int cc = (k + Nr / 2) & (Nr - 1);               // ber_kernel.cuh: bin_active
+                out[k] = (cc >= sys->guard && cc < Nr - sys->guard) ? frames * (sys->S - 1) : 0;
+            }
+        }
     return WOFDM_OK;
 }
 

@@ -1,39 +1,8 @@
 // fp32 instantiations of K1, second generation of the tensor-core-convolution kernel (ber_tconv2.cuh): N = 256, one CTA
 // of 256 threads per frame, two CTAs per SM; N = 512, one CTA of 512 threads per frame and SM; NTILE = tiles of 512 stream
 // samples (tensor-memory accumulators) per frame.
-#include "ber_registry.h"
-#include "ber_tconv2.cuh"
+#include "ber_tconv2_registry.h"
 namespace wofdm {
-namespace {
-template <int N, int NT, int NTILE, int MINB, bool V, int CL = 1, int LB = TCV_LB, bool TXY = false>
-struct Tconv2VariantImpl {
-    // grid = CTAs (a multiple of CL); CL > 1 launches thread-block clusters of CL CTAs
-    static cudaError_t launch(const BerParams& prm, int grid, size_t smem, cudaStream_t st) {
-        if constexpr (CL == 1) {
-            ber_tconv2_kernel<N, NT, NTILE, MINB, V, 1, LB, TXY><<<grid, NT + tconv2_mma_warp_threads(N, NT), smem, st>>>(prm);   // (+ the MMA warp)
-            return cudaGetLastError();
-        } else {
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3(grid); cfg.blockDim = dim3(NT + tconv2_mma_warp_threads(N, NT)); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-            cudaLaunchAttribute at[1];
-            at[0].id = cudaLaunchAttributeClusterDimension;
-            at[0].val.clusterDim.x = CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-            cfg.attrs = at; cfg.numAttrs = 1;
-            return cudaLaunchKernelEx(&cfg, ber_tconv2_kernel<N, NT, NTILE, MINB, V, CL, LB, TXY>, prm);
-        }
-    }
-    static BerVariant make(const char* name) {
-        BerVariant v;
-        v.name = name; v.N = N; v.NT = NT; v.TC = 2 * NTILE; v.LB = LB; v.MINB = MINB; v.CL = CL; v.circ = false; v.txs = true; v.full = false;
-        v.ntile = NTILE; v.gen = 2; v.txy = TXY; v.launch_threads = NT + tconv2_mma_warp_threads(N, NT);
-        v.fp64 = false; v.verify = V;
-        v.layout = &tconv2_smem_layout<N, NT, NTILE, LB>;
-        v.fn = reinterpret_cast<const void*>(&ber_tconv2_kernel<N, NT, NTILE, MINB, V, CL, LB, TXY>);
-        v.launch = &launch;
-        return v;
-    }
-};
-}  // namespace
 #define WOFDM_VARIANT_TCONV2(N, NT, NTILE, MINB)                                                              \
     out.push_back(Tconv2VariantImpl<N, NT, NTILE, MINB, false>::make("ber_f32t2_n" #N "_t" #NT "_tiles" #NTILE "_b" #MINB)); \
     out.push_back(Tconv2VariantImpl<N, NT, NTILE, MINB, true>::make("ber_f32t2_n" #N "_t" #NT "_tiles" #NTILE "_b" #MINB "_verify"));

@@ -85,6 +85,9 @@ struct BerParams {
     // one column of tx_yp floats per symbol (local frame j, symbol s: column j*S + s); the loader does the overlap-adds itself
     const float* tx_y;
     int tx_yp;
+    // RES instantiations (wofdm_ber_run_resolved): counters are [nvar][cell][bins][2] with cell = si*C + ci (res_chan) or si,
+    // bins = N (res_bins: one pair per sub-carrier, accumulated in shared memory) or 1 (the per-warp atomics, re-addressed)
+    int res_chan, res_bins;
 };
 
 // ---- constellation helpers (oracle/wofdm_oracle.py: idx_to_levels / levels_to_idx) --------------
@@ -300,9 +303,46 @@ struct BerSmem {
     int off_x, off_tw, off_geq, off_hf, off_taps, off_wtx, off_wrx, off_red, off_qlut, off_dlut, off_gmask, off_symw;   // byte offsets
     int off_lo, off_bt, off_bar;   // tensor-core convolution policy (ber_tconv.cuh): lo half of the split stream, taps operand, mbarrier
     size_t bytes;
+    int off_res;    // RES instantiations: per-sub-carrier error accumulators, uint32 {bit, sym} per (window pair, bin)
 };
 
-template <typename T, int N, int NT, int TC, int LB>
+// Per-sub-carrier error counts of the RES instantiations (wofdm_ber_run_resolved).  A CTA adds the errors of every decided
+// symbol into 32-bit shared accumulators racc[var][k] = {bit, sym} and moves them to the u64 counters of its current cell only
+// when the cell (SNR point, or SNR point x channel) of its next frame differs, before a 32-bit accumulator could wrap, and at
+// its last frame.  Frames f = (si*C + ci)*ensemble + e are taken round-robin, so a CTA stays in one cell for ensemble / (frames
+// in flight) frames in a row.  Zero accumulators are skipped; the shared atomics of a frame only touch bins with an error.
+// add the errors of x = decided ^ sent (four level codes, byte b = bin k0 + b*kstep) to the accumulators
+__device__ __forceinline__ void res_add4(uint32_t* racc, uint32_t x, uint32_t gxm, int k0, int kstep) {
+#pragma unroll
+    for (int b = 0; b < 4; ++b) {
+        const uint32_t xb = (x >> (8 * b)) & 0xffu;
+        if (xb) {
+            uint32_t* a = racc + 2 * (k0 + b * kstep);
+            atomicAdd(a, code_bit_errors(xb, gxm));
+            atomicAdd(a + 1, 1u);
+        }
+    }
+}
+// move the n accumulator pairs of this CTA into dst (pair e -> dst[2 * (e / nb * cstride + e % nb)]) and zero them.
+// Ordering, both sides by barriers: callers put one in front (every add of the old cell is done), and the next frame's adds
+// come only after the CTA-wide barriers every policy passes before its decisions (the power sums' frame_sync, the pilot's
+// barrier), which every thread reaches only after its part of this loop.  A schedule without such a barrier between the
+// flush and the next decisions needs a second barrier here.
+__device__ __forceinline__ void res_flush(uint32_t* racc, int n, int nb, size_t cstride, unsigned long long* dst, int tid, int nt) {
+    for (int e = tid; e < n; e += nt) {
+        const unsigned sc = racc[2 * e + 1];
+        if (sc == 0u) continue;                        // (no symbol error: no bit error either)
+        const unsigned bb = racc[2 * e];
+        racc[2 * e] = 0u; racc[2 * e + 1] = 0u;
+        unsigned long long* d = dst + 2 * ((size_t)(e / nb) * cstride + (e % nb));
+        atomicAdd(d, (unsigned long long)bb);
+        atomicAdd(d + 1, (unsigned long long)sc);
+    }
+}
+// frames between flushes such that no 32-bit accumulator wraps: a frame adds at most S * bits bit errors to a bin
+__host__ __device__ __forceinline__ unsigned res_frame_limit(int S, int bits) { return 0xffffffffu / (unsigned)(S * (bits > 1 ? bits : 1)); }
+
+template <typename T, int N, int NT, int TC, int LB, bool RES = false>
 __host__ __device__ inline BerSmem ber_smem_layout(int S, int stride, int tail_tx, int tail_rx, int L, int chunk,
                                                    int use_global) {
     using P = FftPlan<N>;
@@ -339,6 +379,8 @@ __host__ __device__ inline BerSmem ber_smem_layout(int S, int stride, int tail_t
     o += 256;                                              m.off_gmask = o;
     o += P::TPF * 32;                                      m.off_symw = o;     // guard band: two uint4 per thread of a transform
     o += S * P::TPF * 16;                                  // constellation-index words of every (symbol, thread)
+    m.off_res = 0;
+    if constexpr (RES) { o = (o + 15) & ~15; m.off_res = o; o += N * 8; }
     m.bytes = ((size_t)o + 15) & ~(size_t)15;
     return m;
 }
@@ -395,7 +437,10 @@ template <int CL> __device__ __forceinline__ void frame_sync() {
 
 // TXS: the Tx stage can take the frame's stream from HBM (BerParams::tx_stream, channel-mask variant).  Always possible in
 // the staged policy; the register-resident kernels get it as separate instantiations so that the main path keeps its code.
-template <typename T, int N, int NT, int TC, int LB, int MINB, bool FULL, bool VERIFY, int CL = 1, bool CIRC = false, bool TXS = false>
+// RES: error counters resolved by sub-carrier and / or channel (BerParams::res_chan / res_bins); in a cluster every CTA keeps
+// and flushes the accumulators of its own symbols
+template <typename T, int N, int NT, int TC, int LB, int MINB, bool FULL, bool VERIFY, int CL = 1, bool CIRC = false, bool TXS = false,
+          bool RES = false>
 __global__ void __launch_bounds__(NT, MINB)
 ber_frame_kernel(const BerParams prm) {
     using P = FftPlan<N>;
@@ -405,6 +450,7 @@ ber_frame_kernel(const BerParams prm) {
     static_assert(NT % TPF == 0 && NT % 32 == 0, "threads per CTA must be a multiple of N/16 and 32");
     constexpr bool REGS = TC > 0;
     static_assert(CL == 1 || REGS, "clusters are a feature of the register-resident policy");
+    static_assert(!RES || (!VERIFY && !TXS), "resolved counters: production kernels");
     static_assert(!CIRC || (REGS && CL == 1 && N <= NT), "circular-interior policy: regs, one CTA per frame, one bin per thread");
     // Register row q of a thread = sub-carriers / samples t + q*TPF.  Only the outer rows can reach the cyclic
     // prefix / suffix, the Tx heads and the Rx overlap-add; the tuned variants look at ER of them (the host
@@ -426,7 +472,7 @@ ber_frame_kernel(const BerParams prm) {
     const int body = beta + sec;                // serialised Tx stream length
     const bool last_rank = rank == CL - 1;
 
-    const BerSmem lay = ber_smem_layout<T, N, NT, TC, LB>(S, stride, beta, prm.tail_rx, L, prm.chunk, prm.use_global);
+    const BerSmem lay = ber_smem_layout<T, N, NT, TC, LB, RES>(S, stride, beta, prm.tail_rx, L, prm.chunk, prm.use_global);
     C2* fbuf = reinterpret_cast<C2*>(smem_raw);
     C2* xbuf = reinterpret_cast<C2*>(smem_raw + lay.off_x);
     C2* tw = reinterpret_cast<C2*>(smem_raw + lay.off_tw);
@@ -465,6 +511,8 @@ ber_frame_kernel(const BerParams prm) {
         qlut[i] = mk2<T>((T)(2 * (i >> hb) - (m - 1)), (T)(2 * (i & (m - 1)) - (m - 1)));
     if (tid == 0 && prm.bits < 8) qlut[255] = mk2<T>(0, 0);              // the null sub-carrier
     const uint32_t gxm = gray_xor_mask(prm.bits, prm.constellation);
+    uint32_t* const racc = reinterpret_cast<uint32_t*>(smem_raw + lay.off_res);   // RES: [N][2] = {bit, sym}
+    if constexpr (RES) { for (int i = tid; i < 2 * N; i += NT) racc[i] = 0u; }
     __syncthreads();
     if (prm.guard > 0) {
         const unsigned d0 = slice_index(mk2<T>(0, 0), hb);                // what the slicer makes of a null bin
@@ -493,6 +541,11 @@ ber_frame_kernel(const BerParams prm) {
         si = (int)(q / prm.C);       ci = (int)(q - (long long)si * prm.C);
         ds = (int)(dq / prm.C);      dc = (int)(dq - (long long)ds * prm.C);
     }
+    // RES: cells of the counters and this CTA's current one
+    const size_t ncell = RES ? (size_t)prm.n_snr * (prm.res_chan ? prm.C : 1) : 0;
+    int rcell = RES ? (prm.res_chan ? si * prm.C + ci : si) : 0;
+    unsigned rfr = 0;
+    const unsigned rlim = RES ? res_frame_limit(prm.S, prm.bits) : 0u;
     for (long long j = fslot; j < prm.n_frames; j += nslots) {
         if constexpr (VERIFY) { ci = (int)f; si = (int)f; }
         const T snr_lin = reinterpret_cast<const T*>(prm.snr_lin)[si];
@@ -903,6 +956,7 @@ ber_frame_kernel(const BerParams prm) {
                     const int txi = sym_byte(w, q);
                     sym_cnt += (dec != txi);                                               // :235
                     bit_cnt += code_bit_errors((uint32_t)(dec ^ txi), gxm);
+                    if constexpr (RES) { if (prm.res_bins && dec != txi) res_add4(racc, (uint32_t)(dec ^ txi), gxm, k, 0); }
                     if constexpr (VERIFY) {
                         const size_t o = ((size_t)f * (prm.S - 1) + (sb + s - 1)) * N + k;
                         prm.eq_out[o] = make_double2((double)e.x * prm.qscale, (double)e.y * prm.qscale);
@@ -913,7 +967,12 @@ ber_frame_kernel(const BerParams prm) {
         }
         bit_cnt = warp_sum(bit_cnt);
         sym_cnt = warp_sum(sym_cnt);
-        if ((tid & 31) == 0) {
+        if constexpr (RES) {
+            if (!prm.res_bins && (tid & 31) == 0) {      // per-cell totals: the per-warp atomics at the cell's address
+                atomicAdd(prm.counters + 2 * rcell, (unsigned long long)bit_cnt);
+                atomicAdd(prm.counters + 2 * rcell + 1, (unsigned long long)sym_cnt);
+            }
+        } else if ((tid & 31) == 0) {
             if constexpr (VERIFY) {
                 atomicAdd(reinterpret_cast<unsigned long long*>(prm.bit_err_f) + f, (unsigned long long)bit_cnt);
                 atomicAdd(reinterpret_cast<unsigned long long*>(prm.sym_err_f) + f, (unsigned long long)sym_cnt);
@@ -935,6 +994,18 @@ ber_frame_kernel(const BerParams prm) {
             ci += dc;
             if (ci >= prm.C) { ci -= prm.C; ++si; }
             si += ds;
+        }
+        if constexpr (RES) {
+            if (prm.res_bins) {                          // uniform: the next frame's cell, the frame count, the last frame
+                const int nc = prm.res_chan ? si * prm.C + ci : si;
+                if (nc != rcell || ++rfr >= rlim || j + nslots >= prm.n_frames) {
+                    __syncthreads();                     // every decision of the cell has been added
+                    res_flush(racc, N, N, ncell * N, prm.counters + (size_t)rcell * N * 2, tid, NT);
+                    rcell = nc; rfr = 0;
+                }
+            } else {
+                rcell = prm.res_chan ? si * prm.C + ci : si;
+            }
         }
     }
     if constexpr (CL > 1) cooperative_groups::this_cluster().sync();   // nobody leaves while a peer may still read its shared memory

@@ -92,6 +92,7 @@ __host__ __device__ constexpr int tconv2_seg_of(int nseg, int ntile, int tt) {
     return k;
 }
 constexpr int TCV2_BAR_STREAM = 14;      // named barrier: "the split stream of this frame is complete"
+constexpr int TCV2_BAR_RES = 15;         // named barrier of the working warps before a flush of the resolved counters (RES)
 
 // N <= 512: the CTA has one more warp that only issues the MMAs.  The register file then leaves the working threads 96
 // registers (two CTAs of 288 threads, or one of 544, per SM), which the N = 256 kernel fits without spills and the N = 512
@@ -185,7 +186,7 @@ static __device__ __forceinline__ void tconv2_load_masked(const float* __restric
     }
 }
 
-template <int N, int NT, int NTILE, int LB = TCV_LB>
+template <int N, int NT, int NTILE, int LB = TCV_LB, bool RES = false>
 __host__ __device__ inline BerSmem tconv2_smem_layout(int S, int stride, int tail_tx, int tail_rx, int L, int nvar, int use_global) {
     using P = FftPlan<N>;
     constexpr int FPP = NT / P::TPF;
@@ -210,6 +211,8 @@ __host__ __device__ inline BerSmem tconv2_smem_layout(int S, int stride, int tai
     o += P::TPF * 32;                         m.off_symw = o;
     o += S * P::TPF * 16;                     m.off_bar = o;
     o += 8 * TCV2_MAXSEG + 8;
+    m.off_res = 0;
+    if constexpr (RES) { o = (o + 15) & ~15; m.off_res = o; o += nv * N * 8; }   // per-sub-carrier error accumulators
     m.off_hf = m.off_taps = m.off_dlut = 0;
     m.bytes = ((size_t)o + 15) & ~(size_t)15;
     (void)L; (void)use_global;
@@ -221,7 +224,9 @@ __host__ __device__ inline BerSmem tconv2_smem_layout(int S, int stride, int tai
 // three times per frame through distributed shared memory: the second CTA takes the first one's last Tx tail and the
 // L - 1 samples of convolution history (PULLED, a few dozen words), the per-warp power partials and the pilot's equaliser
 // taps are PUSHED into both CTAs, so every read is local.
-template <int N, int NT, int NTILE, int MINB, bool VERIFY, int CL = 1, int LB = TCV_LB, bool TXY = false>
+// RES: error counters resolved by sub-carrier and / or channel (BerParams::res_chan / res_bins, ber_kernel.cuh: res_flush);
+// in a cluster every CTA keeps and flushes the accumulators of its own symbols
+template <int N, int NT, int NTILE, int MINB, bool VERIFY, int CL = 1, int LB = TCV_LB, bool TXY = false, bool RES = false>
 __global__ void __launch_bounds__(NT + tconv2_mma_warp_threads(N, NT), MINB)
 ber_tconv2_kernel(const BerParams prm) {
     using T = float;
@@ -235,6 +240,7 @@ ber_tconv2_kernel(const BerParams prm) {
     static_assert(NSEG <= TCV2_MAXSEG, "one mbarrier per segment");
     static_assert(16 * NTILE <= (int)TMEM_COLS, "accumulators of a frame must fit tensor memory");
     static_assert(CL * NW <= 32, "per-warp power partials of all CTAs must fit the reduction scratch");
+    static_assert(!RES || (!VERIFY && !TXY), "resolved counters: production kernels");
 
     extern __shared__ __align__(128) unsigned char tcv_smem[];
     unsigned char* const smem_raw = tcv_smem;
@@ -255,7 +261,7 @@ ber_tconv2_kernel(const BerParams prm) {
 
     const int nvar = (!VERIFY && prm.nvar > 1) ? prm.nvar : 1;     // window pairs evaluated on every frame's symbols
     constexpr int PAD = tconv2_pad(LB), KS = tconv2_ksteps(LB), TBL = tconv2_tbl(LB), ZERO = tconv2_zero(LB);
-    const BerSmem lay = tconv2_smem_layout<N, NT, NTILE, LB>(S, stride, beta, prm.tail_rx, L, nvar, 0);
+    const BerSmem lay = tconv2_smem_layout<N, NT, NTILE, LB, RES>(S, stride, beta, prm.tail_rx, L, nvar, 0);
     uint32_t* const ahi = reinterpret_cast<uint32_t*>(smem_raw);
     uint32_t* const alo = reinterpret_cast<uint32_t*>(smem_raw + lay.off_lo);
     uint32_t* const uh = ahi + PAD;         // uh[i], ul[i]: split stream sample i
@@ -316,6 +322,8 @@ ber_tconv2_kernel(const BerParams prm) {
     build_qtx(0);
     if (tid == 0 && prm.bits < 8) { qlut[255] = mk2<T>(0, 0); qtx[255] = mk2<T>(0, 0); }
     const uint32_t gxm = gray_xor_mask(prm.bits, prm.constellation);
+    uint32_t* const racc = reinterpret_cast<uint32_t*>(smem_raw + lay.off_res);   // RES: [nvar][N][2] = {bit, sym}
+    if constexpr (RES) { for (int i = tid; i < 2 * N * nvar; i += NT) racc[i] = 0u; }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -438,6 +446,11 @@ ber_tconv2_kernel(const BerParams prm) {
         si = (int)(q / prm.C);       ci = (int)(q - (long long)si * prm.C);
         ds = (int)(dq / prm.C);      dc = (int)(dq - (long long)ds * prm.C);
     }
+    // RES: cells of the counters and this CTA's current one
+    const size_t ncell = RES ? (size_t)prm.n_snr * (prm.res_chan ? prm.C : 1) : 0;
+    int rcell = RES ? (prm.res_chan ? si * prm.C + ci : si) : 0;
+    unsigned rfr = 0;
+    const unsigned rlim = RES ? res_frame_limit(prm.S, prm.bits) : 0u;
     for (long long j = fslot; j < prm.n_frames; j += nslots) {
 #if TCV2_TRACE
         const bool trace_on = blockIdx.x == 0 && trace_it >= 3 && trace_it < 6;
@@ -981,6 +994,7 @@ ber_tconv2_kernel(const BerParams prm) {
                     const uint32_t x = d4 ^ w[gq];
                     bit_cnt += code_bit_errors(x, gxm);                                    // :235 (bits) ...
                     sym_cnt += __popc((((x & 0x7f7f7f7fu) + 0x7f7f7f7fu) | x) & 0x80808080u);   // ... and symbols: bytes that differ
+                    if constexpr (RES) { if (prm.res_bins && x) res_add4(racc + 2 * N * var, x, gxm, t + 4 * gq * TPF, TPF); }
                 }
             }
         }
@@ -1001,7 +1015,12 @@ ber_tconv2_kernel(const BerParams prm) {
             __syncthreads();
         }
 #endif
-        if (lane == 0) {
+        if constexpr (RES) {
+            if (!prm.res_bins && lane == 0) {            // per-cell totals: the per-warp atomics at the cell's address
+                atomicAdd(prm.counters + 2 * (var * ncell + rcell), (unsigned long long)bit_cnt);
+                atomicAdd(prm.counters + 2 * (var * ncell + rcell) + 1, (unsigned long long)sym_cnt);
+            }
+        } else if (lane == 0) {
             if constexpr (VERIFY) {
                 atomicAdd(reinterpret_cast<unsigned long long*>(prm.bit_err_f) + f, (unsigned long long)bit_cnt);
                 atomicAdd(reinterpret_cast<unsigned long long*>(prm.sym_err_f) + f, (unsigned long long)sym_cnt);
@@ -1022,6 +1041,19 @@ ber_tconv2_kernel(const BerParams prm) {
             ci += dc;
             if (ci >= prm.C) { ci -= prm.C; ++si; }
             si += ds;
+        }
+        if constexpr (RES) {
+            if (prm.res_bins) {                          // uniform: the next frame's cell, the frame count, the last frame
+                const int nc = prm.res_chan ? si * prm.C + ci : si;
+                if (nc != rcell || ++rfr >= rlim || j + nslots >= prm.n_frames) {
+                    // the working warps only (the MMA warp keeps its own barrier sequence): every decision of the cell is added
+                    asm volatile("bar.sync %0, %1;" :: "n"(TCV2_BAR_RES), "n"(NT) : "memory");
+                    res_flush(racc, nvar * N, N, ncell * N, prm.counters + (size_t)rcell * N * 2, tid, NT);
+                    rcell = nc; rfr = 0;
+                }
+            } else {
+                rcell = prm.res_chan ? si * prm.C + ci : si;
+            }
         }
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");

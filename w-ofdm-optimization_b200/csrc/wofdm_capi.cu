@@ -146,6 +146,9 @@ int wofdm_create_on(wofdm_handle* out, const int* device_ids, int n) {
     register_ber_f32_regs(h->variants);
     register_ber_f32_staged(h->variants);
     register_ber_f64_staged(h->variants);
+    register_ber_f32_tconv2_res(h->variants);
+    register_ber_staged_res(h->variants);
+    register_ber_f32_regs_res(h->variants);
     *out = h;
     return WOFDM_OK;
 }

@@ -84,6 +84,22 @@ class wOFDMSystem:
         np.save(os.path.join(path_to_ser, f"rc_{self.name}_{self.cp_len}.npy"), ser_rc)
         return ser_opt, ser_rc
 
+    def run_simulation_per_subcarrier(self, channel_models, window_tx, window_rx, ensemble, snr_arr, no_symbols):
+        """run_simulation resolved by sub-carrier: the same symbols and noise (same seed), SER of shape (n_snr, N) per
+        FFT bin for the optimised and the RC windows ((ser_opt, ser_rc); 'CP': one array).  Writes no files.  The
+        mean over the active bins is run_simulation's SER."""
+        h = self._h or default_handle()
+        s = self._sys(int(no_symbols))
+        snr = np.asarray(snr_arr, dtype=np.float64)
+        if self.name == "CP":
+            wt, wr = [np.ones(s.n_tx)], [np.ones(s.N + s.tail_rx)]
+        else:
+            wt, wr = [_diag(window_tx), capi.rc_window_tx(s)], [_diag(window_rx), capi.rc_window_rx(s)]
+        r = h.ber_run_resolved(s, wt, wr, channel_models, snr, ensemble, seed=self.seed, variant=0, by_subcarrier=True)
+        tot = r["sym_tot"][:, 0, :]
+        ser = [np.divide(e[:, 0, :], tot, out=np.zeros(tot.shape), where=tot > 0) for e in r["sym_err"]]
+        return ser[0] if self.name == "CP" else (ser[0], ser[1])
+
 
 def load_window_tails(system_design, window_path, cp_len, tail_tx, tail_rx):
     """<window_path>/<sys>_<cp>.npy -> (x_tx, x_rx) reduced variables (wofdm_simulation.py:46-66, SURVEY App. A.4)."""
