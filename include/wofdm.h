@@ -149,6 +149,57 @@ WOFDM_API int wofdm_ber_run_resolved(wofdm_handle h, const wofdm_sys_t* sys, con
                        uint64_t seed, uint32_t variant, int shard_index, int shard_count, int resolve,
                        int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot);
 
+/* Frame segments: a chosen subset of a job's frames.  The job has ensemble_max ensemble indices; its frames are numbered
+ * as in wofdm_ber_run_multi with ensemble = ensemble_max, f = (snr_idx*C + c)*ensemble_max + e, and draw what they draw there.
+ * Segment k = segments[3k .. 3k+2] = {snr_idx, e_begin, e_count} is every frame of that SNR point with any channel c < C
+ * and e in [e_begin, e_begin + e_count).  A call runs its segments as one local index space j: segments in the order given,
+ * channel-major, then e, inside a segment; shards and the handle's devices split j exactly as wofdm_ber_run_multi splits f
+ * (device i of the handle takes j = shard_index + shard_count*i (mod shard_count*ndev)).  Every channel of a point gets
+ * the same frames, so errors / total stays the reference's mean over channels of the mean over the ensemble, and the
+ * counters of disjoint segment lists add up to those of their union: a finished run can be extended where it needs more
+ * precision without repeating a frame.
+ *   resolve = 0: bit_err / sym_err int64[n_var][n_snr], sym_tot int64[n_snr]; non-zero: the layout and semantics of
+ *   wofdm_ber_run_resolved.  sym_tot counts this shard's frames; bit totals are sym_tot * bits.
+ * The call runs the resolved-counter twins with the fallback rules of wofdm_ber_run_resolved.  The segment table is read
+ * on the device, so the twin's counters of [0, e1) and [e1, E) add up to wofdm_ber_run_multi(E) / wofdm_ber_run_resolved(E).
+ * WOFDM_EINVAL: n_seg < 1 or NULL segments; a segment outside [0, n_snr) x [0, ensemble_max) or with e_count < 1; two
+ * overlapping segments of one point; ensemble_max < 1 or n_snr * C * ensemble_max overflowing int64; unknown resolve bits;
+ * and what wofdm_ber_run_multi / _resolved reject.  The handle stays usable after every error. */
+WOFDM_API int wofdm_ber_run_segments(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
+                       const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble_max,
+                       const int64_t* segments /* [n_seg][3] = {snr_idx, e_begin, e_count} */, int n_seg,
+                       uint64_t seed, uint32_t variant, int shard_index, int shard_count, int resolve,
+                       int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot);
+
+/* Stopping rule of Monte-Carlo BER runs: every SNR point runs until it has counted `target` errors or ensemble_max ensemble
+ * indices, in rounds of frame segments (wofdm_ber_run_segments; one plan for the whole call, one segment table upload,
+ * one launch per device and one counter read per round).
+ * Schedule (e_s: ensemble indices point s has run, b_s: its last block):
+ *   round 0 gives every point b = min(first_block, ensemble_max);
+ *   after each round, m_s = the minimum over the window pairs v of point s's cumulative bit errors (target_kind
+ *   WOFDM_TARGET_BIT_ERRORS) or symbol errors (WOFDM_TARGET_SYMBOL_ERRORS);
+ *   point s is done when m_s >= target or e_s == ensemble_max; otherwise its next block is
+ *     min(ensemble_max - e_s, 2*b_s, m_s > 0 ? max(1, ceil((target - m_s) * e_s / m_s)) : 2*b_s)
+ *   in exact integer arithmetic (128-bit, saturating);
+ *   a round's segments are {s, e_s, b_s} of the active points in ascending SNR order.
+ * reduce (optional): called once per round with this process's round counts int64[n_var][n_snr][2] = {bit, sym}, n =
+ * 2*n_var*n_snr; it must overwrite them with their sum over the processes and return 0.  With it every process computes the
+ * same schedule and returns the job's totals.  shard_count > 1 without reduce is WOFDM_EINVAL; a non-zero return fails the
+ * call with WOFDM_EINVAL.  reduce must not call into this handle.
+ * Outputs: ensemble_used[n_snr] (point s ran C * ensemble_used[s] frames: the ensemble indices [0, ensemble_used[s])),
+ * bit_err / sym_err int64[n_var][n_snr] those frames' counters, bit_tot / sym_tot int64[n_snr] their totals, *rounds.
+ * Bias: errors / bits of a run stopped at a target error count is not unbiased -- its relative bias is of order 1/target,
+ * as in inverse binomial sampling; choose target >> 1 (100 gives ~1 %).  Points that stop at ensemble_max are unbiased.
+ * WOFDM_EINVAL additionally: target < 1, an unknown target_kind, first_block < 1, NULL outputs. */
+#define WOFDM_TARGET_BIT_ERRORS    0
+#define WOFDM_TARGET_SYMBOL_ERRORS 1
+typedef int (*wofdm_reduce_fn)(int64_t* counts, int64_t n, void* user);
+WOFDM_API int wofdm_ber_run_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
+                       const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble_max, int64_t first_block,
+                       int target_kind, int64_t target, uint64_t seed, uint32_t variant, int shard_index, int shard_count,
+                       wofdm_reduce_fn reduce, void* reduce_user,
+                       int64_t* ensemble_used, int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot, int* rounds);
+
 /* Device-resident form: inputs are uploaded once, launches are asynchronous. */
 WOFDM_API int wofdm_ber_plan_create(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
                           const double* chan, int L, int C, const double* snr_db, int n_snr,

@@ -14,6 +14,7 @@
 //          reads from settingsData.mat / the channel file inside the function are passed explicitly.
 //   berSNR = wofdm_mex('run_simulation_sweep_multi', ...)   every window variant of a (system, CP) on the same bits, one job
 //   berK = wofdm_mex('run_simulation_per_subcarrier', ...)  the same, BER per sub-carrier: n_snr x N x n_var
+//   [berSNR, ensembleUsed] = wofdm_mex('run_simulation_adaptive', ...)  the same, each SNR point stopped at a bit-error target
 //   [berMasked, ber] = wofdm_mex('run_sim_mc', ...)          run_sim_mc of matlab/main_channel_mask.m:334-337
 //   H = wofdm_mex('window_hessian', ...)                     quad_objective_tx / _rx of matlab/window_optimization.m:596-680
 //   H = wofdm_mex('window_hessian_expected', ...), 'quad_objective_tx_expected', 'quad_objective_rx_expected'
@@ -162,9 +163,13 @@ static std::vector<double> windows_of(const mxArray* a, size_t want, size_t* n_v
 // Returns n_snr x n_var; column v = run_simulation_sweep with pair v (its noise stream: variant v).
 // per_subcarrier = true ('run_simulation_per_subcarrier', the same arguments): BER of every sub-carrier,
 // n_snr x N x n_var (FFT bin order; guard bins 0), from wofdm_ber_run_resolved on the same draws.
-static void do_run_simulation_multi(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[], bool per_subcarrier) {
-    if (nrhs < 14) mexErrMsgIdAndTxt("wofdm:nargin", "%s needs 14 arguments", per_subcarrier ? "run_simulation_per_subcarrier" : "run_simulation_sweep_multi");
-    (void)nlhs;
+// adaptive = true ('run_simulation_adaptive', the 14 arguments, then targetBitErrors, ensembleMax [, seed]): every SNR point
+// runs until each pair has counted targetBitErrors bit errors or ensembleMax ensemble indices (wofdm_ber_run_adaptive);
+// the first argument, ensemble, is the first round's block.  Returns [berSNR (n_snr x n_var), ensembleUsed (n_snr x 1)].
+static void do_run_simulation_multi(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[], bool per_subcarrier,
+                                    bool adaptive = false) {
+    const char* name = adaptive ? "run_simulation_adaptive" : per_subcarrier ? "run_simulation_per_subcarrier" : "run_simulation_sweep_multi";
+    if (nrhs < (adaptive ? 16 : 14)) mexErrMsgIdAndTxt("wofdm:nargin", "%s needs %d arguments", name, adaptive ? 16 : 14);
     wofdm_sys_t s;
     memset(&s, 0, sizeof(s));
     const long long ensemble = (long long)mxGetScalar(prhs[0]);
@@ -181,7 +186,8 @@ static void do_run_simulation_multi(int nlhs, mxArray* plhs[], int nrhs, const m
         mexErrMsgIdAndTxt("wofdm:size", "windowTx / windowRx: cell arrays of the same length (<= %d), or one window", WOFDM_MAX_VARIANTS);
     while (wtx.size() < n_var * n_tx) wtx.insert(wtx.end(), wtx.begin(), wtx.begin() + n_tx);
     while (wrx.size() < n_var * n_wr) wrx.insert(wrx.end(), wrx.begin(), wrx.begin() + n_wr);
-    const unsigned long long seed = nrhs > 14 ? (unsigned long long)mxGetScalar(prhs[14]) : 0ull;
+    const int seed_arg = adaptive ? 16 : 14;
+    const unsigned long long seed = nrhs > seed_arg ? (unsigned long long)mxGetScalar(prhs[seed_arg]) : 0ull;
     const size_t C = mxGetM(prhs[7]), L = mxGetN(prhs[7]);
     std::vector<double> chan(2 * L * C);
     for (size_t c = 0; c < C; ++c) {
@@ -208,6 +214,24 @@ static void do_run_simulation_multi(int nlhs, mxArray* plhs[], int nrhs, const m
         return;
     }
     std::vector<long long> be(n_var * n_snr), se(n_var * n_snr), bt(n_snr), st(n_snr);
+    if (adaptive) {
+        std::vector<long long> used(n_snr);
+        int rounds = 0;
+        check(wofdm_ber_run_adaptive(handle(), &s, wtx.data(), wrx.data(), (int)n_var, chan.data(), (int)L, (int)C, mxGetPr(prhs[8]),
+                                     (int)n_snr, (long long)mxGetScalar(prhs[15]), ensemble, WOFDM_TARGET_BIT_ERRORS,
+                                     (long long)mxGetScalar(prhs[14]), seed, 0, 0, 1, nullptr, nullptr, (int64_t*)used.data(),
+                                     (int64_t*)be.data(), (int64_t*)bt.data(), (int64_t*)se.data(), (int64_t*)st.data(), &rounds),
+              "wofdm_ber_run_adaptive");
+        plhs[0] = mxCreateDoubleMatrix((mwSize)n_snr, (mwSize)n_var, mxREAL);
+        double* out = mxGetPr(plhs[0]);
+        for (size_t v = 0; v < n_var; ++v)
+            for (size_t i = 0; i < n_snr; ++i) out[v * n_snr + i] = bt[i] ? (double)be[v * n_snr + i] / (double)bt[i] : 0.0;
+        if (nlhs > 1) {
+            plhs[1] = mxCreateDoubleMatrix((mwSize)n_snr, 1, mxREAL);
+            for (size_t i = 0; i < n_snr; ++i) mxGetPr(plhs[1])[i] = (double)used[i];
+        }
+        return;
+    }
     check(wofdm_ber_run_multi(handle(), &s, wtx.data(), wrx.data(), (int)n_var, chan.data(), (int)L, (int)C, mxGetPr(prhs[8]), (int)n_snr,
                               ensemble, seed, 0, 0, 1, (int64_t*)be.data(), (int64_t*)bt.data(), (int64_t*)se.data(), (int64_t*)st.data()),
           "wofdm_ber_run_multi");
@@ -379,11 +403,12 @@ static void do_calculate_interference(int nlhs, mxArray* plhs[], int nrhs, const
 extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     char cmd[32];
     if (nrhs < 1 || !mxIsChar(prhs[0]) || mxGetString(prhs[0], cmd, sizeof(cmd)))
-        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_sim_mc', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
+        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_simulation_adaptive', 'run_sim_mc', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
     if (!strcmp(cmd, "run_simulation")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_simulation_sweep")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, true);
     else if (!strcmp(cmd, "run_simulation_sweep_multi")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_simulation_per_subcarrier")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, true);
+    else if (!strcmp(cmd, "run_simulation_adaptive")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, false, true);
     else if (!strcmp(cmd, "run_sim_mc")) do_run_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1);
     else if (!strcmp(cmd, "window_hessian")) do_window_hessian(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "quad_objective_tx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, true, false);

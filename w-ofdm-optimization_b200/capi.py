@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(_HERE, "libwofdm.so")
 
 OK, EINVAL, ECUDA, ENOMEM, ENODEV, EUNSUPPORTED = 0, -1, -2, -3, -4, -5
 WOFDM_BY_SUBCARRIER, WOFDM_BY_CHANNEL = 1, 2         # wofdm_ber_run_resolved: resolve flags
+WOFDM_TARGET_BIT_ERRORS, WOFDM_TARGET_SYMBOL_ERRORS = 0, 1   # wofdm_ber_run_adaptive: target_kind
 _ERRNAME = {EINVAL: "WOFDM_EINVAL", ECUDA: "WOFDM_ECUDA", ENOMEM: "WOFDM_ENOMEM", ENODEV: "WOFDM_ENODEV",
             EUNSUPPORTED: "WOFDM_EUNSUPPORTED"}
 
@@ -57,6 +58,8 @@ class SysT(C.Structure):
 
 _P = C.POINTER
 _dp, _i32p, _i64p = _P(C.c_double), _P(C.c_int32), _P(C.c_int64)
+# wofdm_reduce_fn: int (*)(int64_t* counts, int64_t n, void* user)
+REDUCE_FN = C.CFUNCTYPE(C.c_int, _i64p, C.c_int64, C.c_void_p)
 
 # name -> (restype, argtypes); every symbol include/wofdm.h declares
 SIGNATURES = {
@@ -81,6 +84,11 @@ SIGNATURES = {
                                       C.c_uint64, C.c_uint32, C.c_int, C.c_int, _i64p, _i64p, _i64p, _i64p]),
     "wofdm_ber_run_resolved": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, C.c_int, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
                                          C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_int, _i64p, _i64p, _i64p]),
+    "wofdm_ber_run_segments": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, C.c_int, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
+                                         _i64p, C.c_int, C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_int, _i64p, _i64p, _i64p]),
+    "wofdm_ber_run_adaptive": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, C.c_int, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
+                                         C.c_int64, C.c_int, C.c_int64, C.c_uint64, C.c_uint32, C.c_int, C.c_int, REDUCE_FN,
+                                         C.c_void_p, _i64p, _i64p, _i64p, _i64p, _i64p, _P(C.c_int)]),
     "wofdm_ber_plan_create_multi": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, C.c_int, _dp, C.c_int, C.c_int, _dp, C.c_int,
                                               _P(C.c_void_p)]),
     "wofdm_ber_plan_variants": (C.c_int, [C.c_void_p, _P(C.c_int)]),
@@ -300,6 +308,57 @@ class Handle:
         self._check(rc)
         return dict(bit_err=be, sym_err=se, sym_tot=st, bit_tot=st * int(s.bits))
 
+    def ber_run_segments(self, s, wins_tx, wins_rx, chan, snr_db, ensemble_max, segments, seed=0, variant=0, shard=(0, 1),
+                         by_subcarrier=False, by_channel=False):
+        """A chosen subset of a job's frames (wofdm_ber_run_segments).  segments: (n_seg, 3) {snr_idx, e_begin, e_count}, every
+        channel of point snr_idx at ensemble indices [e_begin, e_begin + e_count) of a job of ensemble_max indices; frames and
+        draws are those of ber_run_multi(..., ensemble=ensemble_max).  Unresolved: bit_err / sym_err (n_var, n_snr), sym_tot /
+        bit_tot (n_snr,); resolved: the shapes of ber_run_resolved."""
+        wt, wr = self._win_multi(s, wins_tx, wins_rx)
+        _, _, chf, L, Cn = self._win_chan(s, wt[0], wr[0], chan)
+        snr = _f64(np.ravel(snr_db))
+        n, nv = snr.size, wt.shape[0]
+        seg = np.ascontiguousarray(np.asarray(segments, dtype=np.int64).reshape(-1, 3))
+        resolve = (WOFDM_BY_SUBCARRIER if by_subcarrier else 0) | (WOFDM_BY_CHANNEL if by_channel else 0)
+        shape = (n, Cn if by_channel else 1, s.N if by_subcarrier else 1) if resolve else (n,)
+        be, se = np.zeros((nv,) + shape, dtype=np.int64), np.zeros((nv,) + shape, dtype=np.int64)
+        st = np.zeros(shape, dtype=np.int64)
+        rc = load().wofdm_ber_run_segments(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), nv, _ptr(chf, _dp), L, Cn,
+                                           _ptr(snr, _dp), n, int(ensemble_max), _ptr(seg, _i64p), seg.shape[0], int(seed),
+                                           int(variant), int(shard[0]), int(shard[1]), int(resolve),
+                                           _ptr(be, _i64p), _ptr(se, _i64p), _ptr(st, _i64p))
+        self._check(rc)
+        return dict(bit_err=be, sym_err=se, sym_tot=st, bit_tot=st * int(s.bits))
+
+    def ber_run_adaptive(self, s, wins_tx, wins_rx, chan, snr_db, ensemble_max, target_bit_errors=None,
+                         target_symbol_errors=None, first_block=1, seed=0, variant=0, shard=(0, 1), reduce=None):
+        """Run every SNR point until the fewest errors over the window pairs reach the target, or to ensemble_max ensemble
+        indices (wofdm_ber_run_adaptive; the schedule is stated in include/wofdm.h).  Exactly one of target_bit_errors /
+        target_symbol_errors.  reduce: None, or a callable on this process's round counts, an int64 array (n_var, n_snr, 2)
+        of {bit, sym}, that returns (or fills in place) their sum over the processes -- sharding.adaptive_allreduce() under
+        torch.distributed.  Returns bit_err / sym_err (n_var, n_snr), bit_tot / sym_tot (n_snr,), ensemble_used (n_snr,)
+        and rounds."""
+        if (target_bit_errors is None) == (target_symbol_errors is None):
+            raise WofdmError(EINVAL, "give exactly one of target_bit_errors / target_symbol_errors")
+        kind, target = ((WOFDM_TARGET_BIT_ERRORS, target_bit_errors) if target_bit_errors is not None
+                        else (WOFDM_TARGET_SYMBOL_ERRORS, target_symbol_errors))
+        wt, wr = self._win_multi(s, wins_tx, wins_rx)
+        _, _, chf, L, Cn = self._win_chan(s, wt[0], wr[0], chan)
+        snr = _f64(np.ravel(snr_db))
+        n, nv = snr.size, wt.shape[0]
+        be, se = np.zeros((nv, n), dtype=np.int64), np.zeros((nv, n), dtype=np.int64)
+        bt, st, used = (np.zeros(n, dtype=np.int64) for _ in range(3))
+        rounds = C.c_int(0)
+        cb = reduce_trampoline(reduce, (nv, n, 2)) if reduce is not None else REDUCE_FN()
+        rc = load().wofdm_ber_run_adaptive(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), nv, _ptr(chf, _dp), L, Cn,
+                                           _ptr(snr, _dp), n, int(ensemble_max), int(first_block), kind, int(target), int(seed),
+                                           int(variant), int(shard[0]), int(shard[1]), cb, None, _ptr(used, _i64p),
+                                           _ptr(be, _i64p), _ptr(bt, _i64p), _ptr(se, _i64p), _ptr(st, _i64p), C.byref(rounds))
+        if reduce is not None and cb.error is not None and rc:
+            raise WofdmError(rc, f"reduce callback raised {cb.error!r}") from cb.error
+        self._check(rc)
+        return dict(bit_err=be, bit_tot=bt, sym_err=se, sym_tot=st, ensemble_used=used, rounds=rounds.value)
+
     def ber_run_masked(self, s, win_tx, win_rx, chan, snr_db, ensemble, seed=0, variant=0, roll_off=10):
         """Channel-mask variant (wofdm_ber_run_masked): counters of the MASKED signal; ber_run with the same `s`
         (s.guard = the script's offset) gives the unmasked ones on the same symbols."""
@@ -474,6 +533,30 @@ class Handle:
                                        _ptr(ph, _dp) if ph is not None else None, _ptr(out, _dp))
         self._check(rc)
         return out.T
+
+
+def reduce_trampoline(fn, shape=None):
+    """A wofdm_reduce_fn calling fn(counts) on the int64 counts of a round (a numpy view, reshaped to `shape`).  fn returns
+    the summed counts (copied back) or None (it summed in place).  An exception is kept in `.error` and reported to the
+    library as a non-zero return, which fails the call: ctypes would otherwise print and swallow it, and the run would go
+    on with unsummed counts.  Keep the returned object alive for the duration of the call."""
+    def tramp(ptr, n, user):
+        try:
+            a = np.ctypeslib.as_array(ptr, shape=(int(n),))
+            v = a.reshape(shape) if shape is not None else a
+            r = fn(v)
+            if r is not None:
+                r = np.asarray(r.cpu() if hasattr(r, "cpu") else r, dtype=np.int64)
+                if r.size != a.size:
+                    raise ValueError(f"reduce returned {r.size} counts, expected {a.size}")
+                a[:] = r.reshape(-1)
+            return 0
+        except BaseException as e:       # noqa: BLE001 -- reported through the return value
+            cb.error = e
+            return 1
+    cb = REDUCE_FN(tramp)
+    cb.error = None
+    return cb
 
 
 class BerPlan:

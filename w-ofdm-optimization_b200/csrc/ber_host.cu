@@ -15,6 +15,7 @@ using namespace wofdm;
 struct PlanDev {
     void *d_wtx = nullptr, *d_wrx = nullptr, *d_tw = nullptr, *d_chan = nullptr, *d_snr = nullptr;
     unsigned long long* d_cnt = nullptr;
+    long long* d_seg = nullptr;    // segment table of wofdm_ber_run_segments / _adaptive (BerParams::seg): [seg_cap][4]
     void* d_scratch = nullptr;
     size_t scratch_bytes = 0;
     int blocks_per_sm = 0;
@@ -39,6 +40,7 @@ struct wofdm_ber_plan_s {
     int resolve = 0;
     const BerVariant* noise_var = nullptr;
     size_t cnt_per_var = 0;        // u64 counters of one window pair: [cells][bins][2] (unresolved: [n_snr][2])
+    int seg_cap = 0;               // entries of the devices' segment tables (PlanDev::d_seg), 0: none
     std::vector<PlanDev> devs;
 };
 
@@ -328,9 +330,11 @@ size_t elem_bytes(const wofdm_sys_t& s) { return s.precision == 1 ? sizeof(doubl
 // transient = true: device buffers come out of the per-device arena (no cudaMalloc / cudaFree per call); such a plan
 // must be destroyed before the arena is used again (wofdm_ber_run_shard does exactly that)
 // resolve != 0 (WOFDM_BY_* flags): counters [n_var][n_snr * Cr][Nr][2] in a buffer of their own (wofdm_ber_run_resolved)
+// seg_cap > 0 (frame segments): the resolved twin runs even with resolve == 0 (counters [n_var][n_snr][2]) and every
+// device gets a segment table of seg_cap entries (BerParams::seg)
 static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
                             const double* chan, int L, int C, const double* snr_db, int n_snr,
-                            wofdm_ber_plan* out, bool transient, int resolve = 0) {
+                            wofdm_ber_plan* out, bool transient, int resolve = 0, int seg_cap = 0) {
     NvtxRange nvtx_("wofdm_ber_plan_create");
     if (!h) return WOFDM_EINVAL;
     if (!out) return fail(h, WOFDM_EINVAL, "plan out pointer is NULL");
@@ -345,6 +349,7 @@ static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double
     wofdm_ber_plan_s* p = new (std::nothrow) wofdm_ber_plan_s();
     if (!p) return fail(h, WOFDM_ENOMEM, "host allocation failed");
     p->ctx = h; p->sys = *sys; p->L = L; p->C = C; p->n_snr = n_snr; p->transient = transient; p->n_var = n_var;
+    p->seg_cap = seg_cap;
     Choice ch;
     size_t cap = h->devs[0].smem_optin;
     for (auto& d : h->devs) cap = std::min(cap, d.smem_optin);
@@ -356,7 +361,7 @@ static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double
     if (rc) { delete p; return rc; }
     p->noise_var = ch.var;
     p->cnt_per_var = (size_t)n_snr * 2;
-    if (resolve) {
+    if (resolve || seg_cap > 0) {
         Choice rch;
         bool rfused = false;
         rc = choose_resolved(h, *sys, L, cap, ch, p->fused, n_var, &rch, &rfused);
@@ -413,7 +418,7 @@ static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double
         pd.scratch_bytes = p->use_global ? (size_t)pd.blocks_per_sm * d.sm_count * 2 * scratch_elems * elem_bytes(*sys) : 0;
         if (e == cudaSuccess && transient) {
             rc = arena_reserve(h, d, t.wtx.size() + t.wrx.size() + t.tw.size() + hchan.size() + hsnr.size() +
-                                         (resolve ? 0 : (size_t)n_var * n_snr * 16) + pd.scratch_bytes);
+                                         (resolve ? 0 : (size_t)n_var * n_snr * 16) + pd.scratch_bytes + (size_t)seg_cap * 32);
             if (rc) { const std::string msg = h->err; wofdm_ber_plan_destroy(p); h->err = msg; return rc; }
         }
         if (e == cudaSuccess) e = up(&pd.d_wtx, t.wtx);
@@ -426,6 +431,7 @@ static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double
         else if (e == cudaSuccess) e = dev_alloc(reinterpret_cast<void**>(&pd.d_cnt), (size_t)n_var * n_snr * 2 * sizeof(unsigned long long));
         if (e == cudaSuccess) e = cudaStreamSynchronize(d.stream);   // host vectors go out of scope
         if (e == cudaSuccess && p->use_global) e = dev_alloc(&pd.d_scratch, pd.scratch_bytes);
+        if (e == cudaSuccess && seg_cap > 0) e = dev_alloc(reinterpret_cast<void**>(&pd.d_seg), (size_t)seg_cap * 32);
         if (e != cudaSuccess) {
             std::string msg = std::string("plan upload: ") + cudaGetErrorString(e);
             wofdm_ber_plan_destroy(p);
@@ -455,9 +461,13 @@ int wofdm_ber_plan_variants(wofdm_ber_plan p, int* fused) {
     return p->n_var;
 }
 
-int wofdm_ber_plan_launch(wofdm_ber_plan p, int slot, int64_t ensemble, uint64_t seed, uint32_t variant,
-                          int shard_index, int shard_count, void* stream, void** d_counters) {
-    NvtxRange nvtx_("wofdm_ber_plan_launch");
+}  // extern "C"
+
+// d_seg != nullptr (a twin plan): the launch runs the n_local frames of the segment table d_seg[n_seg][4] (BerParams::seg)
+// instead of the n_snr * C * ensemble frames of the plan; ensemble is then the job's ensemble_max
+static int plan_launch_impl(wofdm_ber_plan p, int slot, int64_t ensemble, uint64_t seed, uint32_t variant,
+                            int shard_index, int shard_count, void* stream, void** d_counters,
+                            const long long* d_seg = nullptr, int n_seg = 0, long long n_local = 0) {
     if (!p) return WOFDM_EINVAL;
     wofdm_ctx* h = p->ctx;
     if (slot < 0 || slot >= (int)p->devs.size()) return fail(h, WOFDM_EINVAL, "device slot out of range");
@@ -469,7 +479,7 @@ int wofdm_ber_plan_launch(wofdm_ber_plan p, int slot, int64_t ensemble, uint64_t
     cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d.stream;
     WOFDM_CUDA(h, cudaSetDevice(d.dev));
 
-    const long long total = (long long)p->n_snr * p->C * ensemble;
+    const long long total = d_seg ? n_local : (long long)p->n_snr * p->C * ensemble;
     const long long mine = total > shard_index ? (total - shard_index + shard_count - 1) / shard_count : 0;
     BerParams prm;
     fill_sys(prm, p->sys, p->L);
@@ -478,6 +488,7 @@ int wofdm_ber_plan_launch(wofdm_ber_plan p, int slot, int64_t ensemble, uint64_t
     fill_split(prm, *p->noise_var);
     prm.res_chan = (p->resolve & WOFDM_BY_CHANNEL) ? 1 : 0;
     prm.res_bins = (p->resolve & WOFDM_BY_SUBCARRIER) ? 1 : 0;
+    prm.seg = d_seg; prm.n_seg = n_seg;
     prm.win_tx = pd.d_wtx; prm.win_rx = pd.d_wrx; prm.tw = pd.d_tw; prm.chan = pd.d_chan; prm.snr_lin = pd.d_snr;
     prm.C = p->C; prm.n_snr = p->n_snr; prm.ensemble = ensemble;
     prm.seed = seed; prm.variant = variant;
@@ -523,6 +534,35 @@ int wofdm_ber_plan_launch(wofdm_ber_plan p, int slot, int64_t ensemble, uint64_t
     return WOFDM_OK;
 }
 
+// sum of the counter arrays of every slot launched since the last read -> bit_err / sym_err [n_var * cnt_per_var / 2]
+// (the layout of the plan's counters with the {bit, sym} pair split)
+static int read_counters(wofdm_ber_plan p, int64_t* bit_err, int64_t* sym_err) {
+    wofdm_ctx* h = p->ctx;
+    const size_t n_out = (size_t)p->n_var * p->cnt_per_var / 2;
+    std::vector<unsigned long long> tmp;
+    try { tmp.resize(n_out * 2); } catch (const std::bad_alloc&) { return fail(h, WOFDM_ENOMEM, "host allocation failed"); }
+    for (size_t i = 0; i < n_out; ++i) { bit_err[i] = 0; sym_err[i] = 0; }
+    for (size_t i = 0; i < p->devs.size(); ++i) {
+        PlanDev& pd = p->devs[i];
+        if (!pd.pending) continue;
+        cudaError_t e = cudaSetDevice(h->devs[i].dev);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(tmp.data(), pd.d_cnt, n_out * 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, pd.last_stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(pd.last_stream);
+        if (e != cudaSuccess) return fail(h, WOFDM_ECUDA, std::string("counters: ") + cudaGetErrorString(e));
+        for (size_t k = 0; k < n_out; ++k) { bit_err[k] += (int64_t)tmp[2 * k]; sym_err[k] += (int64_t)tmp[2 * k + 1]; }
+        pd.pending = false;
+    }
+    return WOFDM_OK;
+}
+
+extern "C" {
+
+int wofdm_ber_plan_launch(wofdm_ber_plan p, int slot, int64_t ensemble, uint64_t seed, uint32_t variant,
+                          int shard_index, int shard_count, void* stream, void** d_counters) {
+    NvtxRange nvtx_("wofdm_ber_plan_launch");
+    return plan_launch_impl(p, slot, ensemble, seed, variant, shard_index, shard_count, stream, d_counters);
+}
+
 int wofdm_ber_plan_read(wofdm_ber_plan p, int64_t* bit_err, int64_t* sym_err) {
     if (!p) return WOFDM_EINVAL;
     wofdm_ctx* h = p->ctx;
@@ -556,6 +596,7 @@ int wofdm_ber_plan_destroy(wofdm_ber_plan p) {
         cudaFree(pd.d_wtx); cudaFree(pd.d_wrx); cudaFree(pd.d_tw); cudaFree(pd.d_chan); cudaFree(pd.d_snr);
         if (!p->resolve) cudaFree(pd.d_cnt);
         cudaFree(pd.d_scratch);
+        cudaFree(pd.d_seg);
     }
     cudaGetLastError();
     delete p;
@@ -635,21 +676,7 @@ int wofdm_ber_run_resolved(wofdm_handle h, const wofdm_sys_t* sys, const double*
     for (int i = 0; i < nd && rc == WOFDM_OK; ++i)
         rc = wofdm_ber_plan_launch(p, i, ensemble, seed, variant, shard_index + shard_count * i, shard_count * nd,
                                    nullptr, nullptr);
-    std::vector<unsigned long long> tmp;
-    if (rc == WOFDM_OK) {
-        for (size_t i = 0; i < n_out; ++i) { bit_err[i] = 0; sym_err[i] = 0; }
-        try { tmp.resize(n_out * 2); } catch (const std::bad_alloc&) { rc = fail(h, WOFDM_ENOMEM, "host allocation failed"); }
-    }
-    for (int i = 0; i < nd && rc == WOFDM_OK; ++i) {
-        PlanDev& pd = p->devs[i];
-        if (!pd.pending) continue;
-        cudaError_t e = cudaSetDevice(h->devs[i].dev);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(tmp.data(), pd.d_cnt, dev_bytes, cudaMemcpyDeviceToHost, pd.last_stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(pd.last_stream);
-        if (e != cudaSuccess) { rc = fail(h, WOFDM_ECUDA, std::string("resolved counters: ") + cudaGetErrorString(e)); break; }
-        for (size_t k = 0; k < n_out; ++k) { bit_err[k] += (int64_t)tmp[2 * k]; sym_err[k] += (int64_t)tmp[2 * k + 1]; }
-        pd.pending = false;
-    }
+    if (rc == WOFDM_OK) rc = read_counters(p, bit_err, sym_err);
     wofdm_ber_plan_destroy(p);
     if (rc) return rc;
     // frames of this shard per cell (si, c): f in [(si*C + c)*ensemble, +ensemble), f = shard_index (mod shard_count);
@@ -667,6 +694,189 @@ int wofdm_ber_run_resolved(wofdm_handle h, const wofdm_sys_t* sys, const double*
                 out[k] = (cc >= sys->guard && cc < Nr - sys->guard) ? frames * (sys->S - 1) : 0;
             }
         }
+    return WOFDM_OK;
+}
+
+}  // extern "C"
+
+// ---- frame segments (wofdm_ber_run_segments / _adaptive) ---------------------------------------------------------------
+namespace {
+
+// the checks every segment entry point shares with wofdm_ber_run_multi, plus ensemble_max and the size of the frame space
+int check_job(wofdm_handle h, const wofdm_sys_t* sys, int L, int C, int n_snr, int n_var, int64_t ensemble_max,
+              int shard_index, int shard_count) {
+    if (shard_count < 1 || shard_index < 0 || shard_index >= shard_count) return fail(h, WOFDM_EINVAL, "bad shard");
+    if (ensemble_max < 1) return fail(h, WOFDM_EINVAL, "ensemble_max must be >= 1");
+    int rc = validate_sys(h, sys, L);
+    if (rc) return rc;
+    if (C < 1 || n_snr < 1) return fail(h, WOFDM_EINVAL, "C and n_snr must be >= 1");
+    if (n_var < 1 || n_var > WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "n_var must be in [1, WOFDM_MAX_VARIANTS]");
+    int64_t frames = 0;
+    if (__builtin_mul_overflow((int64_t)n_snr, (int64_t)C, &frames) || __builtin_mul_overflow(frames, ensemble_max, &frames))
+        return fail(h, WOFDM_EINVAL, "n_snr * C * ensemble_max overflows int64");
+    return WOFDM_OK;
+}
+
+// device table of `seg` ({snr_idx, e_begin, e_count} each) -> {g0, snr_idx, e_begin, e_count}; *n_local = its frames
+void seg_table(const int64_t* seg, int n_seg, int C, std::vector<long long>& tab, long long* n_local) {
+    tab.resize((size_t)n_seg * 4);
+    long long g = 0;
+    for (int k = 0; k < n_seg; ++k) {
+        tab[4 * k] = g; tab[4 * k + 1] = seg[3 * k]; tab[4 * k + 2] = seg[3 * k + 1]; tab[4 * k + 3] = seg[3 * k + 2];
+        g += (long long)C * seg[3 * k + 2];
+    }
+    *n_local = g;
+}
+
+// one launch of a twin plan over the segment table on every device of the handle (devices split this shard's local
+// indices as wofdm_ber_run_multi splits frame ids), then the summed counters
+int run_segment_table(wofdm_ber_plan p, const std::vector<long long>& tab, long long n_local, int64_t ensemble_max,
+                      uint64_t seed, uint32_t variant, int shard_index, int shard_count, int64_t* bit_err, int64_t* sym_err) {
+    wofdm_ctx* h = p->ctx;
+    const int n_seg = (int)(tab.size() / 4), nd = (int)h->devs.size();
+    if (n_seg > p->seg_cap) return fail(h, WOFDM_EINVAL, "more segments than the plan's segment table holds");
+    for (int i = 0; i < nd; ++i) {
+        DeviceCtx& d = h->devs[i];
+        PlanDev& pd = p->devs[i];
+        WOFDM_CUDA(h, cudaSetDevice(d.dev));
+        // (pageable source: the copy returns once the table is staged; the previous launch on this stream is ordered before it)
+        WOFDM_CUDA(h, cudaMemcpyAsync(pd.d_seg, tab.data(), tab.size() * sizeof(long long), cudaMemcpyHostToDevice, d.stream));
+        const int rc = plan_launch_impl(p, i, ensemble_max, seed, variant, shard_index + shard_count * i, shard_count * nd,
+                                        nullptr, nullptr, pd.d_seg, n_seg, n_local);
+        if (rc) return rc;
+    }
+    return read_counters(p, bit_err, sym_err);
+}
+
+}  // namespace
+
+extern "C" {
+
+int wofdm_ber_run_segments(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
+                           const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble_max,
+                           const int64_t* segments, int n_seg, uint64_t seed, uint32_t variant, int shard_index,
+                           int shard_count, int resolve, int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot) {
+    NvtxRange nvtx_("wofdm_ber_run_segments");
+    if (!h) return WOFDM_EINVAL;
+    if (resolve & ~(WOFDM_BY_SUBCARRIER | WOFDM_BY_CHANNEL))
+        return fail(h, WOFDM_EINVAL, "resolve must be a combination of WOFDM_BY_SUBCARRIER and WOFDM_BY_CHANNEL");
+    if (!bit_err || !sym_err || !sym_tot) return fail(h, WOFDM_EINVAL, "NULL output buffer");
+    int rc = check_job(h, sys, L, C, n_snr, n_var, ensemble_max, shard_index, shard_count);
+    if (rc) return rc;
+    if (!segments || n_seg < 1) return fail(h, WOFDM_EINVAL, "segments must be a non-empty list");
+    {   // inside [0, n_snr) x [0, ensemble_max), no two segments of one point overlap
+        std::vector<std::pair<int64_t, int64_t>> iv((size_t)n_seg);
+        for (int k = 0; k < n_seg; ++k) {
+            const int64_t si = segments[3 * k], e0 = segments[3 * k + 1], ec = segments[3 * k + 2];
+            if (si < 0 || si >= n_snr || e0 < 0 || e0 >= ensemble_max || ec < 1 || ec > ensemble_max - e0)
+                return fail(h, WOFDM_EINVAL, "segment outside [0, n_snr) x [0, ensemble_max) or with e_count < 1");
+            iv[k] = {si * ensemble_max + e0, ec};       // (< n_snr * ensemble_max: no overflow, checked above)
+        }
+        std::sort(iv.begin(), iv.end());
+        for (int k = 1; k < n_seg; ++k)
+            if (iv[k].first < iv[k - 1].first + iv[k - 1].second) return fail(h, WOFDM_EINVAL, "overlapping segments of one SNR point");
+    }
+    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? sys->N : 1;
+    size_t cells = 0, n_out = 0, dev_bytes = 0;
+    if (__builtin_mul_overflow((size_t)n_snr, (size_t)Cr, &cells) || __builtin_mul_overflow(cells, (size_t)Nr, &cells) ||
+        __builtin_mul_overflow(cells, (size_t)n_var, &n_out) || __builtin_mul_overflow(n_out, (size_t)16, &dev_bytes) ||
+        n_out > (size_t)INT64_MAX / 16)
+        return fail(h, WOFDM_EINVAL, "resolved counter array too large");
+    std::vector<long long> tab;
+    long long n_local = 0;
+    seg_table(segments, n_seg, C, tab, &n_local);
+    wofdm_ber_plan p = nullptr;
+    rc = plan_create_impl(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, &p, true, resolve, n_seg);
+    if (rc) return rc;
+    rc = run_segment_table(p, tab, n_local, ensemble_max, seed, variant, shard_index, shard_count, bit_err, sym_err);
+    wofdm_ber_plan_destroy(p);
+    if (rc) return rc;
+    // this shard's frames per cell (si, c): local indices j = shard_index (mod shard_count) in the cell's ranges
+    auto count_upto = [&](long long x) -> long long { return x > shard_index ? (x - shard_index + shard_count - 1) / shard_count : 0; };
+    std::vector<long long> frames((size_t)n_snr * Cr, 0);
+    for (int k = 0; k < n_seg; ++k) {
+        const long long g0 = tab[4 * k], ec = tab[4 * k + 3];
+        for (int c = 0; c < C; ++c)
+            frames[(size_t)tab[4 * k + 1] * Cr + (Cr > 1 ? c : 0)] += count_upto(g0 + (c + 1) * ec) - count_upto(g0 + c * ec);
+    }
+    const long long active = sys->N - 2 * sys->guard;
+    for (size_t cell = 0; cell < (size_t)n_snr * Cr; ++cell) {
+        int64_t* out = sym_tot + cell * Nr;
+        if (Nr == 1) { out[0] = frames[cell] * active * (sys->S - 1); continue; }
+        for (int k = 0; k < Nr; ++k) {
+            const int cc = (k + Nr / 2) & (Nr - 1);                   // ber_kernel.cuh: bin_active
+            out[k] = (cc >= sys->guard && cc < Nr - sys->guard) ? frames[cell] * (sys->S - 1) : 0;
+        }
+    }
+    return WOFDM_OK;
+}
+
+int wofdm_ber_run_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
+                           const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble_max,
+                           int64_t first_block, int target_kind, int64_t target, uint64_t seed, uint32_t variant,
+                           int shard_index, int shard_count, wofdm_reduce_fn reduce, void* reduce_user,
+                           int64_t* ensemble_used, int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot,
+                           int* rounds) {
+    NvtxRange nvtx_("wofdm_ber_run_adaptive");
+    if (!h) return WOFDM_EINVAL;
+    if (!ensemble_used || !bit_err || !bit_tot || !sym_err || !sym_tot || !rounds) return fail(h, WOFDM_EINVAL, "NULL output buffer");
+    int rc = check_job(h, sys, L, C, n_snr, n_var, ensemble_max, shard_index, shard_count);
+    if (rc) return rc;
+    if (target_kind != WOFDM_TARGET_BIT_ERRORS && target_kind != WOFDM_TARGET_SYMBOL_ERRORS) return fail(h, WOFDM_EINVAL, "unknown target_kind");
+    if (target < 1) return fail(h, WOFDM_EINVAL, "target must be >= 1");
+    if (first_block < 1) return fail(h, WOFDM_EINVAL, "first_block must be >= 1");
+    if (shard_count > 1 && !reduce) return fail(h, WOFDM_EINVAL, "shard_count > 1 needs a reduce callback (the schedule needs the job's counts)");
+    wofdm_ber_plan p = nullptr;
+    rc = plan_create_impl(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, &p, true, 0, n_snr);
+    if (rc) return rc;
+    const size_t nv = (size_t)n_var, ns = (size_t)n_snr;
+    std::vector<int64_t> used(ns, 0), block(ns, std::min(first_block, ensemble_max)), rbit(nv * ns), rsym(nv * ns), red(nv * ns * 2);
+    std::vector<int64_t> tbit(nv * ns, 0), tsym(nv * ns, 0);
+    std::vector<char> done(ns, 0);
+    std::vector<long long> tab;
+    int nround = 0;
+    for (;;) {
+        // this round: the active points in ascending SNR order, block[s] ensemble indices each from used[s]
+        std::vector<int64_t> seg;
+        for (size_t s = 0; s < ns; ++s)
+            if (!done[s]) { seg.push_back((int64_t)s); seg.push_back(used[s]); seg.push_back(block[s]); }
+        if (seg.empty()) break;
+        long long n_local = 0;
+        seg_table(seg.data(), (int)(seg.size() / 3), C, tab, &n_local);
+        rc = run_segment_table(p, tab, n_local, ensemble_max, seed, variant, shard_index, shard_count, rbit.data(), rsym.data());
+        if (rc) break;
+        ++nround;
+        for (size_t k = 0; k < nv * ns; ++k) { red[2 * k] = rbit[k]; red[2 * k + 1] = rsym[k]; }   // [n_var][n_snr][2]
+        if (reduce && reduce(red.data(), (int64_t)red.size(), reduce_user) != 0) {
+            rc = fail(h, WOFDM_EINVAL, "the reduce callback failed");
+            break;
+        }
+        for (size_t k = 0; k < nv * ns; ++k) { tbit[k] += red[2 * k]; tsym[k] += red[2 * k + 1]; }
+        for (size_t s = 0; s < ns; ++s) {
+            if (done[s]) continue;
+            used[s] += block[s];
+            int64_t m = INT64_MAX;                      // the fewest errors over the window pairs
+            for (size_t v = 0; v < nv; ++v) m = std::min(m, target_kind == WOFDM_TARGET_BIT_ERRORS ? tbit[v * ns + s] : tsym[v * ns + s]);
+            if (m >= target || used[s] == ensemble_max) { done[s] = 1; continue; }
+            // min(ensemble_max - e, 2b, m > 0 ? max(1, ceil((target - m) * e / m)) : 2b), exact in 128 bits, saturating
+            __int128 nb = std::min<__int128>((__int128)ensemble_max - used[s], (__int128)2 * block[s]);
+            if (m > 0) {
+                const __int128 need = ((__int128)(target - m) * used[s] + m - 1) / m;
+                nb = std::min(nb, std::max<__int128>(1, need));
+            }
+            block[s] = (int64_t)nb;
+        }
+    }
+    wofdm_ber_plan_destroy(p);
+    if (rc) return rc;
+    *rounds = nround;
+    const long long per_frame = (long long)(sys->N - 2 * sys->guard) * (sys->S - 1);
+    for (size_t s = 0; s < ns; ++s) {
+        ensemble_used[s] = used[s];
+        sym_tot[s] = (int64_t)C * used[s] * per_frame;
+        bit_tot[s] = sym_tot[s] * sys->bits;
+    }
+    for (size_t k = 0; k < nv * ns; ++k) { bit_err[k] = tbit[k]; sym_err[k] = tsym[k]; }
     return WOFDM_OK;
 }
 

@@ -88,6 +88,11 @@ struct BerParams {
     // RES instantiations (wofdm_ber_run_resolved): counters are [nvar][cell][bins][2] with cell = si*C + ci (res_chan) or si,
     // bins = N (res_bins: one pair per sub-carrier, accumulated in shared memory) or 1 (the per-warp atomics, re-addressed)
     int res_chan, res_bins;
+    // RES instantiations, frame segments (wofdm_ber_run_segments / _adaptive): seg != nullptr makes frame_begin + j*frame_step
+    // a LOCAL index g into the segment list, seg[k] = {g0, snr_idx, e_begin, e_count} (g0: local index of its first frame,
+    // ascending), channel-major inside a segment; the frame id is f = (snr_idx*C + c)*ensemble + e_begin + e (seg_frame)
+    const long long* seg;
+    int n_seg;
 };
 
 // ---- constellation helpers (oracle/wofdm_oracle.py: idx_to_levels / levels_to_idx) --------------
@@ -339,6 +344,21 @@ __device__ __forceinline__ void res_flush(uint32_t* racc, int n, int nb, size_t 
         atomicAdd(d + 1, (unsigned long long)sc);
     }
 }
+// local index g of a segment launch -> frame id f, SNR point si, channel ci (BerParams::seg).  Uniform over the CTA (and the
+// cluster).  g at or past the end maps to a channel >= C of the last segment: only the loop's exit test follows.
+__device__ __forceinline__ void seg_frame(const BerParams& prm, long long g, long long& f, int& si, int& ci) {
+    int lo = 0, hi = prm.n_seg - 1;                    // the last segment that starts at or before g
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (prm.seg[4 * mid] <= g) lo = mid; else hi = mid - 1;
+    }
+    const long long* sg = prm.seg + 4 * lo;
+    const long long r = g - sg[0], ec = sg[3], c = r / ec;
+    si = (int)sg[1];
+    ci = (int)c;
+    f = ((long long)si * prm.C + c) * prm.ensemble + sg[2] + (r - c * ec);
+}
+
 // frames between flushes such that no 32-bit accumulator wraps: a frame adds at most S * bits bit errors to a bin
 __host__ __device__ __forceinline__ unsigned res_frame_limit(int S, int bits) { return 0xffffffffu / (unsigned)(S * (bits > 1 ? bits : 1)); }
 
@@ -541,6 +561,9 @@ ber_frame_kernel(const BerParams prm) {
         si = (int)(q / prm.C);       ci = (int)(q - (long long)si * prm.C);
         ds = (int)(dq / prm.C);      dc = (int)(dq - (long long)ds * prm.C);
     }
+    // RES with a segment table: f above is the local index g, every frame's (f, si, ci) comes from seg_frame
+    [[maybe_unused]] long long g = f;
+    if constexpr (RES) { if (prm.seg) seg_frame(prm, g, f, si, ci); }
     // RES: cells of the counters and this CTA's current one
     const size_t ncell = RES ? (size_t)prm.n_snr * (prm.res_chan ? prm.C : 1) : 0;
     int rcell = RES ? (prm.res_chan ? si * prm.C + ci : si) : 0;
@@ -996,6 +1019,7 @@ ber_frame_kernel(const BerParams prm) {
             si += ds;
         }
         if constexpr (RES) {
+            if (prm.seg) { g += df; seg_frame(prm, g, f, si, ci); }   // (replaces the incremental decode)
             if (prm.res_bins) {                          // uniform: the next frame's cell, the frame count, the last frame
                 const int nc = prm.res_chan ? si * prm.C + ci : si;
                 if (nc != rcell || ++rfr >= rlim || j + nslots >= prm.n_frames) {

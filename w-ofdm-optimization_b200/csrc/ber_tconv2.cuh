@@ -446,6 +446,10 @@ ber_tconv2_kernel(const BerParams prm) {
         si = (int)(q / prm.C);       ci = (int)(q - (long long)si * prm.C);
         ds = (int)(dq / prm.C);      dc = (int)(dq - (long long)ds * prm.C);
     }
+    // RES with a segment table: f above is the local index g, every frame's (f, si, ci) comes from seg_frame (ber_kernel.cuh);
+    // the CTAs of a cluster share fslot, so they map the same g
+    [[maybe_unused]] long long g = f;
+    if constexpr (RES) { if (prm.seg) seg_frame(prm, g, f, si, ci); }
     // RES: cells of the counters and this CTA's current one
     const size_t ncell = RES ? (size_t)prm.n_snr * (prm.res_chan ? prm.C : 1) : 0;
     int rcell = RES ? (prm.res_chan ? si * prm.C + ci : si) : 0;
@@ -1043,6 +1047,7 @@ ber_tconv2_kernel(const BerParams prm) {
             si += ds;
         }
         if constexpr (RES) {
+            if (prm.seg) { g += df; seg_frame(prm, g, f, si, ci); }   // (replaces the incremental decode)
             if (prm.res_bins) {                          // uniform: the next frame's cell, the frame count, the last frame
                 const int nc = prm.res_chan ? si * prm.C + ci : si;
                 if (nc != rcell || ++rfr >= rlim || j + nslots >= prm.n_frames) {

@@ -100,6 +100,24 @@ class wOFDMSystem:
         ser = [np.divide(e[:, 0, :], tot, out=np.zeros(tot.shape), where=tot > 0) for e in r["sym_err"]]
         return ser[0] if self.name == "CP" else (ser[0], ser[1])
 
+    def run_simulation_adaptive(self, channel_models, window_tx, window_rx, ensemble_max, snr_arr, no_symbols,
+                                target_errors, first_block=1):
+        """run_simulation with a stopping rule: each SNR point runs until both window pairs have counted target_errors
+        symbol errors (the python convention counts symbols) or ensemble_max ensemble indices (Handle.ber_run_adaptive).
+        Frame f of a point is the frame run_simulation(ensemble=ensemble_max) draws.  Returns (ser_opt, ser_rc,
+        ensemble_used) ('CP': (ser, ensemble_used)); writes no files."""
+        h = self._h or default_handle()
+        s = self._sys(int(no_symbols))
+        snr = np.asarray(snr_arr, dtype=np.float64)
+        if self.name == "CP":
+            wt, wr = [np.ones(s.n_tx)], [np.ones(s.N + s.tail_rx)]
+        else:
+            wt, wr = [_diag(window_tx), capi.rc_window_tx(s)], [_diag(window_rx), capi.rc_window_rx(s)]
+        r = h.ber_run_adaptive(s, wt, wr, channel_models, snr, ensemble_max, target_symbol_errors=int(target_errors),
+                               first_block=first_block, seed=self.seed, variant=0)
+        ser = [e / r["sym_tot"] for e in r["sym_err"]]
+        return (ser[0], r["ensemble_used"]) if self.name == "CP" else (ser[0], ser[1], r["ensemble_used"])
+
 
 def load_window_tails(system_design, window_path, cp_len, tail_tx, tail_rx):
     """<window_path>/<sys>_<cp>.npy -> (x_tx, x_rx) reduced variables (wofdm_simulation.py:46-66, SURVEY App. A.4)."""

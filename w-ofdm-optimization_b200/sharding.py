@@ -52,6 +52,26 @@ def allreduce_counters(counters, group=None):
     return t
 
 
+def adaptive_allreduce(group=None):
+    """reduce callable of Handle.ber_run_adaptive under torch.distributed: sums a round's int64 counts over `group` with
+    allreduce_counters (one all-reduce per round).  Every rank then computes the same schedule; each passes its own shard."""
+    def reduce(counts):
+        return allreduce_counters(np.array(counts, dtype=np.int64), group=group)
+    return reduce
+
+
+def segment_frame_ids(segments, C: int, ensemble_max: int, shard=(0, 1)) -> np.ndarray:
+    """Global frame ids of a segment list {snr_idx, e_begin, e_count} in launch order (wofdm_ber_run_segments): segments in
+    the order given, channel-major then e inside a segment; `shard` keeps local indices j = shard[0] (mod shard[1])."""
+    seg = np.asarray(segments, dtype=np.int64).reshape(-1, 3)
+    parts = []
+    for si, e0, ec in seg:
+        c, e = np.divmod(np.arange(int(C) * int(ec), dtype=np.int64), int(ec))
+        parts.append((si * C + c) * int(ensemble_max) + e0 + e)
+    f = np.concatenate(parts) if parts else np.zeros(0, dtype=np.int64)
+    return f[shard[0]::shard[1]]
+
+
 # ---- interference power: channel realisations are independent, rank r takes a contiguous block (SURVEY 8e) ----------
 
 def channel_block(C: int, rank: int, world: int):
