@@ -174,16 +174,6 @@ def setup_case(case, monkeypatch):
     return p, s, [w[0] for w in wins], [w[1] for w in wins], chans, snr, kern, wins
 
 
-def assert_counts(got, want, case, decisions):
-    """bit for bit, except the N = 1024 tensor-core cluster kernel: its production counters move with the frames' assignment
-    to CTAs by a few decisions in 1e7 (test_ber_resolved.test_many_frames_per_cta)"""
-    got, want = np.asarray(got), np.asarray(want)
-    if case != "tconv2_n1024_cluster":
-        assert np.array_equal(got, want), (case, got, want)
-    else:
-        assert np.abs(got - want).sum() <= 6 * (4 + 1e-6 * decisions), (case, got, want)
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", list(CASES))
 def test_unreachable_target_is_the_fixed_run(handle, case, monkeypatch):
@@ -191,13 +181,11 @@ def test_unreachable_target_is_the_fixed_run(handle, case, monkeypatch):
     assert kern in kernel_of(handle, s, wins, chans, snr)
     E = 6
     ref = handle.ber_run_multi(s, wt, wr, chans, snr, E, seed=p.N + 1, variant=3)
-    dec = int(ref["sym_tot"].sum())
     for kw in (dict(target_symbol_errors=10 ** 15), dict(target_bit_errors=10 ** 15)):
         r = handle.ber_run_adaptive(s, wt, wr, chans, snr, E, first_block=1, seed=p.N + 1, variant=3, **kw)
         assert np.array_equal(r["ensemble_used"], np.full(len(snr), E)) and r["rounds"] == 3     # blocks 1, 2, 3
         assert np.array_equal(r["sym_tot"], ref["sym_tot"]) and np.array_equal(r["bit_tot"], ref["bit_tot"])
-        assert_counts(r["sym_err"], ref["sym_err"], case, dec)
-        assert_counts(r["bit_err"], ref["bit_err"], case, dec)
+        assert np.array_equal(r["sym_err"], ref["sym_err"]) and np.array_equal(r["bit_err"], ref["bit_err"]), case
     assert ref["sym_err"].sum() > 0
 
 
@@ -213,13 +201,12 @@ def test_segments_add_up(handle, case, monkeypatch):
     one_call = [hi[2], lo[0], hi[1], lo[2], hi[0], lo[1]]
     split = ([hi[1], lo[0], lo[2]], [lo[1], hi[2], hi[0]])
     ref = handle.ber_run_multi(s, wt, wr, chans, snr, E, seed=seed, variant=1)
-    dec = int(ref["sym_tot"].sum())
     seg = lambda sg, **kw: handle.ber_run_segments(s, wt, wr, chans, snr, E, sg, seed=seed, variant=1, **kw)
     r = seg(one_call)
     parts = [seg(x) for x in split]
     for key in ("bit_err", "sym_err"):
-        assert_counts(r[key], ref[key], case, dec)
-        assert_counts(parts[0][key] + parts[1][key], ref[key], case, dec)
+        assert np.array_equal(r[key], ref[key]), (case, key)
+        assert np.array_equal(parts[0][key] + parts[1][key], ref[key]), (case, key)
     assert np.array_equal(r["sym_tot"], ref["sym_tot"]) and np.array_equal(parts[0]["sym_tot"] + parts[1]["sym_tot"], ref["sym_tot"])
     for bins, chan in ((True, False), (False, True), (True, True)):
         rr = handle.ber_run_resolved(s, wt, wr, chans, snr, E, seed=seed, variant=1, by_subcarrier=bins, by_channel=chan)
@@ -227,7 +214,7 @@ def test_segments_add_up(handle, case, monkeypatch):
         b = seg(split[1], by_subcarrier=bins, by_channel=chan)
         for key in ("bit_err", "sym_err", "sym_tot"):
             assert a[key].shape == rr[key].shape
-            assert_counts(a[key] + b[key], rr[key], case, dec)
+            assert np.array_equal(a[key] + b[key], rr[key]), (case, bins, chan, key)
 
 
 @pytest.mark.gpu

@@ -247,8 +247,7 @@ def test_many_frames_per_cta(handle, case, monkeypatch):
         whose cells (SNR points) change at other frames.  An error put into the wrong cell, a lost flush or a missed reset
         breaks one of them.
     (b) Against the same frames as 47 shards of at most 64 frames, where every CTA decides one frame and flushes once
-        (draws depend on the frame only): every cell bit for bit.  Not for the N = 1024 cluster kernel: its production
-        counters themselves depend on the sharding by a few decisions in 1e7 (wofdm_ber_run_multi shows the same)."""
+        (draws depend on the frame only): every cell bit for bit."""
     monkeypatch.delenv("WOFDM_NO_TCONV", raising=False)
     name, N, cp, ttx, trx, bits, nv, kern = {
         "tconv2_n256": ("WOLA", 256, 16, 8, 10, 4, 1, "f32t2_n256"),
@@ -273,8 +272,6 @@ def test_many_frames_per_cta(handle, case, monkeypatch):
     for key in ("bit_err", "sym_err"):
         assert np.array_equal(both[key].sum(axis=3), long[(False, True)][key][..., 0]), key
         assert np.array_equal(both[key].sum(axis=2), long[(True, False)][key][:, :, 0, :]), key
-    if case == "tconv2_n1024_cluster":
-        return
     for rc in ((True, False), (True, True)):
         acc = {key: np.zeros_like(long[rc][key]) for key in ("bit_err", "sym_err", "sym_tot")}
         for i in range(K):

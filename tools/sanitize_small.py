@@ -1,7 +1,6 @@
 """Small production + verify runs of every tuned K1 policy plus one TF32 interference call: the workload to put under
 `compute-sanitizer --tool memcheck|racecheck|synccheck python tools/sanitize_small.py` where that tool is available
-(it is closed on the round-1 GPU pool; tests/test_ber_gpu.py::test_production_is_deterministic_and_grid_independent
-is the stand-in there)."""
+(it is closed on the round-1 GPU pool; tests/test_ber_frame_invariance.py is the stand-in there)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np

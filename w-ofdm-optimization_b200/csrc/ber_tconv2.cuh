@@ -345,7 +345,7 @@ ber_tconv2_kernel(const BerParams prm) {
     const int warp_u = __shfl_sync(0xffffffffu, warp, 0);      // the warp index as a value the compiler knows to be warp-uniform
     const int tp = TG == 1 ? 0 : (warp_u >> 3);                // this warp's tile set: tiles tp, tp + TG, ...
     const uint32_t tlane = tmem + ((uint32_t)((warp_u & 3) * 32) << 16) + (uint32_t)(8 * ((warp_u >> 2) & 1));
-    uint32_t phase = 0, issuer = blockIdx.x;
+    uint32_t phase = 0;
     constexpr bool MMAW = tconv2_mma_warp_threads(N, NT) > 0;       // a dedicated MMA warp (warp NW)
     constexpr int NTB = NT + tconv2_mma_warp_threads(N, NT);        // threads that meet at the "stream complete" barrier
     // MMA descriptors of tile 0, K step 0 (tile: +2048 B = +128 in the address field, K step: +32 B = +2; B operand: +256 B = +16)
@@ -661,9 +661,16 @@ ber_tconv2_kernel(const BerParams prm) {
         // summed over the whole frame (:135-138; noise_norm 1: over the full convolution, main_BER_calculation.m:260-261,289-292)
         // The MMA warp (above) waits for the whole stream and issues the frame's MMAs; the working warps only announce their
         // stores and go on to the noise draws.  Without an MMA warp (NT = 512), TCV2_NISSUE working warps do its job first.
-        const int irank = (warp_u - (int)issuer) & (NW - 1);          // warp-uniform: issuing warps have irank < TCV2_NISSUE
+        // The issuing warps rotate from frame to frame.  The rotation is keyed on the frame's global id and its noise stream
+        // (variant + var), never on the CTA or on the frames it decided before: the accumulator pass below hands the issuers'
+        // tiles to other warps, so it sets the association of the frame-power sum, and a frame's counters must not depend on
+        // where it runs (shards, segments, devices, a pair alone).  The id is hashed (Fibonacci): a CTA's frames lie
+        // nslots * frame_step apart, often a multiple of 16, which would freeze a rotation by f itself.  (The shuffle keeps the
+        // key and what derives from it in vector registers, as the CTA index was: computed in the uniform datapath the same key
+        // cost 3 % at configs[4], and so did a fixed key -- tools/bench_ber_n1024_rotation.py.  With an MMA warp nobody reads it.)
+        const uint32_t issuer = MMAW ? 0u : __shfl_sync(0xffffffffu, ((uint32_t)f * 0x9E3779B9u >> 28) + prm.variant + (uint32_t)(var + rank), 0);
+        const int irank = (int)(((uint32_t)warp_u - issuer) & (NW - 1));   // warp-uniform: issuing warps have irank < TCV2_NISSUE
         const bool is_issuer = !MMAW && irank < TCV2_NISSUE;
-        ++issuer;
         constexpr bool STAG = !MMAW && TCV2_STAGGER && !TCV2_DEBUG_BARRIERS;
         const int igrp = irank >> 2;                                    // staggered issue: this warp's group
         auto issue_group = [&](auto gc) {                               // group g's quarter of the tiles, shared round-robin by its four warps
@@ -817,7 +824,7 @@ ber_tconv2_kernel(const BerParams prm) {
             // did: the issuers are four consecutive warps), all 16 columns of a row in one tcgen05.ld.x16.
             static_assert(NW == 16, "four warps per tensor-memory lane quarter");
             if (!is_issuer) {
-                const int wi = ((int)(issuer - 1u) + ((warp_u - (int)(issuer - 1u)) & 3)) & (NW - 1);   // the quarter's issuing warp
+                const int wi = (int)((issuer + (((uint32_t)warp_u - issuer) & 3u)) & (NW - 1));   // the quarter's issuing warp
                 const int k = warp_u >> 2, ki = wi >> 2;
                 const int r3 = k - (k > ki ? 1 : 0);                               // my rank among the quarter's three others
                 const uint32_t tq = tmem + ((uint32_t)((warp_u & 3) * 32) << 16);
