@@ -108,7 +108,8 @@ WOFDM_API int wofdm_ber_run(wofdm_handle h, const wofdm_sys_t* sys, const double
                   uint64_t seed, uint32_t variant,
                   int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot);
 /* Same, but only frames f = shard_index (mod shard_count): one process per GPU sums the results
- * with a single all-reduce of the int64 counters (SURVEY.md section 8e). */
+ * with a single all-reduce of the int64 counters (SURVEY.md section 8e).  (The channel-mask chain shards by contiguous
+ * blocks of frames instead: wofdm_ber_run_masked_shard.) */
 WOFDM_API int wofdm_ber_run_shard(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
                         const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
                         uint64_t seed, uint32_t variant, int shard_index, int shard_count,
@@ -277,6 +278,30 @@ WOFDM_API int wofdm_ber_run_masked(wofdm_handle h, const wofdm_sys_t* sys, const
                          const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
                          uint64_t seed, uint32_t variant, int roll_off,
                          int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot);
+/* wofdm_ber_run_masked for the frames of one shard: a CONTIGUOUS block of global frame ids
+ * [floor(total*k/W), floor(total*(k+1)/W)), total = n_snr*C*ensemble, k = shard_index, W = shard_count -- not the
+ * f = shard_index (mod shard_count) rule of wofdm_ber_run_shard: the mask product draws contiguous frame ranges, and the
+ * handle's devices split this block as wofdm_ber_run_masked splits all frames.  *_tot count this shard's frames.  The
+ * counters of the W shards add up to wofdm_ber_run_masked's, bit for bit, and wofdm_ber_run_masked is this call with
+ * (0, 1).  Errors: those of wofdm_ber_run_masked, and WOFDM_EINVAL for a bad shard; the handle stays usable. */
+WOFDM_API int wofdm_ber_run_masked_shard(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                         const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                         uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count,
+                         int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot);
+/* The masked counters resolved as in wofdm_ber_run_resolved (resolve: a non-empty combination of WOFDM_BY_SUBCARRIER and
+ * WOFDM_BY_CHANNEL; the same layout with n_var = 1): bit_err / sym_err int64[n_snr][Cr][Nr], sym_tot int64[n_snr][Cr][Nr]
+ * = this shard's frames of the cell times S-1 on active bins, 0 on guard bins (bit totals: sym_tot * bits).  Shards as in
+ * wofdm_ber_run_masked_shard.  Summed over the cells: wofdm_ber_run_masked_shard's counters, bit for bit -- the call runs
+ * the resolved twin of the K1 kernel the masked chain picks (the same arithmetic and noise numbering).  Where a twin's
+ * accumulators do not fit in shared memory, the staged twin runs with that kernel's noise numbering: it draws the same
+ * noise, but its fp32 arithmetic differs, so the counters agree only up to decisions on a boundary.
+ * Errors: WOFDM_EINVAL for a bad shard, a bad resolve, a NULL output or a counter array whose size overflows;
+ * WOFDM_ENOMEM if the device counter buffer cannot be allocated; and what wofdm_ber_run_masked rejects.  The handle stays
+ * usable after every error. */
+WOFDM_API int wofdm_ber_run_masked_resolved(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                         const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                         uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count, int resolve,
+                         int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot);
 
 /* ---- Window-optimisation Hessian (next-row 8f-2) -------------------------------------------------------------
  * The quadratic form of the interference power in the reduced window variables: OptimizerTx / OptimizerRx /

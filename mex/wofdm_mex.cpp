@@ -16,6 +16,7 @@
 //   berK = wofdm_mex('run_simulation_per_subcarrier', ...)  the same, BER per sub-carrier: n_snr x N x n_var
 //   [berSNR, ensembleUsed] = wofdm_mex('run_simulation_adaptive', ...)  the same, each SNR point stopped at a bit-error target
 //   [berMasked, ber] = wofdm_mex('run_sim_mc', ...)          run_sim_mc of matlab/main_channel_mask.m:334-337
+//   [berMasked, ber] = wofdm_mex('run_sim_mc_per_subcarrier', ...)  the same, BER per sub-carrier: N x 1 each (0 on guard bins)
 //   H = wofdm_mex('window_hessian', ...)                     quad_objective_tx / _rx of matlab/window_optimization.m:596-680
 //   H = wofdm_mex('window_hessian_expected', ...), 'quad_objective_tx_expected', 'quad_objective_rx_expected'
 //       -- the same, averaged over a channel set (C x L, rows = realisations) instead of built from one impulse response
@@ -245,8 +246,11 @@ static void do_run_simulation_multi(int nlhs, mxArray* plhs[], int nrhs, const m
 //                               offset, prefixRemovalLength, circularShiftLength, numSubcar, bitsPerSubcar, symbolsPerTx, rollOff [, seed])
 //   -- the positional arguments of run_sim_mc, matlab/main_channel_mask.m:334-337: the same symbols with and without the
 //      DFT-domain raised-cosine mask, independent noise, averaged over the ensemble.
-static void do_run_sim_mc(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
-    if (nrhs < 16) mexErrMsgIdAndTxt("wofdm:nargin", "run_sim_mc needs 16 arguments");
+// per_subcarrier = true ('run_sim_mc_per_subcarrier', the same arguments): berMasked and ber of every sub-carrier, N x 1 in
+// FFT bin order, 0 on the guard bins; their mean over the active bins is run_sim_mc's result.
+static void do_run_sim_mc(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[], bool per_subcarrier) {
+    const char* name = per_subcarrier ? "run_sim_mc_per_subcarrier" : "run_sim_mc";
+    if (nrhs < 16) mexErrMsgIdAndTxt("wofdm:nargin", "%s needs 16 arguments", name);
     wofdm_sys_t s;
     memset(&s, 0, sizeof(s));
     const long long ensemble = (long long)mxGetScalar(prhs[0]);
@@ -262,6 +266,26 @@ static void do_run_sim_mc(int nlhs, mxArray* plhs[], int nrhs, const mxArray* pr
     const std::vector<double> chan = interleave(prhs[7], (size_t)L, 1, 0);
     const double snr = mxGetScalar(prhs[8]);
     const unsigned long long seed = nrhs > 16 ? (unsigned long long)mxGetScalar(prhs[16]) : 0ull;
+    if (per_subcarrier) {
+        const size_t N = (size_t)s.N;
+        std::vector<long long> be(N), se(N), st(N), bem(N), sem(N), stm(N);
+        check(wofdm_ber_run_resolved(handle(), &s, wtx.data(), wrx.data(), 1, chan.data(), L, 1, &snr, 1, ensemble, seed, 0, 0, 1,
+                                     WOFDM_BY_SUBCARRIER, (int64_t*)be.data(), (int64_t*)se.data(), (int64_t*)st.data()),
+              "wofdm_ber_run_resolved");
+        check(wofdm_ber_run_masked_resolved(handle(), &s, wtx.data(), wrx.data(), chan.data(), L, 1, &snr, 1, ensemble, seed, 1,
+                                            roll_off, 0, 1, WOFDM_BY_SUBCARRIER, (int64_t*)bem.data(), (int64_t*)sem.data(),
+                                            (int64_t*)stm.data()),
+              "wofdm_ber_run_masked_resolved");
+        plhs[0] = mxCreateDoubleMatrix((mwSize)N, 1, mxREAL);
+        double* om = mxGetPr(plhs[0]);
+        for (size_t k = 0; k < N; ++k) om[k] = stm[k] ? (double)bem[k] / (double)(stm[k] * s.bits) : 0.0;
+        if (nlhs > 1) {
+            plhs[1] = mxCreateDoubleMatrix((mwSize)N, 1, mxREAL);
+            double* o = mxGetPr(plhs[1]);
+            for (size_t k = 0; k < N; ++k) o[k] = st[k] ? (double)be[k] / (double)(st[k] * s.bits) : 0.0;
+        }
+        return;
+    }
     long long be = 0, bt = 0, se = 0, st = 0, bem = 0, btm = 0;
     check(wofdm_ber_run(handle(), &s, wtx.data(), wrx.data(), chan.data(), L, 1, &snr, 1, ensemble, seed, 0,
                         (int64_t*)&be, (int64_t*)&bt, (int64_t*)&se, (int64_t*)&st), "wofdm_ber_run");
@@ -403,13 +427,14 @@ static void do_calculate_interference(int nlhs, mxArray* plhs[], int nrhs, const
 extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     char cmd[32];
     if (nrhs < 1 || !mxIsChar(prhs[0]) || mxGetString(prhs[0], cmd, sizeof(cmd)))
-        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_simulation_adaptive', 'run_sim_mc', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
+        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_simulation_adaptive', 'run_sim_mc', 'run_sim_mc_per_subcarrier', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
     if (!strcmp(cmd, "run_simulation")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_simulation_sweep")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, true);
     else if (!strcmp(cmd, "run_simulation_sweep_multi")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_simulation_per_subcarrier")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, true);
     else if (!strcmp(cmd, "run_simulation_adaptive")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, false, true);
-    else if (!strcmp(cmd, "run_sim_mc")) do_run_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1);
+    else if (!strcmp(cmd, "run_sim_mc")) do_run_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1, false);
+    else if (!strcmp(cmd, "run_sim_mc_per_subcarrier")) do_run_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1, true);
     else if (!strcmp(cmd, "window_hessian")) do_window_hessian(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "quad_objective_tx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, true, false);
     else if (!strcmp(cmd, "quad_objective_rx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, false, false);

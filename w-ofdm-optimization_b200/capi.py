@@ -107,6 +107,10 @@ SIGNATURES = {
     "wofdm_interf_last_timing": (C.c_int, [C.c_void_p, _dp, _dp, _dp, _P(C.c_int), _P(C.c_int)]),
     "wofdm_ber_run_masked": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64, C.c_uint64,
                                        C.c_uint32, C.c_int, _i64p, _i64p, _i64p, _i64p]),
+    "wofdm_ber_run_masked_shard": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
+                                             C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_int, _i64p, _i64p, _i64p, _i64p]),
+    "wofdm_ber_run_masked_resolved": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
+                                                C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_int, C.c_int, _i64p, _i64p, _i64p]),
     "wofdm_window_hessian": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, _dp, _P(C.c_int)]),
     "wofdm_window_hessian_parts": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, _dp, C.c_int, _dp, C.c_int, _dp, _dp]),
     "wofdm_window_hessian_set": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, C.c_int, _dp, _P(C.c_int)]),
@@ -359,17 +363,36 @@ class Handle:
         self._check(rc)
         return dict(bit_err=be, bit_tot=bt, sym_err=se, sym_tot=st, ensemble_used=used, rounds=rounds.value)
 
-    def ber_run_masked(self, s, win_tx, win_rx, chan, snr_db, ensemble, seed=0, variant=0, roll_off=10):
-        """Channel-mask variant (wofdm_ber_run_masked): counters of the MASKED signal; ber_run with the same `s`
-        (s.guard = the script's offset) gives the unmasked ones on the same symbols."""
+    def ber_run_masked(self, s, win_tx, win_rx, chan, snr_db, ensemble, seed=0, variant=0, roll_off=10, shard=(0, 1)):
+        """Channel-mask variant (wofdm_ber_run_masked_shard): counters of the MASKED signal; ber_run with the same `s`
+        (s.guard = the script's offset) gives the unmasked ones on the same symbols.  shard=(k, W): the k-th of W
+        contiguous blocks of the frame ids (not f = k mod W as in ber_run); the W shards add up to (0, 1)."""
         wt, wr, chf, L, Cn = self._win_chan(s, win_tx, win_rx, chan)
         snr = _f64(np.ravel(snr_db))
         out = [np.zeros(snr.size, dtype=np.int64) for _ in range(4)]
-        rc = load().wofdm_ber_run_masked(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), _ptr(chf, _dp), L, Cn,
-                                         _ptr(snr, _dp), snr.size, int(ensemble), int(seed), int(variant), int(roll_off),
-                                         *[_ptr(o, _i64p) for o in out])
+        rc = load().wofdm_ber_run_masked_shard(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), _ptr(chf, _dp), L, Cn,
+                                               _ptr(snr, _dp), snr.size, int(ensemble), int(seed), int(variant), int(roll_off),
+                                               int(shard[0]), int(shard[1]), *[_ptr(o, _i64p) for o in out])
         self._check(rc)
         return dict(bit_err=out[0], bit_tot=out[1], sym_err=out[2], sym_tot=out[3])
+
+    def ber_run_masked_resolved(self, s, win_tx, win_rx, chan, snr_db, ensemble, seed=0, variant=0, roll_off=10, shard=(0, 1),
+                                by_subcarrier=True, by_channel=False):
+        """ber_run_masked with the counters resolved by sub-carrier and / or channel (wofdm_ber_run_masked_resolved).
+        bit_err / sym_err / sym_tot / bit_tot: (n_snr, Cr, Nr), Cr = C if by_channel else 1, Nr = N (FFT bin order) if
+        by_subcarrier else 1.  Summed over the last two axes: ber_run_masked's counters of the same shard."""
+        wt, wr, chf, L, Cn = self._win_chan(s, win_tx, win_rx, chan)
+        snr = _f64(np.ravel(snr_db))
+        n = snr.size
+        resolve = (WOFDM_BY_SUBCARRIER if by_subcarrier else 0) | (WOFDM_BY_CHANNEL if by_channel else 0)
+        shape = (n, Cn if by_channel else 1, s.N if by_subcarrier else 1)
+        be, se, st = (np.zeros(shape, dtype=np.int64) for _ in range(3))
+        rc = load().wofdm_ber_run_masked_resolved(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), _ptr(chf, _dp), L, Cn,
+                                                  _ptr(snr, _dp), n, int(ensemble), int(seed), int(variant), int(roll_off),
+                                                  int(shard[0]), int(shard[1]), int(resolve),
+                                                  _ptr(be, _i64p), _ptr(se, _i64p), _ptr(st, _i64p))
+        self._check(rc)
+        return dict(bit_err=be, sym_err=se, sym_tot=st, bit_tot=st * int(s.bits))
 
     def psd_estimate(self, N, cp, cs, tail_tx, win_tx, guard_band=48, n_sym=256, records=1, seed=0, sym_idx=None,
                      bits=4, constellation=0):

@@ -167,9 +167,10 @@ int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, bool verify, bool 
     return WOFDM_OK;
 }
 
-// Resolved counters: the twin (BerVariant::res) of the kernel `prod` that wofdm_ber_run_multi picks, where one is compiled
-// and its accumulators fit (nvar: pairs per launch, 1 = one launch per pair); else the staged twin, which numbers its noise
-// like `prod` through noise_at (BerParams::chunk / split / n48).  *fused_out: the twin evaluates all pairs in one launch.
+// Resolved counters: the twin (BerVariant::res) of the kernel `prod` that wofdm_ber_run_multi (or the channel-mask chain:
+// the same txs / txy) picks, where one is compiled and its accumulators fit (nvar: pairs per launch, 1 = one launch per
+// pair); else the staged twin, which numbers its noise like `prod` through noise_at (BerParams::chunk / split / n48).
+// *fused_out: the twin evaluates all pairs in one launch.
 int choose_resolved(wofdm_ctx* h, const wofdm_sys_t& s, int L, size_t smem_cap, const Choice& prod, bool fused, int n_var,
                     Choice* out, bool* fused_out) {
     const BerVariant& p = *prod.var;
@@ -179,7 +180,7 @@ int choose_resolved(wofdm_ctx* h, const wofdm_sys_t& s, int L, size_t smem_cap, 
         // register policies: the twin of the same instantiation (same arithmetic, same noise blocks)
         for (const auto& v : h->variants) {
             if (!v.res || v.gen != 0 || v.TC != p.TC || v.N != p.N || v.NT != p.NT || v.LB != p.LB || v.MINB != p.MINB || v.CL != p.CL ||
-                v.circ != p.circ || v.full != p.full || v.verify) continue;
+                v.circ != p.circ || v.full != p.full || v.txs != p.txs || v.verify) continue;
             const BerSmem lay = v.layout(s.S / v.CL, stride, s.tail_tx, s.tail_rx, L, prod.chunk, 0);
             if (lay.bytes > smem_cap) break;
             out->var = &v; out->lay = lay; out->chunk = prod.chunk; out->use_global = 0;
@@ -189,7 +190,8 @@ int choose_resolved(wofdm_ctx* h, const wofdm_sys_t& s, int L, size_t smem_cap, 
     }
     if (p.gen == 2 && !staged_only) {
         for (const auto& v : h->variants) {
-            if (!v.res || v.gen != 2 || v.verify || v.N != p.N || v.NT != p.NT || v.ntile != p.ntile || v.LB != p.LB || v.CL != p.CL) continue;
+            if (!v.res || v.gen != 2 || v.verify || v.N != p.N || v.NT != p.NT || v.ntile != p.ntile || v.LB != p.LB || v.CL != p.CL ||
+                v.txy != p.txy) continue;
             // all pairs in one launch where the accumulators of all of them fit, else one launch per pair (same counters)
             for (int nv : {fused ? n_var : 1, 1}) {
                 const BerSmem lay = v.layout(s.S / v.CL, stride, s.tail_tx, s.tail_rx, L, nv, 0);
@@ -1055,21 +1057,32 @@ static void host_fft_pow2(std::vector<double>& a, int n) {
 // Channel-mask variant (include/wofdm.h): frames in batches -- the masked Tx streams of a batch are written to HBM (the dense
 // tensor-core product of mask_gemm.cu, or tx_mask_kernel with WOFDM_MASK_FFT=1), a K1 kernel reads them
 // (BerParams::tx_stream) and does channel, noise, Rx and counting as always.
-int wofdm_ber_run_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
-                         const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
-                         uint64_t seed, uint32_t variant, int roll_off,
-                         int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot) {
-    NvtxRange nvtx_("wofdm_ber_run_masked");
-    if (!h) return WOFDM_EINVAL;
+// The frames [*f_lo, *f_hi) of shard (shard_index, shard_count), a contiguous block of global frame ids.  resolve == 0:
+// bit_err / sym_err [n_snr]; else [n_snr][Cr][Nr] (wofdm_ber_run_resolved's layout, one window pair), counted by the
+// resolved twin of the K1 kernel this chain picks.  outputs_ok: the caller's output pointers are all non-NULL.
+static int run_masked_impl(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                           const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                           uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count, int resolve,
+                           bool outputs_ok, int64_t* bit_err, int64_t* sym_err, long long* f_lo_out, long long* f_hi_out) {
     int rc = validate_sys(h, sys, L);
     if (rc) return rc;
-    if (!win_tx || !win_rx || !chan || !snr_db || !bit_err || !bit_tot || !sym_err || !sym_tot) return fail(h, WOFDM_EINVAL, "NULL buffer");
+    if (!win_tx || !win_rx || !chan || !snr_db || !outputs_ok) return fail(h, WOFDM_EINVAL, "NULL buffer");
     if (C < 1 || n_snr < 1 || ensemble < 1) return fail(h, WOFDM_EINVAL, "C, n_snr and ensemble must be >= 1");
     if (sys->precision != 0) return fail(h, WOFDM_EUNSUPPORTED, "the channel-mask variant runs in fp32");
     const int N = sys->N, n_tx = N + sys->cp + sys->cs, stride = n_tx - sys->tail_tx, M = 2 * n_tx - 1;
     if (N != 128 && N != 256 && N != 512) return fail(h, WOFDM_EUNSUPPORTED, "the channel-mask variant is built for N = 128, 256, 512");
     if (roll_off < 1 || M / 2 + 2 * roll_off > M) return fail(h, WOFDM_EINVAL, "roll_off does not fit the mask");
     if (2 * n_tx > 3 * N + 1) return fail(h, WOFDM_EUNSUPPORTED, "cp + cs too long for the mask kernel (n_tx <= 1.5 N)");
+    if (shard_count < 1 || shard_index < 0 || shard_index >= shard_count) return fail(h, WOFDM_EINVAL, "bad shard");
+    long long total = 0;
+    if (__builtin_mul_overflow((long long)n_snr, (long long)C, &total) || __builtin_mul_overflow(total, (long long)ensemble, &total))
+        return fail(h, WOFDM_EINVAL, "n_snr * C * ensemble overflows int64");
+    // counter pairs [n_snr][Cr][Nr], 16 bytes each on the device: all of it must be representable
+    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? N : 1;
+    size_t ncnt = 0, cnt_bytes = 0;
+    if (__builtin_mul_overflow((size_t)n_snr, (size_t)Cr, &ncnt) || __builtin_mul_overflow(ncnt, (size_t)Nr, &ncnt) ||
+        __builtin_mul_overflow(ncnt, (size_t)16, &cnt_bytes) || ncnt > (size_t)INT64_MAX / 16)
+        return fail(h, WOFDM_EINVAL, "resolved counter array too large");
     DeviceCtx& d0 = h->devs[0];              // (variant selection: the devices of a handle are alike)
     WOFDM_CUDA(h, cudaSetDevice(d0.dev));
     Choice ch, prod;
@@ -1090,9 +1103,20 @@ int wofdm_ber_run_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* w
     rc = choose_variant(h, *sys, L, false, false, d0.smem_optin, &prod, win_tx);     // noise numbering of wofdm_ber_run / _draws
     if (rc) return rc;
     if (prod.var->CL > 1) return fail(h, WOFDM_EUNSUPPORTED, "no channel-mask variant for cluster kernels");
+    // the kernel that runs: ch, or (resolved counters) its twin -- the noise numbering below stays ch's either way, so a
+    // staged fallback draws ch's noise; it reads the assembled stream even where ch gathers from the product itself
+    Choice run = ch;
+    if (resolve) {
+        Choice nz = ch;
+        if (ch.var->TC == 0) nz.chunk = prod.chunk;
+        bool rfused = false;
+        rc = choose_resolved(h, *sys, L, d0.smem_optin, nz, false, 1, &run, &rfused);
+        if (rc) return rc;
+        fused = run.var->txy;
+    }
     int nb = 0;
     long long max_ctas = 0;
-    rc = prepare_kernel(h, *ch.var, ch.lay.bytes, d0.sm_count, &nb, &max_ctas);
+    rc = prepare_kernel(h, *run.var, run.lay.bytes, d0.sm_count, &nb, &max_ctas);
     if (rc) return rc;
     std::vector<double> gd;
     if (!use_gemm) {
@@ -1144,34 +1168,41 @@ int wofdm_ber_run_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* w
         twp.resize(16);
     }
     HostTables t;
-    build_tables(*sys, win_tx, win_rx, t, ch.var->ntile > 0);   // (tx_mask_kernel shares the table: a common factor of its stream)
+    build_tables(*sys, win_tx, win_rx, t, run.var->ntile > 0);   // (tx_mask_kernel shares the table: a common factor of its stream)
     std::vector<unsigned char> hchan, hsnr;
-    cast_chan(false, chan, (size_t)L * C, hchan, L, ch.var->ntile > 0);
+    cast_chan(false, chan, (size_t)L * C, hchan, L, run.var->ntile > 0);
     std::vector<double> lin(n_snr);
     for (int i = 0; i < n_snr; ++i) lin[i] = std::pow(10.0, -0.1 * snr_db[i]);
     cast_any(false, lin, hsnr);
-    const long long total = (long long)n_snr * C * ensemble;
+    // this shard's block of frame ids [f_lo, f_hi); batches and devices take contiguous ranges of it
+    const long long f_lo = (long long)((__int128)total * shard_index / shard_count);
+    const long long f_hi = (long long)((__int128)total * (shard_index + 1) / shard_count), nfr = f_hi - f_lo;
+    *f_lo_out = f_lo; *f_hi_out = f_hi;
+    if (nfr == 0) {
+        for (size_t i = 0; i < ncnt; ++i) { bit_err[i] = 0; sym_err[i] = 0; }
+        return WOFDM_OK;
+    }
     const size_t body = (size_t)sys->tail_tx + (size_t)sys->S * stride;
-    const long long batch = std::min<long long>(total, use_gemm ? 16384 : 8192);
-    const size_t scratch_elems = (size_t)ch.lay.pad + body + 64;
+    const long long batch = std::min<long long>(nfr, use_gemm ? 16384 : 8192);
+    const size_t scratch_elems = (size_t)run.lay.pad + body + 64;
     const int grid_ber = (int)std::min<long long>(batch, max_ctas);
-    const size_t scratch_bytes = ch.use_global ? (size_t)grid_ber * 2 * scratch_elems * sizeof(float2) : 0;
+    const size_t scratch_bytes = run.use_global ? (size_t)grid_ber * 2 * scratch_elems * sizeof(float2) : 0;
     // every device of the handle takes a contiguous range of the frames (frame ids are global: same draws, same counters as
     // on one device); its work is enqueued on its own stream, the counters meet on the host
-    const int nd = (int)std::min<long long>((long long)h->devs.size(), std::max<long long>(1, total / 64));
-    std::vector<std::vector<unsigned long long>> cnts(nd, std::vector<unsigned long long>((size_t)n_snr * 2, 0ull));
+    const int nd = (int)std::min<long long>((long long)h->devs.size(), std::max<long long>(1, nfr / 64));
+    std::vector<std::vector<unsigned long long>> cnts;     // (allocated once the device buffers exist)
     std::vector<void*> d_cnts(nd, nullptr);
     auto run_dev = [&](DeviceCtx& d, long long f_lo, long long f_hi, void** d_cnt_out) -> int {
     WOFDM_CUDA(h, cudaSetDevice(d.dev));
     if (&d != &d0) {
         int nb_ = 0; long long mc_ = 0;
-        const int rcp = prepare_kernel(h, *ch.var, ch.lay.bytes, d.sm_count, &nb_, &mc_);
+        const int rcp = prepare_kernel(h, *run.var, run.lay.bytes, d.sm_count, &nb_, &mc_);
         if (rcp) return rcp;
     }
     MaskGemm mg;
     const size_t mg_bytes = use_gemm ? mask_gemm_plan(*sys, batch, mg) : 0;
     int rc = arena_reserve(h, d, t.wtx.size() + t.wrx.size() + t.tw.size() + twp.size() + hchan.size() + hsnr.size() + g.size() * 4 +
-                                 (size_t)n_snr * 16 + (fused ? 16 : (size_t)batch * body * sizeof(float2)) + scratch_bytes + mg_bytes + 8192);
+                                 cnt_bytes + (fused ? 16 : (size_t)batch * body * sizeof(float2)) + scratch_bytes + mg_bytes + 8192);
     if (rc) return rc;
     auto put = [&](const void* src, size_t bytes, void** dst) -> cudaError_t {
         *dst = arena_take(d, std::max<size_t>(bytes, 16));
@@ -1186,10 +1217,10 @@ int wofdm_ber_run_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* w
     WOFDM_CUDA(h, put(hsnr.data(), hsnr.size(), &d_snr));
     WOFDM_CUDA(h, put(g.data(), g.size() * 4, &d_g));
     WOFDM_CUDA(h, put(twp.data(), twp.size(), &d_twp));
-    WOFDM_CUDA(h, put(nullptr, (size_t)n_snr * 16, &d_cnt));
+    WOFDM_CUDA(h, put(nullptr, cnt_bytes, &d_cnt));
     WOFDM_CUDA(h, put(nullptr, fused ? 16 : (size_t)batch * body * sizeof(float2), &d_stream));
     if (scratch_bytes) WOFDM_CUDA(h, put(nullptr, scratch_bytes, &d_scr));
-    WOFDM_CUDA(h, cudaMemsetAsync(d_cnt, 0, (size_t)n_snr * 16, d.stream));
+    WOFDM_CUDA(h, cudaMemsetAsync(d_cnt, 0, cnt_bytes, d.stream));
     if (use_gemm) {
         rc = mask_gemm_setup(h, d, mg, roll_off, static_cast<const float*>(d_wtx));
         if (rc) return rc;
@@ -1204,7 +1235,7 @@ int wofdm_ber_run_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* w
     mp.seed = seed; mp.stream = static_cast<float2*>(d_stream);
     BerParams prm;
     fill_sys(prm, *sys, L);
-    prm.chunk = ch.var->TC > 0 ? ch.chunk : prod.chunk; prm.use_global = ch.use_global;
+    prm.chunk = ch.var->TC > 0 ? ch.chunk : prod.chunk; prm.use_global = run.use_global;
     fill_flat(prm, *sys, win_tx, win_rx);
     prm.flat_tx = 0;                       // (the Tx stream comes from tx_mask_kernel)
     fill_split(prm, *ch.var);
@@ -1217,6 +1248,8 @@ int wofdm_ber_run_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* w
     prm.C = C; prm.n_snr = n_snr; prm.ensemble = ensemble; prm.seed = seed; prm.variant = variant;
     philox_round_keys(seed, prm.rk);
     prm.counters = static_cast<unsigned long long*>(d_cnt);
+    prm.res_chan = (resolve & WOFDM_BY_CHANNEL) ? 1 : 0;
+    prm.res_bins = (resolve & WOFDM_BY_SUBCARRIER) ? 1 : 0;
     prm.scratch = d_scr; prm.scratch_elems = (long long)scratch_elems;
     prm.tx_stream = static_cast<const float2*>(d_stream);
     if (fused) { prm.tx_y = mg.Y; prm.tx_yp = mg.Yp; }
@@ -1254,33 +1287,93 @@ int wofdm_ber_run_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* w
             }
         }
         prm.frame_begin = f0; prm.frame_step = 1; prm.n_frames = nf;
-        WOFDM_CUDA(h, ch.var->launch(prm, (int)std::min<long long>(nf, max_ctas), ch.lay.bytes, d.stream));
+        WOFDM_CUDA(h, run.var->launch(prm, (int)std::min<long long>(nf, max_ctas), run.lay.bytes, d.stream));
         h->launches += 2;
     }
     *d_cnt_out = d_cnt;
     return WOFDM_OK;
     };   // run_dev
     for (int i = 0; i < nd; ++i) {
-        rc = run_dev(h->devs[i], total * i / nd, total * (i + 1) / nd, &d_cnts[i]);
+        rc = run_dev(h->devs[i], f_lo + nfr * i / nd, f_lo + nfr * (i + 1) / nd, &d_cnts[i]);
         if (rc) break;
+    }
+    if (!rc) {
+        try { cnts.assign(nd, std::vector<unsigned long long>(ncnt * 2, 0ull)); }
+        catch (const std::bad_alloc&) { rc = fail(h, WOFDM_ENOMEM, "host allocation failed"); }
     }
     // (the downloads into pageable memory block the host: only after every device has its work)
     for (int i = 0; i < nd; ++i) {           // (also after a failure: nothing of this call stays in flight)
         cudaSetDevice(h->devs[i].dev);
         cudaError_t es = cudaSuccess;
-        if (!rc && d_cnts[i]) es = cudaMemcpyAsync(cnts[i].data(), d_cnts[i], (size_t)n_snr * 16, cudaMemcpyDeviceToHost, h->devs[i].stream);
+        if (!rc && d_cnts[i]) es = cudaMemcpyAsync(cnts[i].data(), d_cnts[i], cnt_bytes, cudaMemcpyDeviceToHost, h->devs[i].stream);
         if (es == cudaSuccess) es = cudaStreamSynchronize(h->devs[i].stream);
         if (es != cudaSuccess && !rc) rc = fail(h, WOFDM_ECUDA, std::string("wofdm_ber_run_masked: ") + cudaGetErrorString(es));
     }
     cudaSetDevice(d0.dev);
     if (rc) return rc;
-    for (int i = 0; i < n_snr; ++i) {
+    for (size_t i = 0; i < ncnt; ++i) {
         unsigned long long be = 0, se = 0;
         for (int k = 0; k < nd; ++k) { be += cnts[k][2 * i]; se += cnts[k][2 * i + 1]; }
         bit_err[i] = (int64_t)be; sym_err[i] = (int64_t)se;
-        sym_tot[i] = (int64_t)C * ensemble * (N - 2 * sys->guard) * (sys->S - 1);
+    }
+    return WOFDM_OK;
+}
+
+int wofdm_ber_run_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                         const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                         uint64_t seed, uint32_t variant, int roll_off,
+                         int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot) {
+    return wofdm_ber_run_masked_shard(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, seed, variant, roll_off, 0, 1,
+                                      bit_err, bit_tot, sym_err, sym_tot);
+}
+
+int wofdm_ber_run_masked_shard(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                               const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                               uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count,
+                               int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot) {
+    NvtxRange nvtx_("wofdm_ber_run_masked");
+    if (!h) return WOFDM_EINVAL;
+    long long f_lo = 0, f_hi = 0;
+    const int rc = run_masked_impl(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, seed, variant, roll_off,
+                                   shard_index, shard_count, 0, bit_err && bit_tot && sym_err && sym_tot, bit_err, sym_err,
+                                   &f_lo, &f_hi);
+    if (rc) return rc;
+    const long long per_snr = (long long)C * ensemble;
+    for (int i = 0; i < n_snr; ++i) {           // this shard's frames of point i: [i, i+1) * C * ensemble inside [f_lo, f_hi)
+        const long long frames = std::max(0LL, std::min(f_hi, (i + 1) * per_snr) - std::max(f_lo, i * per_snr));
+        sym_tot[i] = frames * (sys->N - 2 * sys->guard) * (sys->S - 1);   // active sub-carriers only
         bit_tot[i] = sym_tot[i] * sys->bits;
     }
+    return WOFDM_OK;
+}
+
+int wofdm_ber_run_masked_resolved(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                                  const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                                  uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count, int resolve,
+                                  int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot) {
+    NvtxRange nvtx_("wofdm_ber_run_masked_resolved");
+    if (!h) return WOFDM_EINVAL;
+    if (resolve == 0 || (resolve & ~(WOFDM_BY_SUBCARRIER | WOFDM_BY_CHANNEL)))
+        return fail(h, WOFDM_EINVAL, "resolve must be a non-empty combination of WOFDM_BY_SUBCARRIER and WOFDM_BY_CHANNEL");
+    if (!bit_err || !sym_err || !sym_tot) return fail(h, WOFDM_EINVAL, "NULL output buffer");
+    long long f_lo = 0, f_hi = 0;
+    const int rc = run_masked_impl(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, seed, variant, roll_off,
+                                   shard_index, shard_count, resolve, true, bit_err, sym_err, &f_lo, &f_hi);
+    if (rc) return rc;
+    // this shard's frames per cell (si, c): [(si*C + c)*ensemble, +ensemble) inside [f_lo, f_hi); guard bins count nothing
+    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? sys->N : 1;
+    const long long active = sys->N - 2 * sys->guard;
+    for (int si = 0; si < n_snr; ++si)
+        for (int c = 0; c < Cr; ++c) {
+            const long long lo = ((long long)si * C + (Cr > 1 ? c : 0)) * ensemble, hi = lo + (Cr > 1 ? 1 : (long long)C) * ensemble;
+            const long long frames = std::max(0LL, std::min(f_hi, hi) - std::max(f_lo, lo));
+            int64_t* out = sym_tot + ((size_t)si * Cr + c) * Nr;
+            if (Nr == 1) { out[0] = frames * active * (sys->S - 1); continue; }
+            for (int k = 0; k < Nr; ++k) {
+                const int cc = (k + Nr / 2) & (Nr - 1);               // ber_kernel.cuh: bin_active
+                out[k] = (cc >= sys->guard && cc < Nr - sys->guard) ? frames * (sys->S - 1) : 0;
+            }
+        }
     return WOFDM_OK;
 }
 

@@ -458,7 +458,7 @@ template <int CL> __device__ __forceinline__ void frame_sync() {
 // TXS: the Tx stage can take the frame's stream from HBM (BerParams::tx_stream, channel-mask variant).  Always possible in
 // the staged policy; the register-resident kernels get it as separate instantiations so that the main path keeps its code.
 // RES: error counters resolved by sub-carrier and / or channel (BerParams::res_chan / res_bins); in a cluster every CTA keeps
-// and flushes the accumulators of its own symbols
+// and flushes the accumulators of its own symbols.  RES && TXS: the twins of the channel-mask chain's TXS kernels
 template <typename T, int N, int NT, int TC, int LB, int MINB, bool FULL, bool VERIFY, int CL = 1, bool CIRC = false, bool TXS = false,
           bool RES = false>
 __global__ void __launch_bounds__(NT, MINB)
@@ -470,7 +470,7 @@ ber_frame_kernel(const BerParams prm) {
     static_assert(NT % TPF == 0 && NT % 32 == 0, "threads per CTA must be a multiple of N/16 and 32");
     constexpr bool REGS = TC > 0;
     static_assert(CL == 1 || REGS, "clusters are a feature of the register-resident policy");
-    static_assert(!RES || (!VERIFY && !TXS), "resolved counters: production kernels");
+    static_assert(!RES || !VERIFY, "resolved counters: production kernels");
     static_assert(!CIRC || (REGS && CL == 1 && N <= NT), "circular-interior policy: regs, one CTA per frame, one bin per thread");
     // Register row q of a thread = sub-carriers / samples t + q*TPF.  Only the outer rows can reach the cyclic
     // prefix / suffix, the Tx heads and the Rx overlap-add; the tuned variants look at ER of them (the host

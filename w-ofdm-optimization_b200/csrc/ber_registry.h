@@ -77,6 +77,9 @@ struct BerVariantImpl {
     out.push_back(BerVariantImpl<T, N, NT, 0, 0, 1, false, false, 1, false, false, true>::make("ber_" tag "_n" #N "_t" #NT "_c0_l0_b1_f0_res"));
 #define WOFDM_VARIANT_RES_REGS(T, N, NT, TC, LB, MINB, FULL, CL, CIRC, tag, sfx)                         \
     out.push_back(BerVariantImpl<T, N, NT, TC, LB, MINB, FULL, false, CL, CIRC, false, true>::make("ber_" tag "_n" #N "_t" #NT "_c" #TC "_l" #LB "_b" #MINB "_f" #FULL "_cl" #CL sfx));
+// ... and the twins of the TXS instantiations (wofdm_ber_run_masked_resolved: the masked Tx stream read from HBM)
+#define WOFDM_VARIANT_RES_TXS(T, N, NT, TC, LB, MINB, FULL, tag)                                         \
+    out.push_back(BerVariantImpl<T, N, NT, TC, LB, MINB, FULL, false, 1, false, true, true>::make("ber_" tag "_n" #N "_t" #NT "_c" #TC "_l" #LB "_b" #MINB "_f" #FULL "_txs_res"));
 
 void register_ber_f32_staged(std::vector<BerVariant>& out);
 void register_ber_f32_tconv(std::vector<BerVariant>& out);
@@ -88,5 +91,7 @@ void register_ber_f32_tconv2_res(std::vector<BerVariant>& out);      // resolved
 void register_ber_f32_tconv2_res_big(std::vector<BerVariant>& out);
 void register_ber_staged_res(std::vector<BerVariant>& out);          // ... staged ...
 void register_ber_f32_regs_res(std::vector<BerVariant>& out);        // ... and register policies
+void register_ber_f32_tconv2_txy_res(std::vector<BerVariant>& out); // the channel-mask chain's twins: tensor-core gather ...
+void register_ber_f32_regs_txs_res(std::vector<BerVariant>& out);    // ... and register kernels on the assembled stream
 
 }  // namespace wofdm

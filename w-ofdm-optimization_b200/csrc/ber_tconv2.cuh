@@ -240,7 +240,7 @@ ber_tconv2_kernel(const BerParams prm) {
     static_assert(NSEG <= TCV2_MAXSEG, "one mbarrier per segment");
     static_assert(16 * NTILE <= (int)TMEM_COLS, "accumulators of a frame must fit tensor memory");
     static_assert(CL * NW <= 32, "per-warp power partials of all CTAs must fit the reduction scratch");
-    static_assert(!RES || (!VERIFY && !TXY), "resolved counters: production kernels");
+    static_assert(!RES || !VERIFY, "resolved counters: production kernels");
 
     extern __shared__ __align__(128) unsigned char tcv_smem[];
     unsigned char* const smem_raw = tcv_smem;

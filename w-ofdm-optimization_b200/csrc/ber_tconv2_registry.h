@@ -34,4 +34,7 @@ struct Tconv2VariantImpl {
 // counters resolved by sub-carrier / channel (wofdm_ber_run_resolved): the production kernels' twins, registered separately
 #define WOFDM_VARIANT_TCONV2_RES(N, NT, NTILE, MINB, CL, LB)                                                  \
     out.push_back(Tconv2VariantImpl<N, NT, NTILE, MINB, false, CL, LB, false, true>::make("ber_f32t2_n" #N "_t" #NT "_tiles" #NTILE "_b" #MINB "_cl" #CL "_l" #LB "_res"));
+// the twins of the TXY instantiations (wofdm_ber_run_masked_resolved: the Tx stream gathered from the mask product)
+#define WOFDM_VARIANT_TCONV2_TXY_RES(N, NT, NTILE, MINB)                                                      \
+    out.push_back(Tconv2VariantImpl<N, NT, NTILE, MINB, false, 1, TCV_LB, true, true>::make("ber_f32t2_n" #N "_t" #NT "_tiles" #NTILE "_b" #MINB "_txy_res"));
 }  // namespace wofdm

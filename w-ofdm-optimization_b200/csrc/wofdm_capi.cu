@@ -149,6 +149,8 @@ int wofdm_create_on(wofdm_handle* out, const int* device_ids, int n) {
     register_ber_f32_tconv2_res(h->variants);
     register_ber_staged_res(h->variants);
     register_ber_f32_regs_res(h->variants);
+    register_ber_f32_tconv2_txy_res(h->variants);
+    register_ber_f32_regs_txs_res(h->variants);
     *out = h;
     return WOFDM_OK;
 }

@@ -215,6 +215,26 @@ def run_sim_mc(ensemble, cpLength, csLength, tailTx, tailRx, windowTx, windowRx,
     return float(rm["bit_err"][0] / rm["bit_tot"][0]), float(r["bit_err"][0] / r["bit_tot"][0])
 
 
+def run_sim_mc_per_subcarrier(ensemble, cpLength, csLength, tailTx, tailRx, windowTx, windowRx, channel, snr, offset,
+                              prefixRemovalLength, circularShiftLength, numSubcar, bitsPerSubcar, symbolsPerTx, rollOff, seed=0,
+                              handle=None):
+    """run_sim_mc resolved by sub-carrier: (berMasked, ber), each of shape (numSubcar,) in FFT bin order, 0 on the guard
+    bins -- where the mask costs errors.  The same symbols with and without the mask, the noise of run_sim_mc with the
+    same seed, so the mean over the active bins is run_sim_mc's result."""
+    h = handle or default_handle()
+    s = capi.SysT(N=int(numSubcar), cp=int(cpLength), cs=int(csLength), tail_tx=int(tailTx), tail_rx=int(tailRx),
+                  rm=int(prefixRemovalLength), shift=int(circularShiftLength), bits=int(bitsPerSubcar),
+                  S=int(symbolsPerTx), noise_norm=1, constellation=1, precision=0, guard=int(offset))
+    wt, wr, ch = _diag(windowTx), _diag(windowRx), np.asarray(channel).ravel()
+    r = h.ber_run_resolved(s, [wt], [wr], ch, [float(snr)], int(ensemble), seed=seed, variant=0, by_subcarrier=True)
+    rm = h.ber_run_masked_resolved(s, wt, wr, ch, [float(snr)], int(ensemble), seed=seed, variant=1, roll_off=int(rollOff),
+                                   by_subcarrier=True)
+    out = []
+    for be, bt in ((rm["bit_err"][0, 0], rm["bit_tot"][0, 0]), (r["bit_err"][0, 0, 0], r["bit_tot"][0, 0])):
+        out.append(np.divide(be, bt, out=np.zeros(bt.shape), where=bt > 0))
+    return out[0], out[1]
+
+
 def calculate_interference(cpLength, typeOFDM, windowTx, windowRx, numSubcar, tailTx, tailRx, channels, mode=0,
                            handle=None):
     """Scalar interference power on the mean of `channels` (rows = realisations, as vehA200channel2 is stored),
