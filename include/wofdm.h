@@ -302,6 +302,40 @@ WOFDM_API int wofdm_ber_run_masked_resolved(wofdm_handle h, const wofdm_sys_t* s
                          const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
                          uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count, int resolve,
                          int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot);
+/* Frame segments of the channel-mask chain: the segments, frame ids, draws and local index j of wofdm_ber_run_segments
+ * (f = (snr_idx*C + c)*ensemble_max + e, the draws of wofdm_ber_run_masked(ensemble = ensemble_max); j runs over the
+ * segments in the order given, channel-major, then e), so disjoint segment lists add up to the full masked run.  Shards
+ * follow the masked chain's rule on j: shard k of W takes the contiguous block [floor(n_local*k/W), floor(n_local*(k+1)/W))
+ * of the n_local local indices, and the handle's devices split that block contiguously.
+ *   resolve = 0: bit_err / sym_err / sym_tot int64[n_snr]; non-zero: the [n_snr][Cr][Nr] layout of
+ *   wofdm_ber_run_masked_resolved.  sym_tot counts this shard's frames; bit totals are sym_tot * bits.
+ * The call always runs the resolved twin of the masked chain's K1 kernel, with the fallback rules of
+ * wofdm_ber_run_masked_resolved.  Errors: what wofdm_ber_run_segments and wofdm_ber_run_masked_resolved reject (NULL or
+ * empty, out-of-range or overlapping segments, e_count < 1, a bad shard, unknown resolve bits, NULL outputs, an overflowing
+ * frame space or counter array, fp64, N outside {128, 256, 512}).  The handle stays usable after every error. */
+WOFDM_API int wofdm_ber_run_masked_segments(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                         const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble_max,
+                         const int64_t* segments /* [n_seg][3] = {snr_idx, e_begin, e_count} */, int n_seg,
+                         uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count, int resolve,
+                         int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot);
+/* run_sim_mc of matlab/main_channel_mask.m with the stopping rule of wofdm_ber_run_adaptive: the masked and the unmasked
+ * chain on the same frames (one window pair, the same sys), every SNR point run until both have counted `target` errors
+ * or ensemble_max ensemble indices.
+ *   row 0 of bit_err / sym_err (int64[2][n_snr]): the masked chain (wofdm_ber_run_masked_segments), noise stream
+ *   variant + 1; row 1: the unmasked chain (wofdm_ber_run_segments), noise stream variant.  variant = 0 gives the draws
+ *   of the two calls run_sim_mc makes.
+ * The schedule is wofdm_ber_run_adaptive's with m_s the minimum over the two rows.  Each row shards by its own chain's
+ * rule (contiguous blocks of the round's local indices for row 0, j = shard_index (mod shard_count) for row 1); reduce
+ * receives this process's round counts int64[2][n_snr][2] = {bit, sym} (n = 4*n_snr) and makes them the job's.
+ * shard_count > 1 without reduce is WOFDM_EINVAL.  Outputs: ensemble_used[n_snr], bit_tot / sym_tot int64[n_snr] (the
+ * same for both rows), *rounds.  The stopped estimator has the relative bias of order 1/target that wofdm_ber_run_adaptive
+ * states; points that stop at ensemble_max are unbiased.  Errors: those of wofdm_ber_run_adaptive and of
+ * wofdm_ber_run_masked; the handle stays usable. */
+WOFDM_API int wofdm_ber_run_masked_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                         const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble_max, int64_t first_block,
+                         int target_kind, int64_t target, uint64_t seed, uint32_t variant, int roll_off, int shard_index,
+                         int shard_count, wofdm_reduce_fn reduce, void* reduce_user,
+                         int64_t* ensemble_used, int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot, int* rounds);
 
 /* ---- Window-optimisation Hessian (next-row 8f-2) -------------------------------------------------------------
  * The quadratic form of the interference power in the reduced window variables: OptimizerTx / OptimizerRx /

@@ -17,6 +17,7 @@
 //   [berSNR, ensembleUsed] = wofdm_mex('run_simulation_adaptive', ...)  the same, each SNR point stopped at a bit-error target
 //   [berMasked, ber] = wofdm_mex('run_sim_mc', ...)          run_sim_mc of matlab/main_channel_mask.m:334-337
 //   [berMasked, ber] = wofdm_mex('run_sim_mc_per_subcarrier', ...)  the same, BER per sub-carrier: N x 1 each (0 on guard bins)
+//   [berMasked, ber, ensembleUsed] = wofdm_mex('run_sim_mc_adaptive', ...)  run_sim_mc, each SNR point stopped at a bit-error target
 //   H = wofdm_mex('window_hessian', ...)                     quad_objective_tx / _rx of matlab/window_optimization.m:596-680
 //   H = wofdm_mex('window_hessian_expected', ...), 'quad_objective_tx_expected', 'quad_objective_rx_expected'
 //       -- the same, averaged over a channel set (C x L, rows = realisations) instead of built from one impulse response
@@ -295,6 +296,48 @@ static void do_run_sim_mc(int nlhs, mxArray* plhs[], int nrhs, const mxArray* pr
     if (nlhs > 1) plhs[1] = mxCreateDoubleScalar(bt ? (double)be / (double)bt : 0.0);
 }
 
+// [berMasked, ber, ensembleUsed] = wofdm_mex('run_sim_mc_adaptive', <the 16 arguments of run_sim_mc>, targetBitErrors,
+//                                            ensembleMax [, seed])
+//   -- run_sim_mc with every SNR point stopped once the masked and the unmasked chain have each counted targetBitErrors
+//      bit errors, or at ensembleMax ensemble indices (wofdm_ber_run_masked_adaptive).  channel: C x L (rows = realisations),
+//      snr: a vector; the first argument, ensemble, is the first round's block.  Each output is n_snr x 1.
+static void do_run_sim_mc_adaptive(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
+    if (nrhs < 18) mexErrMsgIdAndTxt("wofdm:nargin", "run_sim_mc_adaptive needs 18 arguments");
+    wofdm_sys_t s;
+    memset(&s, 0, sizeof(s));
+    const long long first_block = (long long)mxGetScalar(prhs[0]);
+    s.cp = (int)mxGetScalar(prhs[1]); s.cs = (int)mxGetScalar(prhs[2]);
+    s.tail_tx = (int)mxGetScalar(prhs[3]); s.tail_rx = (int)mxGetScalar(prhs[4]);
+    s.guard = (int)mxGetScalar(prhs[9]); s.rm = (int)mxGetScalar(prhs[10]); s.shift = (int)mxGetScalar(prhs[11]);
+    s.N = (int)mxGetScalar(prhs[12]); s.bits = (int)mxGetScalar(prhs[13]); s.S = (int)mxGetScalar(prhs[14]);
+    const int roll_off = (int)mxGetScalar(prhs[15]);
+    s.noise_norm = 1; s.constellation = 1; s.precision = 0;
+    const std::vector<double> wtx = diag_of(prhs[5], (size_t)(s.N + s.cp + s.cs));
+    const std::vector<double> wrx = diag_of(prhs[6], (size_t)(s.N + s.tail_rx));
+    const size_t C = mxGetM(prhs[7]), L = mxGetN(prhs[7]);
+    std::vector<double> chan(2 * L * C);
+    for (size_t c = 0; c < C; ++c) {
+        const std::vector<double> row = interleave(prhs[7], L, C, c);
+        memcpy(chan.data() + 2 * L * c, row.data(), 2 * L * sizeof(double));
+    }
+    const size_t n_snr = mxGetNumberOfElements(prhs[8]);
+    const long long target = (long long)mxGetScalar(prhs[16]), ensemble_max = (long long)mxGetScalar(prhs[17]);
+    const unsigned long long seed = nrhs > 18 ? (unsigned long long)mxGetScalar(prhs[18]) : 0ull;
+    std::vector<long long> be(2 * n_snr), se(2 * n_snr), bt(n_snr), st(n_snr), used(n_snr);
+    int rounds = 0;
+    check(wofdm_ber_run_masked_adaptive(handle(), &s, wtx.data(), wrx.data(), chan.data(), (int)L, (int)C, mxGetPr(prhs[8]),
+                                        (int)n_snr, ensemble_max, first_block, WOFDM_TARGET_BIT_ERRORS, target, seed, 0, roll_off,
+                                        0, 1, nullptr, nullptr, (int64_t*)used.data(), (int64_t*)be.data(), (int64_t*)bt.data(),
+                                        (int64_t*)se.data(), (int64_t*)st.data(), &rounds),
+          "wofdm_ber_run_masked_adaptive");
+    for (int row = 0; row < 3 && row < (nlhs > 0 ? nlhs : 1); ++row) {       // berMasked (row 0), ber (row 1), ensembleUsed
+        plhs[row] = mxCreateDoubleMatrix((mwSize)n_snr, 1, mxREAL);
+        double* out = mxGetPr(plhs[row]);
+        for (size_t i = 0; i < n_snr; ++i)
+            out[i] = row == 2 ? (double)used[i] : bt[i] ? (double)be[row * n_snr + i] / (double)bt[i] : 0.0;
+    }
+}
+
 // H = wofdm_mex('window_hessian', typeOFDM, numSubcar, cpLength, tailTx, tailRx, channel)
 //   -- the quadratic form of the interference power (ICI + ISI) in the REDUCED window variables (tail coefficients), as
 //      python's OptimizerTx/Rx/TxRx.gen_hessian builds it.  channel: ONE impulse response.  (quad_objective_tx / _rx of
@@ -427,7 +470,7 @@ static void do_calculate_interference(int nlhs, mxArray* plhs[], int nrhs, const
 extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     char cmd[32];
     if (nrhs < 1 || !mxIsChar(prhs[0]) || mxGetString(prhs[0], cmd, sizeof(cmd)))
-        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_simulation_adaptive', 'run_sim_mc', 'run_sim_mc_per_subcarrier', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
+        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_simulation_adaptive', 'run_sim_mc', 'run_sim_mc_per_subcarrier', 'run_sim_mc_adaptive', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
     if (!strcmp(cmd, "run_simulation")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_simulation_sweep")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, true);
     else if (!strcmp(cmd, "run_simulation_sweep_multi")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, false);
@@ -435,6 +478,7 @@ extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* 
     else if (!strcmp(cmd, "run_simulation_adaptive")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, false, true);
     else if (!strcmp(cmd, "run_sim_mc")) do_run_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_sim_mc_per_subcarrier")) do_run_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1, true);
+    else if (!strcmp(cmd, "run_sim_mc_adaptive")) do_run_sim_mc_adaptive(nlhs, plhs, nrhs - 1, prhs + 1);
     else if (!strcmp(cmd, "window_hessian")) do_window_hessian(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "quad_objective_tx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, true, false);
     else if (!strcmp(cmd, "quad_objective_rx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, false, false);

@@ -111,6 +111,12 @@ SIGNATURES = {
                                              C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_int, _i64p, _i64p, _i64p, _i64p]),
     "wofdm_ber_run_masked_resolved": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
                                                 C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_int, C.c_int, _i64p, _i64p, _i64p]),
+    "wofdm_ber_run_masked_segments": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
+                                                _i64p, C.c_int, C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_int, C.c_int,
+                                                _i64p, _i64p, _i64p]),
+    "wofdm_ber_run_masked_adaptive": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
+                                                C.c_int64, C.c_int, C.c_int64, C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_int,
+                                                REDUCE_FN, C.c_void_p, _i64p, _i64p, _i64p, _i64p, _i64p, _P(C.c_int)]),
     "wofdm_window_hessian": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, _dp, _P(C.c_int)]),
     "wofdm_window_hessian_parts": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, _dp, C.c_int, _dp, C.c_int, _dp, _dp]),
     "wofdm_window_hessian_set": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, C.c_int, _dp, _P(C.c_int)]),
@@ -393,6 +399,55 @@ class Handle:
                                                   _ptr(be, _i64p), _ptr(se, _i64p), _ptr(st, _i64p))
         self._check(rc)
         return dict(bit_err=be, sym_err=se, sym_tot=st, bit_tot=st * int(s.bits))
+
+    def ber_run_masked_segments(self, s, win_tx, win_rx, chan, snr_db, ensemble_max, segments, seed=0, variant=0, roll_off=10,
+                                shard=(0, 1), by_subcarrier=False, by_channel=False):
+        """A chosen subset of a masked job's frames (wofdm_ber_run_masked_segments).  segments: (n_seg, 3) {snr_idx, e_begin,
+        e_count}, as in ber_run_segments; frames and draws are those of ber_run_masked(..., ensemble=ensemble_max).
+        shard=(k, W): the k-th of W contiguous blocks of the local indices.  Unresolved: bit_err / sym_err / sym_tot / bit_tot
+        (n_snr,); resolved: the (n_snr, Cr, Nr) shapes of ber_run_masked_resolved."""
+        wt, wr, chf, L, Cn = self._win_chan(s, win_tx, win_rx, chan)
+        snr = _f64(np.ravel(snr_db))
+        n = snr.size
+        seg = np.ascontiguousarray(np.asarray(segments, dtype=np.int64).reshape(-1, 3))
+        resolve = (WOFDM_BY_SUBCARRIER if by_subcarrier else 0) | (WOFDM_BY_CHANNEL if by_channel else 0)
+        shape = (n, Cn if by_channel else 1, s.N if by_subcarrier else 1) if resolve else (n,)
+        be, se, st = (np.zeros(shape, dtype=np.int64) for _ in range(3))
+        rc = load().wofdm_ber_run_masked_segments(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), _ptr(chf, _dp), L, Cn,
+                                                  _ptr(snr, _dp), n, int(ensemble_max), _ptr(seg, _i64p), seg.shape[0],
+                                                  int(seed), int(variant), int(roll_off), int(shard[0]), int(shard[1]),
+                                                  int(resolve), _ptr(be, _i64p), _ptr(se, _i64p), _ptr(st, _i64p))
+        self._check(rc)
+        return dict(bit_err=be, sym_err=se, sym_tot=st, bit_tot=st * int(s.bits))
+
+    def ber_run_masked_adaptive(self, s, win_tx, win_rx, chan, snr_db, ensemble_max, target_bit_errors=None,
+                                target_symbol_errors=None, first_block=1, seed=0, variant=0, roll_off=10, shard=(0, 1),
+                                reduce=None):
+        """run_sim_mc with the stopping rule (wofdm_ber_run_masked_adaptive): the masked chain (row 0, noise stream
+        variant + 1) and the unmasked chain (row 1, noise stream variant) on the same frames, every SNR point run until both
+        rows reach the target or ensemble_max ensemble indices.  Exactly one of target_bit_errors / target_symbol_errors.
+        reduce: as in ber_run_adaptive, on int64 counts of shape (2, n_snr, 2).  Returns bit_err / sym_err (2, n_snr),
+        bit_tot / sym_tot (n_snr,), ensemble_used (n_snr,) and rounds."""
+        if (target_bit_errors is None) == (target_symbol_errors is None):
+            raise WofdmError(EINVAL, "give exactly one of target_bit_errors / target_symbol_errors")
+        kind, target = ((WOFDM_TARGET_BIT_ERRORS, target_bit_errors) if target_bit_errors is not None
+                        else (WOFDM_TARGET_SYMBOL_ERRORS, target_symbol_errors))
+        wt, wr, chf, L, Cn = self._win_chan(s, win_tx, win_rx, chan)
+        snr = _f64(np.ravel(snr_db))
+        n = snr.size
+        be, se = np.zeros((2, n), dtype=np.int64), np.zeros((2, n), dtype=np.int64)
+        bt, st, used = (np.zeros(n, dtype=np.int64) for _ in range(3))
+        rounds = C.c_int(0)
+        cb = reduce_trampoline(reduce, (2, n, 2)) if reduce is not None else REDUCE_FN()
+        rc = load().wofdm_ber_run_masked_adaptive(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), _ptr(chf, _dp), L, Cn,
+                                                  _ptr(snr, _dp), n, int(ensemble_max), int(first_block), kind, int(target),
+                                                  int(seed), int(variant), int(roll_off), int(shard[0]), int(shard[1]), cb, None,
+                                                  _ptr(used, _i64p), _ptr(be, _i64p), _ptr(bt, _i64p), _ptr(se, _i64p),
+                                                  _ptr(st, _i64p), C.byref(rounds))
+        if reduce is not None and cb.error is not None and rc:
+            raise WofdmError(rc, f"reduce callback raised {cb.error!r}") from cb.error
+        self._check(rc)
+        return dict(bit_err=be, bit_tot=bt, sym_err=se, sym_tot=st, ensemble_used=used, rounds=rounds.value)
 
     def psd_estimate(self, N, cp, cs, tail_tx, win_tx, guard_band=48, n_sym=256, records=1, seed=0, sym_idx=None,
                      bits=4, constellation=0):

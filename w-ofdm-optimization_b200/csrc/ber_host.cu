@@ -730,6 +730,46 @@ void seg_table(const int64_t* seg, int n_seg, int C, std::vector<long long>& tab
     *n_local = g;
 }
 
+// segments[n_seg][3] of a job: inside [0, n_snr) x [0, ensemble_max), e_count >= 1, no two segments of one point overlap
+int check_segments(wofdm_handle h, const int64_t* segments, int n_seg, int n_snr, int64_t ensemble_max) {
+    if (!segments || n_seg < 1) return fail(h, WOFDM_EINVAL, "segments must be a non-empty list");
+    std::vector<std::pair<int64_t, int64_t>> iv((size_t)n_seg);
+    for (int k = 0; k < n_seg; ++k) {
+        const int64_t si = segments[3 * k], e0 = segments[3 * k + 1], ec = segments[3 * k + 2];
+        if (si < 0 || si >= n_snr || e0 < 0 || e0 >= ensemble_max || ec < 1 || ec > ensemble_max - e0)
+            return fail(h, WOFDM_EINVAL, "segment outside [0, n_snr) x [0, ensemble_max) or with e_count < 1");
+        iv[k] = {si * ensemble_max + e0, ec};       // (< n_snr * ensemble_max: no overflow, checked by the caller)
+    }
+    std::sort(iv.begin(), iv.end());
+    for (int k = 1; k < n_seg; ++k)
+        if (iv[k].first < iv[k - 1].first + iv[k - 1].second) return fail(h, WOFDM_EINVAL, "overlapping segments of one SNR point");
+    return WOFDM_OK;
+}
+
+// the stopping rule's own arguments (wofdm_ber_run_adaptive / wofdm_ber_run_masked_adaptive)
+int check_target(wofdm_handle h, int target_kind, int64_t target, int64_t first_block, int shard_count, wofdm_reduce_fn reduce) {
+    if (target_kind != WOFDM_TARGET_BIT_ERRORS && target_kind != WOFDM_TARGET_SYMBOL_ERRORS) return fail(h, WOFDM_EINVAL, "unknown target_kind");
+    if (target < 1) return fail(h, WOFDM_EINVAL, "target must be >= 1");
+    if (first_block < 1) return fail(h, WOFDM_EINVAL, "first_block must be >= 1");
+    if (shard_count > 1 && !reduce) return fail(h, WOFDM_EINVAL, "shard_count > 1 needs a reduce callback (the schedule needs the job's counts)");
+    return WOFDM_OK;
+}
+
+// The schedule of include/wofdm.h for one point after a round that ran *block more ensemble indices of it: m = its fewest
+// cumulative errors over the rows.  Returns true when the point is done; else *block is its next block.
+bool schedule_step(int64_t m, int64_t target, int64_t ensemble_max, int64_t* used, int64_t* block) {
+    *used += *block;
+    if (m >= target || *used == ensemble_max) return true;
+    // min(ensemble_max - e, 2b, m > 0 ? max(1, ceil((target - m) * e / m)) : 2b), exact in 128 bits, saturating
+    __int128 nb = std::min<__int128>((__int128)ensemble_max - *used, (__int128)2 * *block);
+    if (m > 0) {
+        const __int128 need = ((__int128)(target - m) * *used + m - 1) / m;
+        nb = std::min(nb, std::max<__int128>(1, need));
+    }
+    *block = (int64_t)nb;
+    return false;
+}
+
 // one launch of a twin plan over the segment table on every device of the handle (devices split this shard's local
 // indices as wofdm_ber_run_multi splits frame ids), then the summed counters
 int run_segment_table(wofdm_ber_plan p, const std::vector<long long>& tab, long long n_local, int64_t ensemble_max,
@@ -765,19 +805,8 @@ int wofdm_ber_run_segments(wofdm_handle h, const wofdm_sys_t* sys, const double*
     if (!bit_err || !sym_err || !sym_tot) return fail(h, WOFDM_EINVAL, "NULL output buffer");
     int rc = check_job(h, sys, L, C, n_snr, n_var, ensemble_max, shard_index, shard_count);
     if (rc) return rc;
-    if (!segments || n_seg < 1) return fail(h, WOFDM_EINVAL, "segments must be a non-empty list");
-    {   // inside [0, n_snr) x [0, ensemble_max), no two segments of one point overlap
-        std::vector<std::pair<int64_t, int64_t>> iv((size_t)n_seg);
-        for (int k = 0; k < n_seg; ++k) {
-            const int64_t si = segments[3 * k], e0 = segments[3 * k + 1], ec = segments[3 * k + 2];
-            if (si < 0 || si >= n_snr || e0 < 0 || e0 >= ensemble_max || ec < 1 || ec > ensemble_max - e0)
-                return fail(h, WOFDM_EINVAL, "segment outside [0, n_snr) x [0, ensemble_max) or with e_count < 1");
-            iv[k] = {si * ensemble_max + e0, ec};       // (< n_snr * ensemble_max: no overflow, checked above)
-        }
-        std::sort(iv.begin(), iv.end());
-        for (int k = 1; k < n_seg; ++k)
-            if (iv[k].first < iv[k - 1].first + iv[k - 1].second) return fail(h, WOFDM_EINVAL, "overlapping segments of one SNR point");
-    }
+    rc = check_segments(h, segments, n_seg, n_snr, ensemble_max);
+    if (rc) return rc;
     const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? sys->N : 1;
     size_t cells = 0, n_out = 0, dev_bytes = 0;
     if (__builtin_mul_overflow((size_t)n_snr, (size_t)Cr, &cells) || __builtin_mul_overflow(cells, (size_t)Nr, &cells) ||
@@ -824,10 +853,8 @@ int wofdm_ber_run_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const double*
     if (!ensemble_used || !bit_err || !bit_tot || !sym_err || !sym_tot || !rounds) return fail(h, WOFDM_EINVAL, "NULL output buffer");
     int rc = check_job(h, sys, L, C, n_snr, n_var, ensemble_max, shard_index, shard_count);
     if (rc) return rc;
-    if (target_kind != WOFDM_TARGET_BIT_ERRORS && target_kind != WOFDM_TARGET_SYMBOL_ERRORS) return fail(h, WOFDM_EINVAL, "unknown target_kind");
-    if (target < 1) return fail(h, WOFDM_EINVAL, "target must be >= 1");
-    if (first_block < 1) return fail(h, WOFDM_EINVAL, "first_block must be >= 1");
-    if (shard_count > 1 && !reduce) return fail(h, WOFDM_EINVAL, "shard_count > 1 needs a reduce callback (the schedule needs the job's counts)");
+    rc = check_target(h, target_kind, target, first_block, shard_count, reduce);
+    if (rc) return rc;
     wofdm_ber_plan p = nullptr;
     rc = plan_create_impl(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, &p, true, 0, n_snr);
     if (rc) return rc;
@@ -856,17 +883,9 @@ int wofdm_ber_run_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const double*
         for (size_t k = 0; k < nv * ns; ++k) { tbit[k] += red[2 * k]; tsym[k] += red[2 * k + 1]; }
         for (size_t s = 0; s < ns; ++s) {
             if (done[s]) continue;
-            used[s] += block[s];
             int64_t m = INT64_MAX;                      // the fewest errors over the window pairs
             for (size_t v = 0; v < nv; ++v) m = std::min(m, target_kind == WOFDM_TARGET_BIT_ERRORS ? tbit[v * ns + s] : tsym[v * ns + s]);
-            if (m >= target || used[s] == ensemble_max) { done[s] = 1; continue; }
-            // min(ensemble_max - e, 2b, m > 0 ? max(1, ceil((target - m) * e / m)) : 2b), exact in 128 bits, saturating
-            __int128 nb = std::min<__int128>((__int128)ensemble_max - used[s], (__int128)2 * block[s]);
-            if (m > 0) {
-                const __int128 need = ((__int128)(target - m) * used[s] + m - 1) / m;
-                nb = std::min(nb, std::max<__int128>(1, need));
-            }
-            block[s] = (int64_t)nb;
+            done[s] = schedule_step(m, target, ensemble_max, &used[s], &block[s]);
         }
     }
     wofdm_ber_plan_destroy(p);
@@ -1054,22 +1073,47 @@ static void host_fft_pow2(std::vector<double>& a, int n) {
     }
 }
 
+}  // extern "C"
+
 // Channel-mask variant (include/wofdm.h): frames in batches -- the masked Tx streams of a batch are written to HBM (the dense
 // tensor-core product of mask_gemm.cu, or tx_mask_kernel with WOFDM_MASK_FFT=1), a K1 kernel reads them
 // (BerParams::tx_stream) and does channel, noise, Rx and counting as always.
-// The frames [*f_lo, *f_hi) of shard (shard_index, shard_count), a contiguous block of global frame ids.  resolve == 0:
-// bit_err / sym_err [n_snr]; else [n_snr][Cr][Nr] (wofdm_ber_run_resolved's layout, one window pair), counted by the
-// resolved twin of the K1 kernel this chain picks.  outputs_ok: the caller's output pointers are all non-NULL.
-static int run_masked_impl(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
-                           const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
-                           uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count, int resolve,
-                           bool outputs_ok, int64_t* bit_err, int64_t* sym_err, long long* f_lo_out, long long* f_hi_out) {
+// A call is set up once (masked_setup: kernels, tables, device buffers, the mask product's matrix) and then runs ranges of
+// frames (masked_run): global frame ids, or local indices of a segment table (wofdm_ber_run_masked_segments / _adaptive).
+namespace {
+
+struct MaskedDev {
+    int slot = 0;                          // device of the handle
+    MaskGemm mg{};
+    MaskParams mp{};
+    BerParams prm{};
+    unsigned long long* d_cnt = nullptr;   // counter pairs [n_snr][Cr][Nr]
+    void* d_stream = nullptr;
+    long long* d_seg = nullptr;            // segment table [seg_cap][4]
+};
+
+struct MaskedJob {
+    wofdm_ctx* h = nullptr;
+    wofdm_sys_t sys{};
+    Choice run;                            // the K1 kernel that runs
+    bool use_gemm = false, fused = false;
+    const char* dump_env = nullptr;
+    long long max_ctas = 0, batch = 0, ensemble = 0;
+    size_t ncnt = 0, cnt_bytes = 0, body = 0;
+    int C = 0, seg_cap = 0;
+    std::vector<MaskedDev> devs;           // the devices set up: the first ones of the handle
+};
+
+// what every channel-mask entry point rejects; ensemble: the job's (ensemble_max of a segment call)
+int masked_check(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, const double* chan, int L,
+                 int C, const double* snr_db, int n_snr, int64_t ensemble, int roll_off, int shard_index, int shard_count,
+                 int resolve, bool outputs_ok) {
     int rc = validate_sys(h, sys, L);
     if (rc) return rc;
     if (!win_tx || !win_rx || !chan || !snr_db || !outputs_ok) return fail(h, WOFDM_EINVAL, "NULL buffer");
     if (C < 1 || n_snr < 1 || ensemble < 1) return fail(h, WOFDM_EINVAL, "C, n_snr and ensemble must be >= 1");
     if (sys->precision != 0) return fail(h, WOFDM_EUNSUPPORTED, "the channel-mask variant runs in fp32");
-    const int N = sys->N, n_tx = N + sys->cp + sys->cs, stride = n_tx - sys->tail_tx, M = 2 * n_tx - 1;
+    const int N = sys->N, n_tx = N + sys->cp + sys->cs, M = 2 * n_tx - 1;
     if (N != 128 && N != 256 && N != 512) return fail(h, WOFDM_EUNSUPPORTED, "the channel-mask variant is built for N = 128, 256, 512");
     if (roll_off < 1 || M / 2 + 2 * roll_off > M) return fail(h, WOFDM_EINVAL, "roll_off does not fit the mask");
     if (2 * n_tx > 3 * N + 1) return fail(h, WOFDM_EUNSUPPORTED, "cp + cs too long for the mask kernel (n_tx <= 1.5 N)");
@@ -1083,43 +1127,59 @@ static int run_masked_impl(wofdm_handle h, const wofdm_sys_t* sys, const double*
     if (__builtin_mul_overflow((size_t)n_snr, (size_t)Cr, &ncnt) || __builtin_mul_overflow(ncnt, (size_t)Nr, &ncnt) ||
         __builtin_mul_overflow(ncnt, (size_t)16, &cnt_bytes) || ncnt > (size_t)INT64_MAX / 16)
         return fail(h, WOFDM_EINVAL, "resolved counter array too large");
+    return WOFDM_OK;
+}
+
+// Set-up of a checked channel-mask call: the kernels, the tables, and on every device that takes part (contiguous ranges
+// of at least 64 frames out of max_frames, the most frames one masked_run covers) its buffers and the mask product's
+// matrix.  resolve != 0 or seg_cap > 0: the resolved twin of the K1 kernel (counters [n_snr][Cr][Nr], [n_snr] with
+// resolve 0); seg_cap > 0 also gives every device a segment table of seg_cap entries.
+int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                 const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble, uint64_t seed,
+                 uint32_t variant, int roll_off, int resolve, long long max_frames, int seg_cap) {
+    const int N = sys->N, n_tx = N + sys->cp + sys->cs, stride = n_tx - sys->tail_tx, M = 2 * n_tx - 1;
+    J.h = h; J.sys = *sys; J.C = C; J.ensemble = ensemble; J.seg_cap = seg_cap;
+    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? N : 1;
+    J.ncnt = (size_t)n_snr * Cr * Nr;
+    J.cnt_bytes = J.ncnt * 16;
     DeviceCtx& d0 = h->devs[0];              // (variant selection: the devices of a handle are alike)
     WOFDM_CUDA(h, cudaSetDevice(d0.dev));
     Choice ch, prod;
     // Tx side: the dense tensor-core product of mask_gemm.cu; WOFDM_MASK_FFT=1 keeps the per-symbol FFT kernel (mask_kernel.cuh)
     const char* mask_env = getenv("WOFDM_MASK_FFT");
-    const bool use_gemm = !(mask_env && atoi(mask_env) == 1);
-    const char* dump_env = getenv("WOFDM_MASK_DUMP");
+    J.use_gemm = !(mask_env && atoi(mask_env) == 1);
+    J.dump_env = seg_cap > 0 ? nullptr : getenv("WOFDM_MASK_DUMP");     // (a development aid of the unsegmented calls)
     // a second-generation tensor-core kernel that gathers its stream from the product's output itself (no assembled copy in
     // HBM) where the frame fits one, else a tx_stream kernel (tuned or staged)
-    bool fused = false;
-    if (use_gemm && !(dump_env && *dump_env)) {
+    int rc = WOFDM_OK;
+    if (J.use_gemm && !(J.dump_env && *J.dump_env)) {
         rc = choose_variant(h, *sys, L, false, false, d0.smem_optin, &ch, nullptr, true, true, false, 1, true);
-        fused = rc == WOFDM_OK && ch.var->txy;
+        J.fused = rc == WOFDM_OK && ch.var->txy;
     }
-    if (!fused) rc = choose_variant(h, *sys, L, false, false, d0.smem_optin, &ch, nullptr, true, true);
+    if (!J.fused) rc = choose_variant(h, *sys, L, false, false, d0.smem_optin, &ch, nullptr, true, true);
     if (rc) return rc;
     if (ch.var->CL > 1) return fail(h, WOFDM_EUNSUPPORTED, "no channel-mask variant for cluster kernels");
     rc = choose_variant(h, *sys, L, false, false, d0.smem_optin, &prod, win_tx);     // noise numbering of wofdm_ber_run / _draws
     if (rc) return rc;
     if (prod.var->CL > 1) return fail(h, WOFDM_EUNSUPPORTED, "no channel-mask variant for cluster kernels");
-    // the kernel that runs: ch, or (resolved counters) its twin -- the noise numbering below stays ch's either way, so a
-    // staged fallback draws ch's noise; it reads the assembled stream even where ch gathers from the product itself
-    Choice run = ch;
-    if (resolve) {
+    // the kernel that runs: ch, or (resolved counters, segments) its twin -- the noise numbering below stays ch's either way,
+    // so a staged fallback draws ch's noise; it reads the assembled stream even where ch gathers from the product itself
+    J.run = ch;
+    if (resolve || seg_cap > 0) {
         Choice nz = ch;
         if (ch.var->TC == 0) nz.chunk = prod.chunk;
         bool rfused = false;
-        rc = choose_resolved(h, *sys, L, d0.smem_optin, nz, false, 1, &run, &rfused);
+        rc = choose_resolved(h, *sys, L, d0.smem_optin, nz, false, 1, &J.run, &rfused);
         if (rc) return rc;
-        fused = run.var->txy;
+        J.fused = J.run.var->txy;
     }
+    const Choice& run = J.run;
     int nb = 0;
-    long long max_ctas = 0;
-    rc = prepare_kernel(h, *run.var, run.lay.bytes, d0.sm_count, &nb, &max_ctas);
+    rc = prepare_kernel(h, *run.var, run.lay.bytes, d0.sm_count, &nb, &J.max_ctas);
     if (rc) return rc;
+    if (max_frames == 0) return WOFDM_OK;
     std::vector<double> gd;
-    if (!use_gemm) {
+    if (!J.use_gemm) {
         // g = IDFT_M(ifftshift(windowRC)), main_channel_mask.m:404-412, 477-493
         std::vector<double> wrc(M, 0.0);
         {
@@ -1155,7 +1215,7 @@ static int run_masked_impl(wofdm_handle h, const wofdm_sys_t* sys, const double*
     const int P = 8 * N;
     std::vector<float> g(2 * (size_t)P, 0.f);
     std::vector<unsigned char> twp;
-    if (!use_gemm) {
+    if (!J.use_gemm) {
         std::vector<double> gc(2 * (size_t)P, 0.0);
         for (int mm = -(n_tx - 1); mm <= M - 1; ++mm) {
             const int gi = ((mm % M) + M) % M, ci = ((mm % P) + P) % P;
@@ -1174,150 +1234,228 @@ static int run_masked_impl(wofdm_handle h, const wofdm_sys_t* sys, const double*
     std::vector<double> lin(n_snr);
     for (int i = 0; i < n_snr; ++i) lin[i] = std::pow(10.0, -0.1 * snr_db[i]);
     cast_any(false, lin, hsnr);
-    // this shard's block of frame ids [f_lo, f_hi); batches and devices take contiguous ranges of it
-    const long long f_lo = (long long)((__int128)total * shard_index / shard_count);
-    const long long f_hi = (long long)((__int128)total * (shard_index + 1) / shard_count), nfr = f_hi - f_lo;
-    *f_lo_out = f_lo; *f_hi_out = f_hi;
-    if (nfr == 0) {
-        for (size_t i = 0; i < ncnt; ++i) { bit_err[i] = 0; sym_err[i] = 0; }
-        return WOFDM_OK;
-    }
-    const size_t body = (size_t)sys->tail_tx + (size_t)sys->S * stride;
-    const long long batch = std::min<long long>(nfr, use_gemm ? 16384 : 8192);
-    const size_t scratch_elems = (size_t)run.lay.pad + body + 64;
-    const int grid_ber = (int)std::min<long long>(batch, max_ctas);
+    J.body = (size_t)sys->tail_tx + (size_t)sys->S * stride;
+    J.batch = std::min<long long>(max_frames, J.use_gemm ? 16384 : 8192);
+    const size_t scratch_elems = (size_t)run.lay.pad + J.body + 64;
+    const int grid_ber = (int)std::min<long long>(J.batch, J.max_ctas);
     const size_t scratch_bytes = run.use_global ? (size_t)grid_ber * 2 * scratch_elems * sizeof(float2) : 0;
     // every device of the handle takes a contiguous range of the frames (frame ids are global: same draws, same counters as
     // on one device); its work is enqueued on its own stream, the counters meet on the host
-    const int nd = (int)std::min<long long>((long long)h->devs.size(), std::max<long long>(1, nfr / 64));
-    std::vector<std::vector<unsigned long long>> cnts;     // (allocated once the device buffers exist)
-    std::vector<void*> d_cnts(nd, nullptr);
-    auto run_dev = [&](DeviceCtx& d, long long f_lo, long long f_hi, void** d_cnt_out) -> int {
-    WOFDM_CUDA(h, cudaSetDevice(d.dev));
-    if (&d != &d0) {
-        int nb_ = 0; long long mc_ = 0;
-        const int rcp = prepare_kernel(h, *run.var, run.lay.bytes, d.sm_count, &nb_, &mc_);
-        if (rcp) return rcp;
-    }
-    MaskGemm mg;
-    const size_t mg_bytes = use_gemm ? mask_gemm_plan(*sys, batch, mg) : 0;
-    int rc = arena_reserve(h, d, t.wtx.size() + t.wrx.size() + t.tw.size() + twp.size() + hchan.size() + hsnr.size() + g.size() * 4 +
-                                 cnt_bytes + (fused ? 16 : (size_t)batch * body * sizeof(float2)) + scratch_bytes + mg_bytes + 8192);
-    if (rc) return rc;
-    auto put = [&](const void* src, size_t bytes, void** dst) -> cudaError_t {
-        *dst = arena_take(d, std::max<size_t>(bytes, 16));
-        if (!*dst) return cudaErrorMemoryAllocation;
-        return src ? cudaMemcpyAsync(*dst, src, bytes, cudaMemcpyHostToDevice, d.stream) : cudaSuccess;
-    };
-    void *d_wtx, *d_wrx, *d_tw, *d_twp, *d_chan, *d_snr, *d_g, *d_cnt, *d_stream, *d_scr = nullptr;
-    WOFDM_CUDA(h, put(t.wtx.data(), t.wtx.size(), &d_wtx));
-    WOFDM_CUDA(h, put(t.wrx.data(), t.wrx.size(), &d_wrx));
-    WOFDM_CUDA(h, put(t.tw.data(), t.tw.size(), &d_tw));
-    WOFDM_CUDA(h, put(hchan.data(), hchan.size(), &d_chan));
-    WOFDM_CUDA(h, put(hsnr.data(), hsnr.size(), &d_snr));
-    WOFDM_CUDA(h, put(g.data(), g.size() * 4, &d_g));
-    WOFDM_CUDA(h, put(twp.data(), twp.size(), &d_twp));
-    WOFDM_CUDA(h, put(nullptr, cnt_bytes, &d_cnt));
-    WOFDM_CUDA(h, put(nullptr, fused ? 16 : (size_t)batch * body * sizeof(float2), &d_stream));
-    if (scratch_bytes) WOFDM_CUDA(h, put(nullptr, scratch_bytes, &d_scr));
-    WOFDM_CUDA(h, cudaMemsetAsync(d_cnt, 0, cnt_bytes, d.stream));
-    if (use_gemm) {
-        rc = mask_gemm_setup(h, d, mg, roll_off, static_cast<const float*>(d_wtx));
+    const int nd = (int)std::min<long long>((long long)h->devs.size(), std::max<long long>(1, max_frames / 64));
+    auto setup_dev = [&](MaskedDev& md) -> int {
+        DeviceCtx& d = h->devs[md.slot];
+        WOFDM_CUDA(h, cudaSetDevice(d.dev));
+        if (&d != &d0) {
+            int nb_ = 0; long long mc_ = 0;
+            const int rcp = prepare_kernel(h, *run.var, run.lay.bytes, d.sm_count, &nb_, &mc_);
+            if (rcp) return rcp;
+        }
+        const size_t mg_bytes = J.use_gemm ? mask_gemm_plan(*sys, J.batch, md.mg) : 0;
+        const size_t stream_bytes = J.fused ? 16 : (size_t)J.batch * J.body * sizeof(float2);
+        int rc = arena_reserve(h, d, t.wtx.size() + t.wrx.size() + t.tw.size() + twp.size() + hchan.size() + hsnr.size() + g.size() * 4 +
+                                     J.cnt_bytes + stream_bytes + scratch_bytes + mg_bytes + (size_t)seg_cap * 32 + 8192);
         if (rc) return rc;
-    }
-
-    MaskParams mp;
-    memset(&mp, 0, sizeof(mp));
-    mp.N = N; mp.cp = sys->cp; mp.cs = sys->cs; mp.tail_tx = sys->tail_tx; mp.bits = sys->bits; mp.S = sys->S;
-    mp.n_tx = n_tx; mp.stride = stride; mp.constellation = sys->constellation; mp.guard = sys->guard; mp.M = M;
-    mp.win_tx = static_cast<const float*>(d_wtx); mp.tw = static_cast<const float2*>(d_tw);
-    mp.Gp = static_cast<const float2*>(d_g); mp.twp = static_cast<const float2*>(d_twp);
-    mp.seed = seed; mp.stream = static_cast<float2*>(d_stream);
-    BerParams prm;
-    fill_sys(prm, *sys, L);
-    prm.chunk = ch.var->TC > 0 ? ch.chunk : prod.chunk; prm.use_global = run.use_global;
-    fill_flat(prm, *sys, win_tx, win_rx);
-    prm.flat_tx = 0;                       // (the Tx stream comes from tx_mask_kernel)
-    fill_split(prm, *ch.var);
-    if (ch.var->TC == 0) {                 // staged kernel: the noise numbering of wofdm_ber_run / _draws (noise_at follows it)
-        BerParams tmp = prm;
-        fill_split(tmp, *prod.var);
-        prm.n48 = tmp.n48;
-    }
-    prm.win_tx = d_wtx; prm.win_rx = d_wrx; prm.tw = d_tw; prm.chan = d_chan; prm.snr_lin = d_snr;
-    prm.C = C; prm.n_snr = n_snr; prm.ensemble = ensemble; prm.seed = seed; prm.variant = variant;
-    philox_round_keys(seed, prm.rk);
-    prm.counters = static_cast<unsigned long long*>(d_cnt);
-    prm.res_chan = (resolve & WOFDM_BY_CHANNEL) ? 1 : 0;
-    prm.res_bins = (resolve & WOFDM_BY_SUBCARRIER) ? 1 : 0;
-    prm.scratch = d_scr; prm.scratch_elems = (long long)scratch_elems;
-    prm.tx_stream = static_cast<const float2*>(d_stream);
-    if (fused) { prm.tx_y = mg.Y; prm.tx_yp = mg.Yp; }
-    size_t msm = 0;
-    for (long long f0 = f_lo; f0 < f_hi; f0 += batch) {
-        const long long nf = std::min(batch, f_hi - f0);
-        mp.frame_begin = f0; mp.frame_step = 1; mp.n_frames = nf;
-        const int mgrid = (int)std::min<long long>(nf, (long long)d.sm_count);
-        cudaError_t e = cudaSuccess;
-        if (use_gemm) {
-            rc = mask_gemm_batch(h, d, mg, seed, f0, nf, fused ? nullptr : static_cast<float2*>(d_stream));
+        auto put = [&](const void* src, size_t bytes, void** dst) -> cudaError_t {
+            *dst = arena_take(d, std::max<size_t>(bytes, 16));
+            if (!*dst) return cudaErrorMemoryAllocation;
+            return src ? cudaMemcpyAsync(*dst, src, bytes, cudaMemcpyHostToDevice, d.stream) : cudaSuccess;
+        };
+        void *d_wtx, *d_wrx, *d_tw, *d_twp, *d_chan, *d_snr, *d_g, *d_cnt, *d_seg = nullptr, *d_scr = nullptr;
+        WOFDM_CUDA(h, put(t.wtx.data(), t.wtx.size(), &d_wtx));
+        WOFDM_CUDA(h, put(t.wrx.data(), t.wrx.size(), &d_wrx));
+        WOFDM_CUDA(h, put(t.tw.data(), t.tw.size(), &d_tw));
+        WOFDM_CUDA(h, put(hchan.data(), hchan.size(), &d_chan));
+        WOFDM_CUDA(h, put(hsnr.data(), hsnr.size(), &d_snr));
+        WOFDM_CUDA(h, put(g.data(), g.size() * 4, &d_g));
+        WOFDM_CUDA(h, put(twp.data(), twp.size(), &d_twp));
+        WOFDM_CUDA(h, put(nullptr, J.cnt_bytes, &d_cnt));
+        WOFDM_CUDA(h, put(nullptr, stream_bytes, &md.d_stream));
+        if (scratch_bytes) WOFDM_CUDA(h, put(nullptr, scratch_bytes, &d_scr));
+        if (seg_cap > 0) WOFDM_CUDA(h, put(nullptr, (size_t)seg_cap * 32, &d_seg));
+        md.d_cnt = static_cast<unsigned long long*>(d_cnt);
+        md.d_seg = static_cast<long long*>(d_seg);
+        if (J.use_gemm) {
+            rc = mask_gemm_setup(h, d, md.mg, roll_off, static_cast<const float*>(d_wtx));
             if (rc) return rc;
-        } else
-        switch (N) {
-            case 128: msm = MaskSmem<128>::bytes(sys->S, stride, sys->tail_tx);
-                      e = cudaFuncSetAttribute(tx_mask_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm);
-                      if (e == cudaSuccess) tx_mask_kernel<128><<<mgrid, 256, msm, d.stream>>>(mp); break;
-            case 256: msm = MaskSmem<256>::bytes(sys->S, stride, sys->tail_tx);
-                      e = cudaFuncSetAttribute(tx_mask_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm);
-                      if (e == cudaSuccess) tx_mask_kernel<256><<<mgrid, 256, msm, d.stream>>>(mp); break;
-            default:  msm = MaskSmem<512>::bytes(sys->S, stride, sys->tail_tx);
-                      e = cudaFuncSetAttribute(tx_mask_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm);
-                      if (e == cudaSuccess) tx_mask_kernel<512><<<mgrid, 256, msm, d.stream>>>(mp); break;
         }
-        WOFDM_CUDA(h, e);
-        WOFDM_CUDA(h, cudaGetLastError());
-        if (f0 == 0) {
-            // development aid: WOFDM_MASK_DUMP=<file> writes the masked Tx streams of the first (up to 4) frames as raw float32 pairs
-            const char* dump = dump_env;
-            if (dump && *dump) {
-                std::vector<float> hs(2 * body * (size_t)std::min<long long>(nf, 4));
-                WOFDM_CUDA(h, cudaMemcpyAsync(hs.data(), d_stream, hs.size() * 4, cudaMemcpyDeviceToHost, d.stream));
-                WOFDM_CUDA(h, cudaStreamSynchronize(d.stream));
-                if (FILE* fp = fopen(dump, "wb")) { fwrite(hs.data(), 4, hs.size(), fp); fclose(fp); }
-            }
+        MaskParams& mp = md.mp;
+        memset(&mp, 0, sizeof(mp));
+        mp.N = N; mp.cp = sys->cp; mp.cs = sys->cs; mp.tail_tx = sys->tail_tx; mp.bits = sys->bits; mp.S = sys->S;
+        mp.n_tx = n_tx; mp.stride = stride; mp.constellation = sys->constellation; mp.guard = sys->guard; mp.M = M;
+        mp.win_tx = static_cast<const float*>(d_wtx); mp.tw = static_cast<const float2*>(d_tw);
+        mp.Gp = static_cast<const float2*>(d_g); mp.twp = static_cast<const float2*>(d_twp);
+        mp.seed = seed; mp.stream = static_cast<float2*>(md.d_stream);
+        BerParams& prm = md.prm;
+        fill_sys(prm, *sys, L);
+        prm.chunk = ch.var->TC > 0 ? ch.chunk : prod.chunk; prm.use_global = run.use_global;
+        fill_flat(prm, *sys, win_tx, win_rx);
+        prm.flat_tx = 0;                       // (the Tx stream comes from tx_mask_kernel)
+        fill_split(prm, *ch.var);
+        if (ch.var->TC == 0) {                 // staged kernel: the noise numbering of wofdm_ber_run / _draws (noise_at follows it)
+            BerParams tmp = prm;
+            fill_split(tmp, *prod.var);
+            prm.n48 = tmp.n48;
         }
-        prm.frame_begin = f0; prm.frame_step = 1; prm.n_frames = nf;
-        WOFDM_CUDA(h, run.var->launch(prm, (int)std::min<long long>(nf, max_ctas), run.lay.bytes, d.stream));
-        h->launches += 2;
+        prm.win_tx = d_wtx; prm.win_rx = d_wrx; prm.tw = d_tw; prm.chan = d_chan; prm.snr_lin = d_snr;
+        prm.C = C; prm.n_snr = n_snr; prm.ensemble = ensemble; prm.seed = seed; prm.variant = variant;
+        philox_round_keys(seed, prm.rk);
+        prm.counters = md.d_cnt;
+        prm.res_chan = (resolve & WOFDM_BY_CHANNEL) ? 1 : 0;
+        prm.res_bins = (resolve & WOFDM_BY_SUBCARRIER) ? 1 : 0;
+        prm.scratch = d_scr; prm.scratch_elems = (long long)scratch_elems;
+        prm.tx_stream = static_cast<const float2*>(md.d_stream);
+        if (J.fused) { prm.tx_y = md.mg.Y; prm.tx_yp = md.mg.Yp; }
+        return WOFDM_OK;
+    };
+    J.devs.resize(nd);
+    for (int i = 0; i < nd && rc == WOFDM_OK; ++i) {
+        J.devs[i].slot = i;
+        rc = setup_dev(J.devs[i]);
     }
-    *d_cnt_out = d_cnt;
-    return WOFDM_OK;
-    };   // run_dev
+    // (the host tables may go out of scope: uploads from pageable memory return once staged.  After a failure nothing of
+    //  this call stays in flight.)
+    if (rc)
+        for (int i = 0; i < nd; ++i) { cudaSetDevice(h->devs[i].dev); cudaStreamSynchronize(h->devs[i].stream); }
+    cudaSetDevice(d0.dev);
+    return rc;
+}
+
+// The frames [g_lo, g_hi) of a set-up call: global frame ids, or with `tab` (seg_table's layout, at most seg_cap entries,
+// uploaded to every device) local indices of that segment list.  The devices take contiguous ranges of at least 64.
+// -> bit_err / sym_err [n_snr][Cr][Nr]
+int masked_run(MaskedJob& J, long long g_lo, long long g_hi, const std::vector<long long>* tab, int64_t* bit_err, int64_t* sym_err) {
+    wofdm_ctx* h = J.h;
+    const wofdm_sys_t& sys = J.sys;
+    const int N = sys.N;
+    const long long nfr = g_hi - g_lo;
+    if (nfr == 0) {
+        for (size_t i = 0; i < J.ncnt; ++i) { bit_err[i] = 0; sym_err[i] = 0; }
+        return WOFDM_OK;
+    }
+    const int n_seg = tab ? (int)(tab->size() / 4) : 0;
+    if (n_seg > J.seg_cap) return fail(h, WOFDM_EINVAL, "more segments than the call's segment table holds");
+    const int nd = (int)std::min<long long>((long long)J.devs.size(), std::max<long long>(1, nfr / 64));
+    auto run_dev = [&](MaskedDev& md, long long f_lo, long long f_hi) -> int {
+        DeviceCtx& d = h->devs[md.slot];
+        WOFDM_CUDA(h, cudaSetDevice(d.dev));
+        const long long* seg = tab ? md.d_seg : nullptr;
+        // (pageable source: the copy returns once the table is staged; the previous work on this stream is ordered before it)
+        if (tab) WOFDM_CUDA(h, cudaMemcpyAsync(md.d_seg, tab->data(), tab->size() * sizeof(long long), cudaMemcpyHostToDevice, d.stream));
+        WOFDM_CUDA(h, cudaMemsetAsync(md.d_cnt, 0, J.cnt_bytes, d.stream));
+        MaskSegParams mp;
+        static_cast<MaskParams&>(mp) = md.mp;
+        mp.seg = seg; mp.n_seg = n_seg; mp.C = J.C; mp.ensemble = J.ensemble;
+        BerParams prm = md.prm;
+        prm.seg = seg; prm.n_seg = n_seg;
+        for (long long f0 = f_lo; f0 < f_hi; f0 += J.batch) {
+            const long long nf = std::min(J.batch, f_hi - f0);
+            mp.frame_begin = f0; mp.frame_step = 1; mp.n_frames = nf;
+            const int mgrid = (int)std::min<long long>(nf, (long long)d.sm_count);
+            cudaError_t e = cudaSuccess;
+            if (J.use_gemm) {
+                const int rc = mask_gemm_batch(h, d, md.mg, mp.seed, f0, nf, J.fused ? nullptr : static_cast<float2*>(md.d_stream),
+                                               seg, n_seg, J.C, J.ensemble);
+                if (rc) return rc;
+            } else {
+                // (SEG: the segmented instantiation, whose parameters carry the table)
+                auto launch = [&](auto kern_plain, auto kern_seg, size_t msm) {
+                    cudaError_t es = cudaFuncSetAttribute(seg ? (const void*)kern_seg : (const void*)kern_plain,
+                                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm);
+                    if (es == cudaSuccess && seg) kern_seg<<<mgrid, 256, msm, d.stream>>>(mp);
+                    else if (es == cudaSuccess) kern_plain<<<mgrid, 256, msm, d.stream>>>(static_cast<const MaskParams&>(mp));
+                    return es;
+                };
+                switch (N) {
+                    case 128: e = launch(tx_mask_kernel<128>, tx_mask_kernel<128, true>, MaskSmem<128>::bytes(sys.S, mp.stride, sys.tail_tx)); break;
+                    case 256: e = launch(tx_mask_kernel<256>, tx_mask_kernel<256, true>, MaskSmem<256>::bytes(sys.S, mp.stride, sys.tail_tx)); break;
+                    default:  e = launch(tx_mask_kernel<512>, tx_mask_kernel<512, true>, MaskSmem<512>::bytes(sys.S, mp.stride, sys.tail_tx)); break;
+                }
+            }
+            WOFDM_CUDA(h, e);
+            WOFDM_CUDA(h, cudaGetLastError());
+            if (f0 == 0 && !tab) {
+                // development aid: WOFDM_MASK_DUMP=<file> writes the masked Tx streams of the first (up to 4) frames as raw float32 pairs
+                const char* dump = J.dump_env;
+                if (dump && *dump) {
+                    std::vector<float> hs(2 * J.body * (size_t)std::min<long long>(nf, 4));
+                    WOFDM_CUDA(h, cudaMemcpyAsync(hs.data(), md.d_stream, hs.size() * 4, cudaMemcpyDeviceToHost, d.stream));
+                    WOFDM_CUDA(h, cudaStreamSynchronize(d.stream));
+                    if (FILE* fp = fopen(dump, "wb")) { fwrite(hs.data(), 4, hs.size(), fp); fclose(fp); }
+                }
+            }
+            prm.frame_begin = f0; prm.frame_step = 1; prm.n_frames = nf;
+            WOFDM_CUDA(h, J.run.var->launch(prm, (int)std::min<long long>(nf, J.max_ctas), J.run.lay.bytes, d.stream));
+            h->launches += 2;
+        }
+        return WOFDM_OK;
+    };
+    int rc = WOFDM_OK;
     for (int i = 0; i < nd; ++i) {
-        rc = run_dev(h->devs[i], f_lo + nfr * i / nd, f_lo + nfr * (i + 1) / nd, &d_cnts[i]);
+        rc = run_dev(J.devs[i], g_lo + nfr * i / nd, g_lo + nfr * (i + 1) / nd);
         if (rc) break;
     }
+    std::vector<std::vector<unsigned long long>> cnts;
     if (!rc) {
-        try { cnts.assign(nd, std::vector<unsigned long long>(ncnt * 2, 0ull)); }
+        try { cnts.assign(nd, std::vector<unsigned long long>(J.ncnt * 2, 0ull)); }
         catch (const std::bad_alloc&) { rc = fail(h, WOFDM_ENOMEM, "host allocation failed"); }
     }
     // (the downloads into pageable memory block the host: only after every device has its work)
     for (int i = 0; i < nd; ++i) {           // (also after a failure: nothing of this call stays in flight)
-        cudaSetDevice(h->devs[i].dev);
+        DeviceCtx& d = h->devs[J.devs[i].slot];
+        cudaSetDevice(d.dev);
         cudaError_t es = cudaSuccess;
-        if (!rc && d_cnts[i]) es = cudaMemcpyAsync(cnts[i].data(), d_cnts[i], cnt_bytes, cudaMemcpyDeviceToHost, h->devs[i].stream);
-        if (es == cudaSuccess) es = cudaStreamSynchronize(h->devs[i].stream);
+        if (!rc) es = cudaMemcpyAsync(cnts[i].data(), J.devs[i].d_cnt, J.cnt_bytes, cudaMemcpyDeviceToHost, d.stream);
+        if (es == cudaSuccess) es = cudaStreamSynchronize(d.stream);
         if (es != cudaSuccess && !rc) rc = fail(h, WOFDM_ECUDA, std::string("wofdm_ber_run_masked: ") + cudaGetErrorString(es));
     }
-    cudaSetDevice(d0.dev);
+    cudaSetDevice(h->devs[0].dev);
     if (rc) return rc;
-    for (size_t i = 0; i < ncnt; ++i) {
+    for (size_t i = 0; i < J.ncnt; ++i) {
         unsigned long long be = 0, se = 0;
         for (int k = 0; k < nd; ++k) { be += cnts[k][2 * i]; se += cnts[k][2 * i + 1]; }
         bit_err[i] = (int64_t)be; sym_err[i] = (int64_t)se;
     }
     return WOFDM_OK;
 }
+
+// The frames [*f_lo, *f_hi) of shard (shard_index, shard_count), a contiguous block of global frame ids.  resolve == 0:
+// bit_err / sym_err [n_snr]; else [n_snr][Cr][Nr] (wofdm_ber_run_resolved's layout, one window pair), counted by the
+// resolved twin of the K1 kernel this chain picks.  outputs_ok: the caller's output pointers are all non-NULL.
+int run_masked_impl(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                    const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                    uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count, int resolve,
+                    bool outputs_ok, int64_t* bit_err, int64_t* sym_err, long long* f_lo_out, long long* f_hi_out) {
+    int rc = masked_check(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, roll_off, shard_index, shard_count,
+                          resolve, outputs_ok);
+    if (rc) return rc;
+    // this shard's block of frame ids [f_lo, f_hi); batches and devices take contiguous ranges of it
+    const long long total = (long long)n_snr * C * ensemble;
+    const long long f_lo = (long long)((__int128)total * shard_index / shard_count);
+    const long long f_hi = (long long)((__int128)total * (shard_index + 1) / shard_count);
+    *f_lo_out = f_lo; *f_hi_out = f_hi;
+    MaskedJob J;
+    rc = masked_setup(J, h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, seed, variant, roll_off, resolve, f_hi - f_lo, 0);
+    if (rc) return rc;
+    return masked_run(J, f_lo, f_hi, nullptr, bit_err, sym_err);
+}
+
+// totals of counter cells [n_snr][Cr][Nr] from the frames of each cell (si, c) (c < Cr): S-1 symbols per active bin and
+// frame, 0 on guard bins; Nr == 1: every active bin of the frame
+void cell_totals(const wofdm_sys_t& s, const std::vector<long long>& frames, int Nr, int64_t* sym_tot) {
+    const long long active = s.N - 2 * s.guard;
+    for (size_t cell = 0; cell < frames.size(); ++cell) {
+        int64_t* out = sym_tot + cell * Nr;
+        if (Nr == 1) { out[0] = frames[cell] * active * (s.S - 1); continue; }
+        for (int k = 0; k < Nr; ++k) {
+            const int cc = (k + Nr / 2) & (Nr - 1);                   // ber_kernel.cuh: bin_active
+            out[k] = (cc >= s.guard && cc < Nr - s.guard) ? frames[cell] * (s.S - 1) : 0;
+        }
+    }
+}
+
+}  // namespace
+
+extern "C" {
 
 int wofdm_ber_run_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
                          const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
@@ -1326,7 +1464,6 @@ int wofdm_ber_run_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* w
     return wofdm_ber_run_masked_shard(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, seed, variant, roll_off, 0, 1,
                                       bit_err, bit_tot, sym_err, sym_tot);
 }
-
 int wofdm_ber_run_masked_shard(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
                                const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
                                uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count,
@@ -1374,6 +1511,115 @@ int wofdm_ber_run_masked_resolved(wofdm_handle h, const wofdm_sys_t* sys, const 
                 out[k] = (cc >= sys->guard && cc < Nr - sys->guard) ? frames * (sys->S - 1) : 0;
             }
         }
+    return WOFDM_OK;
+}
+
+
+int wofdm_ber_run_masked_segments(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                                  const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble_max,
+                                  const int64_t* segments, int n_seg, uint64_t seed, uint32_t variant, int roll_off,
+                                  int shard_index, int shard_count, int resolve, int64_t* bit_err, int64_t* sym_err,
+                                  int64_t* sym_tot) {
+    NvtxRange nvtx_("wofdm_ber_run_masked_segments");
+    if (!h) return WOFDM_EINVAL;
+    if (resolve & ~(WOFDM_BY_SUBCARRIER | WOFDM_BY_CHANNEL))
+        return fail(h, WOFDM_EINVAL, "resolve must be a combination of WOFDM_BY_SUBCARRIER and WOFDM_BY_CHANNEL");
+    int rc = masked_check(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, roll_off, shard_index, shard_count,
+                          resolve, bit_err && sym_err && sym_tot);
+    if (rc) return rc;
+    rc = check_segments(h, segments, n_seg, n_snr, ensemble_max);
+    if (rc) return rc;
+    std::vector<long long> tab;
+    long long n_local = 0;
+    seg_table(segments, n_seg, C, tab, &n_local);
+    // this shard's block of local indices [lo, hi), as wofdm_ber_run_masked_shard splits frame ids
+    const long long lo = (long long)((__int128)n_local * shard_index / shard_count);
+    const long long hi = (long long)((__int128)n_local * (shard_index + 1) / shard_count);
+    MaskedJob J;
+    rc = masked_setup(J, h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, seed, variant, roll_off, resolve,
+                      hi - lo, n_seg);
+    if (rc) return rc;
+    rc = masked_run(J, lo, hi, &tab, bit_err, sym_err);
+    if (rc) return rc;
+    // this shard's frames per cell (si, c): the local indices of the cell's ranges inside [lo, hi)
+    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? sys->N : 1;
+    std::vector<long long> frames((size_t)n_snr * Cr, 0);
+    for (int k = 0; k < n_seg; ++k) {
+        const long long g0 = tab[4 * k], ec = tab[4 * k + 3];
+        for (int c = 0; c < C; ++c)
+            frames[(size_t)tab[4 * k + 1] * Cr + (Cr > 1 ? c : 0)] += std::max(0LL, std::min(hi, g0 + (c + 1) * ec) - std::max(lo, g0 + c * ec));
+    }
+    cell_totals(*sys, frames, Nr, sym_tot);
+    return WOFDM_OK;
+}
+
+int wofdm_ber_run_masked_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                                  const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble_max,
+                                  int64_t first_block, int target_kind, int64_t target, uint64_t seed, uint32_t variant,
+                                  int roll_off, int shard_index, int shard_count, wofdm_reduce_fn reduce, void* reduce_user,
+                                  int64_t* ensemble_used, int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot,
+                                  int* rounds) {
+    NvtxRange nvtx_("wofdm_ber_run_masked_adaptive");
+    if (!h) return WOFDM_EINVAL;
+    const bool outputs_ok = ensemble_used && bit_err && bit_tot && sym_err && sym_tot && rounds;
+    int rc = masked_check(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, roll_off, shard_index, shard_count, 0,
+                          outputs_ok);
+    if (rc) return rc;
+    rc = check_target(h, target_kind, target, first_block, shard_count, reduce);
+    if (rc) return rc;
+    if (variant > 0xfffffff0u - WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "variant too large");
+    // row 0: the masked chain (noise stream variant + 1), set up once for the largest round of this shard; row 1: the
+    // unmasked chain, a plan of its own device buffers (the masked chain's live in the arena)
+    const long long total = (long long)n_snr * C * ensemble_max;
+    MaskedJob J;
+    rc = masked_setup(J, h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, seed, variant + 1, roll_off, 0,
+                      (long long)(((__int128)total + shard_count - 1) / shard_count), n_snr);
+    if (rc) return rc;
+    wofdm_ber_plan p = nullptr;
+    rc = plan_create_impl(h, sys, win_tx, win_rx, 1, chan, L, C, snr_db, n_snr, &p, false, 0, n_snr);
+    if (rc) return rc;
+    const size_t ns = (size_t)n_snr;
+    std::vector<int64_t> used(ns, 0), block(ns, std::min(first_block, ensemble_max)), red(4 * ns), tbit(2 * ns, 0), tsym(2 * ns, 0);
+    std::vector<int64_t> rbit(2 * ns), rsym(2 * ns);
+    std::vector<char> done(ns, 0);
+    std::vector<long long> tab;
+    int nround = 0;
+    for (;;) {
+        // this round: the active points in ascending SNR order, block[s] ensemble indices each from used[s]
+        std::vector<int64_t> seg;
+        for (size_t s = 0; s < ns; ++s)
+            if (!done[s]) { seg.push_back((int64_t)s); seg.push_back(used[s]); seg.push_back(block[s]); }
+        if (seg.empty()) break;
+        long long n_local = 0;
+        seg_table(seg.data(), (int)(seg.size() / 3), C, tab, &n_local);
+        const long long lo = (long long)((__int128)n_local * shard_index / shard_count);
+        const long long hi = (long long)((__int128)n_local * (shard_index + 1) / shard_count);
+        rc = masked_run(J, lo, hi, &tab, rbit.data(), rsym.data());
+        if (!rc) rc = run_segment_table(p, tab, n_local, ensemble_max, seed, variant, shard_index, shard_count, rbit.data() + ns, rsym.data() + ns);
+        if (rc) break;
+        ++nround;
+        for (size_t k = 0; k < 2 * ns; ++k) { red[2 * k] = rbit[k]; red[2 * k + 1] = rsym[k]; }   // [2][n_snr][2]
+        if (reduce && reduce(red.data(), (int64_t)red.size(), reduce_user) != 0) {
+            rc = fail(h, WOFDM_EINVAL, "the reduce callback failed");
+            break;
+        }
+        for (size_t k = 0; k < 2 * ns; ++k) { tbit[k] += red[2 * k]; tsym[k] += red[2 * k + 1]; }
+        for (size_t s = 0; s < ns; ++s) {
+            if (done[s]) continue;
+            const std::vector<int64_t>& t = target_kind == WOFDM_TARGET_BIT_ERRORS ? tbit : tsym;
+            done[s] = schedule_step(std::min(t[s], t[ns + s]), target, ensemble_max, &used[s], &block[s]);
+        }
+    }
+    wofdm_ber_plan_destroy(p);
+    if (rc) return rc;
+    *rounds = nround;
+    const long long per_frame = (long long)(sys->N - 2 * sys->guard) * (sys->S - 1);
+    for (size_t s = 0; s < ns; ++s) {
+        ensemble_used[s] = used[s];
+        sym_tot[s] = (int64_t)C * used[s] * per_frame;
+        bit_tot[s] = sym_tot[s] * sys->bits;
+    }
+    for (size_t k = 0; k < 2 * ns; ++k) { bit_err[k] = tbit[k]; sym_err[k] = tsym[k]; }
     return WOFDM_OK;
 }
 

@@ -187,8 +187,8 @@ __global__ void __launch_bounds__(256) mask_split_kernel(const double2* __restri
 // of bins t + q TPF and parks the lattice points of the active ones, (Re, Im) fp16 pairs, in shared memory; the frame's columns
 // then leave as 16-byte chunks (four sub-carriers; consecutive lanes = consecutive columns of a core matrix): into the first
 // half of column frame * S + s (a_s) and into the second half of the next symbol's column (a_{s-1} there; symbol 0's second
-// half stays zero)
-template <int N>
+// half stays zero).  SEG: f0 + fl is a local index into the segment table draw.seg, decoded by seg_frame.
+template <int N, bool SEG = false>
 __global__ void __launch_bounds__(256) mask_sym_kernel(const BerParams draw, long long f0, long long nf, int S, int guard, int nact,
                                                        __half* __restrict__ Bt, int nk) {
     constexpr int TPF = N / 16;
@@ -199,10 +199,12 @@ __global__ void __launch_bounds__(256) mask_sym_kernel(const BerParams draw, lon
     for (int e = threadIdx.x; e < S * rowp; e += blockDim.x) lat[e] = __floats2half2_rn(0.f, 0.f);
     __syncthreads();
     for (long long fl = blockIdx.x; fl < nf; fl += gridDim.x) {
+        long long f = f0 + fl;
+        if constexpr (SEG) { int si, ci; seg_frame(draw, f, f, si, ci); }
         for (int e = threadIdx.x; e < S * TPF; e += blockDim.x) {
             const int s = e / TPF, t = e % TPF;
             uint32_t w[4];
-            load_sym_idx<N, false>(draw, f0 + fl, s, t, w);
+            load_sym_idx<N, false>(draw, f, s, t, w);
 #pragma unroll
             for (int q = 0; q < 16; ++q) {
                 const int bin = t + q * TPF;
@@ -399,25 +401,28 @@ int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, int roll_off, cons
     return WOFDM_OK;
 }
 
-int mask_gemm_batch(wofdm_ctx* h, DeviceCtx& d, const MaskGemm& mg, uint64_t seed, long long f0, long long nf, float2* stream) {
+int mask_gemm_batch(wofdm_ctx* h, DeviceCtx& d, const MaskGemm& mg, uint64_t seed, long long f0, long long nf, float2* stream,
+                    const long long* seg, int n_seg, int C, long long ensemble) {
     if (nf < 1 || nf > mg.batch) return fail(h, WOFDM_EINVAL, "mask product: batch out of range");
     BerParams draw;
     memset(&draw, 0, sizeof(draw));
     draw.seed = seed; philox_round_keys(seed, draw.rk); draw.bits = mg.bits; draw.S = mg.S;
+    draw.C = C; draw.ensemble = ensemble; draw.seg = seg; draw.n_seg = n_seg;
     const long long ncols = nf * mg.S;
     const int grid_s = (int)std::min<long long>(nf, (long long)d.sm_count * 8);
     const size_t sm_s = (size_t)mg.S * (4 * ((mg.nact + 3) / 4) + 4) * sizeof(__half2);
     if (sm_s > d.smem_optin) return fail(h, WOFDM_EUNSUPPORTED, "mask product: too many symbols per frame for the symbol kernel");
-    if (sm_s > 48 * 1024) {                 // (long frames: more than the default dynamic shared memory)
-        const void* fn = mg.N == 128 ? (const void*)mask_sym_kernel<128> : mg.N == 256 ? (const void*)mask_sym_kernel<256> : (const void*)mask_sym_kernel<512>;
-        WOFDM_CUDA(h, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_s));
-    }
+    using SymFn = void (*)(const BerParams, long long, long long, int, int, int, __half*, int);
+    SymFn fn = nullptr;
     switch (mg.N) {
-        case 128: mask_sym_kernel<128><<<grid_s, 256, sm_s, d.stream>>>(draw, f0, nf, mg.S, mg.guard, mg.nact, mg.Bt, mg.nk); break;
-        case 256: mask_sym_kernel<256><<<grid_s, 256, sm_s, d.stream>>>(draw, f0, nf, mg.S, mg.guard, mg.nact, mg.Bt, mg.nk); break;
-        case 512: mask_sym_kernel<512><<<grid_s, 256, sm_s, d.stream>>>(draw, f0, nf, mg.S, mg.guard, mg.nact, mg.Bt, mg.nk); break;
+        case 128: fn = seg ? mask_sym_kernel<128, true> : mask_sym_kernel<128>; break;
+        case 256: fn = seg ? mask_sym_kernel<256, true> : mask_sym_kernel<256>; break;
+        case 512: fn = seg ? mask_sym_kernel<512, true> : mask_sym_kernel<512>; break;
         default: return fail(h, WOFDM_EUNSUPPORTED, "the channel-mask variant is built for N = 128, 256, 512");
     }
+    if (sm_s > 48 * 1024)                   // (long frames: more than the default dynamic shared memory)
+        WOFDM_CUDA(h, cudaFuncSetAttribute((const void*)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_s));
+    fn<<<grid_s, 256, sm_s, d.stream>>>(draw, f0, nf, mg.S, mg.guard, mg.nact, mg.Bt, mg.nk);
     WOFDM_CUDA(h, cudaGetLastError());
     const int CT = (int)((ncols + TN - 1) / TN), n_tiles = CT * mg.RT;
     mask_gemm_f16<<<std::min(n_tiles, d.sm_count), NTHREADS, NSTAGE * STAGE_BYTES, d.stream>>>(mg.At, mg.Bt, mg.Y, mg.scale, mg.nk, mg.RT, n_tiles, mg.Yp, ncols);

@@ -27,7 +27,9 @@ size_t mask_gemm_plan(const wofdm_sys_t& sys, long long batch, MaskGemm& mg);
 // arena buffers + the matrix: the mask of roll_off bins (main_channel_mask.m:404-412, 477-493), d_wtx = K1's Tx table
 int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, int roll_off, const float* d_wtx);
 // masked symbols of frames f0 .. f0 + nf - 1 (nf <= batch) into Y and, if `stream` is not NULL, the serialised Tx streams
-// into stream[nf][tail_tx + S * stride]
-int mask_gemm_batch(wofdm_ctx* h, DeviceCtx& d, const MaskGemm& mg, uint64_t seed, long long f0, long long nf, float2* stream);
+// into stream[nf][tail_tx + S * stride].  seg (a device segment table [n_seg][4], BerParams::seg): f0 .. f0 + nf - 1 are
+// local indices of the segment list of a job with C channels and `ensemble` ensemble indices per point
+int mask_gemm_batch(wofdm_ctx* h, DeviceCtx& d, const MaskGemm& mg, uint64_t seed, long long f0, long long nf, float2* stream,
+                    const long long* seg = nullptr, int n_seg = 0, int C = 0, long long ensemble = 0);
 
 }  // namespace wofdm

@@ -10,6 +10,7 @@
 // [-(n_tx-1), M-1], so it runs as forward FFT_P -> multiply by the precomputed response Gp -> inverse FFT_P with
 // P = 8N >= 4 n_tx - 3 (register FFTs of fft_regs.cuh, P/16 threads per transform).  fp32.
 #pragma once
+#include <type_traits>
 #include "ber_kernel.cuh"
 
 namespace wofdm {
@@ -25,6 +26,14 @@ struct MaskParams {
     long long frame_begin, frame_step, n_frames;
     float2* stream;                // [n_frames][tail_tx + S*stride]
 };
+// SEG instantiations (frame segments): frame_begin + j*frame_step is a local index into the segment table seg[n_seg][4],
+// decoded by seg_frame (BerParams::seg) with C channels and `ensemble` ensemble indices per point.  (A struct of its own:
+// MaskParams keeps its size, and with it the code of the unsegmented kernel.)
+struct MaskSegParams : MaskParams {
+    const long long* seg;
+    int n_seg, C;
+    long long ensemble;
+};
 
 template <int N> struct MaskSmem {
     using PN = FftPlan<N>;
@@ -39,8 +48,8 @@ template <int N> struct MaskSmem {
     }
 };
 
-template <int N>
-__global__ void __launch_bounds__(256) tx_mask_kernel(const MaskParams p) {
+template <int N, bool SEG = false>
+__global__ void __launch_bounds__(256) tx_mask_kernel(const std::conditional_t<SEG, MaskSegParams, MaskParams> p) {
     using MS = MaskSmem<N>;
     using PN = typename MS::PN;
     using PP = typename MS::PP;
@@ -68,12 +77,14 @@ __global__ void __launch_bounds__(256) tx_mask_kernel(const MaskParams p) {
     __syncthreads();
     BerParams draw = {};                                   // only what load_sym_idx reads
     draw.seed = p.seed; philox_round_keys(p.seed, draw.rk); draw.bits = p.bits; draw.S = S;
+    if constexpr (SEG) { draw.C = p.C; draw.ensemble = p.ensemble; draw.seg = p.seg; draw.n_seg = p.n_seg; }
     // symbols per big-transform slot: slot g takes g*half + pass.  At least two, so that symbols filtered at the same time are
     // never neighbours (their stream segments overlap by the Tx tail; S <= FPPP used to put neighbours side by side -- found by
     // the comparison with the mask product, tests/test_drivers_gpu.py::test_channel_mask_product_against_fft_kernel)
     const int half = max(2, (S + FPPP - 1) / FPPP);
     for (long long j = blockIdx.x; j < p.n_frames; j += gridDim.x) {
-        const long long f = p.frame_begin + j * p.frame_step;
+        long long f = p.frame_begin + j * p.frame_step;
+        if constexpr (SEG) { int si, ci; seg_frame(draw, f, f, si, ci); }   // local index -> frame id
         for (int i = tid; i < body; i += NT) us[i] = make_float2(0.f, 0.f);
         // ---- symbols -> IFFT (un-windowed, un-scaled), FPP symbols per pass
         for (int s0 = 0; s0 < S; s0 += FPP) {

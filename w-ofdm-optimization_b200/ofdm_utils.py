@@ -235,6 +235,25 @@ def run_sim_mc_per_subcarrier(ensemble, cpLength, csLength, tailTx, tailRx, wind
     return out[0], out[1]
 
 
+def run_sim_mc_adaptive(ensemble_max, cpLength, csLength, tailTx, tailRx, windowTx, windowRx, channel, snr, offset,
+                        prefixRemovalLength, circularShiftLength, numSubcar, bitsPerSubcar, symbolsPerTx, rollOff,
+                        target_bit_errors, first_block=1, seed=0, handle=None):
+    """run_sim_mc with each SNR point stopped at a bit-error target (wofdm_ber_run_masked_adaptive): every point runs until
+    both the masked and the unmasked chain have counted target_bit_errors bit errors, or ensemble_max ensemble indices.
+    channel: one impulse response, or C x L (rows = realisations); snr: a scalar or a vector.  Returns (berMasked, ber,
+    ensemble_used), arrays over the SNR points, and writes no files.  An unreachable target gives run_sim_mc's result for
+    ensemble = ensemble_max."""
+    h = handle or default_handle()
+    s = capi.SysT(N=int(numSubcar), cp=int(cpLength), cs=int(csLength), tail_tx=int(tailTx), tail_rx=int(tailRx),
+                  rm=int(prefixRemovalLength), shift=int(circularShiftLength), bits=int(bitsPerSubcar),
+                  S=int(symbolsPerTx), noise_norm=1, constellation=1, precision=0, guard=int(offset))
+    ch = np.atleast_2d(np.asarray(channel)).T                         # (L, C)
+    r = h.ber_run_masked_adaptive(s, _diag(windowTx), _diag(windowRx), ch, np.atleast_1d(np.asarray(snr, dtype=np.float64)),
+                                  int(ensemble_max), target_bit_errors=int(target_bit_errors), first_block=int(first_block),
+                                  seed=seed, variant=0, roll_off=int(rollOff))
+    return r["bit_err"][0] / r["bit_tot"], r["bit_err"][1] / r["bit_tot"], r["ensemble_used"]
+
+
 def calculate_interference(cpLength, typeOFDM, windowTx, windowRx, numSubcar, tailTx, tailRx, channels, mode=0,
                            handle=None):
     """Scalar interference power on the mean of `channels` (rows = realisations, as vehA200channel2 is stored),

@@ -60,15 +60,20 @@ def adaptive_allreduce(group=None):
     return reduce
 
 
-def segment_frame_ids(segments, C: int, ensemble_max: int, shard=(0, 1)) -> np.ndarray:
+def segment_frame_ids(segments, C: int, ensemble_max: int, shard=(0, 1), contiguous=False) -> np.ndarray:
     """Global frame ids of a segment list {snr_idx, e_begin, e_count} in launch order (wofdm_ber_run_segments): segments in
-    the order given, channel-major then e inside a segment; `shard` keeps local indices j = shard[0] (mod shard[1])."""
+    the order given, channel-major then e inside a segment; `shard` keeps local indices j = shard[0] (mod shard[1]), or with
+    contiguous=True the channel-mask chain's block [floor(n*k/W), floor(n*(k+1)/W)) of the n local indices
+    (wofdm_ber_run_masked_segments)."""
     seg = np.asarray(segments, dtype=np.int64).reshape(-1, 3)
     parts = []
     for si, e0, ec in seg:
         c, e = np.divmod(np.arange(int(C) * int(ec), dtype=np.int64), int(ec))
         parts.append((si * C + c) * int(ensemble_max) + e0 + e)
     f = np.concatenate(parts) if parts else np.zeros(0, dtype=np.int64)
+    if contiguous:
+        k, w = int(shard[0]), int(shard[1])
+        return f[f.size * k // w: f.size * (k + 1) // w]
     return f[shard[0]::shard[1]]
 
 
