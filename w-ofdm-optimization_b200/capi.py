@@ -239,7 +239,9 @@ class Handle:
     def __exit__(self, *a):
         self.close()
 
-    def _check(self, rc):
+    def _check(self, rc, reduce_cb=None):
+        if rc and getattr(reduce_cb, "error", None) is not None:      # the call failed because its reduce callback raised
+            raise WofdmError(rc, f"reduce callback raised {reduce_cb.error!r}") from reduce_cb.error
         if rc:
             raise WofdmError(rc, (load().wofdm_last_error(self._h) or b"").decode())
 
@@ -308,10 +310,9 @@ class Handle:
         _, _, chf, L, Cn = self._win_chan(s, wt[0], wr[0], chan)
         snr = _f64(np.ravel(snr_db))
         n, nv = snr.size, wt.shape[0]
-        resolve = (WOFDM_BY_SUBCARRIER if by_subcarrier else 0) | (WOFDM_BY_CHANNEL if by_channel else 0)
-        cr, nr = (Cn if by_channel else 1), (s.N if by_subcarrier else 1)
-        be, se = np.zeros((nv, n, cr, nr), dtype=np.int64), np.zeros((nv, n, cr, nr), dtype=np.int64)
-        st = np.zeros((n, cr, nr), dtype=np.int64)
+        resolve, shape = _resolve(s, n, Cn, by_subcarrier, by_channel)
+        be, se = np.zeros((nv,) + shape, dtype=np.int64), np.zeros((nv,) + shape, dtype=np.int64)
+        st = np.zeros(shape, dtype=np.int64)
         rc = load().wofdm_ber_run_resolved(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), nv, _ptr(chf, _dp), L, Cn,
                                            _ptr(snr, _dp), n, int(ensemble), int(seed), int(variant), int(shard[0]),
                                            int(shard[1]), int(resolve), _ptr(be, _i64p), _ptr(se, _i64p), _ptr(st, _i64p))
@@ -329,8 +330,7 @@ class Handle:
         snr = _f64(np.ravel(snr_db))
         n, nv = snr.size, wt.shape[0]
         seg = np.ascontiguousarray(np.asarray(segments, dtype=np.int64).reshape(-1, 3))
-        resolve = (WOFDM_BY_SUBCARRIER if by_subcarrier else 0) | (WOFDM_BY_CHANNEL if by_channel else 0)
-        shape = (n, Cn if by_channel else 1, s.N if by_subcarrier else 1) if resolve else (n,)
+        resolve, shape = _resolve(s, n, Cn, by_subcarrier, by_channel)
         be, se = np.zeros((nv,) + shape, dtype=np.int64), np.zeros((nv,) + shape, dtype=np.int64)
         st = np.zeros(shape, dtype=np.int64)
         rc = load().wofdm_ber_run_segments(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), nv, _ptr(chf, _dp), L, Cn,
@@ -348,10 +348,7 @@ class Handle:
         of {bit, sym}, that returns (or fills in place) their sum over the processes -- sharding.adaptive_allreduce() under
         torch.distributed.  Returns bit_err / sym_err (n_var, n_snr), bit_tot / sym_tot (n_snr,), ensemble_used (n_snr,)
         and rounds."""
-        if (target_bit_errors is None) == (target_symbol_errors is None):
-            raise WofdmError(EINVAL, "give exactly one of target_bit_errors / target_symbol_errors")
-        kind, target = ((WOFDM_TARGET_BIT_ERRORS, target_bit_errors) if target_bit_errors is not None
-                        else (WOFDM_TARGET_SYMBOL_ERRORS, target_symbol_errors))
+        kind, target = _target(target_bit_errors, target_symbol_errors)
         wt, wr = self._win_multi(s, wins_tx, wins_rx)
         _, _, chf, L, Cn = self._win_chan(s, wt[0], wr[0], chan)
         snr = _f64(np.ravel(snr_db))
@@ -364,9 +361,7 @@ class Handle:
                                            _ptr(snr, _dp), n, int(ensemble_max), int(first_block), kind, int(target), int(seed),
                                            int(variant), int(shard[0]), int(shard[1]), cb, None, _ptr(used, _i64p),
                                            _ptr(be, _i64p), _ptr(bt, _i64p), _ptr(se, _i64p), _ptr(st, _i64p), C.byref(rounds))
-        if reduce is not None and cb.error is not None and rc:
-            raise WofdmError(rc, f"reduce callback raised {cb.error!r}") from cb.error
-        self._check(rc)
+        self._check(rc, cb)
         return dict(bit_err=be, bit_tot=bt, sym_err=se, sym_tot=st, ensemble_used=used, rounds=rounds.value)
 
     def ber_run_masked(self, s, win_tx, win_rx, chan, snr_db, ensemble, seed=0, variant=0, roll_off=10, shard=(0, 1)):
@@ -390,8 +385,7 @@ class Handle:
         wt, wr, chf, L, Cn = self._win_chan(s, win_tx, win_rx, chan)
         snr = _f64(np.ravel(snr_db))
         n = snr.size
-        resolve = (WOFDM_BY_SUBCARRIER if by_subcarrier else 0) | (WOFDM_BY_CHANNEL if by_channel else 0)
-        shape = (n, Cn if by_channel else 1, s.N if by_subcarrier else 1)
+        resolve, shape = _resolve(s, n, Cn, by_subcarrier, by_channel)
         be, se, st = (np.zeros(shape, dtype=np.int64) for _ in range(3))
         rc = load().wofdm_ber_run_masked_resolved(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), _ptr(chf, _dp), L, Cn,
                                                   _ptr(snr, _dp), n, int(ensemble), int(seed), int(variant), int(roll_off),
@@ -410,8 +404,7 @@ class Handle:
         snr = _f64(np.ravel(snr_db))
         n = snr.size
         seg = np.ascontiguousarray(np.asarray(segments, dtype=np.int64).reshape(-1, 3))
-        resolve = (WOFDM_BY_SUBCARRIER if by_subcarrier else 0) | (WOFDM_BY_CHANNEL if by_channel else 0)
-        shape = (n, Cn if by_channel else 1, s.N if by_subcarrier else 1) if resolve else (n,)
+        resolve, shape = _resolve(s, n, Cn, by_subcarrier, by_channel)
         be, se, st = (np.zeros(shape, dtype=np.int64) for _ in range(3))
         rc = load().wofdm_ber_run_masked_segments(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), _ptr(chf, _dp), L, Cn,
                                                   _ptr(snr, _dp), n, int(ensemble_max), _ptr(seg, _i64p), seg.shape[0],
@@ -428,10 +421,7 @@ class Handle:
         rows reach the target or ensemble_max ensemble indices.  Exactly one of target_bit_errors / target_symbol_errors.
         reduce: as in ber_run_adaptive, on int64 counts of shape (2, n_snr, 2).  Returns bit_err / sym_err (2, n_snr),
         bit_tot / sym_tot (n_snr,), ensemble_used (n_snr,) and rounds."""
-        if (target_bit_errors is None) == (target_symbol_errors is None):
-            raise WofdmError(EINVAL, "give exactly one of target_bit_errors / target_symbol_errors")
-        kind, target = ((WOFDM_TARGET_BIT_ERRORS, target_bit_errors) if target_bit_errors is not None
-                        else (WOFDM_TARGET_SYMBOL_ERRORS, target_symbol_errors))
+        kind, target = _target(target_bit_errors, target_symbol_errors)
         wt, wr, chf, L, Cn = self._win_chan(s, win_tx, win_rx, chan)
         snr = _f64(np.ravel(snr_db))
         n = snr.size
@@ -444,9 +434,7 @@ class Handle:
                                                   int(seed), int(variant), int(roll_off), int(shard[0]), int(shard[1]), cb, None,
                                                   _ptr(used, _i64p), _ptr(be, _i64p), _ptr(bt, _i64p), _ptr(se, _i64p),
                                                   _ptr(st, _i64p), C.byref(rounds))
-        if reduce is not None and cb.error is not None and rc:
-            raise WofdmError(rc, f"reduce callback raised {cb.error!r}") from cb.error
-        self._check(rc)
+        self._check(rc, cb)
         return dict(bit_err=be, bit_tot=bt, sym_err=se, sym_tot=st, ensemble_used=used, rounds=rounds.value)
 
     def psd_estimate(self, N, cp, cs, tail_tx, win_tx, guard_band=48, n_sym=256, records=1, seed=0, sym_idx=None,
@@ -611,6 +599,20 @@ class Handle:
                                        _ptr(ph, _dp) if ph is not None else None, _ptr(out, _dp))
         self._check(rc)
         return out.T
+
+
+def _resolve(s, n, Cn, by_subcarrier, by_channel):
+    """WOFDM_BY_* flags and the counter shape (n_snr, Cr, Nr) they give, (n_snr,) without them."""
+    resolve = (WOFDM_BY_SUBCARRIER if by_subcarrier else 0) | (WOFDM_BY_CHANNEL if by_channel else 0)
+    return resolve, ((n, Cn if by_channel else 1, s.N if by_subcarrier else 1) if resolve else (n,))
+
+
+def _target(target_bit_errors, target_symbol_errors):
+    """(target_kind, target) of the adaptive calls, from exactly one of the two targets."""
+    if (target_bit_errors is None) == (target_symbol_errors is None):
+        raise WofdmError(EINVAL, "give exactly one of target_bit_errors / target_symbol_errors")
+    return ((WOFDM_TARGET_BIT_ERRORS, target_bit_errors) if target_bit_errors is not None
+            else (WOFDM_TARGET_SYMBOL_ERRORS, target_symbol_errors))
 
 
 def reduce_trampoline(fn, shape=None):

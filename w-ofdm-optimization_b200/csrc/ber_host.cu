@@ -3,6 +3,7 @@
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <new>
 
 #include "host_common.h"
@@ -228,37 +229,17 @@ void cast_any(bool fp64, const std::vector<double>& src, std::vector<unsigned ch
     if (fp64) cast_vec<double>(src, dst); else cast_vec<float>(src, dst);
 }
 
-// host tables shared by plans and the verify path
+// the device inputs of a job in the kernels' precision, shared by plans, the verify path and the channel-mask chain
 struct HostTables {
-    std::vector<unsigned char> wtx, wrx, tw;
+    std::vector<unsigned char> wtx, wrx, tw, chan, snr;
+    size_t bytes() const { return wtx.size() + wrx.size() + tw.size() + chan.size() + snr.size(); }
 };
-
-// unit_peak (tensor-core kernels): the Tx window is divided by its largest magnitude.  Those kernels stage the stream and
-// the taps as fp16 pairs behind fixed power-of-two scales (ber_tconv.cuh: TCV_XSCALE, TCV_HSCALE), so their inputs must
-// have a known range; the chain itself does not care -- a common factor of the Tx signal or of a channel's taps scales
-// r, the noise follows the measured signal power (wofdm_simulation.py:135-138) and the pilot equaliser divides it out (:223-232).
-void build_tables(const wofdm_sys_t& s, const double* win_tx, const double* win_rx, HostTables& t, bool unit_peak = false) {
-    const bool fp64 = s.precision == 1;
-    const int n_tx = s.N + s.cp + s.cs;
-    double k = qam_scale(s) / (double)s.N;   // IDFT 1/N (transmitter.py:58) and constellation scale
-    if (unit_peak) {
-        double mx = 0.0;
-        for (int i = 0; i < n_tx; ++i) mx = std::max(mx, std::fabs(win_tx[i]));
-        if (mx > 0.0 && std::isfinite(mx)) k /= mx;
-    }
-    std::vector<double> a(n_tx), b(s.N + s.tail_rx);
-    for (int i = 0; i < n_tx; ++i) a[i] = win_tx[i] * k;
-    for (int i = 0; i < s.N + s.tail_rx; ++i) b[i] = win_rx[i];
-    cast_any(fp64, a, t.wtx);
-    cast_any(fp64, b, t.wrx);
-    cast_any(fp64, build_twiddles(s.N), t.tw);
-}
 
 // channel matrix L x C column-major complex double -> [C][L] V2<T> (same memory order, cast only).  unit_peak (tensor-core
 // kernels, see build_tables): every channel's taps are divided by their largest component magnitude.
-void cast_chan(bool fp64, const double* chan, size_t n_complex, std::vector<unsigned char>& dst, int L = 0, bool unit_peak = false) {
+void cast_chan(bool fp64, const double* chan, size_t n_complex, std::vector<unsigned char>& dst, int L, bool unit_peak) {
     std::vector<double> v(chan, chan + 2 * n_complex);
-    if (unit_peak && L > 0) {
+    if (unit_peak) {
         for (size_t c = 0; c + (size_t)L <= n_complex; c += (size_t)L) {
             double mx = 0.0;
             for (int i = 0; i < 2 * L; ++i) mx = std::max(mx, std::fabs(v[2 * c + i]));
@@ -269,6 +250,44 @@ void cast_chan(bool fp64, const double* chan, size_t n_complex, std::vector<unsi
         }
     }
     cast_any(fp64, v, dst);
+}
+
+// The tables of n_var window pairs (back to back), the twiddles, C channels of L taps and n_snr SNR points (linear).
+// unit_peak (tensor-core kernels): every Tx window is divided by its largest magnitude.  Those kernels stage the stream and
+// the taps as fp16 pairs behind fixed power-of-two scales (ber_tconv.cuh: TCV_XSCALE, TCV_HSCALE), so their inputs must
+// have a known range; the chain itself does not care -- a common factor of the Tx signal or of a channel's taps scales
+// r, the noise follows the measured signal power (wofdm_simulation.py:135-138) and the pilot equaliser divides it out (:223-232).
+HostTables build_tables(const wofdm_sys_t& s, const double* win_tx, const double* win_rx, int n_var, const double* chan, int L,
+                        int C, const double* snr_db, int n_snr, bool unit_peak) {
+    const bool fp64 = s.precision == 1;
+    const int n_tx = s.N + s.cp + s.cs, n_wr = s.N + s.tail_rx;
+    std::vector<double> a((size_t)n_var * n_tx), b(win_rx, win_rx + (size_t)n_var * n_wr);
+    for (int v = 0; v < n_var; ++v) {
+        const double* wt = win_tx + (size_t)v * n_tx;
+        double k = qam_scale(s) / (double)s.N;   // IDFT 1/N (transmitter.py:58) and constellation scale
+        if (unit_peak) {
+            double mx = 0.0;
+            for (int i = 0; i < n_tx; ++i) mx = std::max(mx, std::fabs(wt[i]));
+            if (mx > 0.0 && std::isfinite(mx)) k /= mx;
+        }
+        for (int i = 0; i < n_tx; ++i) a[(size_t)v * n_tx + i] = wt[i] * k;
+    }
+    std::vector<double> lin(n_snr);
+    for (int i = 0; i < n_snr; ++i) lin[i] = std::pow(10.0, -0.1 * snr_db[i]);   // wofdm_simulation.py:138
+    HostTables t;
+    cast_any(fp64, a, t.wtx);
+    cast_any(fp64, b, t.wrx);
+    cast_any(fp64, build_twiddles(s.N), t.tw);
+    cast_chan(fp64, chan, (size_t)L * C, t.chan, L, unit_peak);
+    cast_any(fp64, lin, t.snr);
+    return t;
+}
+
+// an arena block of max(bytes, 16) on device d, filled from src (unless NULL) on d's stream
+cudaError_t arena_put(DeviceCtx& d, const void* src, size_t bytes, void** dst) {
+    *dst = arena_take(d, std::max<size_t>(bytes, 16));
+    if (!*dst) return cudaErrorMemoryAllocation;
+    return src ? cudaMemcpyAsync(*dst, src, bytes, cudaMemcpyHostToDevice, d.stream) : cudaSuccess;
 }
 
 void fill_sys(BerParams& p, const wofdm_sys_t& s, int L) {
@@ -327,6 +346,179 @@ int prepare_kernel(wofdm_ctx* h, const BerVariant& v, size_t smem, int sm_count,
 
 size_t elem_bytes(const wofdm_sys_t& s) { return s.precision == 1 ? sizeof(double2) : sizeof(float2); }
 
+// ---- argument checks of the wofdm_ber_* entry points ---------------------------------------------------------------------
+// (each call keeps its own order of them: validate_sys and the channel-mask checks can return WOFDM_EUNSUPPORTED, the
+//  others WOFDM_EINVAL, so the order decides the code of a call with several faults)
+
+int check_shard(wofdm_ctx* h, int shard_index, int shard_count) {
+    if (shard_count < 1 || shard_index < 0 || shard_index >= shard_count) return fail(h, WOFDM_EINVAL, "bad shard");
+    return WOFDM_OK;
+}
+
+// resolve: WOFDM_BY_* flags; nonzero: at least one of them
+int check_resolve(wofdm_ctx* h, int resolve, bool nonzero) {
+    if ((nonzero && resolve == 0) || (resolve & ~(WOFDM_BY_SUBCARRIER | WOFDM_BY_CHANNEL)))
+        return fail(h, WOFDM_EINVAL, nonzero ? "resolve must be a non-empty combination of WOFDM_BY_SUBCARRIER and WOFDM_BY_CHANNEL"
+                                             : "resolve must be a combination of WOFDM_BY_SUBCARRIER and WOFDM_BY_CHANNEL");
+    return WOFDM_OK;
+}
+
+int check_shape(wofdm_ctx* h, const wofdm_sys_t* sys, int L, int C, int n_snr, int n_var) {
+    const int rc = validate_sys(h, sys, L);
+    if (rc) return rc;
+    if (C < 1 || n_snr < 1) return fail(h, WOFDM_EINVAL, "C and n_snr must be >= 1");
+    if (n_var < 1 || n_var > WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "n_var must be in [1, WOFDM_MAX_VARIANTS]");
+    return WOFDM_OK;
+}
+
+// the frame ids of a job, n_snr * C * ensemble of them, must be representable
+int check_frames(wofdm_ctx* h, int n_snr, int C, int64_t ensemble) {
+    int64_t frames = 0;
+    if (__builtin_mul_overflow((int64_t)n_snr, (int64_t)C, &frames) || __builtin_mul_overflow(frames, ensemble, &frames))
+        return fail(h, WOFDM_EINVAL, "n_snr * C * ensemble overflows int64");
+    return WOFDM_OK;
+}
+
+// a job of the main chain (ensemble: ensemble_max of the segment calls) and this process's shard of it
+int check_job(wofdm_ctx* h, const wofdm_sys_t* sys, int L, int C, int n_snr, int n_var, int64_t ensemble, int shard_index,
+              int shard_count) {
+    int rc = check_shard(h, shard_index, shard_count);
+    if (rc) return rc;
+    if (ensemble < 1) return fail(h, WOFDM_EINVAL, "ensemble must be >= 1");
+    rc = check_shape(h, sys, L, C, n_snr, n_var);
+    return rc ? rc : check_frames(h, n_snr, C, ensemble);
+}
+
+// counters [n_var][n_snr][Cr][Nr] of `resolve`, 16 bytes each on the device: all of it must be representable
+int check_counters(wofdm_ctx* h, const wofdm_sys_t& s, int C, int n_snr, int n_var, int resolve) {
+    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? s.N : 1;
+    size_t n = 0, bytes = 0;
+    if (__builtin_mul_overflow((size_t)n_snr, (size_t)Cr, &n) || __builtin_mul_overflow(n, (size_t)Nr, &n) ||
+        __builtin_mul_overflow(n, (size_t)n_var, &n) || __builtin_mul_overflow(n, (size_t)16, &bytes) || n > (size_t)INT64_MAX / 16)
+        return fail(h, WOFDM_EINVAL, "resolved counter array too large");
+    return WOFDM_OK;
+}
+
+// a job of the channel-mask chain (one window pair, fp32, N = 128, 256 or 512, a mask that fits) and this process's shard
+// of it; outputs_ok: the caller's output pointers are all non-NULL
+int check_masked(wofdm_ctx* h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, const double* chan, int L,
+                 int C, const double* snr_db, int n_snr, int64_t ensemble, int roll_off, int shard_index, int shard_count,
+                 int resolve, bool outputs_ok) {
+    int rc = check_shape(h, sys, L, C, n_snr, 1);
+    if (rc) return rc;
+    if (!win_tx || !win_rx || !chan || !snr_db || !outputs_ok) return fail(h, WOFDM_EINVAL, "NULL buffer");
+    if (ensemble < 1) return fail(h, WOFDM_EINVAL, "ensemble must be >= 1");
+    if (sys->precision != 0) return fail(h, WOFDM_EUNSUPPORTED, "the channel-mask variant runs in fp32");
+    const int N = sys->N, n_tx = N + sys->cp + sys->cs, M = 2 * n_tx - 1;
+    if (N != 128 && N != 256 && N != 512) return fail(h, WOFDM_EUNSUPPORTED, "the channel-mask variant is built for N = 128, 256, 512");
+    if (roll_off < 1 || M / 2 + 2 * roll_off > M) return fail(h, WOFDM_EINVAL, "roll_off does not fit the mask");
+    if (2 * n_tx > 3 * N + 1) return fail(h, WOFDM_EUNSUPPORTED, "cp + cs too long for the mask kernel (n_tx <= 1.5 N)");
+    rc = check_shard(h, shard_index, shard_count);
+    if (!rc) rc = check_frames(h, n_snr, C, ensemble);
+    return rc ? rc : check_counters(h, *sys, C, n_snr, 1, resolve);
+}
+
+// segments[n_seg][3] of a job: inside [0, n_snr) x [0, ensemble_max), e_count >= 1, no two segments of one point overlap
+int check_segments(wofdm_ctx* h, const int64_t* segments, int n_seg, int n_snr, int64_t ensemble_max) {
+    if (!segments || n_seg < 1) return fail(h, WOFDM_EINVAL, "segments must be a non-empty list");
+    std::vector<std::pair<int64_t, int64_t>> iv((size_t)n_seg);
+    for (int k = 0; k < n_seg; ++k) {
+        const int64_t si = segments[3 * k], e0 = segments[3 * k + 1], ec = segments[3 * k + 2];
+        if (si < 0 || si >= n_snr || e0 < 0 || e0 >= ensemble_max || ec < 1 || ec > ensemble_max - e0)
+            return fail(h, WOFDM_EINVAL, "segment outside [0, n_snr) x [0, ensemble_max) or with e_count < 1");
+        iv[k] = {si * ensemble_max + e0, ec};       // (< n_snr * ensemble_max: no overflow, checked by the caller)
+    }
+    std::sort(iv.begin(), iv.end());
+    for (int k = 1; k < n_seg; ++k)
+        if (iv[k].first < iv[k - 1].first + iv[k - 1].second) return fail(h, WOFDM_EINVAL, "overlapping segments of one SNR point");
+    return WOFDM_OK;
+}
+
+// the stopping rule's own arguments (wofdm_ber_run_adaptive / wofdm_ber_run_masked_adaptive)
+int check_target(wofdm_ctx* h, int target_kind, int64_t target, int64_t first_block, int shard_count, wofdm_reduce_fn reduce) {
+    if (target_kind != WOFDM_TARGET_BIT_ERRORS && target_kind != WOFDM_TARGET_SYMBOL_ERRORS) return fail(h, WOFDM_EINVAL, "unknown target_kind");
+    if (target < 1) return fail(h, WOFDM_EINVAL, "target must be >= 1");
+    if (first_block < 1) return fail(h, WOFDM_EINVAL, "first_block must be >= 1");
+    if (shard_count > 1 && !reduce) return fail(h, WOFDM_EINVAL, "shard_count > 1 needs a reduce callback (the schedule needs the job's counts)");
+    return WOFDM_OK;
+}
+
+// ---- frame sets, shards and totals -----------------------------------------------------------------------------------------
+
+// A list of segments {snr_idx, e_begin, e_count} (every channel of point snr_idx at ensemble indices [e_begin, e_begin +
+// e_count)) as the devices read it (BerParams::seg): tab[k] = {g0, snr_idx, e_begin, e_count}, g0 the local index of
+// segment k's first frame (segments in order, channel-major, then e); n_local frames in all.
+struct Segments {
+    std::vector<long long> tab;
+    long long n_local = 0;
+    int n() const { return (int)(tab.size() / 4); }
+};
+
+Segments seg_table(const int64_t* seg, int n_seg, int C) {
+    Segments s;
+    s.tab.resize((size_t)n_seg * 4);
+    for (int k = 0; k < n_seg; ++k) {
+        long long* t = &s.tab[4 * (size_t)k];
+        t[0] = s.n_local; t[1] = seg[3 * k]; t[2] = seg[3 * k + 1]; t[3] = seg[3 * k + 2];
+        s.n_local += (long long)C * seg[3 * k + 2];
+    }
+    return s;
+}
+
+// the segments {(si, 0, counts[si]) : si < n_snr}.  With counts[si] = ensemble: the whole job of a fixed call, whose local
+// index is exactly the global frame id (si*C + c)*ensemble + e.
+Segments job_segments(int C, const std::vector<int64_t>& counts) {
+    std::vector<int64_t> seg;
+    for (size_t si = 0; si < counts.size(); ++si) { seg.push_back((int64_t)si); seg.push_back(0); seg.push_back(counts[si]); }
+    return seg_table(seg.data(), (int)counts.size(), C);
+}
+
+// The local indices of a frame set that one shard (shard_index, shard_count) owns: strided, j = shard_index (mod
+// shard_count), the main chain's rule; or contiguous, the block [floor(n k / W), floor(n (k+1) / W)) of the n local
+// indices, the channel-mask chain's rule.
+struct ShardRule {
+    bool contiguous;
+    long long index, count;                // strided
+    long long lo, hi;                      // contiguous: [lo, hi)
+    static ShardRule strided(int index, int count) { return {false, index, count, 0, 0}; }
+    static ShardRule block(long long n, int index, int count) {
+        return {true, index, count, (long long)((__int128)n * index / count), (long long)((__int128)n * (index + 1) / count)};
+    }
+    // this shard's local indices in [a, b)
+    long long frames(long long a, long long b) const {
+        if (contiguous) return std::max(0LL, std::min(hi, b) - std::max(lo, a));
+        auto upto = [&](long long x) -> long long { return x > index ? (x - index + count - 1) / count : 0; };
+        return upto(b) - upto(a);
+    }
+};
+
+// this shard's frames per counter cell (si, c) [n_snr][Cr] of a segment list: Cr = C (by channel) or 1
+std::vector<long long> cell_frames(const Segments& sg, int n_snr, int C, int Cr, const ShardRule& r) {
+    std::vector<long long> frames((size_t)n_snr * Cr, 0);
+    for (int k = 0; k < sg.n(); ++k) {
+        const long long g0 = sg.tab[4 * k], si = sg.tab[4 * k + 1], ec = sg.tab[4 * k + 3];
+        const long long w = Cr > 1 ? ec : C * ec;      // local indices of one cell: one channel's, or all of them
+        for (int c = 0; c < Cr; ++c) frames[(size_t)si * Cr + c] += r.frames(g0 + c * w, g0 + (c + 1) * w);
+    }
+    return frames;
+}
+
+// totals of counter cells [n_snr][Cr][Nr] from the frames of each cell (si, c): S-1 symbols per active bin and frame, 0 on
+// guard bins; Nr == 1: every active bin of the frame.  bit_tot (may be NULL) = sym_tot * bits.
+void cell_totals(const wofdm_sys_t& s, const std::vector<long long>& frames, int Nr, int64_t* sym_tot, int64_t* bit_tot) {
+    const long long active = s.N - 2 * s.guard;
+    for (size_t cell = 0; cell < frames.size(); ++cell) {
+        int64_t* out = sym_tot + cell * Nr;
+        if (Nr == 1) { out[0] = frames[cell] * active * (s.S - 1); continue; }
+        for (int k = 0; k < Nr; ++k) {
+            const int cc = (k + Nr / 2) & (Nr - 1);                   // ber_kernel.cuh: bin_active
+            out[k] = (cc >= s.guard && cc < Nr - s.guard) ? frames[cell] * (s.S - 1) : 0;
+        }
+    }
+    if (bit_tot)
+        for (size_t i = 0; i < frames.size() * Nr; ++i) bit_tot[i] = sym_tot[i] * s.bits;
+}
+
 }  // namespace
 
 // transient = true: device buffers come out of the per-device arena (no cudaMalloc / cudaFree per call); such a plan
@@ -341,12 +533,9 @@ static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double
     if (!h) return WOFDM_EINVAL;
     if (!out) return fail(h, WOFDM_EINVAL, "plan out pointer is NULL");
     *out = nullptr;
-    int rc = validate_sys(h, sys, L);
+    int rc = check_shape(h, sys, L, C, n_snr, n_var);
     if (rc) return rc;
     if (!win_tx || !win_rx || !chan || !snr_db) return fail(h, WOFDM_EINVAL, "NULL input buffer");
-    if (C < 1 || n_snr < 1) return fail(h, WOFDM_EINVAL, "C and n_snr must be >= 1");
-    if (n_var < 1 || n_var > WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "n_var must be in [1, WOFDM_MAX_VARIANTS]");
-    const bool fp64 = sys->precision == 1;
 
     wofdm_ber_plan_s* p = new (std::nothrow) wofdm_ber_plan_s();
     if (!p) return fail(h, WOFDM_ENOMEM, "host allocation failed");
@@ -380,21 +569,7 @@ static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double
         p->flat_tx = fp.flat_tx; p->flat_rx = fp.flat_rx;
     }
 
-    HostTables t;
-    const bool unit_peak = p->var->ntile > 0;
-    const int n_tx = sys->N + sys->cp + sys->cs, n_wr = sys->N + sys->tail_rx;
-    for (int v = 0; v < n_var; ++v) {              // tables of the window pairs back to back
-        HostTables tv;
-        build_tables(*sys, win_tx + (size_t)v * n_tx, win_rx + (size_t)v * n_wr, tv, unit_peak);
-        t.wtx.insert(t.wtx.end(), tv.wtx.begin(), tv.wtx.end());
-        t.wrx.insert(t.wrx.end(), tv.wrx.begin(), tv.wrx.end());
-        if (v == 0) t.tw = tv.tw;
-    }
-    std::vector<unsigned char> hchan, hsnr;
-    cast_chan(fp64, chan, (size_t)L * C, hchan, L, unit_peak);
-    std::vector<double> lin(n_snr);
-    for (int i = 0; i < n_snr; ++i) lin[i] = std::pow(10.0, -0.1 * snr_db[i]);   // wofdm_simulation.py:138
-    cast_any(fp64, lin, hsnr);
+    const HostTables t = build_tables(*sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, p->var->ntile > 0);
 
     p->devs.resize(h->devs.size());
     for (size_t i = 0; i < h->devs.size(); ++i) {
@@ -419,15 +594,14 @@ static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double
         const size_t scratch_elems = (size_t)p->lay.pad + sys->tail_tx + (size_t)sys->S * (sys->N + sys->cp + sys->cs - sys->tail_tx) + 64;
         pd.scratch_bytes = p->use_global ? (size_t)pd.blocks_per_sm * d.sm_count * 2 * scratch_elems * elem_bytes(*sys) : 0;
         if (e == cudaSuccess && transient) {
-            rc = arena_reserve(h, d, t.wtx.size() + t.wrx.size() + t.tw.size() + hchan.size() + hsnr.size() +
-                                         (resolve ? 0 : (size_t)n_var * n_snr * 16) + pd.scratch_bytes + (size_t)seg_cap * 32);
+            rc = arena_reserve(h, d, t.bytes() + (resolve ? 0 : (size_t)n_var * n_snr * 16) + pd.scratch_bytes + (size_t)seg_cap * 32);
             if (rc) { const std::string msg = h->err; wofdm_ber_plan_destroy(p); h->err = msg; return rc; }
         }
         if (e == cudaSuccess) e = up(&pd.d_wtx, t.wtx);
         if (e == cudaSuccess) e = up(&pd.d_wrx, t.wrx);
         if (e == cudaSuccess) e = up(&pd.d_tw, t.tw);
-        if (e == cudaSuccess) e = up(&pd.d_chan, hchan);
-        if (e == cudaSuccess) e = up(&pd.d_snr, hsnr);
+        if (e == cudaSuccess) e = up(&pd.d_chan, t.chan);
+        if (e == cudaSuccess) e = up(&pd.d_snr, t.snr);
         // (resolved counters: a buffer of their own, outside the arena -- it can be large, and failing to get it is WOFDM_ENOMEM)
         if (e == cudaSuccess && resolve) e = cudaMalloc(reinterpret_cast<void**>(&pd.d_cnt), n_var * p->cnt_per_var * sizeof(unsigned long long));
         else if (e == cudaSuccess) e = dev_alloc(reinterpret_cast<void**>(&pd.d_cnt), (size_t)n_var * n_snr * 2 * sizeof(unsigned long long));
@@ -567,22 +741,8 @@ int wofdm_ber_plan_launch(wofdm_ber_plan p, int slot, int64_t ensemble, uint64_t
 
 int wofdm_ber_plan_read(wofdm_ber_plan p, int64_t* bit_err, int64_t* sym_err) {
     if (!p) return WOFDM_EINVAL;
-    wofdm_ctx* h = p->ctx;
-    if (!bit_err || !sym_err) return fail(h, WOFDM_EINVAL, "NULL output buffer");
-    const int n_out = p->n_var * p->n_snr;       // [n_var][n_snr]
-    for (int i = 0; i < n_out; ++i) { bit_err[i] = 0; sym_err[i] = 0; }
-    std::vector<unsigned long long> tmp((size_t)n_out * 2);
-    for (size_t s = 0; s < p->devs.size(); ++s) {
-        PlanDev& pd = p->devs[s];
-        if (!pd.pending) continue;
-        WOFDM_CUDA(h, cudaSetDevice(h->devs[s].dev));
-        WOFDM_CUDA(h, cudaMemcpyAsync(tmp.data(), pd.d_cnt, tmp.size() * sizeof(unsigned long long),
-                                      cudaMemcpyDeviceToHost, pd.last_stream));
-        WOFDM_CUDA(h, cudaStreamSynchronize(pd.last_stream));
-        for (int i = 0; i < n_out; ++i) { bit_err[i] += (int64_t)tmp[2 * i]; sym_err[i] += (int64_t)tmp[2 * i + 1]; }
-        pd.pending = false;
-    }
-    return WOFDM_OK;
+    if (!bit_err || !sym_err) return fail(p->ctx, WOFDM_EINVAL, "NULL output buffer");
+    return read_counters(p, bit_err, sym_err);        // [n_var][n_snr]
 }
 
 const char* wofdm_ber_plan_kernel(wofdm_ber_plan p) { return (p && p->var) ? p->var->name : ""; }
@@ -605,155 +765,9 @@ int wofdm_ber_plan_destroy(wofdm_ber_plan p) {
     return WOFDM_OK;
 }
 
-int wofdm_ber_run_shard(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
-                        const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
-                        uint64_t seed, uint32_t variant, int shard_index, int shard_count,
-                        int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot) {
-    return wofdm_ber_run_multi(h, sys, win_tx, win_rx, 1, chan, L, C, snr_db, n_snr, ensemble, seed, variant, shard_index,
-                               shard_count, bit_err, bit_tot, sym_err, sym_tot);
-}
-
-int wofdm_ber_run_multi(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
-                        const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
-                        uint64_t seed, uint32_t variant, int shard_index, int shard_count,
-                        int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot) {
-    NvtxRange nvtx_("wofdm_ber_run_multi");
-    if (!h) return WOFDM_EINVAL;
-    if (!bit_err || !bit_tot || !sym_err || !sym_tot) return fail(h, WOFDM_EINVAL, "NULL output buffer");
-    if (shard_count < 1 || shard_index < 0 || shard_index >= shard_count) return fail(h, WOFDM_EINVAL, "bad shard");
-    if (ensemble < 1) return fail(h, WOFDM_EINVAL, "ensemble must be >= 1");
-    wofdm_ber_plan p = nullptr;
-    int rc = plan_create_impl(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, &p, true);
-    if (rc) return rc;
-    // the handle's devices split this shard's frames between them: device i takes the sub-shard
-    // shard_index + shard_count*i of shard_count*ndev, so results do not depend on the GPU count
-    const int nd = (int)h->devs.size();
-    for (int i = 0; i < nd && rc == WOFDM_OK; ++i)
-        rc = wofdm_ber_plan_launch(p, i, ensemble, seed, variant, shard_index + shard_count * i, shard_count * nd,
-                                   nullptr, nullptr);
-    if (rc == WOFDM_OK) rc = wofdm_ber_plan_read(p, bit_err, sym_err);
-    wofdm_ber_plan_destroy(p);
-    if (rc) return rc;
-    // frames of this shard per SNR point: f = (snr*C + c)*ensemble + e, f = shard_index (mod shard_count)
-    const long long per_snr = (long long)C * ensemble;
-    for (int i = 0; i < n_snr; ++i) {
-        const long long lo = (long long)i * per_snr, hi = lo + per_snr;   // [lo, hi)
-        auto count_upto = [&](long long x) -> long long {                  // #{f < x : f = shard_index mod shard_count}
-            return x > shard_index ? (x - shard_index + shard_count - 1) / shard_count : 0;
-        };
-        const long long frames = count_upto(hi) - count_upto(lo);
-        sym_tot[i] = frames * (long long)(sys->N - 2 * sys->guard) * (sys->S - 1);   // active sub-carriers only
-        bit_tot[i] = sym_tot[i] * sys->bits;
-    }
-    return WOFDM_OK;
-}
-
-int wofdm_ber_run_resolved(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
-                           const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
-                           uint64_t seed, uint32_t variant, int shard_index, int shard_count, int resolve,
-                           int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot) {
-    NvtxRange nvtx_("wofdm_ber_run_resolved");
-    if (!h) return WOFDM_EINVAL;
-    if (resolve == 0 || (resolve & ~(WOFDM_BY_SUBCARRIER | WOFDM_BY_CHANNEL)))
-        return fail(h, WOFDM_EINVAL, "resolve must be a non-empty combination of WOFDM_BY_SUBCARRIER and WOFDM_BY_CHANNEL");
-    if (!bit_err || !sym_err || !sym_tot) return fail(h, WOFDM_EINVAL, "NULL output buffer");
-    if (shard_count < 1 || shard_index < 0 || shard_index >= shard_count) return fail(h, WOFDM_EINVAL, "bad shard");
-    if (ensemble < 1) return fail(h, WOFDM_EINVAL, "ensemble must be >= 1");
-    int rc = validate_sys(h, sys, L);
-    if (rc) return rc;
-    if (C < 1 || n_snr < 1) return fail(h, WOFDM_EINVAL, "C and n_snr must be >= 1");
-    if (n_var < 1 || n_var > WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "n_var must be in [1, WOFDM_MAX_VARIANTS]");
-    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? sys->N : 1;
-    // n_var * n_snr * Cr * Nr counters (x 2 on the device, x 8 bytes): all of it must be representable
-    size_t cells = 0, n_out = 0, dev_bytes = 0;
-    if (__builtin_mul_overflow((size_t)n_snr, (size_t)Cr, &cells) || __builtin_mul_overflow(cells, (size_t)Nr, &cells) ||
-        __builtin_mul_overflow(cells, (size_t)n_var, &n_out) || __builtin_mul_overflow(n_out, (size_t)16, &dev_bytes) ||
-        n_out > (size_t)INT64_MAX / 16)
-        return fail(h, WOFDM_EINVAL, "resolved counter array too large");
-    wofdm_ber_plan p = nullptr;
-    rc = plan_create_impl(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, &p, true, resolve);
-    if (rc) return rc;
-    // the handle's devices split this shard's frames as in wofdm_ber_run_multi; their counter arrays are summed here
-    const int nd = (int)h->devs.size();
-    for (int i = 0; i < nd && rc == WOFDM_OK; ++i)
-        rc = wofdm_ber_plan_launch(p, i, ensemble, seed, variant, shard_index + shard_count * i, shard_count * nd,
-                                   nullptr, nullptr);
-    if (rc == WOFDM_OK) rc = read_counters(p, bit_err, sym_err);
-    wofdm_ber_plan_destroy(p);
-    if (rc) return rc;
-    // frames of this shard per cell (si, c): f in [(si*C + c)*ensemble, +ensemble), f = shard_index (mod shard_count);
-    // guard bins never carry data and count nothing
-    auto count_upto = [&](long long x) -> long long { return x > shard_index ? (x - shard_index + shard_count - 1) / shard_count : 0; };
-    const long long active = sys->N - 2 * sys->guard;
-    for (int si = 0; si < n_snr; ++si)
-        for (int c = 0; c < Cr; ++c) {
-            const long long lo = ((long long)si * C + (Cr > 1 ? c : 0)) * ensemble, hi = lo + (Cr > 1 ? 1 : (long long)C) * ensemble;
-            const long long frames = count_upto(hi) - count_upto(lo);
-            int64_t* out = sym_tot + ((size_t)si * Cr + c) * Nr;
-            if (Nr == 1) { out[0] = frames * active * (sys->S - 1); continue; }
-            for (int k = 0; k < Nr; ++k) {
-                const int cc = (k + Nr / 2) & (Nr - 1);               // ber_kernel.cuh: bin_active
-                out[k] = (cc >= sys->guard && cc < Nr - sys->guard) ? frames * (sys->S - 1) : 0;
-            }
-        }
-    return WOFDM_OK;
-}
-
 }  // extern "C"
 
-// ---- frame segments (wofdm_ber_run_segments / _adaptive) ---------------------------------------------------------------
 namespace {
-
-// the checks every segment entry point shares with wofdm_ber_run_multi, plus ensemble_max and the size of the frame space
-int check_job(wofdm_handle h, const wofdm_sys_t* sys, int L, int C, int n_snr, int n_var, int64_t ensemble_max,
-              int shard_index, int shard_count) {
-    if (shard_count < 1 || shard_index < 0 || shard_index >= shard_count) return fail(h, WOFDM_EINVAL, "bad shard");
-    if (ensemble_max < 1) return fail(h, WOFDM_EINVAL, "ensemble_max must be >= 1");
-    int rc = validate_sys(h, sys, L);
-    if (rc) return rc;
-    if (C < 1 || n_snr < 1) return fail(h, WOFDM_EINVAL, "C and n_snr must be >= 1");
-    if (n_var < 1 || n_var > WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "n_var must be in [1, WOFDM_MAX_VARIANTS]");
-    int64_t frames = 0;
-    if (__builtin_mul_overflow((int64_t)n_snr, (int64_t)C, &frames) || __builtin_mul_overflow(frames, ensemble_max, &frames))
-        return fail(h, WOFDM_EINVAL, "n_snr * C * ensemble_max overflows int64");
-    return WOFDM_OK;
-}
-
-// device table of `seg` ({snr_idx, e_begin, e_count} each) -> {g0, snr_idx, e_begin, e_count}; *n_local = its frames
-void seg_table(const int64_t* seg, int n_seg, int C, std::vector<long long>& tab, long long* n_local) {
-    tab.resize((size_t)n_seg * 4);
-    long long g = 0;
-    for (int k = 0; k < n_seg; ++k) {
-        tab[4 * k] = g; tab[4 * k + 1] = seg[3 * k]; tab[4 * k + 2] = seg[3 * k + 1]; tab[4 * k + 3] = seg[3 * k + 2];
-        g += (long long)C * seg[3 * k + 2];
-    }
-    *n_local = g;
-}
-
-// segments[n_seg][3] of a job: inside [0, n_snr) x [0, ensemble_max), e_count >= 1, no two segments of one point overlap
-int check_segments(wofdm_handle h, const int64_t* segments, int n_seg, int n_snr, int64_t ensemble_max) {
-    if (!segments || n_seg < 1) return fail(h, WOFDM_EINVAL, "segments must be a non-empty list");
-    std::vector<std::pair<int64_t, int64_t>> iv((size_t)n_seg);
-    for (int k = 0; k < n_seg; ++k) {
-        const int64_t si = segments[3 * k], e0 = segments[3 * k + 1], ec = segments[3 * k + 2];
-        if (si < 0 || si >= n_snr || e0 < 0 || e0 >= ensemble_max || ec < 1 || ec > ensemble_max - e0)
-            return fail(h, WOFDM_EINVAL, "segment outside [0, n_snr) x [0, ensemble_max) or with e_count < 1");
-        iv[k] = {si * ensemble_max + e0, ec};       // (< n_snr * ensemble_max: no overflow, checked by the caller)
-    }
-    std::sort(iv.begin(), iv.end());
-    for (int k = 1; k < n_seg; ++k)
-        if (iv[k].first < iv[k - 1].first + iv[k - 1].second) return fail(h, WOFDM_EINVAL, "overlapping segments of one SNR point");
-    return WOFDM_OK;
-}
-
-// the stopping rule's own arguments (wofdm_ber_run_adaptive / wofdm_ber_run_masked_adaptive)
-int check_target(wofdm_handle h, int target_kind, int64_t target, int64_t first_block, int shard_count, wofdm_reduce_fn reduce) {
-    if (target_kind != WOFDM_TARGET_BIT_ERRORS && target_kind != WOFDM_TARGET_SYMBOL_ERRORS) return fail(h, WOFDM_EINVAL, "unknown target_kind");
-    if (target < 1) return fail(h, WOFDM_EINVAL, "target must be >= 1");
-    if (first_block < 1) return fail(h, WOFDM_EINVAL, "first_block must be >= 1");
-    if (shard_count > 1 && !reduce) return fail(h, WOFDM_EINVAL, "shard_count > 1 needs a reduce callback (the schedule needs the job's counts)");
-    return WOFDM_OK;
-}
 
 // The schedule of include/wofdm.h for one point after a round that ran *block more ensemble indices of it: m = its fewest
 // cumulative errors over the rows.  Returns true when the point is done; else *block is its next block.
@@ -770,29 +784,134 @@ bool schedule_step(int64_t m, int64_t target, int64_t ensemble_max, int64_t* use
     return false;
 }
 
-// one launch of a twin plan over the segment table on every device of the handle (devices split this shard's local
-// indices as wofdm_ber_run_multi splits frame ids), then the summed counters
-int run_segment_table(wofdm_ber_plan p, const std::vector<long long>& tab, long long n_local, int64_t ensemble_max,
-                      uint64_t seed, uint32_t variant, int shard_index, int shard_count, int64_t* bit_err, int64_t* sym_err) {
+// One launch of plan p on every device of the handle, then the summed counters.  Device i takes the sub-shard
+// shard_index + shard_count*i of shard_count*ndev, so results do not depend on the GPU count.  segs (twin plans): the
+// launches run the local indices of that segment list, of a job of `ensemble` = ensemble_max indices, instead of the
+// plan's whole job.
+int run_plan(wofdm_ber_plan p, int64_t ensemble, uint64_t seed, uint32_t variant, int shard_index, int shard_count,
+             const Segments* segs, int64_t* bit_err, int64_t* sym_err) {
     wofdm_ctx* h = p->ctx;
-    const int n_seg = (int)(tab.size() / 4), nd = (int)h->devs.size();
-    if (n_seg > p->seg_cap) return fail(h, WOFDM_EINVAL, "more segments than the plan's segment table holds");
+    const int nd = (int)h->devs.size();
+    if (segs && segs->n() > p->seg_cap) return fail(h, WOFDM_EINVAL, "more segments than the plan's segment table holds");
     for (int i = 0; i < nd; ++i) {
         DeviceCtx& d = h->devs[i];
         PlanDev& pd = p->devs[i];
-        WOFDM_CUDA(h, cudaSetDevice(d.dev));
-        // (pageable source: the copy returns once the table is staged; the previous launch on this stream is ordered before it)
-        WOFDM_CUDA(h, cudaMemcpyAsync(pd.d_seg, tab.data(), tab.size() * sizeof(long long), cudaMemcpyHostToDevice, d.stream));
-        const int rc = plan_launch_impl(p, i, ensemble_max, seed, variant, shard_index + shard_count * i, shard_count * nd,
-                                        nullptr, nullptr, pd.d_seg, n_seg, n_local);
+        if (segs) {
+            WOFDM_CUDA(h, cudaSetDevice(d.dev));
+            // (pageable source: the copy returns once the table is staged; the previous launch on this stream is ordered before it)
+            WOFDM_CUDA(h, cudaMemcpyAsync(pd.d_seg, segs->tab.data(), segs->tab.size() * sizeof(long long), cudaMemcpyHostToDevice, d.stream));
+        }
+        const int rc = plan_launch_impl(p, i, ensemble, seed, variant, shard_index + shard_count * i, shard_count * nd, nullptr,
+                                        nullptr, segs ? pd.d_seg : nullptr, segs ? segs->n() : 0, segs ? segs->n_local : 0);
         if (rc) return rc;
     }
     return read_counters(p, bit_err, sym_err);
 }
 
+// A checked job of the main chain on a one-shot plan: the whole job (segs == nullptr: the production kernels, or their
+// resolved twins with resolve != 0) or the frames of a segment list (the twins).  -> counters [n_var][n_snr][Cr][Nr] and
+// this shard's totals [n_snr][Cr][Nr]; bit_tot may be NULL.
+int run_job(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var, const double* chan,
+            int L, int C, const double* snr_db, int n_snr, int64_t ensemble, const Segments* segs, uint64_t seed, uint32_t variant,
+            int shard_index, int shard_count, int resolve, int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot, int64_t* bit_tot) {
+    wofdm_ber_plan p = nullptr;
+    int rc = plan_create_impl(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, &p, true, resolve, segs ? segs->n() : 0);
+    if (rc) return rc;
+    rc = run_plan(p, ensemble, seed, variant, shard_index, shard_count, segs, bit_err, sym_err);
+    wofdm_ber_plan_destroy(p);
+    if (rc) return rc;
+    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? sys->N : 1;
+    const Segments all = segs ? Segments() : job_segments(C, std::vector<int64_t>(n_snr, ensemble));
+    cell_totals(*sys, cell_frames(segs ? *segs : all, n_snr, C, Cr, ShardRule::strided(shard_index, shard_count)), Nr, sym_tot, bit_tot);
+    return WOFDM_OK;
+}
+
+// wofdm_ber_run_multi (resolve 0, bit_tot) and wofdm_ber_run_resolved (a checked resolve)
+int run_fixed(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var, const double* chan,
+              int L, int C, const double* snr_db, int n_snr, int64_t ensemble, uint64_t seed, uint32_t variant, int shard_index,
+              int shard_count, int resolve, int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot, int64_t* bit_tot) {
+    if (!bit_err || !sym_err || !sym_tot || (!resolve && !bit_tot)) return fail(h, WOFDM_EINVAL, "NULL output buffer");
+    int rc = check_job(h, sys, L, C, n_snr, n_var, ensemble, shard_index, shard_count);
+    if (!rc) rc = check_counters(h, *sys, C, n_snr, n_var, resolve);
+    if (rc) return rc;
+    return run_job(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, ensemble, nullptr, seed, variant, shard_index,
+                   shard_count, resolve, bit_err, sym_err, sym_tot, bit_tot);
+}
+
+// The stopping rule of include/wofdm.h over `rows` rows of counters (wofdm_ber_run_adaptive / _masked_adaptive).  Each round
+// runs the next block of every active point, in ascending SNR order, as one segment list: run_round gives this process's
+// counters [rows][n_snr]; reduce (optional) sums them, packed [rows][n_snr][2] = {bit, sym}, over the processes; a point
+// stops when its fewest errors over the rows reach the target.  Fills the call's outputs.
+int run_adaptive(wofdm_ctx* h, const wofdm_sys_t& s, int C, int n_snr, int rows, int64_t ensemble_max, int64_t first_block,
+                 int target_kind, int64_t target, wofdm_reduce_fn reduce, void* reduce_user,
+                 const std::function<int(const Segments&, int64_t*, int64_t*)>& run_round, int64_t* ensemble_used,
+                 int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot, int* rounds) {
+    const size_t nr = (size_t)rows, ns = (size_t)n_snr;
+    std::vector<int64_t> used(ns, 0), block(ns, std::min(first_block, ensemble_max)), rbit(nr * ns), rsym(nr * ns), red(nr * ns * 2);
+    std::vector<int64_t> tbit(nr * ns, 0), tsym(nr * ns, 0);
+    std::vector<char> done(ns, 0);
+    int nround = 0;
+    for (;;) {
+        std::vector<int64_t> seg;
+        for (size_t s = 0; s < ns; ++s)
+            if (!done[s]) { seg.push_back((int64_t)s); seg.push_back(used[s]); seg.push_back(block[s]); }
+        if (seg.empty()) break;
+        const int rc = run_round(seg_table(seg.data(), (int)(seg.size() / 3), C), rbit.data(), rsym.data());
+        if (rc) return rc;
+        ++nround;
+        for (size_t k = 0; k < nr * ns; ++k) { red[2 * k] = rbit[k]; red[2 * k + 1] = rsym[k]; }
+        if (reduce && reduce(red.data(), (int64_t)red.size(), reduce_user) != 0) return fail(h, WOFDM_EINVAL, "the reduce callback failed");
+        for (size_t k = 0; k < nr * ns; ++k) { tbit[k] += red[2 * k]; tsym[k] += red[2 * k + 1]; }
+        const std::vector<int64_t>& t = target_kind == WOFDM_TARGET_BIT_ERRORS ? tbit : tsym;
+        for (size_t s = 0; s < ns; ++s) {
+            if (done[s]) continue;
+            int64_t m = INT64_MAX;
+            for (size_t r = 0; r < nr; ++r) m = std::min(m, t[r * ns + s]);
+            done[s] = schedule_step(m, target, ensemble_max, &used[s], &block[s]);
+        }
+    }
+    *rounds = nround;
+    std::copy(used.begin(), used.end(), ensemble_used);
+    std::copy(tbit.begin(), tbit.end(), bit_err);
+    std::copy(tsym.begin(), tsym.end(), sym_err);
+    // (the job's totals: every process ran the same schedule)
+    cell_totals(s, cell_frames(job_segments(C, used), n_snr, C, 1, ShardRule::strided(0, 1)), 1, sym_tot, bit_tot);
+    return WOFDM_OK;
+}
+
 }  // namespace
 
 extern "C" {
+
+int wofdm_ber_run_shard(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                        const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                        uint64_t seed, uint32_t variant, int shard_index, int shard_count,
+                        int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot) {
+    return wofdm_ber_run_multi(h, sys, win_tx, win_rx, 1, chan, L, C, snr_db, n_snr, ensemble, seed, variant, shard_index,
+                               shard_count, bit_err, bit_tot, sym_err, sym_tot);
+}
+
+int wofdm_ber_run_multi(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
+                        const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                        uint64_t seed, uint32_t variant, int shard_index, int shard_count,
+                        int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot) {
+    NvtxRange nvtx_("wofdm_ber_run_multi");
+    if (!h) return WOFDM_EINVAL;
+    return run_fixed(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, ensemble, seed, variant, shard_index, shard_count,
+                     0, bit_err, sym_err, sym_tot, bit_tot);
+}
+
+int wofdm_ber_run_resolved(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
+                           const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                           uint64_t seed, uint32_t variant, int shard_index, int shard_count, int resolve,
+                           int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot) {
+    NvtxRange nvtx_("wofdm_ber_run_resolved");
+    if (!h) return WOFDM_EINVAL;
+    const int rc = check_resolve(h, resolve, true);
+    if (rc) return rc;
+    return run_fixed(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, ensemble, seed, variant, shard_index, shard_count,
+                     resolve, bit_err, sym_err, sym_tot, nullptr);
+}
 
 int wofdm_ber_run_segments(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
                            const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble_max,
@@ -800,46 +919,16 @@ int wofdm_ber_run_segments(wofdm_handle h, const wofdm_sys_t* sys, const double*
                            int shard_count, int resolve, int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot) {
     NvtxRange nvtx_("wofdm_ber_run_segments");
     if (!h) return WOFDM_EINVAL;
-    if (resolve & ~(WOFDM_BY_SUBCARRIER | WOFDM_BY_CHANNEL))
-        return fail(h, WOFDM_EINVAL, "resolve must be a combination of WOFDM_BY_SUBCARRIER and WOFDM_BY_CHANNEL");
+    int rc = check_resolve(h, resolve, false);
+    if (rc) return rc;
     if (!bit_err || !sym_err || !sym_tot) return fail(h, WOFDM_EINVAL, "NULL output buffer");
-    int rc = check_job(h, sys, L, C, n_snr, n_var, ensemble_max, shard_index, shard_count);
+    rc = check_job(h, sys, L, C, n_snr, n_var, ensemble_max, shard_index, shard_count);
+    if (!rc) rc = check_segments(h, segments, n_seg, n_snr, ensemble_max);
+    if (!rc) rc = check_counters(h, *sys, C, n_snr, n_var, resolve);
     if (rc) return rc;
-    rc = check_segments(h, segments, n_seg, n_snr, ensemble_max);
-    if (rc) return rc;
-    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? sys->N : 1;
-    size_t cells = 0, n_out = 0, dev_bytes = 0;
-    if (__builtin_mul_overflow((size_t)n_snr, (size_t)Cr, &cells) || __builtin_mul_overflow(cells, (size_t)Nr, &cells) ||
-        __builtin_mul_overflow(cells, (size_t)n_var, &n_out) || __builtin_mul_overflow(n_out, (size_t)16, &dev_bytes) ||
-        n_out > (size_t)INT64_MAX / 16)
-        return fail(h, WOFDM_EINVAL, "resolved counter array too large");
-    std::vector<long long> tab;
-    long long n_local = 0;
-    seg_table(segments, n_seg, C, tab, &n_local);
-    wofdm_ber_plan p = nullptr;
-    rc = plan_create_impl(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, &p, true, resolve, n_seg);
-    if (rc) return rc;
-    rc = run_segment_table(p, tab, n_local, ensemble_max, seed, variant, shard_index, shard_count, bit_err, sym_err);
-    wofdm_ber_plan_destroy(p);
-    if (rc) return rc;
-    // this shard's frames per cell (si, c): local indices j = shard_index (mod shard_count) in the cell's ranges
-    auto count_upto = [&](long long x) -> long long { return x > shard_index ? (x - shard_index + shard_count - 1) / shard_count : 0; };
-    std::vector<long long> frames((size_t)n_snr * Cr, 0);
-    for (int k = 0; k < n_seg; ++k) {
-        const long long g0 = tab[4 * k], ec = tab[4 * k + 3];
-        for (int c = 0; c < C; ++c)
-            frames[(size_t)tab[4 * k + 1] * Cr + (Cr > 1 ? c : 0)] += count_upto(g0 + (c + 1) * ec) - count_upto(g0 + c * ec);
-    }
-    const long long active = sys->N - 2 * sys->guard;
-    for (size_t cell = 0; cell < (size_t)n_snr * Cr; ++cell) {
-        int64_t* out = sym_tot + cell * Nr;
-        if (Nr == 1) { out[0] = frames[cell] * active * (sys->S - 1); continue; }
-        for (int k = 0; k < Nr; ++k) {
-            const int cc = (k + Nr / 2) & (Nr - 1);                   // ber_kernel.cuh: bin_active
-            out[k] = (cc >= sys->guard && cc < Nr - sys->guard) ? frames[cell] * (sys->S - 1) : 0;
-        }
-    }
-    return WOFDM_OK;
+    const Segments sg = seg_table(segments, n_seg, C);
+    return run_job(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, ensemble_max, &sg, seed, variant, shard_index,
+                   shard_count, resolve, bit_err, sym_err, sym_tot, nullptr);
 }
 
 int wofdm_ber_run_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
@@ -852,53 +941,18 @@ int wofdm_ber_run_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const double*
     if (!h) return WOFDM_EINVAL;
     if (!ensemble_used || !bit_err || !bit_tot || !sym_err || !sym_tot || !rounds) return fail(h, WOFDM_EINVAL, "NULL output buffer");
     int rc = check_job(h, sys, L, C, n_snr, n_var, ensemble_max, shard_index, shard_count);
-    if (rc) return rc;
-    rc = check_target(h, target_kind, target, first_block, shard_count, reduce);
+    if (!rc) rc = check_target(h, target_kind, target, first_block, shard_count, reduce);
     if (rc) return rc;
     wofdm_ber_plan p = nullptr;
     rc = plan_create_impl(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, &p, true, 0, n_snr);
     if (rc) return rc;
-    const size_t nv = (size_t)n_var, ns = (size_t)n_snr;
-    std::vector<int64_t> used(ns, 0), block(ns, std::min(first_block, ensemble_max)), rbit(nv * ns), rsym(nv * ns), red(nv * ns * 2);
-    std::vector<int64_t> tbit(nv * ns, 0), tsym(nv * ns, 0);
-    std::vector<char> done(ns, 0);
-    std::vector<long long> tab;
-    int nround = 0;
-    for (;;) {
-        // this round: the active points in ascending SNR order, block[s] ensemble indices each from used[s]
-        std::vector<int64_t> seg;
-        for (size_t s = 0; s < ns; ++s)
-            if (!done[s]) { seg.push_back((int64_t)s); seg.push_back(used[s]); seg.push_back(block[s]); }
-        if (seg.empty()) break;
-        long long n_local = 0;
-        seg_table(seg.data(), (int)(seg.size() / 3), C, tab, &n_local);
-        rc = run_segment_table(p, tab, n_local, ensemble_max, seed, variant, shard_index, shard_count, rbit.data(), rsym.data());
-        if (rc) break;
-        ++nround;
-        for (size_t k = 0; k < nv * ns; ++k) { red[2 * k] = rbit[k]; red[2 * k + 1] = rsym[k]; }   // [n_var][n_snr][2]
-        if (reduce && reduce(red.data(), (int64_t)red.size(), reduce_user) != 0) {
-            rc = fail(h, WOFDM_EINVAL, "the reduce callback failed");
-            break;
-        }
-        for (size_t k = 0; k < nv * ns; ++k) { tbit[k] += red[2 * k]; tsym[k] += red[2 * k + 1]; }
-        for (size_t s = 0; s < ns; ++s) {
-            if (done[s]) continue;
-            int64_t m = INT64_MAX;                      // the fewest errors over the window pairs
-            for (size_t v = 0; v < nv; ++v) m = std::min(m, target_kind == WOFDM_TARGET_BIT_ERRORS ? tbit[v * ns + s] : tsym[v * ns + s]);
-            done[s] = schedule_step(m, target, ensemble_max, &used[s], &block[s]);
-        }
-    }
+    rc = run_adaptive(h, *sys, C, n_snr, n_var, ensemble_max, first_block, target_kind, target, reduce, reduce_user,
+                      [&](const Segments& sg, int64_t* be, int64_t* se) {
+                          return run_plan(p, ensemble_max, seed, variant, shard_index, shard_count, &sg, be, se);
+                      },
+                      ensemble_used, bit_err, bit_tot, sym_err, sym_tot, rounds);
     wofdm_ber_plan_destroy(p);
-    if (rc) return rc;
-    *rounds = nround;
-    const long long per_frame = (long long)(sys->N - 2 * sys->guard) * (sys->S - 1);
-    for (size_t s = 0; s < ns; ++s) {
-        ensemble_used[s] = used[s];
-        sym_tot[s] = (int64_t)C * used[s] * per_frame;
-        bit_tot[s] = sym_tot[s] * sys->bits;
-    }
-    for (size_t k = 0; k < nv * ns; ++k) { bit_err[k] = tbit[k]; sym_err[k] = tsym[k]; }
-    return WOFDM_OK;
+    return rc;
 }
 
 int wofdm_ber_run(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
@@ -920,7 +974,6 @@ int wofdm_ber_verify(wofdm_handle h, const wofdm_sys_t* sys, const double* win_t
     if (!win_tx || !win_rx || !chan || !snr_db || !sym_idx || !noise || !eq_out || !dec_idx || !bit_err || !sym_err)
         return fail(h, WOFDM_EINVAL, "NULL buffer");
     if (F < 1) return fail(h, WOFDM_EINVAL, "F must be >= 1");
-    const bool fp64 = sys->precision == 1;
     const int M = 1 << sys->bits;
     const size_t n_sym = (size_t)sys->N * sys->S * F;
     for (size_t i = 0; i < n_sym; ++i)
@@ -938,40 +991,27 @@ int wofdm_ber_verify(wofdm_handle h, const wofdm_sys_t* sys, const double* win_t
     if (rc) return rc;
     const int grid = (int)std::min<long long>(F, std::max<long long>(max_ctas / ch.var->CL, 1)) * ch.var->CL;
 
-    HostTables t;
-    build_tables(*sys, win_tx, win_rx, t, ch.var->ntile > 0);
-    std::vector<unsigned char> hchan, hsnr;
-    cast_chan(fp64, chan, (size_t)L * F, hchan, L, ch.var->ntile > 0);
-    std::vector<double> lin(F);
-    for (int i = 0; i < F; ++i) lin[i] = std::pow(10.0, -0.1 * snr_db[i]);
-    cast_any(fp64, lin, hsnr);
+    const HostTables t = build_tables(*sys, win_tx, win_rx, 1, chan, L, F, snr_db, F, ch.var->ntile > 0);   // (frame f: channel f, SNR f)
     const size_t nlen = (size_t)noise_len(*sys, L);
     const size_t n_eq = (size_t)sys->N * (sys->S - 1) * F;
     const size_t scratch_elems = (size_t)ch.lay.pad + sys->tail_tx + (size_t)sys->S * (sys->N + sys->cp + sys->cs - sys->tail_tx) + 64;
     const size_t scratch_bytes = ch.use_global ? (size_t)grid * 2 * scratch_elems * elem_bytes(*sys) : 0;
 
-    const size_t total = t.wtx.size() + t.wrx.size() + t.tw.size() + hchan.size() + hsnr.size() + n_sym * 4 +
-                         nlen * F * 16 + n_eq * 16 + n_eq * 4 + (size_t)F * 16 + scratch_bytes;
-    rc = arena_reserve(h, d, total);
+    rc = arena_reserve(h, d, t.bytes() + n_sym * 4 + nlen * F * 16 + n_eq * 16 + n_eq * 4 + (size_t)F * 16 + scratch_bytes);
     if (rc) return rc;
-    auto put = [&](const void* src, size_t bytes, void** dst) -> cudaError_t {
-        *dst = arena_take(d, std::max<size_t>(bytes, 16));
-        if (!*dst) return cudaErrorMemoryAllocation;
-        return src ? cudaMemcpyAsync(*dst, src, bytes, cudaMemcpyHostToDevice, d.stream) : cudaSuccess;
-    };
     void *d_wtx, *d_wrx, *d_tw, *d_chan, *d_snr, *d_sym, *d_noise, *d_eq, *d_dec, *d_be, *d_se, *d_scr = nullptr;
-    WOFDM_CUDA(h, put(t.wtx.data(), t.wtx.size(), &d_wtx));
-    WOFDM_CUDA(h, put(t.wrx.data(), t.wrx.size(), &d_wrx));
-    WOFDM_CUDA(h, put(t.tw.data(), t.tw.size(), &d_tw));
-    WOFDM_CUDA(h, put(hchan.data(), hchan.size(), &d_chan));
-    WOFDM_CUDA(h, put(hsnr.data(), hsnr.size(), &d_snr));
-    WOFDM_CUDA(h, put(sym_idx, n_sym * 4, &d_sym));
-    WOFDM_CUDA(h, put(noise, nlen * F * 16, &d_noise));
-    WOFDM_CUDA(h, put(nullptr, n_eq * 16, &d_eq));
-    WOFDM_CUDA(h, put(nullptr, n_eq * 4, &d_dec));
-    WOFDM_CUDA(h, put(nullptr, (size_t)F * 8, &d_be));
-    WOFDM_CUDA(h, put(nullptr, (size_t)F * 8, &d_se));
-    if (scratch_bytes) WOFDM_CUDA(h, put(nullptr, scratch_bytes, &d_scr));
+    WOFDM_CUDA(h, arena_put(d, t.wtx.data(), t.wtx.size(), &d_wtx));
+    WOFDM_CUDA(h, arena_put(d, t.wrx.data(), t.wrx.size(), &d_wrx));
+    WOFDM_CUDA(h, arena_put(d, t.tw.data(), t.tw.size(), &d_tw));
+    WOFDM_CUDA(h, arena_put(d, t.chan.data(), t.chan.size(), &d_chan));
+    WOFDM_CUDA(h, arena_put(d, t.snr.data(), t.snr.size(), &d_snr));
+    WOFDM_CUDA(h, arena_put(d, sym_idx, n_sym * 4, &d_sym));
+    WOFDM_CUDA(h, arena_put(d, noise, nlen * F * 16, &d_noise));
+    WOFDM_CUDA(h, arena_put(d, nullptr, n_eq * 16, &d_eq));
+    WOFDM_CUDA(h, arena_put(d, nullptr, n_eq * 4, &d_dec));
+    WOFDM_CUDA(h, arena_put(d, nullptr, (size_t)F * 8, &d_be));
+    WOFDM_CUDA(h, arena_put(d, nullptr, (size_t)F * 8, &d_se));
+    if (scratch_bytes) WOFDM_CUDA(h, arena_put(d, nullptr, scratch_bytes, &d_scr));
     WOFDM_CUDA(h, cudaMemsetAsync(d_be, 0, (size_t)F * 8, d.stream));
     WOFDM_CUDA(h, cudaMemsetAsync(d_se, 0, (size_t)F * 8, d.stream));
 
@@ -1104,32 +1144,6 @@ struct MaskedJob {
     std::vector<MaskedDev> devs;           // the devices set up: the first ones of the handle
 };
 
-// what every channel-mask entry point rejects; ensemble: the job's (ensemble_max of a segment call)
-int masked_check(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, const double* chan, int L,
-                 int C, const double* snr_db, int n_snr, int64_t ensemble, int roll_off, int shard_index, int shard_count,
-                 int resolve, bool outputs_ok) {
-    int rc = validate_sys(h, sys, L);
-    if (rc) return rc;
-    if (!win_tx || !win_rx || !chan || !snr_db || !outputs_ok) return fail(h, WOFDM_EINVAL, "NULL buffer");
-    if (C < 1 || n_snr < 1 || ensemble < 1) return fail(h, WOFDM_EINVAL, "C, n_snr and ensemble must be >= 1");
-    if (sys->precision != 0) return fail(h, WOFDM_EUNSUPPORTED, "the channel-mask variant runs in fp32");
-    const int N = sys->N, n_tx = N + sys->cp + sys->cs, M = 2 * n_tx - 1;
-    if (N != 128 && N != 256 && N != 512) return fail(h, WOFDM_EUNSUPPORTED, "the channel-mask variant is built for N = 128, 256, 512");
-    if (roll_off < 1 || M / 2 + 2 * roll_off > M) return fail(h, WOFDM_EINVAL, "roll_off does not fit the mask");
-    if (2 * n_tx > 3 * N + 1) return fail(h, WOFDM_EUNSUPPORTED, "cp + cs too long for the mask kernel (n_tx <= 1.5 N)");
-    if (shard_count < 1 || shard_index < 0 || shard_index >= shard_count) return fail(h, WOFDM_EINVAL, "bad shard");
-    long long total = 0;
-    if (__builtin_mul_overflow((long long)n_snr, (long long)C, &total) || __builtin_mul_overflow(total, (long long)ensemble, &total))
-        return fail(h, WOFDM_EINVAL, "n_snr * C * ensemble overflows int64");
-    // counter pairs [n_snr][Cr][Nr], 16 bytes each on the device: all of it must be representable
-    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? N : 1;
-    size_t ncnt = 0, cnt_bytes = 0;
-    if (__builtin_mul_overflow((size_t)n_snr, (size_t)Cr, &ncnt) || __builtin_mul_overflow(ncnt, (size_t)Nr, &ncnt) ||
-        __builtin_mul_overflow(ncnt, (size_t)16, &cnt_bytes) || ncnt > (size_t)INT64_MAX / 16)
-        return fail(h, WOFDM_EINVAL, "resolved counter array too large");
-    return WOFDM_OK;
-}
-
 // Set-up of a checked channel-mask call: the kernels, the tables, and on every device that takes part (contiguous ranges
 // of at least 64 frames out of max_frames, the most frames one masked_run covers) its buffers and the mask product's
 // matrix.  resolve != 0 or seg_cap > 0: the resolved twin of the K1 kernel (counters [n_snr][Cr][Nr], [n_snr] with
@@ -1227,13 +1241,8 @@ int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const dou
     } else {
         twp.resize(16);
     }
-    HostTables t;
-    build_tables(*sys, win_tx, win_rx, t, run.var->ntile > 0);   // (tx_mask_kernel shares the table: a common factor of its stream)
-    std::vector<unsigned char> hchan, hsnr;
-    cast_chan(false, chan, (size_t)L * C, hchan, L, run.var->ntile > 0);
-    std::vector<double> lin(n_snr);
-    for (int i = 0; i < n_snr; ++i) lin[i] = std::pow(10.0, -0.1 * snr_db[i]);
-    cast_any(false, lin, hsnr);
+    // (tx_mask_kernel shares the Tx window's table: a common factor of its stream)
+    const HostTables t = build_tables(*sys, win_tx, win_rx, 1, chan, L, C, snr_db, n_snr, run.var->ntile > 0);
     J.body = (size_t)sys->tail_tx + (size_t)sys->S * stride;
     J.batch = std::min<long long>(max_frames, J.use_gemm ? 16384 : 8192);
     const size_t scratch_elems = (size_t)run.lay.pad + J.body + 64;
@@ -1252,26 +1261,21 @@ int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const dou
         }
         const size_t mg_bytes = J.use_gemm ? mask_gemm_plan(*sys, J.batch, md.mg) : 0;
         const size_t stream_bytes = J.fused ? 16 : (size_t)J.batch * J.body * sizeof(float2);
-        int rc = arena_reserve(h, d, t.wtx.size() + t.wrx.size() + t.tw.size() + twp.size() + hchan.size() + hsnr.size() + g.size() * 4 +
-                                     J.cnt_bytes + stream_bytes + scratch_bytes + mg_bytes + (size_t)seg_cap * 32 + 8192);
+        int rc = arena_reserve(h, d, t.bytes() + twp.size() + g.size() * 4 + J.cnt_bytes + stream_bytes + scratch_bytes + mg_bytes +
+                                     (size_t)seg_cap * 32 + 8192);
         if (rc) return rc;
-        auto put = [&](const void* src, size_t bytes, void** dst) -> cudaError_t {
-            *dst = arena_take(d, std::max<size_t>(bytes, 16));
-            if (!*dst) return cudaErrorMemoryAllocation;
-            return src ? cudaMemcpyAsync(*dst, src, bytes, cudaMemcpyHostToDevice, d.stream) : cudaSuccess;
-        };
         void *d_wtx, *d_wrx, *d_tw, *d_twp, *d_chan, *d_snr, *d_g, *d_cnt, *d_seg = nullptr, *d_scr = nullptr;
-        WOFDM_CUDA(h, put(t.wtx.data(), t.wtx.size(), &d_wtx));
-        WOFDM_CUDA(h, put(t.wrx.data(), t.wrx.size(), &d_wrx));
-        WOFDM_CUDA(h, put(t.tw.data(), t.tw.size(), &d_tw));
-        WOFDM_CUDA(h, put(hchan.data(), hchan.size(), &d_chan));
-        WOFDM_CUDA(h, put(hsnr.data(), hsnr.size(), &d_snr));
-        WOFDM_CUDA(h, put(g.data(), g.size() * 4, &d_g));
-        WOFDM_CUDA(h, put(twp.data(), twp.size(), &d_twp));
-        WOFDM_CUDA(h, put(nullptr, J.cnt_bytes, &d_cnt));
-        WOFDM_CUDA(h, put(nullptr, stream_bytes, &md.d_stream));
-        if (scratch_bytes) WOFDM_CUDA(h, put(nullptr, scratch_bytes, &d_scr));
-        if (seg_cap > 0) WOFDM_CUDA(h, put(nullptr, (size_t)seg_cap * 32, &d_seg));
+        WOFDM_CUDA(h, arena_put(d, t.wtx.data(), t.wtx.size(), &d_wtx));
+        WOFDM_CUDA(h, arena_put(d, t.wrx.data(), t.wrx.size(), &d_wrx));
+        WOFDM_CUDA(h, arena_put(d, t.tw.data(), t.tw.size(), &d_tw));
+        WOFDM_CUDA(h, arena_put(d, t.chan.data(), t.chan.size(), &d_chan));
+        WOFDM_CUDA(h, arena_put(d, t.snr.data(), t.snr.size(), &d_snr));
+        WOFDM_CUDA(h, arena_put(d, g.data(), g.size() * 4, &d_g));
+        WOFDM_CUDA(h, arena_put(d, twp.data(), twp.size(), &d_twp));
+        WOFDM_CUDA(h, arena_put(d, nullptr, J.cnt_bytes, &d_cnt));
+        WOFDM_CUDA(h, arena_put(d, nullptr, stream_bytes, &md.d_stream));
+        if (scratch_bytes) WOFDM_CUDA(h, arena_put(d, nullptr, scratch_bytes, &d_scr));
+        if (seg_cap > 0) WOFDM_CUDA(h, arena_put(d, nullptr, (size_t)seg_cap * 32, &d_seg));
         md.d_cnt = static_cast<unsigned long long*>(d_cnt);
         md.d_seg = static_cast<long long*>(d_seg);
         if (J.use_gemm) {
@@ -1320,10 +1324,10 @@ int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const dou
     return rc;
 }
 
-// The frames [g_lo, g_hi) of a set-up call: global frame ids, or with `tab` (seg_table's layout, at most seg_cap entries,
-// uploaded to every device) local indices of that segment list.  The devices take contiguous ranges of at least 64.
+// The frames [g_lo, g_hi) of a set-up call: global frame ids, or with `segs` (at most seg_cap segments, its table uploaded to
+// every device) local indices of that segment list.  The devices take contiguous ranges of at least 64.
 // -> bit_err / sym_err [n_snr][Cr][Nr]
-int masked_run(MaskedJob& J, long long g_lo, long long g_hi, const std::vector<long long>* tab, int64_t* bit_err, int64_t* sym_err) {
+int masked_run(MaskedJob& J, long long g_lo, long long g_hi, const Segments* segs, int64_t* bit_err, int64_t* sym_err) {
     wofdm_ctx* h = J.h;
     const wofdm_sys_t& sys = J.sys;
     const int N = sys.N;
@@ -1332,15 +1336,15 @@ int masked_run(MaskedJob& J, long long g_lo, long long g_hi, const std::vector<l
         for (size_t i = 0; i < J.ncnt; ++i) { bit_err[i] = 0; sym_err[i] = 0; }
         return WOFDM_OK;
     }
-    const int n_seg = tab ? (int)(tab->size() / 4) : 0;
+    const int n_seg = segs ? segs->n() : 0;
     if (n_seg > J.seg_cap) return fail(h, WOFDM_EINVAL, "more segments than the call's segment table holds");
     const int nd = (int)std::min<long long>((long long)J.devs.size(), std::max<long long>(1, nfr / 64));
     auto run_dev = [&](MaskedDev& md, long long f_lo, long long f_hi) -> int {
         DeviceCtx& d = h->devs[md.slot];
         WOFDM_CUDA(h, cudaSetDevice(d.dev));
-        const long long* seg = tab ? md.d_seg : nullptr;
+        const long long* seg = segs ? md.d_seg : nullptr;
         // (pageable source: the copy returns once the table is staged; the previous work on this stream is ordered before it)
-        if (tab) WOFDM_CUDA(h, cudaMemcpyAsync(md.d_seg, tab->data(), tab->size() * sizeof(long long), cudaMemcpyHostToDevice, d.stream));
+        if (segs) WOFDM_CUDA(h, cudaMemcpyAsync(md.d_seg, segs->tab.data(), segs->tab.size() * sizeof(long long), cudaMemcpyHostToDevice, d.stream));
         WOFDM_CUDA(h, cudaMemsetAsync(md.d_cnt, 0, J.cnt_bytes, d.stream));
         MaskSegParams mp;
         static_cast<MaskParams&>(mp) = md.mp;
@@ -1373,7 +1377,7 @@ int masked_run(MaskedJob& J, long long g_lo, long long g_hi, const std::vector<l
             }
             WOFDM_CUDA(h, e);
             WOFDM_CUDA(h, cudaGetLastError());
-            if (f0 == 0 && !tab) {
+            if (f0 == 0 && !segs) {
                 // development aid: WOFDM_MASK_DUMP=<file> writes the masked Tx streams of the first (up to 4) frames as raw float32 pairs
                 const char* dump = J.dump_env;
                 if (dump && *dump) {
@@ -1418,39 +1422,25 @@ int masked_run(MaskedJob& J, long long g_lo, long long g_hi, const std::vector<l
     return WOFDM_OK;
 }
 
-// The frames [*f_lo, *f_hi) of shard (shard_index, shard_count), a contiguous block of global frame ids.  resolve == 0:
+// A checked job of the channel-mask chain: the whole job (segs == nullptr: global frame ids, the unsegmented kernels) or
+// the frames of a segment list, in either case this shard's contiguous block of the local indices.  resolve == 0:
 // bit_err / sym_err [n_snr]; else [n_snr][Cr][Nr] (wofdm_ber_run_resolved's layout, one window pair), counted by the
-// resolved twin of the K1 kernel this chain picks.  outputs_ok: the caller's output pointers are all non-NULL.
-int run_masked_impl(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
-                    const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
-                    uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count, int resolve,
-                    bool outputs_ok, int64_t* bit_err, int64_t* sym_err, long long* f_lo_out, long long* f_hi_out) {
-    int rc = masked_check(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, roll_off, shard_index, shard_count,
-                          resolve, outputs_ok);
-    if (rc) return rc;
-    // this shard's block of frame ids [f_lo, f_hi); batches and devices take contiguous ranges of it
-    const long long total = (long long)n_snr * C * ensemble;
-    const long long f_lo = (long long)((__int128)total * shard_index / shard_count);
-    const long long f_hi = (long long)((__int128)total * (shard_index + 1) / shard_count);
-    *f_lo_out = f_lo; *f_hi_out = f_hi;
+// resolved twin of the K1 kernel this chain picks.  Totals as in run_job; bit_tot may be NULL.
+int run_masked_impl(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, const double* chan,
+                    int L, int C, const double* snr_db, int n_snr, int64_t ensemble, const Segments* segs, uint64_t seed,
+                    uint32_t variant, int roll_off, int shard_index, int shard_count, int resolve, int64_t* bit_err,
+                    int64_t* sym_err, int64_t* sym_tot, int64_t* bit_tot) {
+    const Segments all = segs ? Segments() : job_segments(C, std::vector<int64_t>(n_snr, ensemble));
+    const Segments& sg = segs ? *segs : all;
+    const ShardRule r = ShardRule::block(sg.n_local, shard_index, shard_count);
     MaskedJob J;
-    rc = masked_setup(J, h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, seed, variant, roll_off, resolve, f_hi - f_lo, 0);
+    int rc = masked_setup(J, h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, seed, variant, roll_off, resolve,
+                          r.hi - r.lo, segs ? segs->n() : 0);
+    if (!rc) rc = masked_run(J, r.lo, r.hi, segs, bit_err, sym_err);
     if (rc) return rc;
-    return masked_run(J, f_lo, f_hi, nullptr, bit_err, sym_err);
-}
-
-// totals of counter cells [n_snr][Cr][Nr] from the frames of each cell (si, c) (c < Cr): S-1 symbols per active bin and
-// frame, 0 on guard bins; Nr == 1: every active bin of the frame
-void cell_totals(const wofdm_sys_t& s, const std::vector<long long>& frames, int Nr, int64_t* sym_tot) {
-    const long long active = s.N - 2 * s.guard;
-    for (size_t cell = 0; cell < frames.size(); ++cell) {
-        int64_t* out = sym_tot + cell * Nr;
-        if (Nr == 1) { out[0] = frames[cell] * active * (s.S - 1); continue; }
-        for (int k = 0; k < Nr; ++k) {
-            const int cc = (k + Nr / 2) & (Nr - 1);                   // ber_kernel.cuh: bin_active
-            out[k] = (cc >= s.guard && cc < Nr - s.guard) ? frames[cell] * (s.S - 1) : 0;
-        }
-    }
+    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? sys->N : 1;
+    cell_totals(*sys, cell_frames(sg, n_snr, C, Cr, r), Nr, sym_tot, bit_tot);
+    return WOFDM_OK;
 }
 
 }  // namespace
@@ -1470,18 +1460,11 @@ int wofdm_ber_run_masked_shard(wofdm_handle h, const wofdm_sys_t* sys, const dou
                                int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot) {
     NvtxRange nvtx_("wofdm_ber_run_masked");
     if (!h) return WOFDM_EINVAL;
-    long long f_lo = 0, f_hi = 0;
-    const int rc = run_masked_impl(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, seed, variant, roll_off,
-                                   shard_index, shard_count, 0, bit_err && bit_tot && sym_err && sym_tot, bit_err, sym_err,
-                                   &f_lo, &f_hi);
+    const int rc = check_masked(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, roll_off, shard_index, shard_count, 0,
+                                bit_err && bit_tot && sym_err && sym_tot);
     if (rc) return rc;
-    const long long per_snr = (long long)C * ensemble;
-    for (int i = 0; i < n_snr; ++i) {           // this shard's frames of point i: [i, i+1) * C * ensemble inside [f_lo, f_hi)
-        const long long frames = std::max(0LL, std::min(f_hi, (i + 1) * per_snr) - std::max(f_lo, i * per_snr));
-        sym_tot[i] = frames * (sys->N - 2 * sys->guard) * (sys->S - 1);   // active sub-carriers only
-        bit_tot[i] = sym_tot[i] * sys->bits;
-    }
-    return WOFDM_OK;
+    return run_masked_impl(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, nullptr, seed, variant, roll_off,
+                           shard_index, shard_count, 0, bit_err, sym_err, sym_tot, bit_tot);
 }
 
 int wofdm_ber_run_masked_resolved(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
@@ -1490,30 +1473,14 @@ int wofdm_ber_run_masked_resolved(wofdm_handle h, const wofdm_sys_t* sys, const 
                                   int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot) {
     NvtxRange nvtx_("wofdm_ber_run_masked_resolved");
     if (!h) return WOFDM_EINVAL;
-    if (resolve == 0 || (resolve & ~(WOFDM_BY_SUBCARRIER | WOFDM_BY_CHANNEL)))
-        return fail(h, WOFDM_EINVAL, "resolve must be a non-empty combination of WOFDM_BY_SUBCARRIER and WOFDM_BY_CHANNEL");
-    if (!bit_err || !sym_err || !sym_tot) return fail(h, WOFDM_EINVAL, "NULL output buffer");
-    long long f_lo = 0, f_hi = 0;
-    const int rc = run_masked_impl(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, seed, variant, roll_off,
-                                   shard_index, shard_count, resolve, true, bit_err, sym_err, &f_lo, &f_hi);
+    int rc = check_resolve(h, resolve, true);
     if (rc) return rc;
-    // this shard's frames per cell (si, c): [(si*C + c)*ensemble, +ensemble) inside [f_lo, f_hi); guard bins count nothing
-    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? sys->N : 1;
-    const long long active = sys->N - 2 * sys->guard;
-    for (int si = 0; si < n_snr; ++si)
-        for (int c = 0; c < Cr; ++c) {
-            const long long lo = ((long long)si * C + (Cr > 1 ? c : 0)) * ensemble, hi = lo + (Cr > 1 ? 1 : (long long)C) * ensemble;
-            const long long frames = std::max(0LL, std::min(f_hi, hi) - std::max(f_lo, lo));
-            int64_t* out = sym_tot + ((size_t)si * Cr + c) * Nr;
-            if (Nr == 1) { out[0] = frames * active * (sys->S - 1); continue; }
-            for (int k = 0; k < Nr; ++k) {
-                const int cc = (k + Nr / 2) & (Nr - 1);               // ber_kernel.cuh: bin_active
-                out[k] = (cc >= sys->guard && cc < Nr - sys->guard) ? frames * (sys->S - 1) : 0;
-            }
-        }
-    return WOFDM_OK;
+    if (!bit_err || !sym_err || !sym_tot) return fail(h, WOFDM_EINVAL, "NULL output buffer");
+    rc = check_masked(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, roll_off, shard_index, shard_count, resolve, true);
+    if (rc) return rc;
+    return run_masked_impl(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, nullptr, seed, variant, roll_off,
+                           shard_index, shard_count, resolve, bit_err, sym_err, sym_tot, nullptr);
 }
-
 
 int wofdm_ber_run_masked_segments(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
                                   const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble_max,
@@ -1522,35 +1489,14 @@ int wofdm_ber_run_masked_segments(wofdm_handle h, const wofdm_sys_t* sys, const 
                                   int64_t* sym_tot) {
     NvtxRange nvtx_("wofdm_ber_run_masked_segments");
     if (!h) return WOFDM_EINVAL;
-    if (resolve & ~(WOFDM_BY_SUBCARRIER | WOFDM_BY_CHANNEL))
-        return fail(h, WOFDM_EINVAL, "resolve must be a combination of WOFDM_BY_SUBCARRIER and WOFDM_BY_CHANNEL");
-    int rc = masked_check(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, roll_off, shard_index, shard_count,
-                          resolve, bit_err && sym_err && sym_tot);
+    int rc = check_resolve(h, resolve, false);
+    if (!rc) rc = check_masked(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, roll_off, shard_index, shard_count,
+                               resolve, bit_err && sym_err && sym_tot);
+    if (!rc) rc = check_segments(h, segments, n_seg, n_snr, ensemble_max);
     if (rc) return rc;
-    rc = check_segments(h, segments, n_seg, n_snr, ensemble_max);
-    if (rc) return rc;
-    std::vector<long long> tab;
-    long long n_local = 0;
-    seg_table(segments, n_seg, C, tab, &n_local);
-    // this shard's block of local indices [lo, hi), as wofdm_ber_run_masked_shard splits frame ids
-    const long long lo = (long long)((__int128)n_local * shard_index / shard_count);
-    const long long hi = (long long)((__int128)n_local * (shard_index + 1) / shard_count);
-    MaskedJob J;
-    rc = masked_setup(J, h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, seed, variant, roll_off, resolve,
-                      hi - lo, n_seg);
-    if (rc) return rc;
-    rc = masked_run(J, lo, hi, &tab, bit_err, sym_err);
-    if (rc) return rc;
-    // this shard's frames per cell (si, c): the local indices of the cell's ranges inside [lo, hi)
-    const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? sys->N : 1;
-    std::vector<long long> frames((size_t)n_snr * Cr, 0);
-    for (int k = 0; k < n_seg; ++k) {
-        const long long g0 = tab[4 * k], ec = tab[4 * k + 3];
-        for (int c = 0; c < C; ++c)
-            frames[(size_t)tab[4 * k + 1] * Cr + (Cr > 1 ? c : 0)] += std::max(0LL, std::min(hi, g0 + (c + 1) * ec) - std::max(lo, g0 + c * ec));
-    }
-    cell_totals(*sys, frames, Nr, sym_tot);
-    return WOFDM_OK;
+    const Segments sg = seg_table(segments, n_seg, C);
+    return run_masked_impl(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, &sg, seed, variant, roll_off,
+                           shard_index, shard_count, resolve, bit_err, sym_err, sym_tot, nullptr);
 }
 
 int wofdm_ber_run_masked_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
@@ -1562,14 +1508,14 @@ int wofdm_ber_run_masked_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const 
     NvtxRange nvtx_("wofdm_ber_run_masked_adaptive");
     if (!h) return WOFDM_EINVAL;
     const bool outputs_ok = ensemble_used && bit_err && bit_tot && sym_err && sym_tot && rounds;
-    int rc = masked_check(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, roll_off, shard_index, shard_count, 0,
+    int rc = check_masked(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, roll_off, shard_index, shard_count, 0,
                           outputs_ok);
-    if (rc) return rc;
-    rc = check_target(h, target_kind, target, first_block, shard_count, reduce);
+    if (!rc) rc = check_target(h, target_kind, target, first_block, shard_count, reduce);
     if (rc) return rc;
     if (variant > 0xfffffff0u - WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "variant too large");
     // row 0: the masked chain (noise stream variant + 1), set up once for the largest round of this shard; row 1: the
-    // unmasked chain, a plan of its own device buffers (the masked chain's live in the arena)
+    // unmasked chain, a plan of its own device buffers (the masked chain's live in the arena).  Each row shards by its
+    // chain's rule.
     const long long total = (long long)n_snr * C * ensemble_max;
     MaskedJob J;
     rc = masked_setup(J, h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, seed, variant + 1, roll_off, 0,
@@ -1578,49 +1524,16 @@ int wofdm_ber_run_masked_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const 
     wofdm_ber_plan p = nullptr;
     rc = plan_create_impl(h, sys, win_tx, win_rx, 1, chan, L, C, snr_db, n_snr, &p, false, 0, n_snr);
     if (rc) return rc;
-    const size_t ns = (size_t)n_snr;
-    std::vector<int64_t> used(ns, 0), block(ns, std::min(first_block, ensemble_max)), red(4 * ns), tbit(2 * ns, 0), tsym(2 * ns, 0);
-    std::vector<int64_t> rbit(2 * ns), rsym(2 * ns);
-    std::vector<char> done(ns, 0);
-    std::vector<long long> tab;
-    int nround = 0;
-    for (;;) {
-        // this round: the active points in ascending SNR order, block[s] ensemble indices each from used[s]
-        std::vector<int64_t> seg;
-        for (size_t s = 0; s < ns; ++s)
-            if (!done[s]) { seg.push_back((int64_t)s); seg.push_back(used[s]); seg.push_back(block[s]); }
-        if (seg.empty()) break;
-        long long n_local = 0;
-        seg_table(seg.data(), (int)(seg.size() / 3), C, tab, &n_local);
-        const long long lo = (long long)((__int128)n_local * shard_index / shard_count);
-        const long long hi = (long long)((__int128)n_local * (shard_index + 1) / shard_count);
-        rc = masked_run(J, lo, hi, &tab, rbit.data(), rsym.data());
-        if (!rc) rc = run_segment_table(p, tab, n_local, ensemble_max, seed, variant, shard_index, shard_count, rbit.data() + ns, rsym.data() + ns);
-        if (rc) break;
-        ++nround;
-        for (size_t k = 0; k < 2 * ns; ++k) { red[2 * k] = rbit[k]; red[2 * k + 1] = rsym[k]; }   // [2][n_snr][2]
-        if (reduce && reduce(red.data(), (int64_t)red.size(), reduce_user) != 0) {
-            rc = fail(h, WOFDM_EINVAL, "the reduce callback failed");
-            break;
-        }
-        for (size_t k = 0; k < 2 * ns; ++k) { tbit[k] += red[2 * k]; tsym[k] += red[2 * k + 1]; }
-        for (size_t s = 0; s < ns; ++s) {
-            if (done[s]) continue;
-            const std::vector<int64_t>& t = target_kind == WOFDM_TARGET_BIT_ERRORS ? tbit : tsym;
-            done[s] = schedule_step(std::min(t[s], t[ns + s]), target, ensemble_max, &used[s], &block[s]);
-        }
-    }
+    rc = run_adaptive(h, *sys, C, n_snr, 2, ensemble_max, first_block, target_kind, target, reduce, reduce_user,
+                      [&](const Segments& sg, int64_t* be, int64_t* se) {
+                          const ShardRule r = ShardRule::block(sg.n_local, shard_index, shard_count);
+                          const int rc_m = masked_run(J, r.lo, r.hi, &sg, be, se);
+                          if (rc_m) return rc_m;
+                          return run_plan(p, ensemble_max, seed, variant, shard_index, shard_count, &sg, be + n_snr, se + n_snr);
+                      },
+                      ensemble_used, bit_err, bit_tot, sym_err, sym_tot, rounds);
     wofdm_ber_plan_destroy(p);
-    if (rc) return rc;
-    *rounds = nround;
-    const long long per_frame = (long long)(sys->N - 2 * sys->guard) * (sys->S - 1);
-    for (size_t s = 0; s < ns; ++s) {
-        ensemble_used[s] = used[s];
-        sym_tot[s] = (int64_t)C * used[s] * per_frame;
-        bit_tot[s] = sym_tot[s] * sys->bits;
-    }
-    for (size_t k = 0; k < 2 * ns; ++k) { bit_err[k] = tbit[k]; sym_err[k] = tsym[k]; }
-    return WOFDM_OK;
+    return rc;
 }
 
 }  // extern "C"
