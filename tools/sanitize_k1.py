@@ -1,6 +1,6 @@
 """The K1 production kernels with SEVERAL frames per CTA (the reuse of shared memory from frame to frame without a closing
 barrier is what a race checker should look at), small enough for `compute-sanitizer --tool racecheck`:
-    compute-sanitizer --tool racecheck python tools/sanitize_k1.py [n256|multi|n1024]"""
+    compute-sanitizer --tool racecheck python tools/sanitize_k1.py [n256|multi|wtx|n1024]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -16,6 +16,13 @@ if which == "n512":
     s = W.params_from_name("CPW", 512, 32, 16, 20, bits=6, S=16, noise_norm=1, constellation=1)
     vt, vr = capi.rc_window_tx(s), capi.rc_window_rx(s)
     r = h.ber_run(s, vt, vr, chan, snr, 80, seed=1)                      # 480 frames on 148 CTAs
+elif which == "wtx":                                                     # the fixed-shape instance (ber_tconv2.cuh: HS)
+    s = W.params_from_name("wtx", 256, 16, 8, 0, bits=4, S=16, noise_norm=1, constellation=1)
+    vt, vr = capi.rc_window_tx(s), capi.rc_window_rx(s)
+    plan = h.ber_plan(s, vt, vr, chan, snr)
+    print("KERNEL", plan.kernel)
+    plan.close()
+    r = h.ber_run(s, vt, vr, chan, snr, 150, seed=1)                     # 900 frames on <= 296 CTAs
 elif which in ("n256", "multi"):
     s = W.params_from_name("WOLA", 256, 16, 8, 10, bits=4, S=16, noise_norm=0, constellation=0)
     vt, vr = capi.rc_window_tx(s), capi.rc_window_rx(s)

@@ -53,6 +53,20 @@ struct Choice {
     int chunk = 0, use_global = 0;
 };
 
+// a Tx window that is one non-zero value between its tails, which lie inside the prefix and the suffix
+bool flat_tx_window(const wofdm_sys_t& s, const double* wt) {
+    const int n_tx = s.N + s.cp + s.cs;
+    bool ft = s.cp >= s.tail_tx && s.cs >= s.tail_tx && wt[s.tail_tx] != 0.0;
+    for (int i = s.tail_tx; ft && i < n_tx - s.tail_tx; ++i) ft = wt[i] == wt[s.tail_tx];
+    return ft;
+}
+
+// the shape class of the fixed-shape tensor-core kernels (ber_tconv2.cuh: HS): one window pair with a flat Tx window
+// (BerParams::flat_tx), no Rx window tails, no guard band, symbols drawn in the kernel (no Tx stream from the mask chain)
+bool tconv2_fixed_shape(const wofdm_sys_t& s, const double* win_tx, int nvar, bool want_txs, bool want_txy) {
+    return win_tx != nullptr && nvar == 1 && !want_txs && !want_txy && s.tail_rx == 0 && s.guard == 0 && flat_tx_window(s, win_tx);
+}
+
 // tensor-core kernel: windows that are one value between their tails (BerParams::flat_tx / flat_rx)
 // (n_var window pairs back to back: bit v of flat_tx / flat_rx = pair v)
 void fill_flat(BerParams& prm, const wofdm_sys_t& s, const double* win_tx, const double* win_rx, int n_var = 1) {
@@ -61,8 +75,7 @@ void fill_flat(BerParams& prm, const wofdm_sys_t& s, const double* win_tx, const
     for (int v = 0; v < n_var; ++v) {
         const double* wt = win_tx + (size_t)v * n_tx;
         const double* wr = win_rx + (size_t)v * n_wr;
-        bool ft = s.cp >= s.tail_tx && s.cs >= s.tail_tx && wt[s.tail_tx] != 0.0;
-        for (int i = s.tail_tx; ft && i < n_tx - s.tail_tx; ++i) ft = wt[i] == wt[s.tail_tx];
+        const bool ft = flat_tx_window(s, wt);
         bool fr = wr[s.tail_rx] != 0.0;
         for (int i = s.tail_rx; fr && i < s.N; ++i) fr = wr[i] == wr[s.tail_rx];
         prm.flat_tx |= (ft ? 1 : 0) << v;
@@ -93,6 +106,7 @@ int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, bool verify, bool 
     const char* want = getenv("WOFDM_VARIANT");
     if (no_tconv || getenv("WOFDM_NO_TCONV")) no_tconv = true;
     const int tconv_gen = getenv("WOFDM_TCONV_GEN") ? atoi(getenv("WOFDM_TCONV_GEN")) : 2;   // 1: ber_tconv.cuh, 2: ber_tconv2.cuh
+    const bool fixed_shape = tconv2_fixed_shape(s, win_tx, nvar, want_txs, want_txy);
     if (!fp64 && !force_staged) {
         for (const auto& v : h->variants) {
             if (v.TC == 0 || v.fp64 || v.verify != verify || v.N != s.N) continue;
@@ -108,6 +122,7 @@ int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, bool verify, bool 
                 if (no_tconv || S_cta > v.NT / tpf || L > v.LB) continue;
                 if (v.gen != tconv_gen) continue;
                 if (v.txy != want_txy) continue;                     // (the mask product's consumers serve the channel-mask variant only)
+                if (v.fixed_shape && !fixed_shape) continue;
                 if (v.CL > 1 && want_txs) continue;                  // (the masked Tx stream is a one-CTA-per-frame feature)
                 // second generation: a receiver thread holds at most N48_MAXLEV noise samples besides its 16 FFT rows
                 if (v.gen == 2 && (stride - s.N + (s.noise_norm == 1 ? s.tail_tx + L - 1 : 0) + tpf - 1) / tpf > (v.LB > TCV_LB ? N48_MAXLEV : N48_MAXLEV_SHORT)) continue;
@@ -117,8 +132,10 @@ int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, bool verify, bool 
                 if (nvar > 1 && v.gen != 2) continue;                // (several window pairs per launch: ber_tconv2.cuh only)
                 const BerSmem lay = v.layout(S_cta, stride, s.tail_tx, s.tail_rx, L, v.gen == 2 ? nvar : 0, 0);
                 if (lay.bytes > smem_cap) continue;
-                // fewest taps of history first (MMAs per tile), then fewest tiles
-                if (!best.var || best.var->ntile == 0 || v.LB < best.var->LB || (v.LB == best.var->LB && v.ntile < best.var->ntile)) {
+                // fewest taps of history first (MMAs per tile), then fewest tiles, then the fixed-shape instance
+                // (same noise numbering and arithmetic, counters bit for bit: 3856 SASS instructions instead of 4976)
+                if (!best.var || best.var->ntile == 0 || v.LB < best.var->LB ||
+                    (v.LB == best.var->LB && (v.ntile < best.var->ntile || (v.ntile == best.var->ntile && v.fixed_shape)))) {
                     best.var = &v; best.lay = lay; best.chunk = 0;
                 }
                 continue;
@@ -548,7 +565,8 @@ static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double
     // their tables; otherwise the pairs are launched one after the other on the same draws (same counters either way)
     rc = choose_variant(h, *sys, L, false, false, cap, &ch, win_tx, false, false, false, n_var);
     p->fused = rc == WOFDM_OK && n_var > 1 && ch.var->gen == 2;
-    if (n_var > 1 && !p->fused) rc = choose_variant(h, *sys, L, false, false, cap, &ch, win_tx, /*no_circ=*/true);
+    // (one launch per pair: no Tx window is passed, so no kernel that relies on the flatness of pair 0's is chosen)
+    if (n_var > 1 && !p->fused) rc = choose_variant(h, *sys, L, false, false, cap, &ch, nullptr, /*no_circ=*/true);
     if (rc) { delete p; return rc; }
     p->noise_var = ch.var;
     p->cnt_per_var = (size_t)n_snr * 2;

@@ -18,6 +18,7 @@ struct BerVariant {
     int gen;                   // tensor-core kernels: 1 = ber_tconv.cuh (64-bit noise draws by position), 2 = ber_tconv2.cuh (48-bit draws)
     bool txy = false;          // ber_tconv2.cuh: takes the Tx stream from the mask product's output (BerParams::tx_y) and nothing else
     bool res = false;          // counters resolved by sub-carrier / channel (BerParams::res_bins / res_chan) and nothing else
+    bool fixed_shape = false;  // ber_tconv2.cuh HS: the switches of one shape class as constants (ber_host.cu: tconv2_fixed_shape)
     bool fp64, verify;
     BerSmem (*layout)(int S, int stride, int tail_tx, int tail_rx, int L, int chunk, int use_global);
     const void* fn;
@@ -84,6 +85,7 @@ struct BerVariantImpl {
 void register_ber_f32_staged(std::vector<BerVariant>& out);
 void register_ber_f32_tconv(std::vector<BerVariant>& out);
 void register_ber_f32_tconv2(std::vector<BerVariant>& out);
+void register_ber_f32_tconv2_hs(std::vector<BerVariant>& out);       // ... its fixed-shape instances
 void register_ber_f64_staged(std::vector<BerVariant>& out);
 void register_ber_f32_regs(std::vector<BerVariant>& out);
 void register_ber_f32_regs_big(std::vector<BerVariant>& out);

@@ -226,7 +226,11 @@ __host__ __device__ inline BerSmem tconv2_smem_layout(int S, int stride, int tai
 // taps are PUSHED into both CTAs, so every read is local.
 // RES: error counters resolved by sub-carrier and / or channel (BerParams::res_chan / res_bins, ber_kernel.cuh: res_flush);
 // in a cluster every CTA keeps and flushes the accumulators of its own symbols
-template <int N, int NT, int NTILE, int MINB, bool VERIFY, int CL = 1, int LB = TCV_LB, bool TXY = false, bool RES = false>
+// HS: the frame loop of the common shape class compiled with its switches as constants (ber_host.cu: tconv2_fixed_shape):
+// a flat Tx window with cp, cs >= tail_tx, tail_rx = 0, one window pair, no guard band, the symbols drawn in the kernel.
+// N, S, L, the Rx window's flatness and the conventions (noise_norm, constellation) stay run-time.
+template <int N, int NT, int NTILE, int MINB, bool VERIFY, int CL = 1, int LB = TCV_LB, bool TXY = false, bool RES = false,
+          bool HS = false>
 __global__ void __launch_bounds__(NT + tconv2_mma_warp_threads(N, NT), MINB)
 ber_tconv2_kernel(const BerParams prm) {
     using T = float;
@@ -241,6 +245,7 @@ ber_tconv2_kernel(const BerParams prm) {
     static_assert(16 * NTILE <= (int)TMEM_COLS, "accumulators of a frame must fit tensor memory");
     static_assert(CL * NW <= 32, "per-warp power partials of all CTAs must fit the reduction scratch");
     static_assert(!RES || !VERIFY, "resolved counters: production kernels");
+    static_assert(!HS || (CL == 1 && !VERIFY && !TXY && !RES), "the fixed-shape frame loop: one-CTA production kernels");
 
     extern __shared__ __align__(128) unsigned char tcv_smem[];
     unsigned char* const smem_raw = tcv_smem;
@@ -253,13 +258,13 @@ ber_tconv2_kernel(const BerParams prm) {
     const int S = prm.S / CL, sb = rank * S;    // this CTA's symbols: sb .. sb + S - 1 (the whole frame when CL == 1)
     const int stride = prm.stride, n_tx = prm.n_tx, beta = prm.tail_tx, L = prm.L;
     const int cp = prm.cp, cs = prm.cs;
-    const int hh = prm.tail_rx >> 1;
+    const int hh = HS ? 0 : prm.tail_rx >> 1;
     const int hb = prm.bits >> 1, m = 1 << hb;
     const int sec = S * stride;                 // samples kept after the channel (this CTA's)
     const int body = beta + sec;                // serialised Tx stream length
     const int npow = (prm.noise_norm == 1 && last_rank) ? body + L - 1 : sec;   // samples inside the frame-wide power sums
 
-    const int nvar = (!VERIFY && prm.nvar > 1) ? prm.nvar : 1;     // window pairs evaluated on every frame's symbols
+    const int nvar = (!VERIFY && !HS && prm.nvar > 1) ? prm.nvar : 1;     // window pairs evaluated on every frame's symbols
     constexpr int PAD = tconv2_pad(LB), KS = tconv2_ksteps(LB), TBL = tconv2_tbl(LB), ZERO = tconv2_zero(LB);
     const BerSmem lay = tconv2_smem_layout<N, NT, NTILE, LB, RES>(S, stride, beta, prm.tail_rx, L, nvar, 0);
     uint32_t* const ahi = reinterpret_cast<uint32_t*>(smem_raw);
@@ -328,7 +333,7 @@ ber_tconv2_kernel(const BerParams prm) {
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem = *tmem_slot;
-    if (prm.guard > 0) {
+    if (!HS && prm.guard > 0) {
         const unsigned d0 = slice_index(mk2<T>(0, 0), hb);
         for (int tt = tid; tt < TPF; tt += NT) {
             uint32_t ff[4] = {0, 0, 0, 0}, dd[4] = {0, 0, 0, 0};
@@ -466,7 +471,7 @@ ber_tconv2_kernel(const BerParams prm) {
       // every window pair of the plan on this frame's symbols (drawn once), each with its own noise stream
       // (wofdm_simulation.py:183-236: optimised and RC windows on one signal_digmod; main_BER_calculation.m:118-198)
       for (int var = 0; var < nvar; ++var) {
-        const bool flat_tx = (prm.flat_tx >> var) & 1, flat_rx = (prm.flat_rx >> var) & 1;
+        const bool flat_tx = HS || ((prm.flat_tx >> var) & 1), flat_rx = (prm.flat_rx >> var) & 1;
         const T* const wtx = wtx_all + var * WTXL;
         const T* const wrx = wrx_all + var * WRXL;
         // ---- taps operand of this frame: n = 2o + comp (o < 4), K pair jj = sample offset in the row, tap l = LB-1 + o - jj
@@ -505,7 +510,7 @@ ber_tconv2_kernel(const BerParams prm) {
         }
 
         // =========================== transmitter ===========================
-        if (prm.tx_stream != nullptr) {          // uniform: masked Tx stream from tx_mask_kernel (mask_kernel.cuh)
+        if (!HS && prm.tx_stream != nullptr) {          // uniform: masked Tx stream from tx_mask_kernel (mask_kernel.cuh)
             for (int e = tid; e < S * TPF; e += NT) {
                 const int tt = e % TPF;
                 uint32_t w[4];
@@ -549,7 +554,7 @@ ber_tconv2_kernel(const BerParams prm) {
                 }
 #pragma unroll
                 for (int jw = 0; jw < 4; ++jw) wq[jw] = w[jw];
-                if (prm.guard > 0) {
+                if (!HS && prm.guard > 0) {
                     const uint4 gf = gmask[2 * t], gd = gmask[2 * t + 1];
                     const uint32_t ff[4] = {gf.x, gf.y, gf.z, gf.w}, dd[4] = {gd.x, gd.y, gd.z, gd.w};
 #pragma unroll
@@ -632,7 +637,7 @@ ber_tconv2_kernel(const BerParams prm) {
                         }
                     }
                 }
-                if (cp < beta) {
+                if (!HS && cp < beta) {
 #pragma unroll
                     for (int q = 0; q < ER; ++q) {
                         const int i = t + q * TPF + cp;
@@ -741,6 +746,18 @@ ber_tconv2_kernel(const BerParams prm) {
         //  count in the noise power and are dropped)
         C2 nz[16], nx[2];
         C2 pr2 = mk2<T>(0, 0), pn2 = mk2<T>(0, 0), pnx = mk2<T>(0, 0);
+        // HS: the draws are register arithmetic only, and with the switches as constants ptxas hoists most of them above the
+        // bar.arrive above (468 SASS instructions between the Tx barrier and the arrive instead of 112): the MMA warp then waits
+        // for every working warp's draws before it issues, and the accumulator pass waits for the MMAs.  So there the draws key
+        // on a frame id that passes through a shared-memory load behind the arrive (ahi[0], the operand's zero pad: always 0),
+        // which ptxas does not move across the barrier.
+        long long fn = f;
+        if constexpr (HS) {
+            static_assert(CL == 1, "ahi[0] is zero only with one CTA per frame: a CTA of rank > 0 writes its neighbour's history there");
+            uint32_t z;
+            asm volatile("ld.volatile.shared.u32 %0, [%1];" : "=r"(z) : "r"(tcv_smem_u32(ahi)) : "memory");
+            fn += z;
+        }
         {
             const bool act = slot < S;
             const int se = act ? TCV2_SLOT_SYMBOL(slot, S) : S - 1;
@@ -762,8 +779,8 @@ ber_tconv2_kernel(const BerParams prm) {
                 const uint32_t q0 = (uint32_t)(sg * TPF + t) * (uint32_t)N48_CALLS;
 #pragma unroll
                 for (int gq = 0; gq < 2; ++gq) {
-                    const uint4 ca = noise48_call(prm, f, q0 + 3 * gq, var), cb = noise48_call(prm, f, q0 + 3 * gq + 1, var);
-                    const uint4 cc = noise48_call(prm, f, q0 + 3 * gq + 2, var);
+                    const uint4 ca = noise48_call(prm, fn, q0 + 3 * gq, var), cb = noise48_call(prm, fn, q0 + 3 * gq + 1, var);
+                    const uint4 cc = noise48_call(prm, fn, q0 + 3 * gq + 2, var);
                     gauss_quad48(ca.x, ca.y, cc.x, nz[8 * gq + 0], nz[8 * gq + 1]);
                     gauss_quad48(ca.z, ca.w, cc.y, nz[8 * gq + 2], nz[8 * gq + 3]);
                     gauss_quad48(cb.x, cb.y, cc.z, nz[8 * gq + 4], nz[8 * gq + 5]);
@@ -772,21 +789,21 @@ ber_tconv2_kernel(const BerParams prm) {
                 }
                 nx[0] = nx[1] = mk2<T>(0, 0);
                 if (nlev > 0) {                                          // uniform per transform group
-                    const uint4 c6 = noise48_call(prm, f, q0 + 6, var);
+                    const uint4 c6 = noise48_call(prm, fn, q0 + 6, var);
                     gauss_quad48(c6.y, c6.z, c6.x, nx[0], nx[1]);
                     if (xt >= xas) nx[0] = mk2<T>(0, 0);
                     if (xt + TPF >= xas) nx[1] = mk2<T>(0, 0);
                     // further level pairs (long prefixes; the last symbol under MATLAB's full-convolution sums): rare, out of line
                     if constexpr (LB > TCV_LB) {
-                        if (nlev > 2) pnx = n48_more_extras(prm, f, q0, var, nlev, xt, TPF, xas);
+                        if (nlev > 2) pnx = n48_more_extras(prm, fn, q0, var, nlev, xt, TPF, xas);
                     } else if (nlev > 2) {                               // (at most N48_MAXLEV_SHORT = 6 levels: ber_host.cu)
-                        const uint4 c7 = noise48_call(prm, f, q0 + 7, var);
+                        const uint4 c7 = noise48_call(prm, fn, q0 + 7, var);
                         C2 e2, e3;
                         gauss_quad48(c7.x, c7.y, c6.w, e2, e3);
                         if (xt + 2 * TPF < xas) pnx = csq_acc(e2, pnx);
                         if (xt + 3 * TPF < xas) pnx = csq_acc(e3, pnx);
                         if (nlev > 4) {
-                            const uint4 c8 = noise48_call(prm, f, q0 + 8, var);
+                            const uint4 c8 = noise48_call(prm, fn, q0 + 8, var);
                             gauss_quad48(c7.w, c8.x, c7.z, e2, e3);
                             if (xt + 4 * TPF < xas) pnx = csq_acc(e2, pnx);
                             if (xt + 5 * TPF < xas) pnx = csq_acc(e3, pnx);
@@ -964,7 +981,7 @@ ber_tconv2_kernel(const BerParams prm) {
                     const C2 y0 = geq[k];
                     const C2 x0 = qlut[pil[(k % TPF) * 16 + k / TPF]];
                     C2 gk = cscale(((TCV2_FOLD_SLICER && !VERIFY) ? (T)0.5 : (T)1) * recip(y0.x * y0.x + y0.y * y0.y), cmulc(x0, y0));
-                    if (prm.guard > 0 && !bin_active<N>(k, prm.guard)) gk = mk2<T>(0, 0);
+                    if (!HS && prm.guard > 0 && !bin_active<N>(k, prm.guard)) gk = mk2<T>(0, 0);
                     geq[k] = gk;
                     if constexpr (CL > 1) {
 #pragma unroll

@@ -143,6 +143,7 @@ int wofdm_create_on(wofdm_handle* out, const int* device_ids, int n) {
     }
     register_ber_f32_tconv(h->variants);
     register_ber_f32_tconv2(h->variants);
+    register_ber_f32_tconv2_hs(h->variants);
     register_ber_f32_regs(h->variants);
     register_ber_f32_staged(h->variants);
     register_ber_f64_staged(h->variants);
