@@ -31,7 +31,6 @@ ROWS = {
     "tconv2_n512": ("CPW", 512, 32, 16, 20, 4, 21, 2, 0, {}, ["f32t2_n512"], 1, 0, 4, 2500),
     "tconv2_n1024": ("WOLA", 1024, 64, 32, 40, 6, 21, 2, 0, {}, ["f32t2_n1024", "_cl2"], 0, 0, 4, 10000),
     "tconv2_n1024_l84": ("CPW", 1024, 64, 32, 40, 6, 84, 1, 0, {}, ["f32t2_n1024", "_l84"], 1, 0, 4, 20000),
-    "tconv1_n256": ("WOLA", 256, 16, 8, 10, 4, 21, 1, 0, {"WOFDM_TCONV_GEN": "1"}, ["ber_f32t_n256"], 0, 0, 4, 10000),
     "regs_n256_exact_fit": ("WOLA", 256, 16, 8, 10, 4, 21, 1, 0, {"WOFDM_NO_TCONV": "1"}, ["ber_f32r_n256", "_ftrue", "!_circ"], 1, 0, 4, 10000),
     "regs_n256_circ": ("wrx", 256, 16, 0, 10, 4, 21, 1, 0, {"WOFDM_NO_TCONV": "1"}, ["ber_f32r_n256", "_circ"], 0, 0, 4, 10000),
     "regs_n512": ("WOLA", 512, 32, 16, 20, 4, 21, 2, 0, {"WOFDM_NO_TCONV": "1"}, ["ber_f32r_n512"], 0, 0, 4, 2500),
@@ -43,7 +42,7 @@ ROWS = {
     "guard_tconv2_n1024": ("WOLA", 1024, 64, 32, 40, 6, 21, 1, 0, {}, ["f32t2_n1024"], 1, 256, 4, 20000),
 }
 BIG = 3e8                                    # decisions per reassignment of the fp32 tensor-core and register rows
-ENV = ("WOFDM_NO_TCONV", "WOFDM_TCONV_GEN", "WOFDM_MAX_CTAS_PER_SM", "WOFDM_DEBUG")
+ENV = ("WOFDM_NO_TCONV", "WOFDM_MAX_CTAS_PER_SM", "WOFDM_DEBUG")
 
 
 @pytest.fixture(scope="module")
@@ -159,18 +158,16 @@ def test_counters_depend_on_the_frame_alone(handle, row, monkeypatch, capfd):
     # 3. shards summed
     for K in (2, 47):
         check(f"{K} shards", summed([multi(shard=(i, K)) for i in range(K)]))
-    # 4. and 5. the resolved-counter twin of the production kernel; the first-generation tensor-core kernel has none (its
-    #    resolved calls run the staged kernel, whose fp32 arithmetic is another)
-    if "ber_f32t_" not in kernel:
-        rng = np.random.default_rng(F)
-        segs = random_segments(rng, len(snr), E, 3)
-        check("segments", summed([handle.ber_run_segments(s, wt, wr, chans, snr, E, sg, seed=seed, variant=variant) for sg in segs]))
-        kw = dict(seed=seed, variant=variant, by_subcarrier=True, by_channel=True)
-        res = handle.ber_run_resolved(s, wt, wr, chans, snr, E, **kw)
-        check("resolved, summed over channels and bins", {k: res[k].sum(axis=(-2, -1)) for k in ("bit_err", "sym_err", "sym_tot", "bit_tot")})
-        K = 47
-        parts = summed([handle.ber_run_resolved(s, wt, wr, chans, snr, E, shard=(i, K), **kw) for i in range(K)])
-        check(f"resolved, {K} shards, cell by cell", parts, want=res)
+    # 4. and 5. the resolved-counter twin of the production kernel
+    rng = np.random.default_rng(F)
+    segs = random_segments(rng, len(snr), E, 3)
+    check("segments", summed([handle.ber_run_segments(s, wt, wr, chans, snr, E, sg, seed=seed, variant=variant) for sg in segs]))
+    kw = dict(seed=seed, variant=variant, by_subcarrier=True, by_channel=True)
+    res = handle.ber_run_resolved(s, wt, wr, chans, snr, E, **kw)
+    check("resolved, summed over channels and bins", {k: res[k].sum(axis=(-2, -1)) for k in ("bit_err", "sym_err", "sym_tot", "bit_tot")})
+    K = 47
+    parts = summed([handle.ber_run_resolved(s, wt, wr, chans, snr, E, shard=(i, K), **kw) for i in range(K)])
+    check(f"resolved, {K} shards, cell by cell", parts, want=res)
     # 6. each window pair alone
     if nv > 1:
         for v in range(nv):

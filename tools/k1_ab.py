@@ -1,5 +1,6 @@
-"""A/B timing of K1 kernel generations / variants on one GPU (development aid, not the bench).
-usage: k1_ab.py [N] [ens]   -- env WOFDM_* select variants inside the library; this script loops WOFDM_TCONV_GEN over 1, 2."""
+"""Timing of the K1 kernel a plan picks, per case, on one GPU (development aid, not the bench).
+usage: k1_ab.py [N] [ens]   -- env WOFDM_* select variants inside the library (a third argument, the kernel generations
+of earlier versions of this script, is ignored)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -9,7 +10,6 @@ from wofdm_b200 import capi
 
 N = int(sys.argv[1]) if len(sys.argv) > 1 else 256
 ens = int(sys.argv[2]) if len(sys.argv) > 2 else 27
-gens = [int(x) for x in (sys.argv[3].split(",") if len(sys.argv) > 3 else ["1", "2"])]
 scale = N // 256
 h = W.Handle([0])
 rng = np.random.default_rng(0)
@@ -31,26 +31,22 @@ for name, cp, nn, conv in cases:
     if name in ("CP", "wtx", "CPwtx"): trx = 0
     s = W.params_from_name(name, N, cp * (1 if N == 256 else 1), ttx, trx, bits=4 if N == 256 else 6, S=16, noise_norm=nn, constellation=conv)
     vt, vr = capi.rc_window_tx(s), capi.rc_window_rx(s)
-    row = []
-    for gen in gens:
-        os.environ["WOFDM_TCONV_GEN"] = str(gen)
-        plan = h.ber_plan(s, vt, vr, chan, snr)
-        for _ in range(3):
-            plan.launch(ens, seed=1, stream=st)
-        torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        K = 6
-        e0.record()
-        for k in range(K):
-            plan.launch(ens, seed=2 + k, stream=st)
-        e1.record()
-        torch.cuda.synchronize()
-        ms = e0.elapsed_time(e1) / K
-        syms = 30 * C * ens * 16
-        be, se = plan.read()
-        bt, stot = plan.totals(ens)
-        row.append((gen, plan.kernel, ms, syms / ms * 1e3, (se / stot)[[0, 15, 29]]))
-        plan.close()
-    for gen, k, ms, rate, ser in row:
-        print(f"{name:6s} cp={cp:3d} nn={nn} conv={conv} gen{gen} {k:34s} {ms:8.3f} ms {rate:.4g} sym/s  SER {np.round(ser, 5)}", flush=True)
+    plan = h.ber_plan(s, vt, vr, chan, snr)
+    for _ in range(3):
+        plan.launch(ens, seed=1, stream=st)
+    torch.cuda.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    K = 6
+    e0.record()
+    for k in range(K):
+        plan.launch(ens, seed=2 + k, stream=st)
+    e1.record()
+    torch.cuda.synchronize()
+    ms = e0.elapsed_time(e1) / K
+    syms = 30 * C * ens * 16
+    be, se = plan.read()
+    bt, stot = plan.totals(ens)
+    ser = (se / stot)[[0, 15, 29]]
+    print(f"{name:6s} cp={cp:3d} nn={nn} conv={conv} {plan.kernel:34s} {ms:8.3f} ms {syms / ms * 1e3:.4g} sym/s  SER {np.round(ser, 5)}", flush=True)
+    plan.close()
 h.close()

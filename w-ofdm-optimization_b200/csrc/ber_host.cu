@@ -61,10 +61,26 @@ bool flat_tx_window(const wofdm_sys_t& s, const double* wt) {
     return ft;
 }
 
+// where a kernel takes the Tx stream from: drawn in the kernel, read from HBM (BerParams::tx_stream, BerVariant::txs), or
+// gathered from the mask product's output (BerParams::tx_y, BerVariant::txy)
+enum class TxSource { drawn, stream, gather };
+
+// what a caller of choose_variant asks for
+struct KernelRequest {
+    bool verify = false;              // the verify instantiations (wofdm_ber_verify)
+    bool staged_only = false;
+    bool no_tconv = false;            // no tensor-core kernels
+    bool no_circ = false;             // no circular-interior kernels
+    const double* win_tx = nullptr;   // Tx window whose flatness the circular-interior and HS kernels need; NULL: neither
+    int nvar = 1;                     // window pairs per launch
+    TxSource tx = TxSource::drawn;
+};
+
 // the shape class of the fixed-shape tensor-core kernels (ber_tconv2.cuh: HS): one window pair with a flat Tx window
 // (BerParams::flat_tx), no Rx window tails, no guard band, symbols drawn in the kernel (no Tx stream from the mask chain)
-bool tconv2_fixed_shape(const wofdm_sys_t& s, const double* win_tx, int nvar, bool want_txs, bool want_txy) {
-    return win_tx != nullptr && nvar == 1 && !want_txs && !want_txy && s.tail_rx == 0 && s.guard == 0 && flat_tx_window(s, win_tx);
+bool tconv2_fixed_shape(const wofdm_sys_t& s, const KernelRequest& rq) {
+    return rq.win_tx != nullptr && rq.nvar == 1 && rq.tx == TxSource::drawn && s.tail_rx == 0 && s.guard == 0 &&
+           flat_tx_window(s, rq.win_tx);
 }
 
 // tensor-core kernel: windows that are one value between their tails (BerParams::flat_tx / flat_rx)
@@ -87,50 +103,67 @@ void fill_flat(BerParams& prm, const wofdm_sys_t& s, const double* win_tx, const
 void fill_split(BerParams& prm, const BerVariant& v) {
     prm.split = v.CL > 1 ? prm.S * prm.stride / v.CL : 0;
     prm.split_nt = v.CL > 1 ? v.NT : 0;
-    prm.n48 = v.gen == 2 ? 1 : 0;      // 48-bit noise draws in receiver layout (ber_kernel.cuh: noise_draw48)
+    prm.n48 = v.ntile > 0 ? 1 : 0;     // 48-bit noise draws in receiver layout (ber_kernel.cuh: noise_draw48)
 }
 
-// win_tx (may be NULL): the circular-interior kernels need it flat between the tails; no_circ excludes them
-int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, bool verify, bool force_staged, size_t smem_cap,
-                   Choice* out, const double* win_tx = nullptr, bool no_circ = false, bool want_txs = false,
-                   bool no_tconv = false, int nvar = 1, bool want_txy = false, bool want_resolved = false) {
+// the staged kernel (verify / resolved-counter instance) of the frame's N and precision, with noise block `chunk`: frame
+// buffers in shared memory where they fit, else in global memory (use_global)
+int choose_staged(wofdm_ctx* h, const wofdm_sys_t& s, int L, size_t smem_cap, bool verify, bool res, int chunk, Choice* out) {
+    const int stride = s.N + s.cp + s.cs - s.tail_tx;
+    for (const auto& v : h->variants) {
+        if (v.TC != 0 || v.fp64 != (s.precision == 1) || v.verify != verify || v.res != res || v.N != s.N) continue;
+        Choice c;
+        c.var = &v;
+        c.chunk = chunk;
+        c.lay = v.layout(s.S, stride, s.tail_tx, s.tail_rx, L, 0, 0);
+        if (c.lay.bytes > smem_cap) {
+            c.use_global = 1;
+            c.lay = v.layout(s.S, stride, s.tail_tx, s.tail_rx, L, 0, 1);
+            if (c.lay.bytes > smem_cap) return fail(h, WOFDM_EUNSUPPORTED, "frame does not fit the staged kernel's shared memory");
+        }
+        *out = c;
+        return WOFDM_OK;
+    }
+    return fail(h, WOFDM_EUNSUPPORTED, res ? "no compiled resolved-counter kernel for this N / precision"
+                                           : "no compiled kernel variant for this N / precision");
+}
+
+// The kernel of request rq, among those without resolved counters (BerVariant::res): a tensor-core kernel wherever one
+// applies, else a register kernel, else the staged kernel.  WOFDM_NO_TCONV and WOFDM_NO_CIRC add no_tconv / no_circ;
+// WOFDM_VARIANT=<substring> restricts the tensor-core and register candidates (kernel tuning aid, e.g. "_b2").
+int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, size_t smem_cap, const KernelRequest& rq, Choice* out) {
     const int stride = s.N + s.cp + s.cs - s.tail_tx;
     const int sec = s.S * stride;
-    const bool fp64 = s.precision == 1;
-    Choice best;
-    bool flat = win_tx != nullptr && !no_circ && !getenv("WOFDM_NO_CIRC");
+    const bool want_txs = rq.tx != TxSource::drawn, want_txy = rq.tx == TxSource::gather;
+    const bool no_tconv = rq.no_tconv || getenv("WOFDM_NO_TCONV");
+    const char* want = getenv("WOFDM_VARIANT");
+    bool flat = rq.win_tx != nullptr && !rq.no_circ && !getenv("WOFDM_NO_CIRC");
     if (flat)
         for (int i = s.tail_tx; i < s.N + s.cp + s.cs - s.tail_tx; ++i)
-            if (win_tx[i] != win_tx[s.tail_tx]) { flat = false; break; }
-    // WOFDM_VARIANT=<substring> restricts the tuned candidates (kernel tuning aid, e.g. "_b2")
-    const char* want = getenv("WOFDM_VARIANT");
-    if (no_tconv || getenv("WOFDM_NO_TCONV")) no_tconv = true;
-    const int tconv_gen = getenv("WOFDM_TCONV_GEN") ? atoi(getenv("WOFDM_TCONV_GEN")) : 2;   // 1: ber_tconv.cuh, 2: ber_tconv2.cuh
-    const bool fixed_shape = tconv2_fixed_shape(s, win_tx, nvar, want_txs, want_txy);
-    if (!fp64 && !force_staged) {
+            if (rq.win_tx[i] != rq.win_tx[s.tail_tx]) { flat = false; break; }
+    const bool fixed_shape = tconv2_fixed_shape(s, rq);
+    Choice best;
+    if (s.precision != 1 && !rq.staged_only) {
         for (const auto& v : h->variants) {
-            if (v.TC == 0 || v.fp64 || v.verify != verify || v.N != s.N) continue;
-            if (v.res != want_resolved) continue;                // (the resolved-counter twins serve wofdm_ber_run_resolved only)
+            if (v.TC == 0 || v.fp64 || v.verify != rq.verify || v.N != s.N || v.res) continue;
             if (want && !strstr(v.name, want)) continue;
             if (v.ntile > 0) {
-                // channel convolution on the tensor cores (ber_tconv.cuh): first choice wherever it applies -- one Tx pass,
-                // L <= 21, prefix / suffix / tails inside the outer register rows, power sums and the zeros behind the
-                // stream inside the frame's tiles.  Noise numbering: draw = position (chunk 0).  Takes tx_stream too.
+                // channel convolution on the tensor cores (ber_tconv2.cuh): first choice wherever it applies -- one Tx pass,
+                // L <= LB, prefix / suffix / tails inside the outer register rows, power sums and the zeros behind the
+                // stream inside the frame's tiles.  Takes tx_stream too.
                 // CL CTAs share a frame: S/CL consecutive symbols each, in one Tx pass of the CTA
                 if (s.S % v.CL != 0) continue;
                 const int tpf = s.N / 16, S_cta = s.S / v.CL, sec_cta = sec / v.CL, body = s.tail_tx + sec_cta;
                 if (no_tconv || S_cta > v.NT / tpf || L > v.LB) continue;
-                if (v.gen != tconv_gen) continue;
                 if (v.txy != want_txy) continue;                     // (the mask product's consumers serve the channel-mask variant only)
                 if (v.fixed_shape && !fixed_shape) continue;
                 if (v.CL > 1 && want_txs) continue;                  // (the masked Tx stream is a one-CTA-per-frame feature)
-                // second generation: a receiver thread holds at most N48_MAXLEV noise samples besides its 16 FFT rows
-                if (v.gen == 2 && (stride - s.N + (s.noise_norm == 1 ? s.tail_tx + L - 1 : 0) + tpf - 1) / tpf > (v.LB > TCV_LB ? N48_MAXLEV : N48_MAXLEV_SHORT)) continue;
+                // a receiver thread holds at most N48_MAXLEV noise samples besides its 16 FFT rows
+                if ((stride - s.N + (s.noise_norm == 1 ? s.tail_tx + L - 1 : 0) + tpf - 1) / tpf > (v.LB > TCV_LB ? N48_MAXLEV : N48_MAXLEV_SHORT)) continue;
                 if (s.cp > 2 * tpf || s.cs > 2 * tpf || s.tail_tx > 2 * tpf || s.tail_rx / 2 > tpf || s.shift > tpf) continue;
-                const int need = std::max(s.noise_norm == 1 ? body + L - 1 : sec_cta, body + (v.gen == 2 ? tconv2_zero(v.LB) : TCV_ZERO));
+                const int need = std::max(s.noise_norm == 1 ? body + L - 1 : sec_cta, body + tconv2_zero(v.LB));
                 if (need > 512 * v.ntile || sec_cta <= 512 * (v.ntile - 2)) continue;   // (the kernel range-checks its last two tiles only)
-                if (nvar > 1 && v.gen != 2) continue;                // (several window pairs per launch: ber_tconv2.cuh only)
-                const BerSmem lay = v.layout(S_cta, stride, s.tail_tx, s.tail_rx, L, v.gen == 2 ? nvar : 0, 0);
+                const BerSmem lay = v.layout(S_cta, stride, s.tail_tx, s.tail_rx, L, rq.nvar, 0);
                 if (lay.bytes > smem_cap) continue;
                 // fewest taps of history first (MMAs per tile), then fewest tiles, then the fixed-shape instance
                 // (same noise numbering and arithmetic, counters bit for bit: 3856 SASS instructions instead of 4976)
@@ -164,77 +197,38 @@ int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, bool verify, bool 
             if (better) { best.var = &v; best.lay = lay; best.chunk = chunk; }
         }
     }
-    if (!best.var) {
-        for (const auto& v : h->variants) {
-            if (v.TC != 0 || v.fp64 != fp64 || v.verify != verify || v.N != s.N) continue;
-            if (v.res != want_resolved) continue;
-            best.var = &v;
-            best.chunk = ((sec + 255) / 256) | 1;   // noise block B of the staged policy (any odd number)
-            best.lay = v.layout(s.S, stride, s.tail_tx, s.tail_rx, L, 0, 0);
-            best.use_global = 0;
-            if (best.lay.bytes > smem_cap) {
-                best.use_global = 1;
-                best.lay = v.layout(s.S, stride, s.tail_tx, s.tail_rx, L, 0, 1);
-                if (best.lay.bytes > smem_cap) return fail(h, WOFDM_EUNSUPPORTED, "frame does not fit the staged kernel's shared memory");
-            }
-            break;
-        }
-    }
-    if (!best.var) return fail(h, WOFDM_EUNSUPPORTED, "no compiled kernel variant for this N / precision");
+    if (!best.var) return choose_staged(h, s, L, smem_cap, rq.verify, false, ((sec + 255) / 256) | 1, out);   // (noise block B of the staged policy: any odd number)
     *out = best;
     return WOFDM_OK;
 }
 
-// Resolved counters: the twin (BerVariant::res) of the kernel `prod` that wofdm_ber_run_multi (or the channel-mask chain:
-// the same txs / txy) picks, where one is compiled and its accumulators fit (nvar: pairs per launch, 1 = one launch per
-// pair); else the staged twin, which numbers its noise like `prod` through noise_at (BerParams::chunk / split / n48).
-// *fused_out: the twin evaluates all pairs in one launch.
+// Resolved counters: the twin of the kernel `prod` that wofdm_ber_run_multi (or the channel-mask chain) picks -- the
+// resolved-counter instance with the same key (BerVariant::key: same arithmetic, same noise blocks) -- where its
+// accumulators fit (fused: all n_var pairs in one launch, else one launch per pair); else the staged twin, which numbers
+// its noise like `prod` through noise_at (BerParams::chunk / split / n48).  *fused_out: the twin evaluates all pairs in one
+// launch.
 int choose_resolved(wofdm_ctx* h, const wofdm_sys_t& s, int L, size_t smem_cap, const Choice& prod, bool fused, int n_var,
                     Choice* out, bool* fused_out) {
     const BerVariant& p = *prod.var;
     const int stride = s.N + s.cp + s.cs - s.tail_tx;
+    *fused_out = false;
     const bool staged_only = getenv("WOFDM_RESOLVED_STAGED") != nullptr;   // test aid: the staged twin with production's numbering
-    if (p.gen == 0 && p.TC > 0 && !staged_only) {
-        // register policies: the twin of the same instantiation (same arithmetic, same noise blocks)
+    if (p.TC > 0 && !staged_only) {
         for (const auto& v : h->variants) {
-            if (!v.res || v.gen != 0 || v.TC != p.TC || v.N != p.N || v.NT != p.NT || v.LB != p.LB || v.MINB != p.MINB || v.CL != p.CL ||
-                v.circ != p.circ || v.full != p.full || v.txs != p.txs || v.verify) continue;
-            const BerSmem lay = v.layout(s.S / v.CL, stride, s.tail_tx, s.tail_rx, L, prod.chunk, 0);
-            if (lay.bytes > smem_cap) break;
-            out->var = &v; out->lay = lay; out->chunk = prod.chunk; out->use_global = 0;
-            *fused_out = false;
-            return WOFDM_OK;
-        }
-    }
-    if (p.gen == 2 && !staged_only) {
-        for (const auto& v : h->variants) {
-            if (!v.res || v.gen != 2 || v.verify || v.N != p.N || v.NT != p.NT || v.ntile != p.ntile || v.LB != p.LB || v.CL != p.CL ||
-                v.txy != p.txy) continue;
-            // all pairs in one launch where the accumulators of all of them fit, else one launch per pair (same counters)
+            if (!v.res || v.verify || v.key() != p.key()) continue;
+            // tensor-core twins: all pairs in one launch where the accumulators of all of them fit, else one launch per pair
+            // (same counters); register twins: production's noise block
             for (int nv : {fused ? n_var : 1, 1}) {
-                const BerSmem lay = v.layout(s.S / v.CL, stride, s.tail_tx, s.tail_rx, L, nv, 0);
+                const BerSmem lay = v.layout(s.S / v.CL, stride, s.tail_tx, s.tail_rx, L, v.ntile > 0 ? nv : prod.chunk, 0);
                 if (lay.bytes > smem_cap) continue;
-                out->var = &v; out->lay = lay; out->chunk = 0; out->use_global = 0;
+                out->var = &v; out->lay = lay; out->chunk = prod.chunk; out->use_global = 0;
                 *fused_out = fused && nv == n_var;
                 return WOFDM_OK;
             }
+            break;
         }
     }
-    for (const auto& v : h->variants) {
-        if (!v.res || v.TC != 0 || v.fp64 != (s.precision == 1) || v.verify || v.N != s.N) continue;
-        out->var = &v;
-        out->chunk = prod.chunk;
-        out->use_global = 0;
-        out->lay = v.layout(s.S, stride, s.tail_tx, s.tail_rx, L, 0, 0);
-        if (out->lay.bytes > smem_cap) {
-            out->use_global = 1;
-            out->lay = v.layout(s.S, stride, s.tail_tx, s.tail_rx, L, 0, 1);
-            if (out->lay.bytes > smem_cap) return fail(h, WOFDM_EUNSUPPORTED, "frame does not fit the staged kernel's shared memory");
-        }
-        *fused_out = false;
-        return WOFDM_OK;
-    }
-    return fail(h, WOFDM_EUNSUPPORTED, "no compiled resolved-counter kernel for this N / precision");
+    return choose_staged(h, s, L, smem_cap, false, true, prod.chunk, out);
 }
 
 template <typename T> void cast_vec(const std::vector<double>& src, std::vector<unsigned char>& dst) {
@@ -563,10 +557,19 @@ static int plan_create_impl(wofdm_handle h, const wofdm_sys_t* sys, const double
     for (auto& d : h->devs) cap = std::min(cap, d.smem_optin);
     // several window pairs: one launch for all of them where the second-generation tensor-core kernel applies and holds
     // their tables; otherwise the pairs are launched one after the other on the same draws (same counters either way)
-    rc = choose_variant(h, *sys, L, false, false, cap, &ch, win_tx, false, false, false, n_var);
-    p->fused = rc == WOFDM_OK && n_var > 1 && ch.var->gen == 2;
+    {
+        KernelRequest rq;
+        rq.win_tx = win_tx;
+        rq.nvar = n_var;
+        rc = choose_variant(h, *sys, L, cap, rq, &ch);
+    }
+    p->fused = rc == WOFDM_OK && n_var > 1 && ch.var->ntile > 0;
     // (one launch per pair: no Tx window is passed, so no kernel that relies on the flatness of pair 0's is chosen)
-    if (n_var > 1 && !p->fused) rc = choose_variant(h, *sys, L, false, false, cap, &ch, nullptr, /*no_circ=*/true);
+    if (n_var > 1 && !p->fused) {
+        KernelRequest rq;
+        rq.no_circ = true;
+        rc = choose_variant(h, *sys, L, cap, rq, &ch);
+    }
     if (rc) { delete p; return rc; }
     p->noise_var = ch.var;
     p->cnt_per_var = (size_t)n_snr * 2;
@@ -1000,8 +1003,13 @@ int wofdm_ber_verify(wofdm_handle h, const wofdm_sys_t* sys, const double* win_t
     DeviceCtx& d = h->devs[0];
     WOFDM_CUDA(h, cudaSetDevice(d.dev));
     Choice ch;
-    rc = choose_variant(h, *sys, L, true, variant_kernel == 1, d.smem_optin, &ch, win_tx, variant_kernel == 2, false,
-                        variant_kernel == 2 || variant_kernel == 3);
+    KernelRequest rq;
+    rq.verify = true;
+    rq.staged_only = variant_kernel == 1;
+    rq.no_tconv = variant_kernel == 2 || variant_kernel == 3;
+    rq.no_circ = variant_kernel == 2;
+    rq.win_tx = win_tx;
+    rc = choose_variant(h, *sys, L, d.smem_optin, rq, &ch);
     if (rc) return rc;
     int nb = 0;
     long long max_ctas = 0;
@@ -1082,7 +1090,7 @@ int wofdm_ber_draws(wofdm_handle h, const wofdm_sys_t* sys, int L, uint64_t seed
     philox_round_keys(seed, prm.rk);
     {   // the noise block B is a property of the kernel variant production mode dispatches to
         Choice ch;
-        rc = choose_variant(h, *sys, L, false, false, d.smem_optin, &ch);
+        rc = choose_variant(h, *sys, L, d.smem_optin, KernelRequest{}, &ch);
         if (rc) return rc;
         prm.chunk = ch.chunk;
         fill_split(prm, *ch.var);
@@ -1185,13 +1193,25 @@ int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const dou
     // HBM) where the frame fits one, else a tx_stream kernel (tuned or staged)
     int rc = WOFDM_OK;
     if (J.use_gemm && !(J.dump_env && *J.dump_env)) {
-        rc = choose_variant(h, *sys, L, false, false, d0.smem_optin, &ch, nullptr, true, true, false, 1, true);
+        KernelRequest rq;
+        rq.no_circ = true;
+        rq.tx = TxSource::gather;
+        rc = choose_variant(h, *sys, L, d0.smem_optin, rq, &ch);
         J.fused = rc == WOFDM_OK && ch.var->txy;
     }
-    if (!J.fused) rc = choose_variant(h, *sys, L, false, false, d0.smem_optin, &ch, nullptr, true, true);
+    if (!J.fused) {
+        KernelRequest rq;
+        rq.no_circ = true;
+        rq.tx = TxSource::stream;
+        rc = choose_variant(h, *sys, L, d0.smem_optin, rq, &ch);
+    }
     if (rc) return rc;
     if (ch.var->CL > 1) return fail(h, WOFDM_EUNSUPPORTED, "no channel-mask variant for cluster kernels");
-    rc = choose_variant(h, *sys, L, false, false, d0.smem_optin, &prod, win_tx);     // noise numbering of wofdm_ber_run / _draws
+    {
+        KernelRequest rq;                   // noise numbering of wofdm_ber_run / _draws
+        rq.win_tx = win_tx;
+        rc = choose_variant(h, *sys, L, d0.smem_optin, rq, &prod);
+    }
     if (rc) return rc;
     if (prod.var->CL > 1) return fail(h, WOFDM_EUNSUPPORTED, "no channel-mask variant for cluster kernels");
     // the kernel that runs: ch, or (resolved counters, segments) its twin -- the noise numbering below stays ch's either way,

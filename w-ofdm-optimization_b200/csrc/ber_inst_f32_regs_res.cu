@@ -3,17 +3,17 @@
 #include "ber_registry.h"
 namespace wofdm {
 void register_ber_f32_regs_res(std::vector<BerVariant>& out) {
-    WOFDM_VARIANT_RES_REGS(float, 256, 256, 17, 21, 2, true, 1, false, "f32r", "_res")
-    WOFDM_VARIANT_RES_REGS(float, 256, 256, 17, 21, 2, false, 1, false, "f32r", "_res")
-    WOFDM_VARIANT_RES_REGS(float, 256, 256, 19, 21, 2, false, 1, false, "f32r", "_res")
-    WOFDM_VARIANT_RES_REGS(float, 256, 256, 17, 21, 2, true, 1, true, "f32r", "_circ_res")
-    WOFDM_VARIANT_RES_REGS(float, 256, 256, 17, 21, 2, false, 1, true, "f32r", "_circ_res")
-    WOFDM_VARIANT_RES_REGS(float, 256, 256, 19, 21, 2, false, 1, true, "f32r", "_circ_res")
-    WOFDM_VARIANT_RES_REGS(float, 512, 512, 17, 21, 1, true, 1, false, "f32r", "_res")
-    WOFDM_VARIANT_RES_REGS(float, 512, 512, 17, 21, 1, false, 1, false, "f32r", "_res")
-    WOFDM_VARIANT_RES_REGS(float, 512, 512, 19, 21, 1, false, 1, false, "f32r", "_res")
-    WOFDM_VARIANT_RES_REGS(float, 1024, 512, 17, 21, 1, true, 2, false, "f32r", "_res")
-    WOFDM_VARIANT_RES_REGS(float, 1024, 512, 17, 21, 1, false, 2, false, "f32r", "_res")
-    WOFDM_VARIANT_RES_REGS(float, 1024, 512, 19, 21, 1, false, 2, false, "f32r", "_res")
+    WOFDM_VARIANT("f32r", "_cl1_res", float, 256, 256, 17, 21, 2, true, false, 1, false, false, true)
+    WOFDM_VARIANT("f32r", "_cl1_res", float, 256, 256, 17, 21, 2, false, false, 1, false, false, true)
+    WOFDM_VARIANT("f32r", "_cl1_res", float, 256, 256, 19, 21, 2, false, false, 1, false, false, true)
+    WOFDM_VARIANT("f32r", "_cl1_circ_res", float, 256, 256, 17, 21, 2, true, false, 1, true, false, true)
+    WOFDM_VARIANT("f32r", "_cl1_circ_res", float, 256, 256, 17, 21, 2, false, false, 1, true, false, true)
+    WOFDM_VARIANT("f32r", "_cl1_circ_res", float, 256, 256, 19, 21, 2, false, false, 1, true, false, true)
+    WOFDM_VARIANT("f32r", "_cl1_res", float, 512, 512, 17, 21, 1, true, false, 1, false, false, true)
+    WOFDM_VARIANT("f32r", "_cl1_res", float, 512, 512, 17, 21, 1, false, false, 1, false, false, true)
+    WOFDM_VARIANT("f32r", "_cl1_res", float, 512, 512, 19, 21, 1, false, false, 1, false, false, true)
+    WOFDM_VARIANT("f32r", "_cl2_res", float, 1024, 512, 17, 21, 1, true, false, 2, false, false, true)
+    WOFDM_VARIANT("f32r", "_cl2_res", float, 1024, 512, 17, 21, 1, false, false, 2, false, false, true)
+    WOFDM_VARIANT("f32r", "_cl2_res", float, 1024, 512, 19, 21, 1, false, false, 2, false, false, true)
 }
 }  // namespace wofdm

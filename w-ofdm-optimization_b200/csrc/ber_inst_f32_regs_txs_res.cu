@@ -3,8 +3,8 @@
 #include "ber_registry.h"
 namespace wofdm {
 void register_ber_f32_regs_txs_res(std::vector<BerVariant>& out) {
-    WOFDM_VARIANT_RES_TXS(float, 256, 256, 17, 21, 2, true, "f32r")
-    WOFDM_VARIANT_RES_TXS(float, 256, 256, 17, 21, 2, false, "f32r")
-    WOFDM_VARIANT_RES_TXS(float, 256, 256, 19, 21, 2, false, "f32r")
+    WOFDM_VARIANT("f32r", "_txs_res", float, 256, 256, 17, 21, 2, true, false, 1, false, true, true)
+    WOFDM_VARIANT("f32r", "_txs_res", float, 256, 256, 17, 21, 2, false, false, 1, false, true, true)
+    WOFDM_VARIANT("f32r", "_txs_res", float, 256, 256, 19, 21, 2, false, false, 1, false, true, true)
 }
 }  // namespace wofdm

@@ -4,7 +4,7 @@
 #include "ber_tconv2_registry.h"
 namespace wofdm {
 void register_ber_f32_tconv2_hs(std::vector<BerVariant>& out) {
-    WOFDM_VARIANT_TCONV2_HS(256, 256, 9, 2)
-    WOFDM_VARIANT_TCONV2_HS(256, 256, 10, 2)
+    WOFDM_TCONV2_VARIANT("_hs", 256, 256, 9, 2, false, 1, TCV_LB, false, false, true)
+    WOFDM_TCONV2_VARIANT("_hs", 256, 256, 10, 2, false, 1, TCV_LB, false, false, true)
 }
 }  // namespace wofdm

@@ -3,9 +3,9 @@
 #include "ber_tconv2_registry.h"
 namespace wofdm {
 void register_ber_f32_tconv2_txy_res(std::vector<BerVariant>& out) {
-    WOFDM_VARIANT_TCONV2_TXY_RES(256, 256, 9, 2)
-    WOFDM_VARIANT_TCONV2_TXY_RES(256, 256, 10, 2)
-    WOFDM_VARIANT_TCONV2_TXY_RES(512, 512, 18, 1)
-    WOFDM_VARIANT_TCONV2_TXY_RES(512, 512, 19, 1)
+    WOFDM_TCONV2_VARIANT("_txy_res", 256, 256, 9, 2, false, 1, TCV_LB, true, true)
+    WOFDM_TCONV2_VARIANT("_txy_res", 256, 256, 10, 2, false, 1, TCV_LB, true, true)
+    WOFDM_TCONV2_VARIANT("_txy_res", 512, 512, 18, 1, false, 1, TCV_LB, true, true)
+    WOFDM_TCONV2_VARIANT("_txy_res", 512, 512, 19, 1, false, 1, TCV_LB, true, true)
 }
 }  // namespace wofdm

@@ -41,7 +41,7 @@ struct BerParams {
     int N, cp, cs, tail_tx, tail_rx, rm, shift, bits, S;
     int n_tx, stride, L;
     int noise_norm, constellation;
-    int flat_tx, flat_rx;      // tensor-core kernel (ber_tconv.cuh): the window is one value between its tails (and cp, cs >= tail_tx
+    int flat_tx, flat_rx;      // tensor-core kernel (ber_tconv2.cuh): the window is one value between its tails (and cp, cs >= tail_tx
                                // for Tx): that value moves into the constellation table / is divided out, the flat rows skip the product
                                // (bit v = window pair v of a multi-variant plan)
     int nvar;                  // ber_tconv2.cuh: window pairs evaluated on every frame's symbols in one launch (<= 1: one);
@@ -306,7 +306,7 @@ struct BerSmem {
     int flen;       // frame-stream buffer elements incl. pad and tail slack (0: lives in global scratch)
     int xlen;       // second buffer elements: staged -> conv output / FFT exchange; regs -> noise / FFT exchange
     int off_x, off_tw, off_geq, off_hf, off_taps, off_wtx, off_wrx, off_red, off_qlut, off_dlut, off_gmask, off_symw;   // byte offsets
-    int off_lo, off_bt, off_bar;   // tensor-core convolution policy (ber_tconv.cuh): lo half of the split stream, taps operand, mbarrier
+    int off_lo, off_bt, off_bar;   // tensor-core convolution policy (ber_tconv2.cuh): lo half of the split stream, taps operand, mbarrier
     size_t bytes;
     int off_res;    // RES instantiations: per-sub-carrier error accumulators, uint32 {bit, sym} per (window pair, bin)
 };

@@ -1,34 +1,18 @@
-// ber_tconv.cuh -- K1 with the channel convolution on the 5th-generation tensor cores (tcgen05, sm_100a).
+// ber_tconv.cuh -- the pieces of K1's channel convolution on the 5th-generation tensor cores (tcgen05, sm_100a) that the
+// frame kernel of ber_tconv2.cuh builds on: the Hankel operand, its fp16 split, its scales, and the tcgen05 wrappers.
 //
-// Same chain, same draws-by-position, same Tx / Rx stages as ber_frame_kernel (ber_kernel.cuh; reference loop body
-// python/ofdm_utils/wofdm_simulation.py:171-240, matlab/main_BER_calculation.m:245-273).  What changes is the L-tap
-// tapped-delay-line convolution r = conv(h, u) (wofdm_simulation.py:206, main_BER_calculation.m:260): in the register
-// policy it is 2 L packed FMAs per sample on the FP32 dispatch port, which is the port that bounds the kernel.  Here the
-// frame stream itself is the A operand of a tensor-core product:
+// The L-tap tapped-delay-line convolution r = conv(h, u) (wofdm_simulation.py:206, main_BER_calculation.m:260) is a
+// tensor-core product whose A operand is the frame stream itself:
 //
-//   * the Tx stage stores every stream sample split in two fp16 pairs, u = hi + lo (|u - hi - lo| <= 2^-22 |u|), as
-//     half2 words (re, im) in two arrays ahi[], alo[];
+//   * every stream sample is split in two fp16 pairs, u = hi + lo (|u - hi - lo| <= 2^-22 |u|), stored as half2 words
+//     (re, im) in two arrays ahi[], alo[];
 //   * row r of the operand is the 24 samples 4r-20 .. 4r+3 (K = 48 halves).  Rows are 16 bytes apart -- exactly the
 //     pitch of the rows inside an 8 x 16-byte core matrix of the K-major, no-swizzle UMMA layout -- so the raw array IS
 //     a canonical operand of the (overlapping) Hankel matrix: LBO = 16 B (next K chunk = next 4 samples), SBO = 128 B
 //     (next 8 rows).  Nothing is gathered or copied;
 //   * B (16 x 48, K-major) holds the taps, rebuilt per frame: output column 2o / 2o+1 = Re / Im of r[4 row + o], o < 4, from
 //     T_hi; columns 8 + (2o, 2o+1) the same from T_lo.  r = hi.[T_hi | T_lo] + lo.[T_hi | 0]: two 128 x 16 x 16 MMAs per
-//     (tile of 512 samples, K step of 8 samples), fp32 accumulation in tensor memory (16 columns per tile);
-//   * the MMAs of a frame (6 per tile; one elected lane of each of TCV_NISSUE warps issues them on the uniform datapath and
-//     commits them to an mbarrier) run while all threads draw the frame's noise (Philox + Box-Muller, kept in registers:
-//     nothing is parked in shared memory); the accumulators are read with tcgen05.ld once for the frame-wide signal
-//     power and once more for y = r + g n, which is written as plain fp32 over the (dead) split stream for the Rx stage.
-// Outputs past the kept samples (MATLAB's full-length noise normalisation) are more rows of the same product: the
-// stream is followed by zeros.  Noise numbering: stream sample i uses draw i (BerParams::chunk == 0), thread-independent.
-// Around the convolution: a Tx window that is one value between its tails rides on the constellation table, an Rx window
-// of that kind is divided out (BerParams::flat_tx / flat_rx, host-checked; arbitrary windows take the general path); the
-// slicer packs the decisions of four sub-carriers into a word and counts bit and symbol errors per word; six CTA
-// barriers per frame (none at its end: see the comment there).
-// fp32; N = 256: one CTA of 256 threads per frame, two CTAs per SM (256 of the 512 tensor-memory columns each); N = 512:
-// one CTA of 512 threads per frame and SM (all 512 columns; the two sets of eight warps take the even / odd tiles);
-// S <= 16 symbols in one Tx pass, L <= 21, prefix / suffix / tails within the outer register rows (the host checks,
-// ber_host.cu:choose_variant).
+//     (tile of 512 samples, K step of 8 samples), fp32 accumulation in tensor memory (16 columns per tile).
 #pragma once
 #include <cuda_fp16.h>
 #include "ber_kernel.cuh"
@@ -36,50 +20,10 @@
 namespace wofdm {
 
 constexpr int TCV_LB = 21;            // taps of the Hankel operand (row r = samples 4r - (LB-1) .. 4r + 3)
-constexpr int TCV_PAD = TCV_LB - 1;   // zero samples in front of the stream
-constexpr int TCV_SLACK = 0;
-constexpr int TCV_ZERO = 24;          // zero samples written behind the stream every frame
 constexpr float TCV_XSCALE = 64.0f;   // stream and taps are scaled by powers of two into the comfortable fp16 range;
 constexpr float TCV_HSCALE = 16.0f;   // everything behind the channel is scale-invariant (measured powers, pilot equaliser)
-constexpr uint32_t TCV_IDESC = (1u << 4) | ((16u >> 3) << 17) | ((128u >> 4) << 24);   // D f32, A = B = f16, K-major, N 16, M 128
 // tensor-memory columns a CTA allocates: 16 per tile, a power of two (two CTAs per SM when 256 are enough)
 __host__ __device__ constexpr uint32_t tconv_tmem_cols(int ntile) { return 16 * ntile <= 256 ? 256u : 512u; }
-#ifndef TCV_NISSUE
-#define TCV_NISSUE 4                   // warps that issue a frame's MMAs (one elected lane each, tiles round-robin); measured on
-                                      // the quick bench: 1 -> 6.42 ms, 2 -> 6.47, 4 -> 6.34, 8 -> 6.51
-#endif
-
-__host__ __device__ constexpr int tconv_alen(int ntile) { return TCV_PAD + ntile * 512 + TCV_SLACK; }
-
-template <int N, int NT, int NTILE>
-__host__ __device__ inline BerSmem tconv_smem_layout(int S, int stride, int tail_tx, int tail_rx, int L, int chunk, int use_global) {
-    using P = FftPlan<N>;
-    constexpr int FPP = NT / P::TPF;
-    BerSmem m;
-    m.pad = TCV_PAD;
-    m.flen = tconv_alen(NTILE);
-    m.xlen = FPP * P::XLEN;
-    int o = 0;
-    o += m.flen * 4;                 m.off_lo = o;        // ahi
-    o += m.flen * 4;                                      // alo (the received stream y lies over ahi | alo from byte 80)
-    o = (o + 15) & ~15;              m.off_x = o;
-    o += m.xlen * 8;                 m.off_tw = o;
-    o += P::NTW * 8;                 m.off_geq = o;
-    o += N * 8;                      m.off_bt = o;
-    o += 3 * 768;                    m.off_wtx = o;       // [T_hi | T_lo | zeros], 8 rows x 48 halves each
-    o += ((stride + tail_tx + 3) & ~3) * 4;   m.off_wrx = o;
-    o += ((N + tail_rx + 3) & ~3) * 4;        m.off_red = o;
-    o += 64 * 4;                              m.off_qlut = o;
-    o += 2 * 256 * 8;                         m.off_dlut = o;       // lattice points: Rx (pilot) copy, Tx copy (carries the flat window value)
-    o += 4 * 256 * 4;                         m.off_gmask = o;      // decision tables, one per byte lane of a packed word
-    o += P::TPF * 32;                         m.off_symw = o;
-    o += S * P::TPF * 16;                     m.off_bar = o;
-    o += 16;
-    m.off_hf = m.off_taps = 0;
-    m.bytes = ((size_t)o + 15) & ~(size_t)15;
-    (void)L; (void)chunk; (void)use_global;
-    return m;
-}
 
 __device__ __forceinline__ uint32_t tcv_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ uint64_t tcv_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
@@ -91,10 +35,11 @@ __device__ __forceinline__ uint64_t tcv_desc(uint32_t saddr, uint32_t lbo, uint3
     return d;
 }
 __device__ __forceinline__ void tcv_mma(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t accumulate) {
+    constexpr uint32_t idesc = (1u << 4) | ((16u >> 3) << 17) | ((128u >> 4) << 24);   // D f32, A = B = f16, K-major, N 16, M 128
     asm volatile(
         "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
         "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-        :: "r"(tmem_d), "l"(da), "l"(db), "r"(TCV_IDESC), "r"(accumulate) : "memory");
+        :: "r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate) : "memory");
 }
 __device__ __forceinline__ void tcv_mbar_wait(uint32_t bar, uint32_t parity) {
     uint32_t done = 0;
@@ -148,481 +93,5 @@ __device__ __forceinline__ void split_h2(float2 v, uint32_t& hi, uint32_t& lo) {
     lo = h2_bits(__floats2half2_rn(dx, dy));
 }
 __device__ __forceinline__ float2 join_h2(uint32_t hi, uint32_t lo) { return add2(__half22float2(bits_h2(hi)), __half22float2(bits_h2(lo))); }
-
-template <int N, int NT, int NTILE, int MINB, bool VERIFY>
-__global__ void __launch_bounds__(NT, MINB)
-ber_tconv_kernel(const BerParams prm) {
-    using T = float;
-    using C2 = float2;
-    using P = FftPlan<N>;
-    constexpr int TPF = P::TPF, FPP = NT / TPF, ER = 2, NW = NT / 32;
-    // 256 threads: warps 0-3 / 4-7 take outputs 0,1 / 2,3 of their rows in every tile.  512 threads (N = 512): a second
-    // set of eight warps, and the two sets take the even / the odd tiles.
-    static_assert(NT == 256 || NT == 512, "eight warps read a tile's accumulators");
-    constexpr int TG = NT / 256, NTH = (NTILE + TG - 1) / TG;             // tile sets; tiles per thread
-    constexpr uint32_t TMEM_COLS = tconv_tmem_cols(NTILE);
-    static_assert(16 * NTILE <= (int)TMEM_COLS, "accumulators of a frame must fit tensor memory");
-
-    extern __shared__ __align__(128) unsigned char tcv_smem[];
-    unsigned char* const smem_raw = tcv_smem;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int slot = tid / TPF, t = tid % TPF;
-    const int S = prm.S, stride = prm.stride, n_tx = prm.n_tx, beta = prm.tail_tx, L = prm.L;
-    const int cp = prm.cp, cs = prm.cs;
-    const int hh = prm.tail_rx >> 1;
-    const int hb = prm.bits >> 1, m = 1 << hb;
-    const int sec = S * stride;                 // samples kept after the channel
-    const int body = beta + sec;                // serialised Tx stream length
-    const int npow = prm.noise_norm == 1 ? body + L - 1 : sec;   // samples inside the frame-wide power sums
-
-    const BerSmem lay = tconv_smem_layout<N, NT, NTILE>(S, stride, beta, prm.tail_rx, L, 0, 0);
-    uint32_t* const ahi = reinterpret_cast<uint32_t*>(smem_raw);
-    uint32_t* const alo = reinterpret_cast<uint32_t*>(smem_raw + lay.off_lo);
-    uint32_t* const uh = ahi + TCV_PAD;         // uh[i], ul[i]: split stream sample i
-    uint32_t* const ul = alo + TCV_PAD;
-    C2* const yb = reinterpret_cast<C2*>(smem_raw + TCV_PAD * 4);   // received stream y[i], over the dead split stream (keeps ahi's zero pad)
-    static_assert((TCV_PAD * 4) % 16 == 0, "y is stored in 16-byte pairs");
-    C2* xbuf = reinterpret_cast<C2*>(smem_raw + lay.off_x);
-    C2* tw = reinterpret_cast<C2*>(smem_raw + lay.off_tw);
-    C2* geq = reinterpret_cast<C2*>(smem_raw + lay.off_geq);
-    unsigned char* bt = smem_raw + lay.off_bt;
-    T* wtx = reinterpret_cast<T*>(smem_raw + lay.off_wtx);
-    T* wrx = reinterpret_cast<T*>(smem_raw + lay.off_wrx);
-    T* red = reinterpret_cast<T*>(smem_raw + lay.off_red);
-    C2* qlut = reinterpret_cast<C2*>(smem_raw + lay.off_qlut);
-    C2* qtx = qlut + 256;
-    uint32_t* dlut4 = reinterpret_cast<uint32_t*>(smem_raw + lay.off_dlut);   // [b][(re level << hb) | im level] = index << 8b
-    uint4* gmask = reinterpret_cast<uint4*>(smem_raw + lay.off_gmask);
-    uint4* symw = reinterpret_cast<uint4*>(smem_raw + lay.off_symw);
-    unsigned long long* bar = reinterpret_cast<unsigned long long*>(smem_raw + lay.off_bar);
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem_raw + lay.off_bar + 8);
-    C2* const xb = xbuf + slot * P::XLEN;
-
-    // ---- one-time: tensor memory, barrier, tables ----
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(tcv_smem_u32(tmem_slot)), "r"(TMEM_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(tcv_smem_u32(bar)), "r"(TCV_NISSUE) : "memory");   // one commit per issuing warp and frame
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    for (int i = tid; i < P::NTW; i += NT) tw[i] = reinterpret_cast<const C2*>(prm.tw)[i];
-    // flat windows (host-checked): the Tx window's flat value rides on the constellation table and wtx holds the ratio to it
-    // (1 on every body row: no product there); the Rx window is divided by its flat value (a common factor of the
-    // received signal cancels in the pilot equaliser) and rows 1..13 of the Rx gather skip the product
-    const bool flat_tx = prm.flat_tx != 0, flat_rx = prm.flat_rx != 0;
-    const T wflat = flat_tx ? reinterpret_cast<const T*>(prm.win_tx)[beta] : (T)1;
-    const T rflat = flat_rx ? reinterpret_cast<const T*>(prm.win_rx)[prm.tail_rx] : (T)1;
-    for (int i = tid; i < n_tx; i += NT)
-        wtx[i] = flat_tx ? reinterpret_cast<const T*>(prm.win_tx)[i] / wflat : reinterpret_cast<const T*>(prm.win_tx)[i] * TCV_XSCALE;
-    for (int i = tid; i < N + prm.tail_rx; i += NT) wrx[i] = reinterpret_cast<const T*>(prm.win_rx)[i] / rflat;
-    for (int i = tid; i < TCV_PAD; i += NT) ahi[i] = 0u;
-    for (int i = tid; i < 768 / 4; i += NT) reinterpret_cast<uint32_t*>(bt + 1536)[i] = 0u;
-    for (int i = tid; i < (1 << prm.bits); i += NT) {
-        int a, c;
-        idx_to_levels(i, hb, m, prm.constellation, a, c);
-        qlut[i] = mk2<T>((T)(2 * a - (m - 1)), (T)(2 * c - (m - 1)));
-        qtx[i] = flat_tx ? cscale(wflat * TCV_XSCALE, qlut[i]) : qlut[i];
-#pragma unroll
-        for (int b = 0; b < 4; ++b) dlut4[b * 256 + ((a << hb) | c)] = (uint32_t)i << (8 * b);
-    }
-    if (tid == 0 && prm.bits < 8) { qlut[255] = mk2<T>(0, 0); qtx[255] = mk2<T>(0, 0); }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem = *tmem_slot;
-    if (prm.guard > 0) {
-        const unsigned d0 = dlut4[slice_index(mk2<T>(0, 0), hb)];
-        for (int tt = tid; tt < TPF; tt += NT) {
-            uint32_t ff[4] = {0, 0, 0, 0}, dd[4] = {0, 0, 0, 0};
-            for (int q = 0; q < 16; ++q)
-                if (!bin_active<N>(tt + q * TPF, prm.guard)) { ff[q >> 2] |= 0xffu << (8 * (q & 3)); dd[q >> 2] |= d0 << (8 * (q & 3)); }
-            gmask[2 * tt] = make_uint4(ff[0], ff[1], ff[2], ff[3]);
-            gmask[2 * tt + 1] = make_uint4(dd[0], dd[1], dd[2], dd[3]);
-        }
-        __syncthreads();
-    }
-
-    // this thread's operand row inside every tile (TMEM lane) and its half of the row's four outputs
-    const int wg = (warp >> 2) & 1, row = (warp & 3) * 32 + lane;
-    const int warp_u = __shfl_sync(0xffffffffu, warp, 0);      // the warp index as a value the compiler knows to be warp-uniform
-    const int tp = TG == 1 ? 0 : (warp_u >> 3);                // this warp's tile set: tiles tp, tp + TG, ...
-    const uint32_t tlane = tmem + ((uint32_t)((warp_u & 3) * 32) << 16) + (uint32_t)(4 * ((warp_u >> 2) & 1));
-    uint32_t phase = 0, issuer = blockIdx.x;
-
-    const long long fslot = blockIdx.x, nslots = gridDim.x;
-    long long f = prm.frame_begin + fslot * prm.frame_step;
-    const long long df = nslots * prm.frame_step;
-    long long fe = 0, de = 0;
-    int ci = 0, si = 0, dc = 0, ds = 0;
-    if constexpr (!VERIFY) {
-        const long long q = f / prm.ensemble, dq = df / prm.ensemble;
-        fe = f - q * prm.ensemble;   de = df - dq * prm.ensemble;
-        si = (int)(q / prm.C);       ci = (int)(q - (long long)si * prm.C);
-        ds = (int)(dq / prm.C);      dc = (int)(dq - (long long)ds * prm.C);
-    }
-    for (long long j = fslot; j < prm.n_frames; j += nslots) {
-        if constexpr (VERIFY) { ci = (int)f; si = (int)f; }
-        const T snr_lin = reinterpret_cast<const T*>(prm.snr_lin)[si];
-        // ---- taps operand of this frame: n = 2o + comp (o < 4), K pair jj = sample offset in the row, tap l = LB-1 + o - jj
-        if (tid < 8 * 24) {
-            const int n = tid / 24, jj = tid % 24;
-            const int o = n >> 1, l = TCV_LB - 1 + o - jj;
-            C2 tp = mk2<T>(0, 0);
-            if (l >= 0 && l < L) tp = reinterpret_cast<const C2*>(prm.chan)[(size_t)ci * L + l];
-            tp = cscale(TCV_HSCALE, tp);
-            const C2 v = (n & 1) ? mk2<T>(tp.y, tp.x) : mk2<T>(tp.x, -tp.y);     // multiplies (Re u, Im u)
-            uint32_t hi, lo;
-            split_h2(v, hi, lo);
-            const int off = (jj >> 2) * 128 + n * 16 + (jj & 3) * 4;
-            *reinterpret_cast<uint32_t*>(bt + off) = hi;
-            *reinterpret_cast<uint32_t*>(bt + 768 + off) = lo;
-        } else if (tid < 8 * 24 + TCV_PAD) {
-            alo[tid - 8 * 24] = 0u;                                              // (y of the previous frame lay over it)
-        } else if (tid - (8 * 24 + TCV_PAD) < TCV_ZERO) {
-            const int i = body + tid - (8 * 24 + TCV_PAD);                       // the linear convolution sees zeros behind the stream
-            uh[i] = 0u; ul[i] = 0u;
-        }
-
-        // =========================== transmitter ===========================
-        if (prm.tx_stream != nullptr) {          // uniform: masked Tx stream from tx_mask_kernel (mask_kernel.cuh)
-            for (int e = tid; e < S * TPF; e += NT) {
-                const int tt = e % TPF;
-                uint32_t w[4];
-                load_sym_idx<N, VERIFY>(prm, f, e / TPF, tt, w);
-                if (prm.guard > 0) {
-                    const uint4 gf = gmask[2 * tt], gd = gmask[2 * tt + 1];
-                    w[0] = (w[0] & ~gf.x) | gd.x; w[1] = (w[1] & ~gf.y) | gd.y;
-                    w[2] = (w[2] & ~gf.z) | gd.z; w[3] = (w[3] & ~gf.w) | gd.w;
-                }
-                symw[e] = make_uint4(w[0], w[1], w[2], w[3]);
-            }
-            const float2* src = prm.tx_stream + (size_t)j * body;
-            for (int i = tid; i < body; i += NT) {
-                uint32_t hi, lo;
-                split_h2(cscale(TCV_XSCALE, src[i]), hi, lo);
-                uh[i] = hi; ul[i] = lo;
-            }
-        } else {
-            const int s = slot;
-            const bool act = s < S;
-            const int se = act ? s : S - 1;     // idle slots shadow the last symbol (identical stores)
-            const bool first = se == 0;         // the frame's first symbol has no predecessor
-            C2 v[16];
-            {
-                uint32_t w[4], wq[4];
-                load_sym_idx<N, VERIFY>(prm, f, se, t, w);
-#pragma unroll
-                for (int jw = 0; jw < 4; ++jw) wq[jw] = w[jw];
-                if (prm.guard > 0) {
-                    const uint4 gf = gmask[2 * t], gd = gmask[2 * t + 1];
-                    const uint32_t ff[4] = {gf.x, gf.y, gf.z, gf.w}, dd[4] = {gd.x, gd.y, gd.z, gd.w};
-#pragma unroll
-                    for (int jw = 0; jw < 4; ++jw) { wq[jw] = w[jw] | ff[jw]; w[jw] = (w[jw] & ~ff[jw]) | dd[jw]; }
-                }
-                symw[se * TPF + t] = make_uint4(w[0], w[1], w[2], w[3]);
-#pragma unroll
-                for (int q = 0; q < 16; ++q) v[q] = qtx[sym_byte(wq, q)];
-            }
-            fft_regs<T, N, +1, FPP>(v, t, xb, tw, slot);
-            // CP/CS insertion + Tx window (transmitter.py:13-35, 61-87); heads i < tail_tx overlap the previous symbol's
-            // falling tail (wofdm_simulation.py:190-203) and are added after the barrier
-            uint32_t* const sh = uh + se * stride;
-            uint32_t* const sl = ul + se * stride;
-            if (flat_tx) {                        // uniform (implies cp, cs >= tail_tx: the body lies in the flat part)
-#pragma unroll
-                for (int q = 0; q < 16; ++q) {
-                    uint32_t hi, lo;
-                    split_h2(v[q], hi, lo);
-                    sh[t + q * TPF + cp] = hi; sl[t + q * TPF + cp] = lo;
-                }
-            } else if (cp >= beta) {
-                T wv[16];
-#pragma unroll
-                for (int q = 0; q < 16; ++q) wv[q] = wtx[t + q * TPF + cp];
-#pragma unroll
-                for (int q = 0; q < 16; ++q) {
-                    uint32_t hi, lo;
-                    split_h2(cscale(wv[q], v[q]), hi, lo);
-                    sh[t + q * TPF + cp] = hi; sl[t + q * TPF + cp] = lo;
-                }
-            } else {
-#pragma unroll
-                for (int q = 0; q < 16; ++q) {
-                    const int i = t + q * TPF + cp;
-                    if (q >= ER || i >= beta || first) {
-                        uint32_t hi, lo;
-                        split_h2(cscale(wtx[i], v[q]), hi, lo);
-                        sh[i] = hi; sl[i] = lo;
-                    }
-                }
-            }
-#pragma unroll
-            for (int q = 16 - ER; q < 16; ++q) {
-                if (q * TPF + TPF > N - cp) {             // uniform: this register row reaches the prefix
-                    const int i = t + q * TPF - (N - cp);
-                    if (i >= 0 && (i >= beta || first)) {
-                        uint32_t hi, lo;
-                        split_h2(cscale(wtx[i], v[q]), hi, lo);
-                        sh[i] = hi; sl[i] = lo;
-                    }
-                }
-            }
-#pragma unroll
-            for (int q = 0; q < ER; ++q) {
-                if (q * TPF < cs) {                        // uniform: ... the suffix
-                    const int i = t + q * TPF + cp + N;
-                    if (i < n_tx) {
-                        uint32_t hi, lo;
-                        split_h2(cscale(wtx[i], v[q]), hi, lo);
-                        sh[i] = hi; sl[i] = lo;
-                    }
-                }
-            }
-            __syncthreads();
-            if (beta > 0 && act && !first) {
-#pragma unroll
-                for (int q = 16 - ER; q < 16; ++q) {
-                    if (q * TPF + TPF > N - cp) {
-                        const int i = t + q * TPF - (N - cp);
-                        if (i >= 0 && i < beta) {
-                            uint32_t hi, lo;
-                            split_h2(caxpy(wtx[i], v[q], join_h2(sh[i], sl[i])), hi, lo);
-                            sh[i] = hi; sl[i] = lo;
-                        }
-                    }
-                }
-                if (cp < beta) {
-#pragma unroll
-                    for (int q = 0; q < ER; ++q) {
-                        const int i = t + q * TPF + cp;
-                        if (i < beta) {
-                            uint32_t hi, lo;
-                            split_h2(caxpy(wtx[i], v[q], join_h2(sh[i], sl[i])), hi, lo);
-                            sh[i] = hi; sl[i] = lo;
-                        }
-                    }
-                }
-            }
-        }
-        // the tensor core reads shared memory through the async proxy
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-
-        // =========================== channel + AWGN ===========================
-        // r = conv(h, u) (wofdm_simulation.py:206-209) on the tensor cores; y = r + sqrt(Pr*10^(-snr/10)/Pn) n with Pr, Pn
-        // summed over the whole frame (:135-138; noise_norm 1: over the full convolution, main_BER_calculation.m:260-261,289-292)
-        // One elected lane of each of TCV_NISSUE warps issues its share of the frame's MMAs (uniform datapath: 6 UTCHMMA per
-        // tile back to back) in front of the warp's noise draws; the tensor core then works through them (~40 cycles each,
-        // bound by its shared-memory reads) while every warp draws noise.  The issuing warps rotate from frame to frame
-        // so that no scheduler carries them every time.
-        const int irank = (warp_u - (int)issuer) & (NW - 1);          // warp-uniform: issuing warps have irank < TCV_NISSUE
-        const bool is_issuer = irank < TCV_NISSUE;
-        ++issuer;
-        if (is_issuer) asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        const uint32_t a_hi = tcv_smem_u32(ahi), a_lo = tcv_smem_u32(alo), b0 = tcv_smem_u32(bt);
-        if (is_issuer) {
-            if (tcv_elect_one()) {
-#pragma unroll
-                for (int ti = 0; ti < NTILE; ++ti) {
-                    if (ti % TCV_NISSUE != irank) continue;              // the issuing warps share the tiles round-robin
-                    const uint32_t tacc = tmem + (uint32_t)(16 * ti);
-#pragma unroll
-                    for (int k = 0; k < 3; ++k) {
-                        tcv_mma(tacc, tcv_desc(a_hi + ti * 2048 + k * 32, 16, 128), tcv_desc(b0 + k * 256, 128, 768), k != 0);
-                        tcv_mma(tacc, tcv_desc(a_lo + ti * 2048 + k * 32, 16, 128), tcv_desc(b0 + k * 256, 128, 1536), 1u);
-                    }
-                }
-                // completes when all of this warp's MMAs have
-                asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(tcv_smem_u32(bar)) : "memory");
-            }
-            __syncwarp();
-        }
-        // ---- noise of this thread's samples p, p+1 of its tiles, p = 512 tile + 4 row + 2 wg (draw = position), |n|^2 partial
-        C2 nz[NTH][2];
-        C2 pr2 = mk2<T>(0, 0), pn2 = mk2<T>(0, 0);
-#pragma unroll
-        for (int kt = 0; kt < NTH; ++kt) {
-            const int tt = TG * kt + tp;
-            const int p = 512 * tt + 4 * row + 2 * wg;
-            C2 n0 = mk2<T>(0, 0), n1 = mk2<T>(0, 0);
-            if (tt < NTILE - 2 || (tt < NTILE && 512 * tt + 128 * (warp & 3) < npow)) {   // warp-uniform; every tile but the last two lies inside the sums
-                if constexpr (VERIFY) {
-                    const double2* nin = prm.noise_in + (size_t)f * prm.noise_len;
-                    if (p < npow) n0 = to_v2<T>(nin[p]);
-                    if (p + 1 < npow) n1 = to_v2<T>(nin[p + 1]);
-                } else {
-                    noise_pair<T>(prm, f, (uint32_t)(p >> 1), n0, n1);
-                    if (tt >= NTILE - 2 && 512 * (tt + 1) > npow) {   // uniform: only the last tiles hold samples past the sums
-                        if (p >= npow) n0 = mk2<T>(0, 0);
-                        if (p + 1 >= npow) n1 = mk2<T>(0, 0);
-                    }
-                }
-            }
-            nz[kt][0] = n0; nz[kt][1] = n1;
-            pn2 = csq_acc(n0, pn2);
-            pn2 = csq_acc(n1, pn2);
-        }
-        // ---- signal power from the accumulators
-        tcv_mbar_wait(tcv_smem_u32(bar), phase);
-        phase ^= 1u;
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        constexpr int GT = 3;                      // tiles per batch of accumulator loads (one wait per batch)
-#pragma unroll
-        for (int t0 = 0; t0 < NTH; t0 += GT) {
-            C2 a0[GT], a1[GT], b0[GT], b1[GT];
-#pragma unroll
-            for (int u = 0; u < GT; ++u) {
-                if (t0 + u < NTH) {
-                    const int tt = min(TG * (t0 + u) + tp, NTILE - 1);      // (a set's tile past the frame: result masked below)
-                    tcv_ld4(tlane + (uint32_t)(16 * tt), a0[u], a1[u]);
-                    tcv_ld4(tlane + (uint32_t)(16 * tt + 8), b0[u], b1[u]);
-                }
-            }
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-            for (int u = 0; u < GT; ++u) {
-                if (t0 + u < NTH) {
-                    const int tt = TG * (t0 + u) + tp, p = 512 * tt + 4 * row + 2 * wg;
-                    C2 r0 = cadd(a0[u], b0[u]), r1 = cadd(a1[u], b1[u]);
-                    if (tt >= NTILE - 2 && 512 * (tt + 1) > npow) {
-                        if (p >= npow) r0 = mk2<T>(0, 0);
-                        if (p + 1 >= npow) r1 = mk2<T>(0, 0);
-                    }
-                    pr2 = csq_acc(r0, pr2);
-                    pr2 = csq_acc(r1, pr2);
-                }
-            }
-        }
-        T pr = warp_sum(pr2.x + pr2.y), pn = warp_sum(pn2.x + pn2.y);
-        if (lane == 0) { red[warp] = pr; red[32 + warp] = pn; }
-        __syncthreads();                           // also: every thread has seen the MMAs complete -- the split stream is dead
-        const T g = noise_gain(block_total<NW>(red), snr_lin, block_total<NW>(red + 32));
-#pragma unroll
-        for (int t0 = 0; t0 < NTH; t0 += GT) {
-            C2 a0[GT], a1[GT], b0[GT], b1[GT];
-#pragma unroll
-            for (int u = 0; u < GT; ++u) {
-                if (t0 + u < NTH) {
-                    const int tt = min(TG * (t0 + u) + tp, NTILE - 1);
-                    tcv_ld4(tlane + (uint32_t)(16 * tt), a0[u], a1[u]);
-                    tcv_ld4(tlane + (uint32_t)(16 * tt + 8), b0[u], b1[u]);
-                }
-            }
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-            for (int u = 0; u < GT; ++u) {
-                if (t0 + u < NTH) {
-                    const int tt = TG * (t0 + u) + tp, p = 512 * tt + 4 * row + 2 * wg;
-                    const C2 y0 = caxpy(g, nz[t0 + u][0], cadd(a0[u], b0[u])), y1 = caxpy(g, nz[t0 + u][1], cadd(a1[u], b1[u]));
-                    if (tt < NTILE - 2 || p + 1 < sec) *reinterpret_cast<float4*>(yb + p) = make_float4(y0.x, y0.y, y1.x, y1.y);
-                    else if (p < sec) yb[p] = y0;
-                }
-            }
-        }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-
-        // =========================== receiver ===========================
-        // block s: z[k] = wrx[k]*y[s*stride + rm + k]; o[n] = sum_{k = n + hh (mod N)} z[k];
-        // q[n] = o[(n + shift) mod N]; Y = DFT(q)   (receiver.py:13-133)
-        unsigned bit_cnt = 0, sym_cnt = 0;
-        {
-            const int s = slot;
-            const bool act = s < S;
-            const int se = act ? s : S - 1;
-            C2 v[16];
-            const C2* ys = yb + se * stride + prm.rm + hh;
-            const T* wr = wrx + hh;
-#pragma unroll
-            for (int q = 0; q < 16; ++q) {
-                if (q >= 1 && q <= 13) {
-                    // tail_rx/2, shift <= TPF: rows 1..13 neither wrap nor touch the overlap-add margins (nor the window tails)
-                    const int n = t + q * TPF + prm.shift;
-                    v[q] = flat_rx ? ys[n] : cscale(wr[n], ys[n]);
-                    continue;
-                }
-                const int a0 = (q * TPF + prm.shift) & (N - 1);
-                const int n = (t + q * TPF + prm.shift) & (N - 1);
-                C2 o = cscale(wr[n], ys[n]);
-                if (hh > 0) {
-                    const bool wraps = a0 + TPF > N;
-                    if (wraps || a0 < hh) { if (n < hh) o = caxpy(wr[n + N], ys[n + N], o); }
-                    if (wraps || a0 + TPF > N - hh) { if (n >= N - hh) o = caxpy(wr[n - N], ys[n - N], o); }
-                }
-                v[q] = o;
-            }
-            fft_regs<T, N, -1, FPP>(v, t, xb, tw, slot);
-            const uint4 wv = symw[se * TPF + t];
-            const uint32_t w[4] = {wv.x, wv.y, wv.z, wv.w};
-            // pilot (wofdm_simulation.py:223): the pilot's threads publish Y0, then every thread turns one bin into the
-            // equaliser tap G[k] = X0[k] / Y0[k] (lattice units)
-            if (se == 0) {
-#pragma unroll
-                for (int q = 0; q < 16; ++q) geq[t + q * TPF] = v[q];
-            }
-            __syncthreads();
-            const unsigned char* pil = reinterpret_cast<const unsigned char*>(symw);
-            for (int k = tid; k < N; k += NT) {
-                const C2 y0 = geq[k];
-                const C2 x0 = qlut[pil[(k % TPF) * 16 + k / TPF]];
-                C2 gk = cscale(recip(y0.x * y0.x + y0.y * y0.y), cmulc(x0, y0));
-                if (prm.guard > 0 && !bin_active<N>(k, prm.guard)) gk = mk2<T>(0, 0);
-                geq[k] = gk;
-            }
-            __syncthreads();
-            if (act && s > 0) {
-                // decisions of four sub-carriers packed like the stored Tx indices (byte q & 3 of word q >> 2): one XOR,
-                // one population count for the bit errors and one (of the non-zero bytes) for the symbol errors per word
-#pragma unroll
-                for (int gq = 0; gq < 4; ++gq) {
-                    uint32_t d4 = 0;
-#pragma unroll
-                    for (int b = 0; b < 4; ++b) {
-                        const int q = 4 * gq + b, k = t + q * TPF;
-                        const C2 e = cmul(v[q], geq[k]);                                   // :231
-                        const uint32_t dq = dlut4[b * 256 + slice_index(e, hb)];           // :233
-                        d4 |= dq;
-                        if constexpr (VERIFY) {
-                            const size_t o = ((size_t)f * (prm.S - 1) + (s - 1)) * N + k;
-                            prm.eq_out[o] = make_double2((double)e.x * prm.qscale, (double)e.y * prm.qscale);
-                            prm.dec_out[o] = (int32_t)(dq >> (8 * b));
-                        }
-                    }
-                    const uint32_t x = d4 ^ w[gq];
-                    bit_cnt += __popc(x);                                                  // :235 (bits) ...
-                    sym_cnt += __popc((((x & 0x7f7f7f7fu) + 0x7f7f7f7fu) | x) & 0x80808080u);   // ... and symbols: bytes that differ
-                }
-            }
-        }
-        bit_cnt = warp_sum(bit_cnt);
-        sym_cnt = warp_sum(sym_cnt);
-        if (lane == 0) {
-            if constexpr (VERIFY) {
-                atomicAdd(reinterpret_cast<unsigned long long*>(prm.bit_err_f) + f, (unsigned long long)bit_cnt);
-                atomicAdd(reinterpret_cast<unsigned long long*>(prm.sym_err_f) + f, (unsigned long long)sym_cnt);
-            } else {
-                atomicAdd(prm.counters + 2 * si, (unsigned long long)bit_cnt);
-                atomicAdd(prm.counters + 2 * si + 1, (unsigned long long)sym_cnt);
-            }
-        }
-        // No barrier here: what the next frame's Tx stage overwrites (the split stream over y, the symbol words, the taps
-        // operand, the exchange buffers) was last read before the pilot barriers above by every thread; geq, red and the
-        // tensor-memory accumulators are rewritten only behind the next frame's own barriers.
-        f += df;
-        if constexpr (!VERIFY) {
-            fe += de;
-            if (fe >= prm.ensemble) { fe -= prm.ensemble; ++ci; }
-            ci += dc;
-            if (ci >= prm.C) { ci -= prm.C; ++si; }
-            si += ds;
-        }
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"(TMEM_COLS) : "memory");
-}
 
 }  // namespace wofdm

@@ -196,7 +196,7 @@ __host__ __device__ inline BerSmem tconv2_smem_layout(int S, int stride, int tai
     m.xlen = FPP * P::XLEN;
     int o = 0;
     o += m.flen * 4;                 m.off_lo = o;        // ahi
-    o += m.flen * 4;                                      // alo (r lies over ahi | alo from byte 4 * TCV_PAD, two halves of
+    o += m.flen * 4;                                      // alo (r lies over ahi | alo from byte 4 * (TCV_LB - 1), two halves of
     o += 64;                                              //      128 NTILE + 4 chunks of 16 bytes)
     o = (o + 15) & ~15;              m.off_x = o;
     o += m.xlen * 8;                 m.off_tw = o;

@@ -141,7 +141,6 @@ int wofdm_create_on(wofdm_handle* out, const int* device_ids, int n) {
         d.smem_optin = prop.sharedMemPerBlockOptin;
         h->devs.push_back(d);
     }
-    register_ber_f32_tconv(h->variants);
     register_ber_f32_tconv2(h->variants);
     register_ber_f32_tconv2_hs(h->variants);
     register_ber_f32_regs(h->variants);
