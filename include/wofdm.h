@@ -403,6 +403,28 @@ WOFDM_API int wofdm_psd_estimate(wofdm_handle h, int N, int cp, int cs, int tail
                        const double* win_tx, int guard_band, int n_sym, int64_t records, uint64_t seed,
                        const int32_t* sym_idx, double* psd);
 
+/* PSD of the channel-mask chain's Tx streams (matlab/main_channel_mask.m), masked and unmasked, on the frames of its BER
+ * calls: frames f0 .. f0 + n_frames - 1 carry exactly the symbols wofdm_ber_run_masked / wofdm_ber_run give frame f with
+ * the same seed (wofdm_ber_draws exports them).  A frame is sys->S symbols on the guard-band allocation (sys->guard),
+ * windowed with win_tx (n_tx values), overlap-added with the frame stride into tail_tx + S * stride samples; the masked
+ * stream passes the mask of roll_off bins exactly as in the BER chain (the last symbol's filter tail is dropped), the
+ * unmasked one is the same symbols without it.  Each non-NULL output gets the 8N-point fftshifted PSD averaged over
+ * the slices of every frame; a NULL output skips that half of the work, and at least one must be non-NULL.  Ranges add
+ * up: the PSD of [a, c) is the frame-weighted mean of [a, b) and [b, c) up to the order of fp64 additions.
+ *   estimator 0: __psd_estimate of the reference (python/ofdm_utils/timefreq_simulation.py:104-123, as
+ *                wofdm_psd_estimate): floor(len / 8N) non-overlapping slices plus the zero-padded remainder, averaged over
+ *                floor + 1 slices.
+ *   estimator 1: Hann-tapered slices w[n] = sin^2(pi n / 8N) at a hop of 4N (50 % overlap), no remainder slice, each
+ *                periodogram scaled by 8N / sum(w^2) = 8/3 (a white stream reads the same level under both).
+ * The Tx fields of sys as wofdm_ber_run_masked accepts them (fp32, N = 128 / 256 / 512, bits < 8 with a guard band,
+ * roll_off that fits the mask); the Rx fields are ignored.  Device slot 0 only.  Errors: WOFDM_EINVAL for a NULL win_tx,
+ * both outputs NULL, f0 < 0, n_frames < 1, an overflowing frame range, a bad estimator or roll_off, or a stream shorter
+ * than one slice (tail_tx + S * stride < 8N); WOFDM_EUNSUPPORTED for fp64, another N, or a frame the mask product's
+ * symbol kernel cannot hold in shared memory.  The handle stays usable after every error. */
+WOFDM_API int wofdm_psd_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, int roll_off,
+                       uint64_t seed, int64_t f0, int64_t n_frames, int estimator,
+                       double* psd_masked /* 8N or NULL */, double* psd_unmasked /* 8N or NULL */);
+
 #ifdef __cplusplus
 }
 #endif

@@ -18,6 +18,7 @@
 //   [berMasked, ber] = wofdm_mex('run_sim_mc', ...)          run_sim_mc of matlab/main_channel_mask.m:334-337
 //   [berMasked, ber] = wofdm_mex('run_sim_mc_per_subcarrier', ...)  the same, BER per sub-carrier: N x 1 each (0 on guard bins)
 //   [berMasked, ber, ensembleUsed] = wofdm_mex('run_sim_mc_adaptive', ...)  run_sim_mc, each SNR point stopped at a bit-error target
+//   [psdMasked, psd] = wofdm_mex('psd_sim_mc', ...)         the Tx spectra of run_sim_mc's frames with and without the mask
 //   H = wofdm_mex('window_hessian', ...)                     quad_objective_tx / _rx of matlab/window_optimization.m:596-680
 //   H = wofdm_mex('window_hessian_expected', ...), 'quad_objective_tx_expected', 'quad_objective_rx_expected'
 //       -- the same, averaged over a channel set (C x L, rows = realisations) instead of built from one impulse response
@@ -467,10 +468,48 @@ static void do_calculate_interference(int nlhs, mxArray* plhs[], int nrhs, const
     plhs[0] = mxCreateDoubleScalar(P);
 }
 
+// [psdMasked, psd] = wofdm_mex('psd_sim_mc', numFrames, cpLength, csLength, tailTx, windowTx, offset, numSubcar,
+//                               bitsPerSubcar, symbolsPerTx, rollOff [, seed [, estimator]])
+//   -- the 8N-point fftshifted PSD (8N x 1 each) of the Tx signal of run_sim_mc's frames 0 .. numFrames-1 (the symbols
+//      run_sim_mc draws with the same seed), with and without the DFT-domain raised-cosine mask (wofdm_psd_masked).
+//      estimator: 'reference' / 0 (__psd_estimate's slices, the default) or 'hann' / 1 (sin^2 taper, 50 % overlap).
+static void do_psd_sim_mc(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
+    if (nrhs < 10) mexErrMsgIdAndTxt("wofdm:nargin", "psd_sim_mc needs 10 arguments");
+    wofdm_sys_t s;
+    memset(&s, 0, sizeof(s));
+    const long long n_frames = (long long)mxGetScalar(prhs[0]);
+    s.cp = (int)mxGetScalar(prhs[1]); s.cs = (int)mxGetScalar(prhs[2]); s.tail_tx = (int)mxGetScalar(prhs[3]);
+    s.guard = (int)mxGetScalar(prhs[5]); s.N = (int)mxGetScalar(prhs[6]); s.bits = (int)mxGetScalar(prhs[7]);
+    s.S = (int)mxGetScalar(prhs[8]);
+    const int roll_off = (int)mxGetScalar(prhs[9]);
+    s.noise_norm = 1; s.constellation = 1; s.precision = 0;
+    const std::vector<double> wtx = diag_of(prhs[4], (size_t)(s.N + s.cp + s.cs));
+    const unsigned long long seed = nrhs > 10 ? (unsigned long long)mxGetScalar(prhs[10]) : 0ull;
+    int estimator = 0;
+    if (nrhs > 11) {
+        char est[16];
+        if (mxIsChar(prhs[11])) {
+            if (mxGetString(prhs[11], est, sizeof(est))) mexErrMsgIdAndTxt("wofdm:usage", "estimator: 'reference' or 'hann'");
+            if (!strcmp(est, "hann")) estimator = 1;
+            else if (strcmp(est, "reference")) mexErrMsgIdAndTxt("wofdm:usage", "estimator: 'reference' or 'hann'");
+        } else {
+            estimator = (int)mxGetScalar(prhs[11]);
+        }
+    }
+    const size_t P = 8 * (size_t)(s.N > 0 ? s.N : 0);
+    std::vector<double> xm(P), xu(P);
+    check(wofdm_psd_masked(handle(), &s, wtx.data(), roll_off, seed, 0, n_frames, estimator, xm.data(), xu.data()),
+          "wofdm_psd_masked");
+    for (int k = 0; k < 2 && k < (nlhs > 0 ? nlhs : 1); ++k) {
+        plhs[k] = mxCreateDoubleMatrix((mwSize)P, 1, mxREAL);
+        memcpy(mxGetPr(plhs[k]), (k == 0 ? xm : xu).data(), P * sizeof(double));
+    }
+}
+
 extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     char cmd[32];
     if (nrhs < 1 || !mxIsChar(prhs[0]) || mxGetString(prhs[0], cmd, sizeof(cmd)))
-        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_simulation_adaptive', 'run_sim_mc', 'run_sim_mc_per_subcarrier', 'run_sim_mc_adaptive', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
+        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_simulation_adaptive', 'run_sim_mc', 'run_sim_mc_per_subcarrier', 'run_sim_mc_adaptive', 'psd_sim_mc', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
     if (!strcmp(cmd, "run_simulation")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_simulation_sweep")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, true);
     else if (!strcmp(cmd, "run_simulation_sweep_multi")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, false);
@@ -479,6 +518,7 @@ extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* 
     else if (!strcmp(cmd, "run_sim_mc")) do_run_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_sim_mc_per_subcarrier")) do_run_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1, true);
     else if (!strcmp(cmd, "run_sim_mc_adaptive")) do_run_sim_mc_adaptive(nlhs, plhs, nrhs - 1, prhs + 1);
+    else if (!strcmp(cmd, "psd_sim_mc")) do_psd_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1);
     else if (!strcmp(cmd, "window_hessian")) do_window_hessian(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "quad_objective_tx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, true, false);
     else if (!strcmp(cmd, "quad_objective_rx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, false, false);

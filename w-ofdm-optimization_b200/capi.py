@@ -128,6 +128,7 @@ SIGNATURES = {
                                      C.c_uint64, _dp, _dp]),
     "wofdm_psd_estimate": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _dp, C.c_int, C.c_int,
                                      C.c_int64, C.c_uint64, _i32p, _dp]),
+    "wofdm_psd_masked": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, C.c_uint64, C.c_int64, C.c_int64, C.c_int, _dp, _dp]),
 }
 
 _lib = None
@@ -454,6 +455,23 @@ class Handle:
                                        records, seed, _ptr(si, _i32p) if si is not None else None, _ptr(out, _dp))
         self._check(rc)
         return out
+
+    def psd_masked(self, s, win_tx, roll_off=10, frames=1, f0=0, seed=0, estimator="reference", masked=True, unmasked=True):
+        """PSD of the channel-mask chain's Tx streams (wofdm_psd_masked): frames f0 .. f0 + frames - 1, the symbols
+        ber_run_masked / ber_run give them with the same `s` and seed; estimator "reference" (__psd_estimate) or "hann"
+        (sin^2 taper, 50 % overlap).  Returns (masked, unmasked), each 8N doubles (fftshifted) or None where not asked for."""
+        w = _f64(np.ravel(win_tx))
+        if w.size != s.n_tx:
+            raise WofdmError(EINVAL, f"psd_masked: win_tx must have n_tx={s.n_tx} entries")
+        est = {"reference": 0, "hann": 1}.get(estimator)
+        if est is None:
+            raise WofdmError(EINVAL, f"psd_masked: estimator must be 'reference' or 'hann', not {estimator!r}")
+        om = np.empty(8 * s.N, dtype=np.float64) if masked else None
+        ou = np.empty(8 * s.N, dtype=np.float64) if unmasked else None
+        rc = load().wofdm_psd_masked(self._h, C.byref(s), _ptr(w, _dp), int(roll_off), int(seed), int(f0), int(frames), est,
+                                     _ptr(om, _dp) if om is not None else None, _ptr(ou, _dp) if ou is not None else None)
+        self._check(rc)
+        return om, ou
 
     def ber_plan_multi(self, s, wins_tx, wins_rx, chan, snr_db):
         """Device-resident plan of n_var window pairs (wofdm_ber_plan_create_multi)."""

@@ -45,6 +45,19 @@ struct wofdm_ber_plan_s {
     std::vector<PlanDev> devs;
 };
 
+std::vector<double> wofdm::tx_table(const wofdm_sys_t& s, const double* win_tx, bool unit_peak) {
+    const int n_tx = s.N + s.cp + s.cs;
+    double k = qam_scale(s) / (double)s.N;   // IDFT 1/N (transmitter.py:58) and constellation scale
+    if (unit_peak) {
+        double mx = 0.0;
+        for (int i = 0; i < n_tx; ++i) mx = std::max(mx, std::fabs(win_tx[i]));
+        if (mx > 0.0 && std::isfinite(mx)) k /= mx;
+    }
+    std::vector<double> a(n_tx);
+    for (int i = 0; i < n_tx; ++i) a[i] = win_tx[i] * k;
+    return a;
+}
+
 namespace {
 
 struct Choice {
@@ -274,14 +287,8 @@ HostTables build_tables(const wofdm_sys_t& s, const double* win_tx, const double
     const int n_tx = s.N + s.cp + s.cs, n_wr = s.N + s.tail_rx;
     std::vector<double> a((size_t)n_var * n_tx), b(win_rx, win_rx + (size_t)n_var * n_wr);
     for (int v = 0; v < n_var; ++v) {
-        const double* wt = win_tx + (size_t)v * n_tx;
-        double k = qam_scale(s) / (double)s.N;   // IDFT 1/N (transmitter.py:58) and constellation scale
-        if (unit_peak) {
-            double mx = 0.0;
-            for (int i = 0; i < n_tx; ++i) mx = std::max(mx, std::fabs(wt[i]));
-            if (mx > 0.0 && std::isfinite(mx)) k /= mx;
-        }
-        for (int i = 0; i < n_tx; ++i) a[(size_t)v * n_tx + i] = wt[i] * k;
+        const std::vector<double> wt = tx_table(s, win_tx + (size_t)v * n_tx, unit_peak);
+        std::copy(wt.begin(), wt.end(), a.begin() + (size_t)v * n_tx);
     }
     std::vector<double> lin(n_snr);
     for (int i = 0; i < n_snr; ++i) lin[i] = std::pow(10.0, -0.1 * snr_db[i]);   // wofdm_simulation.py:138

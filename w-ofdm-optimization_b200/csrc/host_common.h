@@ -82,4 +82,8 @@ inline int noise_len(const wofdm_sys_t& s, int L) {
 // FFT twiddle sections in the layout fft_regs.cuh documents, as interleaved doubles (re, im)
 std::vector<double> build_twiddles(int N);
 
+// the kernels' Tx window table of one window (n_tx values): v_tx * qam_scale / N; unit_peak (the tensor-core BER kernels,
+// ber_host.cu: build_tables) also divides by the window's largest magnitude
+std::vector<double> tx_table(const wofdm_sys_t& s, const double* win_tx, bool unit_peak);
+
 }  // namespace wofdm

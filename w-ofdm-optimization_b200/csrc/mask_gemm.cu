@@ -376,7 +376,7 @@ size_t mask_gemm_plan(const wofdm_sys_t& sys, long long batch, MaskGemm& mg) {
     return (size_t)mg.RT * mg.nk * 2 * A_BYTES + cols * mg.Kp * 2 + cols * mg.Yp * 4 + (size_t)mg.M * 16 + (size_t)mg.M * mg.nact * 16 + 4096;
 }
 
-int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, int roll_off, const float* d_wtx) {
+int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, int roll_off, const float* d_wtx, bool unit_impulse) {
     const size_t cols = (size_t)((mg.batch * mg.S + TN - 1) / TN) * TN;
     const size_t at_b = (size_t)mg.RT * mg.nk * 2 * A_BYTES, bt_b = cols * mg.Kp * 2, y_b = cols * mg.Yp * 4;
     mg.At = static_cast<__half*>(arena_take(d, at_b));
@@ -387,8 +387,14 @@ int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, int roll_off, cons
     mg.scale = static_cast<float*>(arena_take(d, 16));
     mg.maxbits = static_cast<unsigned*>(arena_take(d, 16));
     if (!mg.At || !mg.Bt || !mg.Y || !mg.g || !mg.Mm || !mg.scale || !mg.maxbits) return fail(h, WOFDM_ENOMEM, "mask product: arena exhausted");
-    mask_response_kernel<<<(mg.M + 63) / 64, 64, (size_t)mg.M * 24, d.stream>>>(mg.g, mg.M, roll_off);
-    WOFDM_CUDA(h, cudaGetLastError());
+    if (unit_impulse) {
+        const double2 one = make_double2(1.0, 0.0);       // (pageable source: the copy returns once it is staged)
+        WOFDM_CUDA(h, cudaMemsetAsync(mg.g, 0, (size_t)mg.M * 16, d.stream));
+        WOFDM_CUDA(h, cudaMemcpyAsync(mg.g, &one, sizeof(one), cudaMemcpyHostToDevice, d.stream));
+    } else {
+        mask_response_kernel<<<(mg.M + 63) / 64, 64, (size_t)mg.M * 24, d.stream>>>(mg.g, mg.M, roll_off);
+        WOFDM_CUDA(h, cudaGetLastError());
+    }
     WOFDM_CUDA(h, cudaMemsetAsync(mg.maxbits, 0, 4, d.stream));
     WOFDM_CUDA(h, cudaMemsetAsync(mg.Bt, 0, bt_b, d.stream));      // K padding and the columns behind the batch stay zero
     const int ne = mg.M * mg.nact;
@@ -397,7 +403,7 @@ int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, int roll_off, cons
     mask_split_kernel<<<2 * d.sm_count, 256, 0, d.stream>>>(mg.Mm, mg.maxbits, mg.At, mg.scale, mg.M, mg.n_tx, mg.nact, mg.Kp, mg.RT);
     WOFDM_CUDA(h, cudaGetLastError());
     WOFDM_CUDA(h, cudaFuncSetAttribute(mask_gemm_f16, cudaFuncAttributeMaxDynamicSharedMemorySize, NSTAGE * STAGE_BYTES));
-    h->launches += 3;
+    h->launches += unit_impulse ? 2 : 3;
     return WOFDM_OK;
 }
 

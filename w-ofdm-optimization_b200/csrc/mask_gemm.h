@@ -24,8 +24,10 @@ struct MaskGemm {
 
 // dimensions for `sys` and `batch` frames; returns the device bytes mask_gemm_setup takes from the arena
 size_t mask_gemm_plan(const wofdm_sys_t& sys, long long batch, MaskGemm& mg);
-// arena buffers + the matrix: the mask of roll_off bins (main_channel_mask.m:404-412, 477-493), d_wtx = K1's Tx table
-int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, int roll_off, const float* d_wtx);
+// arena buffers + the matrix: the mask of roll_off bins (main_channel_mask.m:404-412, 477-493), d_wtx = K1's Tx table.
+// unit_impulse: g = delta instead of the mask (roll_off unused), so Mtop = the windowed, CP-extended IDFT columns and
+// Mbot = 0 -- the UNMASKED symbols through the same product (wofdm_psd_masked's second spectrum)
+int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, int roll_off, const float* d_wtx, bool unit_impulse = false);
 // masked symbols of frames f0 .. f0 + nf - 1 (nf <= batch) into Y and, if `stream` is not NULL, the serialised Tx streams
 // into stream[nf][tail_tx + S * stride].  seg (a device segment table [n_seg][4], BerParams::seg): f0 .. f0 + nf - 1 are
 // local indices of the segment list of a job with C channels and `ensemble` ensemble indices per point

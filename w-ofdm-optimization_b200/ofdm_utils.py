@@ -7,6 +7,7 @@ Same names, argument meaning, file side effects and error behaviour (Python exce
 * ``ofdm_utils.interf_power(sys, [Vtx, Vrx], N, cp, tail_tx, tail_rx)``   python/ofdm_utils/interf_calc.py:20-113
 * ``run_simulation(ensemble, symbolsPerTx, ...)`` matlab/main_BER_calculation.m:230-274 (what the MEX gateway calls)
 * ``calculate_interference(cpLength, typeOFDM, windowTx, windowRx, ...)`` matlab/main_interference_calculation.m:177-225
+* ``run_sim_mc(...)`` / ``psd_sim_mc(...)``         matlab/main_channel_mask.m: the masked chain's BER and Tx spectra
 
 so a reference driver switches backend by importing this module instead of ``ofdm_utils`` (INTEGRATION.md).
 Everything numeric happens on the GPU through the C-ABI; there is no CPU fallback.  Documented deviations:
@@ -252,6 +253,36 @@ def run_sim_mc_adaptive(ensemble_max, cpLength, csLength, tailTx, tailRx, window
                                   int(ensemble_max), target_bit_errors=int(target_bit_errors), first_block=int(first_block),
                                   seed=seed, variant=0, roll_off=int(rollOff))
     return r["bit_err"][0] / r["bit_tot"], r["bit_err"][1] / r["bit_tot"], r["ensemble_used"]
+
+
+def obr_split(x, offset):
+    """(obr, mf_band) of an 8N-point fftshifted PSD of a guard-band signal: the guard band is the first and the last
+    8*offset bins (8x interpolation), its mean the out-of-band radiation; mf_band the bins in between."""
+    gb = 8 * int(offset)
+    if gb < 1 or 2 * gb >= len(x):
+        raise ValueError("the OBR needs 1 <= offset < numSubcar/2")
+    return float(np.mean(np.hstack((x[:gb], x[-gb:])))), x[gb:len(x) - gb]
+
+
+def psd_sim_mc(numFrames, cpLength, csLength, tailTx, windowTx, offset, numSubcar, bitsPerSubcar, symbolsPerTx, rollOff,
+               seed=0, estimator="reference", handle=None):
+    """PSD of the Tx signal of run_sim_mc (matlab/main_channel_mask.m:334-431) with and without the DFT-domain
+    raised-cosine mask, on frames 0 .. numFrames-1 of run_sim_mc's draws with the same seed (Handle.psd_masked).
+    MATLAB conventions (Gray unit-power QAM), guard = offset; windowTx a diagonal matrix or a vector.  estimator:
+    "reference" (__psd_estimate's slices) or "hann" (sin^2 taper, 50 % overlap).  Returns estimate_obr-style keys:
+    X_est_masked / X_est (8N bins, fftshifted), obr_masked / obr (mean over the guard band), mf_band_masked / mf_band (the
+    bins in between) and f_axis in cycles per sample."""
+    if int(offset) < 1:
+        raise ValueError("the OBR needs offset >= 1")
+    h = handle or default_handle()
+    N = int(numSubcar)
+    s = capi.SysT(N=N, cp=int(cpLength), cs=int(csLength), tail_tx=int(tailTx), bits=int(bitsPerSubcar),
+                  S=int(symbolsPerTx), noise_norm=1, constellation=1, precision=0, guard=int(offset))
+    xm, xu = h.psd_masked(s, _diag(windowTx), roll_off=int(rollOff), frames=int(numFrames), seed=seed, estimator=estimator)
+    out = {"X_est_masked": xm, "X_est": xu, "f_axis": np.linspace(-.5, .5 - 1 / (8 * N), 8 * N)}
+    out["obr_masked"], out["mf_band_masked"] = obr_split(xm, offset)
+    out["obr"], out["mf_band"] = obr_split(xu, offset)
+    return out
 
 
 def calculate_interference(cpLength, typeOFDM, windowTx, windowRx, numSubcar, tailTx, tailRx, channels, mode=0,
