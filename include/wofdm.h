@@ -288,6 +288,22 @@ WOFDM_API int wofdm_ber_run_masked_shard(wofdm_handle h, const wofdm_sys_t* sys,
                          const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
                          uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count,
                          int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot);
+/* n_var window pairs of the channel-mask chain on the same frames in one call (1 <= n_var <= WOFDM_MAX_VARIANTS): pair v =
+ * (win_tx + v*n_tx, win_rx + v*(N+tail_rx), roll_off[v]) gets exactly the counters of wofdm_ber_run_masked_shard with that
+ * pair, variant + v and the same shard, bit for bit -- the symbols depend on (seed, frame) only, pair v's noise on (seed,
+ * frame, variant + v).  Shards and the split over the handle's devices as in wofdm_ber_run_masked_shard.  A batch's symbols
+ * are drawn once and one tensor-core product covers the mask matrices of all pairs; K1 evaluates all pairs of a frame in
+ * one launch where its tables fit (else one launch per pair on the same product output).
+ *   bit_err / sym_err: int64[n_var][n_snr]; bit_tot / sym_tot: int64[n_snr] (the same for every pair).
+ * Errors: WOFDM_EINVAL for n_var outside [1, WOFDM_MAX_VARIANTS], a NULL roll_off, and what wofdm_ber_run_masked_shard
+ * rejects for any pair (a roll-off that does not fit the mask among them).  The handle stays usable after every error. */
+WOFDM_API int wofdm_ber_run_masked_multi(wofdm_handle h, const wofdm_sys_t* sys,
+                         const double* win_tx /* n_var x n_tx */, const double* win_rx /* n_var x (N + tail_rx) */,
+                         const int* roll_off /* n_var */, int n_var,
+                         const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                         uint64_t seed, uint32_t variant, int shard_index, int shard_count,
+                         int64_t* bit_err /* n_var x n_snr */, int64_t* bit_tot /* n_snr */,
+                         int64_t* sym_err /* n_var x n_snr */, int64_t* sym_tot /* n_snr */);
 /* The masked counters resolved as in wofdm_ber_run_resolved (resolve: a non-empty combination of WOFDM_BY_SUBCARRIER and
  * WOFDM_BY_CHANNEL; the same layout with n_var = 1): bit_err / sym_err int64[n_snr][Cr][Nr], sym_tot int64[n_snr][Cr][Nr]
  * = this shard's frames of the cell times S-1 on active bins, 0 on guard bins (bit totals: sym_tot * bits).  Shards as in

@@ -18,6 +18,7 @@
 //   [berMasked, ber] = wofdm_mex('run_sim_mc', ...)          run_sim_mc of matlab/main_channel_mask.m:334-337
 //   [berMasked, ber] = wofdm_mex('run_sim_mc_per_subcarrier', ...)  the same, BER per sub-carrier: N x 1 each (0 on guard bins)
 //   [berMasked, ber, ensembleUsed] = wofdm_mex('run_sim_mc_adaptive', ...)  run_sim_mc, each SNR point stopped at a bit-error target
+//   [berMasked, ber] = wofdm_mex('run_sim_mc_multi', ...)    run_sim_mc for several window pairs / roll-offs on the same symbols
 //   [psdMasked, psd] = wofdm_mex('psd_sim_mc', ...)         the Tx spectra of run_sim_mc's frames with and without the mask
 //   H = wofdm_mex('window_hessian', ...)                     quad_objective_tx / _rx of matlab/window_optimization.m:596-680
 //   H = wofdm_mex('window_hessian_expected', ...), 'quad_objective_tx_expected', 'quad_objective_rx_expected'
@@ -297,6 +298,51 @@ static void do_run_sim_mc(int nlhs, mxArray* plhs[], int nrhs, const mxArray* pr
     if (nlhs > 1) plhs[1] = mxCreateDoubleScalar(bt ? (double)be / (double)bt : 0.0);
 }
 
+// [berMasked, ber] = wofdm_mex('run_sim_mc_multi', <the 16 arguments of run_sim_mc> [, seed]) with windowTx and windowRx CELL
+// ARRAYS of n_var windows and rollOff a vector of n_var, channel C x L (rows = realisations) and snr a vector
+//   -- every configuration v = (windowTx{v}, windowRx{v}, rollOff(v)) on the same symbols: the unmasked chain in one call
+//      (wofdm_ber_run_multi, noise stream v), the masked chain in one (wofdm_ber_run_masked_multi, noise stream n_var + v).
+//      Each output is n_snr x n_var.
+static void do_run_sim_mc_multi(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
+    if (nrhs < 16) mexErrMsgIdAndTxt("wofdm:nargin", "run_sim_mc_multi needs 16 arguments");
+    wofdm_sys_t s;
+    memset(&s, 0, sizeof(s));
+    const long long ensemble = (long long)mxGetScalar(prhs[0]);
+    s.cp = (int)mxGetScalar(prhs[1]); s.cs = (int)mxGetScalar(prhs[2]);
+    s.tail_tx = (int)mxGetScalar(prhs[3]); s.tail_rx = (int)mxGetScalar(prhs[4]);
+    s.guard = (int)mxGetScalar(prhs[9]); s.rm = (int)mxGetScalar(prhs[10]); s.shift = (int)mxGetScalar(prhs[11]);
+    s.N = (int)mxGetScalar(prhs[12]); s.bits = (int)mxGetScalar(prhs[13]); s.S = (int)mxGetScalar(prhs[14]);
+    s.noise_norm = 1; s.constellation = 1; s.precision = 0;
+    size_t nvt = 0, nvr = 0;
+    const std::vector<double> wtx = windows_of(prhs[5], (size_t)(s.N + s.cp + s.cs), &nvt);
+    const std::vector<double> wrx = windows_of(prhs[6], (size_t)(s.N + s.tail_rx), &nvr);
+    const size_t n_var = mxGetNumberOfElements(prhs[15]);
+    if (nvt != n_var || nvr != n_var || n_var < 1 || n_var > WOFDM_MAX_VARIANTS)
+        mexErrMsgIdAndTxt("wofdm:size", "windowTx, windowRx (cell arrays) and rollOff must all hold n_var <= %d entries", WOFDM_MAX_VARIANTS);
+    std::vector<int> roll_off(n_var);
+    for (size_t v = 0; v < n_var; ++v) roll_off[v] = (int)mxGetPr(prhs[15])[v];
+    int L = 0, C = 0;
+    const std::vector<double> chan = channel_rows(prhs[7], &L, &C);
+    const size_t n_snr = mxGetNumberOfElements(prhs[8]);
+    const unsigned long long seed = nrhs > 16 ? (unsigned long long)mxGetScalar(prhs[16]) : 0ull;
+    std::vector<long long> be(n_var * n_snr), se(n_var * n_snr), bt(n_snr), st(n_snr), bem(n_var * n_snr), sem(n_var * n_snr), btm(n_snr);
+    check(wofdm_ber_run_multi(handle(), &s, wtx.data(), wrx.data(), (int)n_var, chan.data(), L, C, mxGetPr(prhs[8]), (int)n_snr,
+                              ensemble, seed, 0, 0, 1, (int64_t*)be.data(), (int64_t*)bt.data(), (int64_t*)se.data(), (int64_t*)st.data()),
+          "wofdm_ber_run_multi");
+    check(wofdm_ber_run_masked_multi(handle(), &s, wtx.data(), wrx.data(), roll_off.data(), (int)n_var, chan.data(), L, C,
+                                     mxGetPr(prhs[8]), (int)n_snr, ensemble, seed, (uint32_t)n_var, 0, 1, (int64_t*)bem.data(),
+                                     (int64_t*)btm.data(), (int64_t*)sem.data(), (int64_t*)st.data()),
+          "wofdm_ber_run_masked_multi");
+    for (int row = 0; row < 2 && row < (nlhs > 0 ? nlhs : 1); ++row) {      // berMasked, ber
+        const std::vector<long long>& e = row == 0 ? bem : be;
+        const std::vector<long long>& t = row == 0 ? btm : bt;
+        plhs[row] = mxCreateDoubleMatrix((mwSize)n_snr, (mwSize)n_var, mxREAL);
+        double* out = mxGetPr(plhs[row]);
+        for (size_t v = 0; v < n_var; ++v)
+            for (size_t i = 0; i < n_snr; ++i) out[v * n_snr + i] = t[i] ? (double)e[v * n_snr + i] / (double)t[i] : 0.0;
+    }
+}
+
 // [berMasked, ber, ensembleUsed] = wofdm_mex('run_sim_mc_adaptive', <the 16 arguments of run_sim_mc>, targetBitErrors,
 //                                            ensembleMax [, seed])
 //   -- run_sim_mc with every SNR point stopped once the masked and the unmasked chain have each counted targetBitErrors
@@ -509,7 +555,7 @@ static void do_psd_sim_mc(int nlhs, mxArray* plhs[], int nrhs, const mxArray* pr
 extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     char cmd[32];
     if (nrhs < 1 || !mxIsChar(prhs[0]) || mxGetString(prhs[0], cmd, sizeof(cmd)))
-        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_simulation_adaptive', 'run_sim_mc', 'run_sim_mc_per_subcarrier', 'run_sim_mc_adaptive', 'psd_sim_mc', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
+        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_simulation_adaptive', 'run_sim_mc', 'run_sim_mc_per_subcarrier', 'run_sim_mc_adaptive', 'run_sim_mc_multi', 'psd_sim_mc', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
     if (!strcmp(cmd, "run_simulation")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_simulation_sweep")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, true);
     else if (!strcmp(cmd, "run_simulation_sweep_multi")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, false);
@@ -518,6 +564,7 @@ extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* 
     else if (!strcmp(cmd, "run_sim_mc")) do_run_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_sim_mc_per_subcarrier")) do_run_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1, true);
     else if (!strcmp(cmd, "run_sim_mc_adaptive")) do_run_sim_mc_adaptive(nlhs, plhs, nrhs - 1, prhs + 1);
+    else if (!strcmp(cmd, "run_sim_mc_multi")) do_run_sim_mc_multi(nlhs, plhs, nrhs - 1, prhs + 1);
     else if (!strcmp(cmd, "psd_sim_mc")) do_psd_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1);
     else if (!strcmp(cmd, "window_hessian")) do_window_hessian(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "quad_objective_tx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, true, false);

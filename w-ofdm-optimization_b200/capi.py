@@ -109,6 +109,9 @@ SIGNATURES = {
                                        C.c_uint32, C.c_int, _i64p, _i64p, _i64p, _i64p]),
     "wofdm_ber_run_masked_shard": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
                                              C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_int, _i64p, _i64p, _i64p, _i64p]),
+    "wofdm_ber_run_masked_multi": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _P(C.c_int), C.c_int, _dp, C.c_int, C.c_int, _dp,
+                                             C.c_int, C.c_int64, C.c_uint64, C.c_uint32, C.c_int, C.c_int, _i64p, _i64p, _i64p,
+                                             _i64p]),
     "wofdm_ber_run_masked_resolved": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
                                                 C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_int, C.c_int, _i64p, _i64p, _i64p]),
     "wofdm_ber_run_masked_segments": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
@@ -378,6 +381,25 @@ class Handle:
         self._check(rc)
         return dict(bit_err=out[0], bit_tot=out[1], sym_err=out[2], sym_tot=out[3])
 
+    def ber_run_masked_multi(self, s, wins_tx, wins_rx, chan, snr_db, ensemble, seed=0, variant=0, roll_offs=10, shard=(0, 1)):
+        """n_var window pairs of the channel-mask chain on the same frames (wofdm_ber_run_masked_multi): pair v = ber_run_masked(
+        ..., variant=variant + v, roll_off=roll_offs[v], shard=shard) with its windows, bit for bit.  roll_offs: one value for
+        every pair, or n_var values.  bit_err / sym_err: (n_var, n_snr); bit_tot / sym_tot: (n_snr,)."""
+        wt, wr = self._win_multi(s, wins_tx, wins_rx)
+        _, _, chf, L, Cn = self._win_chan(s, wt[0], wr[0], chan)
+        nv = wt.shape[0]
+        ro = _roll_offs(roll_offs, nv)
+        snr = _f64(np.ravel(snr_db))
+        n = snr.size
+        be, se = np.zeros((nv, n), dtype=np.int64), np.zeros((nv, n), dtype=np.int64)
+        bt, st = np.zeros(n, dtype=np.int64), np.zeros(n, dtype=np.int64)
+        rc = load().wofdm_ber_run_masked_multi(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), _ptr(ro, _P(C.c_int)), nv,
+                                               _ptr(chf, _dp), L, Cn, _ptr(snr, _dp), n, int(ensemble), int(seed), int(variant),
+                                               int(shard[0]), int(shard[1]), _ptr(be, _i64p), _ptr(bt, _i64p), _ptr(se, _i64p),
+                                               _ptr(st, _i64p))
+        self._check(rc)
+        return dict(bit_err=be, bit_tot=bt, sym_err=se, sym_tot=st)
+
     def ber_run_masked_resolved(self, s, win_tx, win_rx, chan, snr_db, ensemble, seed=0, variant=0, roll_off=10, shard=(0, 1),
                                 by_subcarrier=True, by_channel=False):
         """ber_run_masked with the counters resolved by sub-carrier and / or channel (wofdm_ber_run_masked_resolved).
@@ -617,6 +639,14 @@ class Handle:
                                        _ptr(ph, _dp) if ph is not None else None, _ptr(out, _dp))
         self._check(rc)
         return out.T
+
+
+def _roll_offs(roll_offs, n_var):
+    """a scalar roll-off for every pair, or n_var of them -> contiguous int32 (n_var,)"""
+    ro = np.atleast_1d(np.asarray(roll_offs))
+    if ro.ndim != 1 or ro.size not in (1, n_var) or not np.all(ro == np.round(ro)):
+        raise WofdmError(EINVAL, f"roll_offs must be one integer or {n_var} of them (one per window pair)")
+    return np.ascontiguousarray(np.broadcast_to(ro, (n_var,)), dtype=np.int32)
 
 
 def _resolve(s, n, Cn, by_subcarrier, by_channel):

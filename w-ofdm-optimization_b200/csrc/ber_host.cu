@@ -1151,16 +1151,18 @@ static void host_fft_pow2(std::vector<double>& a, int n) {
 // Channel-mask variant (include/wofdm.h): frames in batches -- the masked Tx streams of a batch are written to HBM (the dense
 // tensor-core product of mask_gemm.cu, or tx_mask_kernel with WOFDM_MASK_FFT=1), a K1 kernel reads them
 // (BerParams::tx_stream) and does channel, noise, Rx and counting as always.
-// A call is set up once (masked_setup: kernels, tables, device buffers, the mask product's matrix) and then runs ranges of
+// A call is set up once (masked_setup: kernels, tables, device buffers, the mask product's matrices) and then runs ranges of
 // frames (masked_run): global frame ids, or local indices of a segment table (wofdm_ber_run_masked_segments / _adaptive).
+// n_var window pairs (wofdm_ber_run_masked_multi) share the batch's symbol draw and one product; K1 evaluates them in one
+// launch where the gathering kernel holds all their tables, else one launch per pair.
 namespace {
 
 struct MaskedDev {
     int slot = 0;                          // device of the handle
     MaskGemm mg{};
-    MaskParams mp{};
-    BerParams prm{};
-    unsigned long long* d_cnt = nullptr;   // counter pairs [n_snr][Cr][Nr]
+    MaskParams mp{};                       // pair 0's; pair v: its Tx table and mask response (WOFDM_MASK_FFT=1)
+    std::vector<BerParams> prm;            // one K1 launch each: all pairs, or pair v
+    unsigned long long* d_cnt = nullptr;   // counter pairs [n_var][n_snr][Cr][Nr]
     void* d_stream = nullptr;
     long long* d_seg = nullptr;            // segment table [seg_cap][4]
 };
@@ -1172,26 +1174,28 @@ struct MaskedJob {
     bool use_gemm = false, fused = false;
     const char* dump_env = nullptr;
     long long max_ctas = 0, batch = 0, ensemble = 0;
-    size_t ncnt = 0, cnt_bytes = 0, body = 0;
-    int C = 0, seg_cap = 0;
+    size_t ncnt = 0, cnt_bytes = 0, body = 0;   // (of one pair)
+    int C = 0, seg_cap = 0, n_var = 1;
     std::vector<MaskedDev> devs;           // the devices set up: the first ones of the handle
 };
 
-// Set-up of a checked channel-mask call: the kernels, the tables, and on every device that takes part (contiguous ranges
-// of at least 64 frames out of max_frames, the most frames one masked_run covers) its buffers and the mask product's
-// matrix.  resolve != 0 or seg_cap > 0: the resolved twin of the K1 kernel (counters [n_snr][Cr][Nr], [n_snr] with
+// Set-up of a checked channel-mask call of n_var window pairs (win_tx / win_rx back to back, roll_off[n_var]; pair v's
+// noise stream is variant + v): the kernels, the tables, and on every device that takes part (contiguous ranges of at least
+// 64 frames out of max_frames, the most frames one masked_run covers) its buffers and the mask product's matrices.
+// resolve != 0 or seg_cap > 0 (n_var = 1 only): the resolved twin of the K1 kernel (counters [n_snr][Cr][Nr], [n_snr] with
 // resolve 0); seg_cap > 0 also gives every device a segment table of seg_cap entries.
-int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
-                 const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble, uint64_t seed,
-                 uint32_t variant, int roll_off, int resolve, long long max_frames, int seg_cap) {
-    const int N = sys->N, n_tx = N + sys->cp + sys->cs, stride = n_tx - sys->tail_tx, M = 2 * n_tx - 1;
-    J.h = h; J.sys = *sys; J.C = C; J.ensemble = ensemble; J.seg_cap = seg_cap;
+int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
+                 const int* roll_off, const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                 uint64_t seed, uint32_t variant, int resolve, long long max_frames, int seg_cap) {
+    const int N = sys->N, n_tx = N + sys->cp + sys->cs, stride = n_tx - sys->tail_tx, M = 2 * n_tx - 1, n_wr = N + sys->tail_rx;
+    J.h = h; J.sys = *sys; J.C = C; J.ensemble = ensemble; J.seg_cap = seg_cap; J.n_var = n_var;
     const int Cr = (resolve & WOFDM_BY_CHANNEL) ? C : 1, Nr = (resolve & WOFDM_BY_SUBCARRIER) ? N : 1;
     J.ncnt = (size_t)n_snr * Cr * Nr;
     J.cnt_bytes = J.ncnt * 16;
     DeviceCtx& d0 = h->devs[0];              // (variant selection: the devices of a handle are alike)
     WOFDM_CUDA(h, cudaSetDevice(d0.dev));
-    Choice ch, prod;
+    Choice ch;
+    std::vector<Choice> prod(n_var);
     // Tx side: the dense tensor-core product of mask_gemm.cu; WOFDM_MASK_FFT=1 keeps the per-symbol FFT kernel (mask_kernel.cuh)
     const char* mask_env = getenv("WOFDM_MASK_FFT");
     J.use_gemm = !(mask_env && atoi(mask_env) == 1);
@@ -1214,19 +1218,26 @@ int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const dou
     }
     if (rc) return rc;
     if (ch.var->CL > 1) return fail(h, WOFDM_EUNSUPPORTED, "no channel-mask variant for cluster kernels");
-    {
-        KernelRequest rq;                   // noise numbering of wofdm_ber_run / _draws
-        rq.win_tx = win_tx;
-        rc = choose_variant(h, *sys, L, d0.smem_optin, rq, &prod);
+    for (int v = 0; v < n_var; ++v) {
+        KernelRequest rq;                   // noise numbering of wofdm_ber_run / _draws with pair v's Tx window
+        rq.win_tx = win_tx + (size_t)v * n_tx;
+        rc = choose_variant(h, *sys, L, d0.smem_optin, rq, &prod[v]);
+        if (rc) return rc;
+        if (prod[v].var->CL > 1) return fail(h, WOFDM_EUNSUPPORTED, "no channel-mask variant for cluster kernels");
     }
-    if (rc) return rc;
-    if (prod.var->CL > 1) return fail(h, WOFDM_EUNSUPPORTED, "no channel-mask variant for cluster kernels");
+    // several pairs: one launch of the gathering kernel for all of them where it holds all their tables (the same kernel
+    // as for one pair, so the same counters); else one launch per pair
+    int nv_launch = 1;
+    if (J.fused && n_var > 1) {
+        const BerSmem lay = ch.var->layout(sys->S, stride, sys->tail_tx, sys->tail_rx, L, n_var, 0);
+        if (lay.bytes <= d0.smem_optin) { nv_launch = n_var; ch.lay = lay; }
+    }
     // the kernel that runs: ch, or (resolved counters, segments) its twin -- the noise numbering below stays ch's either way,
     // so a staged fallback draws ch's noise; it reads the assembled stream even where ch gathers from the product itself
     J.run = ch;
     if (resolve || seg_cap > 0) {
         Choice nz = ch;
-        if (ch.var->TC == 0) nz.chunk = prod.chunk;
+        if (ch.var->TC == 0) nz.chunk = prod[0].chunk;
         bool rfused = false;
         rc = choose_resolved(h, *sys, L, d0.smem_optin, nz, false, 1, &J.run, &rfused);
         if (rc) return rc;
@@ -1237,21 +1248,27 @@ int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const dou
     rc = prepare_kernel(h, *run.var, run.lay.bytes, d0.sm_count, &nb, &J.max_ctas);
     if (rc) return rc;
     if (max_frames == 0) return WOFDM_OK;
-    std::vector<double> gd;
-    if (!J.use_gemm) {
+    // the circular convolution (mod M) of an n_tx-sample symbol = a linear one with the periodic extension of g on
+    // [-(n_tx-1), M-1]: Gp = FFT_P of that sequence laid out circularly in P = 8N >= 4 n_tx - 3 points, times 1/P
+    // (WOFDM_MASK_FFT=1: [n_var][P], pair v's mask)
+    const int P = 8 * N;
+    std::vector<float> g(J.use_gemm ? 2 : 2 * (size_t)P * n_var, 0.f);
+    std::vector<unsigned char> twp;
+    for (int v = 0; v < n_var && !J.use_gemm; ++v) {
+        const int ro = roll_off[v];
         // g = IDFT_M(ifftshift(windowRC)), main_channel_mask.m:404-412, 477-493
         std::vector<double> wrc(M, 0.0);
         {
-            const int wl = M / 2, rest = M - wl - 2 * roll_off, zl = rest / 2;
-            for (int i = 0; i < roll_off; ++i) {
-                const double ax = -(roll_off + 1) / 2.0 + 1.0 + i;
-                const double v = std::sin(1.5707963267948966 * (0.5 + ax / roll_off));
-                wrc[zl + i] = v * v;
-                wrc[zl + roll_off + wl + (roll_off - 1 - i)] = v * v;
+            const int wl = M / 2, rest = M - wl - 2 * ro, zl = rest / 2;
+            for (int i = 0; i < ro; ++i) {
+                const double ax = -(ro + 1) / 2.0 + 1.0 + i;
+                const double x = std::sin(1.5707963267948966 * (0.5 + ax / ro));
+                wrc[zl + i] = x * x;
+                wrc[zl + ro + wl + (ro - 1 - i)] = x * x;
             }
-            for (int i = 0; i < wl; ++i) wrc[zl + roll_off + i] = 1.0;
+            for (int i = 0; i < wl; ++i) wrc[zl + ro + i] = 1.0;
         }
-        gd.resize(2 * (size_t)M);
+        std::vector<double> gd(2 * (size_t)M);
         std::vector<double> phc(M), phs(M);
         for (int i = 0; i < M; ++i) {
             const double a = 6.283185307179586476925286766559 * (double)i / (double)M;
@@ -1268,26 +1285,18 @@ int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const dou
             }
             gd[2 * n] = re / M; gd[2 * n + 1] = im / M;
         }
-    }
-    // the circular convolution (mod M) of an n_tx-sample symbol = a linear one with the periodic extension of g on
-    // [-(n_tx-1), M-1]: Gp = FFT_P of that sequence laid out circularly in P = 8N >= 4 n_tx - 3 points, times 1/P
-    const int P = 8 * N;
-    std::vector<float> g(2 * (size_t)P, 0.f);
-    std::vector<unsigned char> twp;
-    if (!J.use_gemm) {
         std::vector<double> gc(2 * (size_t)P, 0.0);
         for (int mm = -(n_tx - 1); mm <= M - 1; ++mm) {
             const int gi = ((mm % M) + M) % M, ci = ((mm % P) + P) % P;
             gc[2 * ci] = gd[2 * gi]; gc[2 * ci + 1] = gd[2 * gi + 1];
         }
         host_fft_pow2(gc, P);
-        for (size_t i = 0; i < g.size(); ++i) g[i] = (float)(gc[i] / P);
-        cast_any(false, build_twiddles(P), twp);
-    } else {
-        twp.resize(16);
+        for (size_t i = 0; i < gc.size(); ++i) g[2 * (size_t)P * v + i] = (float)(gc[i] / P);
     }
+    if (!J.use_gemm) cast_any(false, build_twiddles(P), twp);
+    else twp.resize(16);
     // (tx_mask_kernel shares the Tx window's table: a common factor of its stream)
-    const HostTables t = build_tables(*sys, win_tx, win_rx, 1, chan, L, C, snr_db, n_snr, run.var->ntile > 0);
+    const HostTables t = build_tables(*sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, run.var->ntile > 0);
     J.body = (size_t)sys->tail_tx + (size_t)sys->S * stride;
     J.batch = std::min<long long>(max_frames, J.use_gemm ? 16384 : 8192);
     const size_t scratch_elems = (size_t)run.lay.pad + J.body + 64;
@@ -1304,10 +1313,10 @@ int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const dou
             const int rcp = prepare_kernel(h, *run.var, run.lay.bytes, d.sm_count, &nb_, &mc_);
             if (rcp) return rcp;
         }
-        const size_t mg_bytes = J.use_gemm ? mask_gemm_plan(*sys, J.batch, md.mg) : 0;
+        const size_t mg_bytes = J.use_gemm ? mask_gemm_plan(*sys, J.batch, n_var, md.mg) : 0;
         const size_t stream_bytes = J.fused ? 16 : (size_t)J.batch * J.body * sizeof(float2);
-        int rc = arena_reserve(h, d, t.bytes() + twp.size() + g.size() * 4 + J.cnt_bytes + stream_bytes + scratch_bytes + mg_bytes +
-                                     (size_t)seg_cap * 32 + 8192);
+        int rc = arena_reserve(h, d, t.bytes() + twp.size() + g.size() * 4 + n_var * J.cnt_bytes + stream_bytes + scratch_bytes +
+                                     mg_bytes + (size_t)seg_cap * 32 + 8192);
         if (rc) return rc;
         void *d_wtx, *d_wrx, *d_tw, *d_twp, *d_chan, *d_snr, *d_g, *d_cnt, *d_seg = nullptr, *d_scr = nullptr;
         WOFDM_CUDA(h, arena_put(d, t.wtx.data(), t.wtx.size(), &d_wtx));
@@ -1317,7 +1326,7 @@ int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const dou
         WOFDM_CUDA(h, arena_put(d, t.snr.data(), t.snr.size(), &d_snr));
         WOFDM_CUDA(h, arena_put(d, g.data(), g.size() * 4, &d_g));
         WOFDM_CUDA(h, arena_put(d, twp.data(), twp.size(), &d_twp));
-        WOFDM_CUDA(h, arena_put(d, nullptr, J.cnt_bytes, &d_cnt));
+        WOFDM_CUDA(h, arena_put(d, nullptr, n_var * J.cnt_bytes, &d_cnt));
         WOFDM_CUDA(h, arena_put(d, nullptr, stream_bytes, &md.d_stream));
         if (scratch_bytes) WOFDM_CUDA(h, arena_put(d, nullptr, scratch_bytes, &d_scr));
         if (seg_cap > 0) WOFDM_CUDA(h, arena_put(d, nullptr, (size_t)seg_cap * 32, &d_seg));
@@ -1334,26 +1343,33 @@ int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const dou
         mp.win_tx = static_cast<const float*>(d_wtx); mp.tw = static_cast<const float2*>(d_tw);
         mp.Gp = static_cast<const float2*>(d_g); mp.twp = static_cast<const float2*>(d_twp);
         mp.seed = seed; mp.stream = static_cast<float2*>(md.d_stream);
-        BerParams& prm = md.prm;
-        fill_sys(prm, *sys, L);
-        prm.chunk = ch.var->TC > 0 ? ch.chunk : prod.chunk; prm.use_global = run.use_global;
-        fill_flat(prm, *sys, win_tx, win_rx);
-        prm.flat_tx = 0;                       // (the Tx stream comes from tx_mask_kernel)
-        fill_split(prm, *ch.var);
-        if (ch.var->TC == 0) {                 // staged kernel: the noise numbering of wofdm_ber_run / _draws (noise_at follows it)
-            BerParams tmp = prm;
-            fill_split(tmp, *prod.var);
-            prm.n48 = tmp.n48;
+        // the K1 launches: pairs v .. v + nv_launch - 1 each (the tables, counters and product outputs of pair v on)
+        md.prm.assign(n_var / nv_launch, BerParams{});
+        for (int v = 0; v < n_var; v += nv_launch) {
+            BerParams& prm = md.prm[v / nv_launch];
+            fill_sys(prm, *sys, L);
+            prm.chunk = ch.var->TC > 0 ? ch.chunk : prod[v].chunk; prm.use_global = run.use_global;
+            fill_flat(prm, *sys, win_tx + (size_t)v * n_tx, win_rx + (size_t)v * n_wr, nv_launch);
+            prm.flat_tx = 0;                       // (the Tx stream comes from tx_mask_kernel)
+            prm.nvar = nv_launch;
+            fill_split(prm, *ch.var);
+            if (ch.var->TC == 0) {                 // staged kernel: the noise numbering of wofdm_ber_run / _draws (noise_at follows it)
+                BerParams tmp = prm;
+                fill_split(tmp, *prod[v].var);
+                prm.n48 = tmp.n48;
+            }
+            prm.win_tx = static_cast<const float*>(d_wtx) + (size_t)v * n_tx;
+            prm.win_rx = static_cast<const float*>(d_wrx) + (size_t)v * n_wr;
+            prm.tw = d_tw; prm.chan = d_chan; prm.snr_lin = d_snr;
+            prm.C = C; prm.n_snr = n_snr; prm.ensemble = ensemble; prm.seed = seed; prm.variant = variant + (uint32_t)v;
+            philox_round_keys(seed, prm.rk);
+            prm.counters = md.d_cnt + (size_t)v * J.ncnt * 2;
+            prm.res_chan = (resolve & WOFDM_BY_CHANNEL) ? 1 : 0;
+            prm.res_bins = (resolve & WOFDM_BY_SUBCARRIER) ? 1 : 0;
+            prm.scratch = d_scr; prm.scratch_elems = (long long)scratch_elems;
+            prm.tx_stream = static_cast<const float2*>(md.d_stream);
+            if (J.fused) { prm.tx_y = md.mg.Y + (size_t)v * md.mg.ypair; prm.tx_yp = md.mg.Yp; prm.tx_ypair = md.mg.ypair; }
         }
-        prm.win_tx = d_wtx; prm.win_rx = d_wrx; prm.tw = d_tw; prm.chan = d_chan; prm.snr_lin = d_snr;
-        prm.C = C; prm.n_snr = n_snr; prm.ensemble = ensemble; prm.seed = seed; prm.variant = variant;
-        philox_round_keys(seed, prm.rk);
-        prm.counters = md.d_cnt;
-        prm.res_chan = (resolve & WOFDM_BY_CHANNEL) ? 1 : 0;
-        prm.res_bins = (resolve & WOFDM_BY_SUBCARRIER) ? 1 : 0;
-        prm.scratch = d_scr; prm.scratch_elems = (long long)scratch_elems;
-        prm.tx_stream = static_cast<const float2*>(md.d_stream);
-        if (J.fused) { prm.tx_y = md.mg.Y; prm.tx_yp = md.mg.Yp; }
         return WOFDM_OK;
     };
     J.devs.resize(nd);
@@ -1371,14 +1387,15 @@ int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const dou
 
 // The frames [g_lo, g_hi) of a set-up call: global frame ids, or with `segs` (at most seg_cap segments, its table uploaded to
 // every device) local indices of that segment list.  The devices take contiguous ranges of at least 64.
-// -> bit_err / sym_err [n_snr][Cr][Nr]
+// -> bit_err / sym_err [n_var][n_snr][Cr][Nr]
 int masked_run(MaskedJob& J, long long g_lo, long long g_hi, const Segments* segs, int64_t* bit_err, int64_t* sym_err) {
     wofdm_ctx* h = J.h;
     const wofdm_sys_t& sys = J.sys;
     const int N = sys.N;
     const long long nfr = g_hi - g_lo;
+    const size_t nout = (size_t)J.n_var * J.ncnt;
     if (nfr == 0) {
-        for (size_t i = 0; i < J.ncnt; ++i) { bit_err[i] = 0; sym_err[i] = 0; }
+        for (size_t i = 0; i < nout; ++i) { bit_err[i] = 0; sym_err[i] = 0; }
         return WOFDM_OK;
     }
     const int n_seg = segs ? segs->n() : 0;
@@ -1390,51 +1407,63 @@ int masked_run(MaskedJob& J, long long g_lo, long long g_hi, const Segments* seg
         const long long* seg = segs ? md.d_seg : nullptr;
         // (pageable source: the copy returns once the table is staged; the previous work on this stream is ordered before it)
         if (segs) WOFDM_CUDA(h, cudaMemcpyAsync(md.d_seg, segs->tab.data(), segs->tab.size() * sizeof(long long), cudaMemcpyHostToDevice, d.stream));
-        WOFDM_CUDA(h, cudaMemsetAsync(md.d_cnt, 0, J.cnt_bytes, d.stream));
+        WOFDM_CUDA(h, cudaMemsetAsync(md.d_cnt, 0, J.n_var * J.cnt_bytes, d.stream));
         MaskSegParams mp;
         static_cast<MaskParams&>(mp) = md.mp;
         mp.seg = seg; mp.n_seg = n_seg; mp.C = J.C; mp.ensemble = J.ensemble;
-        BerParams prm = md.prm;
-        prm.seg = seg; prm.n_seg = n_seg;
+        const int P = 8 * N, nvl = J.n_var / (int)md.prm.size();     // pairs per K1 launch
         for (long long f0 = f_lo; f0 < f_hi; f0 += J.batch) {
             const long long nf = std::min(J.batch, f_hi - f0);
             mp.frame_begin = f0; mp.frame_step = 1; mp.n_frames = nf;
             const int mgrid = (int)std::min<long long>(nf, (long long)d.sm_count);
-            cudaError_t e = cudaSuccess;
-            if (J.use_gemm) {
-                const int rc = mask_gemm_batch(h, d, md.mg, mp.seed, f0, nf, J.fused ? nullptr : static_cast<float2*>(md.d_stream),
-                                               seg, n_seg, J.C, J.ensemble);
+            if (J.use_gemm) {      // every pair's masked symbols of the batch, one symbol draw and one product
+                const int rc = mask_gemm_batch(h, d, md.mg, mp.seed, f0, nf, seg, n_seg, J.C, J.ensemble);
                 if (rc) return rc;
-            } else {
-                // (SEG: the segmented instantiation, whose parameters carry the table)
-                auto launch = [&](auto kern_plain, auto kern_seg, size_t msm) {
-                    cudaError_t es = cudaFuncSetAttribute(seg ? (const void*)kern_seg : (const void*)kern_plain,
-                                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm);
-                    if (es == cudaSuccess && seg) kern_seg<<<mgrid, 256, msm, d.stream>>>(mp);
-                    else if (es == cudaSuccess) kern_plain<<<mgrid, 256, msm, d.stream>>>(static_cast<const MaskParams&>(mp));
-                    return es;
-                };
-                switch (N) {
-                    case 128: e = launch(tx_mask_kernel<128>, tx_mask_kernel<128, true>, MaskSmem<128>::bytes(sys.S, mp.stride, sys.tail_tx)); break;
-                    case 256: e = launch(tx_mask_kernel<256>, tx_mask_kernel<256, true>, MaskSmem<256>::bytes(sys.S, mp.stride, sys.tail_tx)); break;
-                    default:  e = launch(tx_mask_kernel<512>, tx_mask_kernel<512, true>, MaskSmem<512>::bytes(sys.S, mp.stride, sys.tail_tx)); break;
-                }
             }
-            WOFDM_CUDA(h, e);
-            WOFDM_CUDA(h, cudaGetLastError());
-            if (f0 == 0 && !segs) {
-                // development aid: WOFDM_MASK_DUMP=<file> writes the masked Tx streams of the first (up to 4) frames as raw float32 pairs
-                const char* dump = J.dump_env;
-                if (dump && *dump) {
-                    std::vector<float> hs(2 * J.body * (size_t)std::min<long long>(nf, 4));
-                    WOFDM_CUDA(h, cudaMemcpyAsync(hs.data(), md.d_stream, hs.size() * 4, cudaMemcpyDeviceToHost, d.stream));
-                    WOFDM_CUDA(h, cudaStreamSynchronize(d.stream));
-                    if (FILE* fp = fopen(dump, "wb")) { fwrite(hs.data(), 4, hs.size(), fp); fclose(fp); }
+            for (size_t k = 0; k < md.prm.size(); ++k) {
+                const int v = (int)k * nvl;                              // (first) pair of this K1 launch
+                cudaError_t e = cudaSuccess;
+                if (J.use_gemm) {
+                    // the K1 kernel gathers from Y itself (ber_tconv2.cuh, tconv2_load_masked), or reads pair v's assembled stream
+                    if (!J.fused) {
+                        const int rc = mask_gemm_assemble(h, d, md.mg, v, nf, static_cast<float2*>(md.d_stream));
+                        if (rc) return rc;
+                    }
+                } else {
+                    mp.win_tx = md.mp.win_tx + (size_t)v * mp.n_tx;
+                    mp.Gp = md.mp.Gp + (size_t)v * P;
+                    // (SEG: the segmented instantiation, whose parameters carry the table)
+                    auto launch = [&](auto kern_plain, auto kern_seg, size_t msm) {
+                        cudaError_t es = cudaFuncSetAttribute(seg ? (const void*)kern_seg : (const void*)kern_plain,
+                                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm);
+                        if (es == cudaSuccess && seg) kern_seg<<<mgrid, 256, msm, d.stream>>>(mp);
+                        else if (es == cudaSuccess) kern_plain<<<mgrid, 256, msm, d.stream>>>(static_cast<const MaskParams&>(mp));
+                        return es;
+                    };
+                    switch (N) {
+                        case 128: e = launch(tx_mask_kernel<128>, tx_mask_kernel<128, true>, MaskSmem<128>::bytes(sys.S, mp.stride, sys.tail_tx)); break;
+                        case 256: e = launch(tx_mask_kernel<256>, tx_mask_kernel<256, true>, MaskSmem<256>::bytes(sys.S, mp.stride, sys.tail_tx)); break;
+                        default:  e = launch(tx_mask_kernel<512>, tx_mask_kernel<512, true>, MaskSmem<512>::bytes(sys.S, mp.stride, sys.tail_tx)); break;
+                    }
                 }
+                WOFDM_CUDA(h, e);
+                WOFDM_CUDA(h, cudaGetLastError());
+                if (f0 == 0 && !segs && v == 0) {
+                    // development aid: WOFDM_MASK_DUMP=<file> writes the masked Tx streams of the first (up to 4) frames as raw float32 pairs
+                    const char* dump = J.dump_env;
+                    if (dump && *dump) {
+                        std::vector<float> hs(2 * J.body * (size_t)std::min<long long>(nf, 4));
+                        WOFDM_CUDA(h, cudaMemcpyAsync(hs.data(), md.d_stream, hs.size() * 4, cudaMemcpyDeviceToHost, d.stream));
+                        WOFDM_CUDA(h, cudaStreamSynchronize(d.stream));
+                        if (FILE* fp = fopen(dump, "wb")) { fwrite(hs.data(), 4, hs.size(), fp); fclose(fp); }
+                    }
+                }
+                BerParams prm = md.prm[k];
+                prm.seg = seg; prm.n_seg = n_seg;
+                prm.frame_begin = f0; prm.frame_step = 1; prm.n_frames = nf;
+                WOFDM_CUDA(h, J.run.var->launch(prm, (int)std::min<long long>(nf, J.max_ctas), J.run.lay.bytes, d.stream));
+                h->launches += 2;
             }
-            prm.frame_begin = f0; prm.frame_step = 1; prm.n_frames = nf;
-            WOFDM_CUDA(h, J.run.var->launch(prm, (int)std::min<long long>(nf, J.max_ctas), J.run.lay.bytes, d.stream));
-            h->launches += 2;
         }
         return WOFDM_OK;
     };
@@ -1445,7 +1474,7 @@ int masked_run(MaskedJob& J, long long g_lo, long long g_hi, const Segments* seg
     }
     std::vector<std::vector<unsigned long long>> cnts;
     if (!rc) {
-        try { cnts.assign(nd, std::vector<unsigned long long>(J.ncnt * 2, 0ull)); }
+        try { cnts.assign(nd, std::vector<unsigned long long>(nout * 2, 0ull)); }
         catch (const std::bad_alloc&) { rc = fail(h, WOFDM_ENOMEM, "host allocation failed"); }
     }
     // (the downloads into pageable memory block the host: only after every device has its work)
@@ -1453,13 +1482,13 @@ int masked_run(MaskedJob& J, long long g_lo, long long g_hi, const Segments* seg
         DeviceCtx& d = h->devs[J.devs[i].slot];
         cudaSetDevice(d.dev);
         cudaError_t es = cudaSuccess;
-        if (!rc) es = cudaMemcpyAsync(cnts[i].data(), J.devs[i].d_cnt, J.cnt_bytes, cudaMemcpyDeviceToHost, d.stream);
+        if (!rc) es = cudaMemcpyAsync(cnts[i].data(), J.devs[i].d_cnt, J.n_var * J.cnt_bytes, cudaMemcpyDeviceToHost, d.stream);
         if (es == cudaSuccess) es = cudaStreamSynchronize(d.stream);
         if (es != cudaSuccess && !rc) rc = fail(h, WOFDM_ECUDA, std::string("wofdm_ber_run_masked: ") + cudaGetErrorString(es));
     }
     cudaSetDevice(h->devs[0].dev);
     if (rc) return rc;
-    for (size_t i = 0; i < J.ncnt; ++i) {
+    for (size_t i = 0; i < nout; ++i) {
         unsigned long long be = 0, se = 0;
         for (int k = 0; k < nd; ++k) { be += cnts[k][2 * i]; se += cnts[k][2 * i + 1]; }
         bit_err[i] = (int64_t)be; sym_err[i] = (int64_t)se;
@@ -1467,19 +1496,19 @@ int masked_run(MaskedJob& J, long long g_lo, long long g_hi, const Segments* seg
     return WOFDM_OK;
 }
 
-// A checked job of the channel-mask chain: the whole job (segs == nullptr: global frame ids, the unsegmented kernels) or
-// the frames of a segment list, in either case this shard's contiguous block of the local indices.  resolve == 0:
-// bit_err / sym_err [n_snr]; else [n_snr][Cr][Nr] (wofdm_ber_run_resolved's layout, one window pair), counted by the
-// resolved twin of the K1 kernel this chain picks.  Totals as in run_job; bit_tot may be NULL.
-int run_masked_impl(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, const double* chan,
-                    int L, int C, const double* snr_db, int n_snr, int64_t ensemble, const Segments* segs, uint64_t seed,
-                    uint32_t variant, int roll_off, int shard_index, int shard_count, int resolve, int64_t* bit_err,
-                    int64_t* sym_err, int64_t* sym_tot, int64_t* bit_tot) {
+// A checked job of the channel-mask chain for n_var window pairs: the whole job (segs == nullptr: global frame ids, the
+// unsegmented kernels) or the frames of a segment list, in either case this shard's contiguous block of the local indices.
+// resolve == 0: bit_err / sym_err [n_var][n_snr]; else [n_snr][Cr][Nr] (wofdm_ber_run_resolved's layout, one window pair),
+// counted by the resolved twin of the K1 kernel this chain picks.  Totals as in run_job; bit_tot may be NULL.
+int run_masked_impl(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
+                    const int* roll_off, const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
+                    const Segments* segs, uint64_t seed, uint32_t variant, int shard_index, int shard_count, int resolve,
+                    int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot, int64_t* bit_tot) {
     const Segments all = segs ? Segments() : job_segments(C, std::vector<int64_t>(n_snr, ensemble));
     const Segments& sg = segs ? *segs : all;
     const ShardRule r = ShardRule::block(sg.n_local, shard_index, shard_count);
     MaskedJob J;
-    int rc = masked_setup(J, h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, seed, variant, roll_off, resolve,
+    int rc = masked_setup(J, h, sys, win_tx, win_rx, n_var, roll_off, chan, L, C, snr_db, n_snr, ensemble, seed, variant, resolve,
                           r.hi - r.lo, segs ? segs->n() : 0);
     if (!rc) rc = masked_run(J, r.lo, r.hi, segs, bit_err, sym_err);
     if (rc) return rc;
@@ -1508,7 +1537,24 @@ int wofdm_ber_run_masked_shard(wofdm_handle h, const wofdm_sys_t* sys, const dou
     const int rc = check_masked(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, roll_off, shard_index, shard_count, 0,
                                 bit_err && bit_tot && sym_err && sym_tot);
     if (rc) return rc;
-    return run_masked_impl(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, nullptr, seed, variant, roll_off,
+    return run_masked_impl(h, sys, win_tx, win_rx, 1, &roll_off, chan, L, C, snr_db, n_snr, ensemble, nullptr, seed, variant,
+                           shard_index, shard_count, 0, bit_err, sym_err, sym_tot, bit_tot);
+}
+
+int wofdm_ber_run_masked_multi(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                               const int* roll_off, int n_var, const double* chan, int L, int C, const double* snr_db, int n_snr,
+                               int64_t ensemble, uint64_t seed, uint32_t variant, int shard_index, int shard_count,
+                               int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot) {
+    NvtxRange nvtx_("wofdm_ber_run_masked_multi");
+    if (!h) return WOFDM_EINVAL;
+    if (n_var < 1 || n_var > WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "n_var must be in [1, WOFDM_MAX_VARIANTS]");
+    if (!roll_off) return fail(h, WOFDM_EINVAL, "NULL roll_off");
+    for (int v = 0; v < n_var; ++v) {         // (the pairs differ only in what check_masked reads of roll_off)
+        const int rc = check_masked(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, roll_off[v], shard_index,
+                                    shard_count, 0, bit_err && bit_tot && sym_err && sym_tot);
+        if (rc) return rc;
+    }
+    return run_masked_impl(h, sys, win_tx, win_rx, n_var, roll_off, chan, L, C, snr_db, n_snr, ensemble, nullptr, seed, variant,
                            shard_index, shard_count, 0, bit_err, sym_err, sym_tot, bit_tot);
 }
 
@@ -1523,7 +1569,7 @@ int wofdm_ber_run_masked_resolved(wofdm_handle h, const wofdm_sys_t* sys, const 
     if (!bit_err || !sym_err || !sym_tot) return fail(h, WOFDM_EINVAL, "NULL output buffer");
     rc = check_masked(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, roll_off, shard_index, shard_count, resolve, true);
     if (rc) return rc;
-    return run_masked_impl(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, nullptr, seed, variant, roll_off,
+    return run_masked_impl(h, sys, win_tx, win_rx, 1, &roll_off, chan, L, C, snr_db, n_snr, ensemble, nullptr, seed, variant,
                            shard_index, shard_count, resolve, bit_err, sym_err, sym_tot, nullptr);
 }
 
@@ -1540,7 +1586,7 @@ int wofdm_ber_run_masked_segments(wofdm_handle h, const wofdm_sys_t* sys, const 
     if (!rc) rc = check_segments(h, segments, n_seg, n_snr, ensemble_max);
     if (rc) return rc;
     const Segments sg = seg_table(segments, n_seg, C);
-    return run_masked_impl(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, &sg, seed, variant, roll_off,
+    return run_masked_impl(h, sys, win_tx, win_rx, 1, &roll_off, chan, L, C, snr_db, n_snr, ensemble_max, &sg, seed, variant,
                            shard_index, shard_count, resolve, bit_err, sym_err, sym_tot, nullptr);
 }
 
@@ -1563,7 +1609,7 @@ int wofdm_ber_run_masked_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const 
     // chain's rule.
     const long long total = (long long)n_snr * C * ensemble_max;
     MaskedJob J;
-    rc = masked_setup(J, h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, seed, variant + 1, roll_off, 0,
+    rc = masked_setup(J, h, sys, win_tx, win_rx, 1, &roll_off, chan, L, C, snr_db, n_snr, ensemble_max, seed, variant + 1, 0,
                       (long long)(((__int128)total + shard_count - 1) / shard_count), n_snr);
     if (rc) return rc;
     wofdm_ber_plan p = nullptr;

@@ -93,6 +93,8 @@ struct BerParams {
     // ascending), channel-major inside a segment; the frame id is f = (snr_idx*C + c)*ensemble + e_begin + e (seg_frame)
     const long long* seg;
     int n_seg;
+    // TXY instantiations with nvar > 1 (wofdm_ber_run_masked_multi): window pair v reads its columns at tx_y + v * tx_ypair
+    long long tx_ypair;
 };
 
 // ---- constellation helpers (oracle/wofdm_oracle.py: idx_to_levels / levels_to_idx) --------------

@@ -511,6 +511,8 @@ ber_tconv2_kernel(const BerParams prm) {
 
         // =========================== transmitter ===========================
         if (!HS && prm.tx_stream != nullptr) {          // uniform: masked Tx stream from tx_mask_kernel (mask_kernel.cuh)
+            // (TXY: every window pair transmits the same symbols -- the first one stores them)
+            if (!TXY || var == 0)
             for (int e = tid; e < S * TPF; e += NT) {
                 const int tt = e % TPF;
                 uint32_t w[4];
@@ -523,12 +525,17 @@ ber_tconv2_kernel(const BerParams prm) {
                 symw[e] = make_uint4(w[0], w[1], w[2], w[3]);
             }
             if constexpr (TXY) {             // (its own instantiations: the production kernels stay as they are)
-                // the frame this CTA takes next: its S columns of Y are contiguous -- one bulk prefetch into L2 (the loader is
-                // bound by the latency of its gather, and the product wrote Y through to HBM)
-                if (tid == 0 && j + nslots < prm.n_frames)
-                    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" :: "l"(prm.tx_y + (size_t)(j + nslots) * S * prm.tx_yp),
+                // the (frame, window pair) this CTA takes next -- the next pair of this frame, or the first pair of its next
+                // frame: its S columns of Y are contiguous -- one bulk prefetch into L2 (the loader is bound by the latency of
+                // its gather, and the product wrote Y through to HBM).  Pair v's columns start at tx_y + v * tx_ypair.
+                const bool last_var = var + 1 == nvar;
+                if (tid == 0 && (!last_var || j + nslots < prm.n_frames))
+                    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;"
+                                 :: "l"(prm.tx_y + (last_var ? (size_t)(j + nslots) * S * prm.tx_yp
+                                                             : (size_t)(var + 1) * prm.tx_ypair + (size_t)j * S * prm.tx_yp)),
                                  "r"((uint32_t)(S * prm.tx_yp * 4)) : "memory");
-                tconv2_load_masked<NT>(prm.tx_y + (size_t)j * S * prm.tx_yp, prm.tx_yp, S, stride, n_tx, body, uh, ul, tid);
+                tconv2_load_masked<NT>(prm.tx_y + (size_t)var * prm.tx_ypair + (size_t)j * S * prm.tx_yp, prm.tx_yp, S, stride, n_tx, body,
+                                       uh, ul, tid);
             } else {
                 const float2* src = prm.tx_stream + (size_t)j * body;
                 for (int i = tid; i < body; i += NT) {

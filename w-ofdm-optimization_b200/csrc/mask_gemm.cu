@@ -29,7 +29,9 @@
 //                                            into pre-tiled hi | lo operands
 //   mask_sym_kernel                          the Philox symbol draws of K1 (load_sym_idx) -> lattice points as fp16 B tiles
 //   mask_gemm_f16                            persistent, warp-specialised: bulk-copy producer, one MMA thread, four epilogue
-//                                            warps; two 128 x 256 accumulators in tensor memory, three 64 KB stages
+//                                            warps; two 128 x 256 accumulators in tensor memory, three 64 KB stages.  The
+//                                            mask matrices of n_var window pairs are stacked as row tiles of A: one launch
+//                                            for all pairs, each B tile read by all of their row tiles
 //   mask_assemble_kernel                     (K1 kernels other than ber_tconv2.cuh, which gathers from Y itself:) the filtered
 //                                            symbols overlap-added with the frame stride (tx2rx, :420-431): the serialised
 //                                            stream K1 reads (BerParams::tx_stream)
@@ -227,10 +229,14 @@ __global__ void __launch_bounds__(256) mask_sym_kernel(const BerParams draw, lon
     }
 }
 
-// Persistent: CTA q takes the tiles q, q + grid, ...; tile p = (column tile p / RT, row tile p % RT) -- CTAs that run side by
-// side share their B tile in L2.  Warps 0-3 = epilogue (TMEM lanes 32w..32w+31), warp 4 = producer, warp 5 = MMA issuer.
+// Persistent: CTA q takes the tiles q, q + grid, ...; tile p = (column tile p / RA, row tile p % RA), RA = nvar RT row tiles
+// of all pairs -- CTAs that run side by side share their B tile in L2.  Row tile rr belongs to pair rr / RT: its output goes
+// to that pair's Y (+ (rr / RT) ypair), scaled by that pair's inverse scale.  Warps 0-3 = epilogue (TMEM lanes
+// 32w..32w+31), warp 4 = producer, warp 5 = MMA issuer.
 __global__ void __launch_bounds__(NTHREADS, 1) mask_gemm_f16(const __half* __restrict__ At, const __half* __restrict__ Bt, float* __restrict__ Y,
-                                                            const float* __restrict__ scale, int nk, int RT, int n_tiles, int Yp, long long ncols) {
+                                                            const float* __restrict__ scale, int nk, int RT, int nvar, int n_tiles, int Yp,
+                                                            long long ypair, long long ncols) {
+    const int RA = nvar * RT;
     extern __shared__ __align__(1024) unsigned char sm[];
     __shared__ __align__(8) unsigned long long full_bar[NSTAGE], empty_bar[NSTAGE], acc_full[2], acc_empty[2];
     __shared__ uint32_t tmem_base_s;
@@ -261,8 +267,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) mask_gemm_f16(const __half* __res
             // ===== producer: two bulk copies per stage (A hi | lo, B), K blocks numbered through all of this CTA's tiles =====
             int it = 0;
             for (int p = blockIdx.x; p < n_tiles; p += gridDim.x) {
-                const __half* ra = At + (size_t)(p % RT) * nk * (2 * (size_t)A_HALVES);
-                const __half* rb = Bt + (size_t)(p / RT) * nk * (size_t)B_HALVES;
+                const __half* ra = At + (size_t)(p % RA) * nk * (2 * (size_t)A_HALVES);
+                const __half* rb = Bt + (size_t)(p / RA) * nk * (size_t)B_HALVES;
                 for (int kb = 0; kb < nk; ++kb, ++it) {
                     const int st = it % NSTAGE;
                     if (it >= NSTAGE) mbar_wait(smem_u32(&empty_bar[st]), (uint32_t)(((it / NSTAGE) - 1) & 1));
@@ -304,15 +310,16 @@ __global__ void __launch_bounds__(NTHREADS, 1) mask_gemm_f16(const __half* __res
     } else {
         // ===== epilogue warps: thread = one row of the tile (TMEM lane 32 warp + lane): for every column (symbol) the warp
         //       stores 32 consecutive floats of Y =====
-        const float descale = scale[1];
         int tl = 0;
         for (int p = blockIdx.x; p < n_tiles; p += gridDim.x, ++tl) {
             const int buf = tl & 1;
-            const long long col0 = (long long)(p / RT) * TN;
-            const int r = (p % RT) * TM + warp * 32 + lane;
+            const long long col0 = (long long)(p / RA) * TN;
+            const int rr = p % RA, v = rr / RT;
+            const int r = (rr - v * RT) * TM + warp * 32 + lane;
+            const float descale = scale[2 * v + 1];
             mbar_wait(smem_u32(&acc_full[buf]), (uint32_t)((tl >> 1) & 1));
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            float* yrow = Y + (size_t)col0 * Yp + r;
+            float* yrow = Y + (size_t)v * ypair + (size_t)col0 * Yp + r;
 #pragma unroll 1
             for (int cc = 0; cc < TN / 32; ++cc) {
                 uint32_t v[32];
@@ -364,50 +371,57 @@ __global__ void __launch_bounds__(256) mask_assemble_kernel(const float* __restr
 
 }  // namespace
 
-size_t mask_gemm_plan(const wofdm_sys_t& sys, long long batch, MaskGemm& mg) {
+size_t mask_gemm_plan(const wofdm_sys_t& sys, long long batch, int nvar, MaskGemm& mg) {
     memset(&mg, 0, sizeof(mg));
     mg.N = sys.N; mg.S = sys.S; mg.cp = sys.cp; mg.bits = sys.bits; mg.guard = sys.guard; mg.tail_tx = sys.tail_tx;
     mg.n_tx = sys.N + sys.cp + sys.cs; mg.stride = mg.n_tx - sys.tail_tx; mg.M = 2 * mg.n_tx - 1;
     mg.nact = sys.N - 2 * sys.guard;
     mg.Kp = 2 * ((2 * mg.nact + KB - 1) / KB * KB); mg.nk = mg.Kp / KB;          // [a_s | a_{s-1}], each half padded to the K block
     mg.RT = (2 * mg.n_tx + TM - 1) / TM; mg.Yp = mg.RT * TM;
-    mg.batch = batch;
+    mg.batch = batch; mg.nvar = nvar;
     const size_t cols = (size_t)((batch * sys.S + TN - 1) / TN) * TN;
-    return (size_t)mg.RT * mg.nk * 2 * A_BYTES + cols * mg.Kp * 2 + cols * mg.Yp * 4 + (size_t)mg.M * 16 + (size_t)mg.M * mg.nact * 16 + 4096;
+    mg.ypair = (long long)(cols * mg.Yp);
+    return (size_t)nvar * ((size_t)mg.RT * mg.nk * 2 * A_BYTES + cols * mg.Yp * 4) + cols * mg.Kp * 2 + (size_t)mg.M * 16 +
+           (size_t)mg.M * mg.nact * 16 + (size_t)nvar * 32 + 4096;
 }
 
-int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, int roll_off, const float* d_wtx, bool unit_impulse) {
+int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, const int* roll_off, const float* d_wtx, bool unit_impulse) {
     const size_t cols = (size_t)((mg.batch * mg.S + TN - 1) / TN) * TN;
     const size_t at_b = (size_t)mg.RT * mg.nk * 2 * A_BYTES, bt_b = cols * mg.Kp * 2, y_b = cols * mg.Yp * 4;
-    mg.At = static_cast<__half*>(arena_take(d, at_b));
+    mg.At = static_cast<__half*>(arena_take(d, mg.nvar * at_b));
     mg.Bt = static_cast<__half*>(arena_take(d, bt_b));
-    mg.Y = static_cast<float*>(arena_take(d, y_b));
+    mg.Y = static_cast<float*>(arena_take(d, mg.nvar * y_b));
     mg.g = static_cast<double2*>(arena_take(d, (size_t)mg.M * 16));
     mg.Mm = static_cast<double2*>(arena_take(d, (size_t)mg.M * mg.nact * 16));
-    mg.scale = static_cast<float*>(arena_take(d, 16));
-    mg.maxbits = static_cast<unsigned*>(arena_take(d, 16));
+    mg.scale = static_cast<float*>(arena_take(d, (size_t)mg.nvar * 8));
+    mg.maxbits = static_cast<unsigned*>(arena_take(d, (size_t)mg.nvar * 4));
     if (!mg.At || !mg.Bt || !mg.Y || !mg.g || !mg.Mm || !mg.scale || !mg.maxbits) return fail(h, WOFDM_ENOMEM, "mask product: arena exhausted");
-    if (unit_impulse) {
-        const double2 one = make_double2(1.0, 0.0);       // (pageable source: the copy returns once it is staged)
-        WOFDM_CUDA(h, cudaMemsetAsync(mg.g, 0, (size_t)mg.M * 16, d.stream));
-        WOFDM_CUDA(h, cudaMemcpyAsync(mg.g, &one, sizeof(one), cudaMemcpyHostToDevice, d.stream));
-    } else {
-        mask_response_kernel<<<(mg.M + 63) / 64, 64, (size_t)mg.M * 24, d.stream>>>(mg.g, mg.M, roll_off);
-        WOFDM_CUDA(h, cudaGetLastError());
-    }
-    WOFDM_CUDA(h, cudaMemsetAsync(mg.maxbits, 0, 4, d.stream));
+    WOFDM_CUDA(h, cudaMemsetAsync(mg.maxbits, 0, (size_t)mg.nvar * 4, d.stream));
     WOFDM_CUDA(h, cudaMemsetAsync(mg.Bt, 0, bt_b, d.stream));      // K padding and the columns behind the batch stay zero
-    const int ne = mg.M * mg.nact;
-    mask_matrix_kernel<<<(ne + 255) / 256, 256, (size_t)mg.N * 16, d.stream>>>(mg.g, d_wtx, mg.Mm, mg.maxbits, mg.N, mg.n_tx, mg.cp, mg.guard, mg.M, mg.nact);
-    WOFDM_CUDA(h, cudaGetLastError());
-    mask_split_kernel<<<2 * d.sm_count, 256, 0, d.stream>>>(mg.Mm, mg.maxbits, mg.At, mg.scale, mg.M, mg.n_tx, mg.nact, mg.Kp, mg.RT);
-    WOFDM_CUDA(h, cudaGetLastError());
+    // pair by pair on one g / Mm (the stream orders them)
+    for (int v = 0; v < mg.nvar; ++v) {
+        if (unit_impulse) {
+            const double2 one = make_double2(1.0, 0.0);       // (pageable source: the copy returns once it is staged)
+            WOFDM_CUDA(h, cudaMemsetAsync(mg.g, 0, (size_t)mg.M * 16, d.stream));
+            WOFDM_CUDA(h, cudaMemcpyAsync(mg.g, &one, sizeof(one), cudaMemcpyHostToDevice, d.stream));
+        } else {
+            mask_response_kernel<<<(mg.M + 63) / 64, 64, (size_t)mg.M * 24, d.stream>>>(mg.g, mg.M, roll_off[v]);
+            WOFDM_CUDA(h, cudaGetLastError());
+        }
+        const int ne = mg.M * mg.nact;
+        mask_matrix_kernel<<<(ne + 255) / 256, 256, (size_t)mg.N * 16, d.stream>>>(mg.g, d_wtx + (size_t)v * mg.n_tx, mg.Mm, mg.maxbits + v,
+                                                                                    mg.N, mg.n_tx, mg.cp, mg.guard, mg.M, mg.nact);
+        WOFDM_CUDA(h, cudaGetLastError());
+        mask_split_kernel<<<2 * d.sm_count, 256, 0, d.stream>>>(mg.Mm, mg.maxbits + v, mg.At + v * at_b / sizeof(__half), mg.scale + 2 * v,
+                                                                mg.M, mg.n_tx, mg.nact, mg.Kp, mg.RT);
+        WOFDM_CUDA(h, cudaGetLastError());
+        h->launches += unit_impulse ? 2 : 3;
+    }
     WOFDM_CUDA(h, cudaFuncSetAttribute(mask_gemm_f16, cudaFuncAttributeMaxDynamicSharedMemorySize, NSTAGE * STAGE_BYTES));
-    h->launches += unit_impulse ? 2 : 3;
     return WOFDM_OK;
 }
 
-int mask_gemm_batch(wofdm_ctx* h, DeviceCtx& d, const MaskGemm& mg, uint64_t seed, long long f0, long long nf, float2* stream,
+int mask_gemm_batch(wofdm_ctx* h, DeviceCtx& d, const MaskGemm& mg, uint64_t seed, long long f0, long long nf,
                     const long long* seg, int n_seg, int C, long long ensemble) {
     if (nf < 1 || nf > mg.batch) return fail(h, WOFDM_EINVAL, "mask product: batch out of range");
     BerParams draw;
@@ -430,14 +444,18 @@ int mask_gemm_batch(wofdm_ctx* h, DeviceCtx& d, const MaskGemm& mg, uint64_t see
         WOFDM_CUDA(h, cudaFuncSetAttribute((const void*)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_s));
     fn<<<grid_s, 256, sm_s, d.stream>>>(draw, f0, nf, mg.S, mg.guard, mg.nact, mg.Bt, mg.nk);
     WOFDM_CUDA(h, cudaGetLastError());
-    const int CT = (int)((ncols + TN - 1) / TN), n_tiles = CT * mg.RT;
-    mask_gemm_f16<<<std::min(n_tiles, d.sm_count), NTHREADS, NSTAGE * STAGE_BYTES, d.stream>>>(mg.At, mg.Bt, mg.Y, mg.scale, mg.nk, mg.RT, n_tiles, mg.Yp, ncols);
+    const int CT = (int)((ncols + TN - 1) / TN), n_tiles = CT * mg.RT * mg.nvar;
+    mask_gemm_f16<<<std::min(n_tiles, d.sm_count), NTHREADS, NSTAGE * STAGE_BYTES, d.stream>>>(mg.At, mg.Bt, mg.Y, mg.scale, mg.nk, mg.RT, mg.nvar,
+                                                                                           n_tiles, mg.Yp, mg.ypair, ncols);
     WOFDM_CUDA(h, cudaGetLastError());
     h->launches += 2;
-    if (!stream) return WOFDM_OK;          // (the K1 kernel gathers from Y itself: ber_tconv2.cuh, tconv2_load_masked)
+    return WOFDM_OK;
+}
+
+int mask_gemm_assemble(wofdm_ctx* h, DeviceCtx& d, const MaskGemm& mg, int v, long long nf, float2* stream) {
     const long long total = nf * (mg.tail_tx + (long long)mg.S * mg.stride);
     mask_assemble_kernel<<<(int)std::min<long long>((total + 255) / 256, (long long)d.sm_count * 16), 256, 0, d.stream>>>(
-        mg.Y, stream, nf, mg.S, mg.stride, mg.n_tx, mg.tail_tx, mg.Yp);
+        mg.Y + (size_t)v * mg.ypair, stream, nf, mg.S, mg.stride, mg.n_tx, mg.tail_tx, mg.Yp);
     WOFDM_CUDA(h, cudaGetLastError());
     h->launches += 1;
     return WOFDM_OK;

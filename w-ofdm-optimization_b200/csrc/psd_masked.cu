@@ -158,7 +158,7 @@ extern "C" int wofdm_psd_masked(wofdm_handle h, const wofdm_sys_t* sys, const do
     MaskGemm mg[2];
     size_t need = wf.size() * 4 + twf.size() * 4 + 2 * (size_t)P * 8;
     for (int k = 0; k < 2; ++k)
-        if (outs[k]) need += mask_gemm_plan(*sys, batch, mg[k]);
+        if (outs[k]) need += mask_gemm_plan(*sys, batch, 1, mg[k]);
     rc = arena_reserve(h, d, need);
     if (rc) return rc;
     float* d_w = static_cast<float*>(arena_take(d, wf.size() * 4));
@@ -172,7 +172,7 @@ extern "C" int wofdm_psd_masked(wofdm_handle h, const wofdm_sys_t* sys, const do
     auto run = [&]() -> int {
         for (int k = 0; k < 2; ++k) {
             if (!outs[k]) continue;
-            const int r = mask_gemm_setup(h, d, mg[k], roll_off, d_w, k == 1);
+            const int r = mask_gemm_setup(h, d, mg[k], &roll_off, d_w, k == 1);
             if (r) return r;
         }
         PsdMaskedParams p;
@@ -183,7 +183,7 @@ extern "C" int wofdm_psd_masked(wofdm_handle h, const wofdm_sys_t* sys, const do
             const long long nf = std::min(batch, f0 + n_frames - fb);
             for (int k = 0; k < 2; ++k) {
                 if (!outs[k]) continue;
-                const int r = mask_gemm_batch(h, d, mg[k], seed, fb, nf, nullptr);
+                const int r = mask_gemm_batch(h, d, mg[k], seed, fb, nf);
                 if (r) return r;
                 p.Y = mg[k].Y; p.items = nf * groups; p.psd = d_psd + (size_t)k * P;
                 cudaError_t e = cudaSuccess;

@@ -216,6 +216,29 @@ def run_sim_mc(ensemble, cpLength, csLength, tailTx, tailRx, windowTx, windowRx,
     return float(rm["bit_err"][0] / rm["bit_tot"][0]), float(r["bit_err"][0] / r["bit_tot"][0])
 
 
+def run_sim_mc_multi(ensemble, cpLength, csLength, tailTx, tailRx, windowTx, windowRx, channel, snr, offset,
+                     prefixRemovalLength, circularShiftLength, numSubcar, bitsPerSubcar, symbolsPerTx, rollOff, seed=0,
+                     handle=None):
+    """run_sim_mc for n_var configurations on the same symbols in one masked and one unmasked call: windowTx, windowRx and
+    rollOff are lists of n_var (diagonal matrices or vectors; integers).  Returns (berMasked, ber), arrays of n_var.
+    Configuration v's unmasked chain has noise stream v (Handle.ber_run_multi), its masked chain n_var + v
+    (Handle.ber_run_masked_multi), so no two streams meet; with one configuration this is run_sim_mc's result exactly."""
+    wts, wrs, ros = list(windowTx), list(windowRx), list(np.atleast_1d(rollOff))
+    if not (len(wts) == len(wrs) == len(ros)) or not wts:
+        raise ValueError(f"windowTx, windowRx and rollOff must be lists of the same length "
+                         f"(got {len(wts)}, {len(wrs)}, {len(ros)})")
+    h = handle or default_handle()
+    s = capi.SysT(N=int(numSubcar), cp=int(cpLength), cs=int(csLength), tail_tx=int(tailTx), tail_rx=int(tailRx),
+                  rm=int(prefixRemovalLength), shift=int(circularShiftLength), bits=int(bitsPerSubcar),
+                  S=int(symbolsPerTx), noise_norm=1, constellation=1, precision=0, guard=int(offset))
+    wt, wr, ch = [_diag(w) for w in wts], [_diag(w) for w in wrs], np.asarray(channel).ravel()
+    nv = len(wt)
+    r = h.ber_run_multi(s, wt, wr, ch, [float(snr)], int(ensemble), seed=seed, variant=0)
+    rm = h.ber_run_masked_multi(s, wt, wr, ch, [float(snr)], int(ensemble), seed=seed, variant=nv,
+                                roll_offs=[int(x) for x in ros])
+    return rm["bit_err"][:, 0] / rm["bit_tot"][0], r["bit_err"][:, 0] / r["bit_tot"][0]
+
+
 def run_sim_mc_per_subcarrier(ensemble, cpLength, csLength, tailTx, tailRx, windowTx, windowRx, channel, snr, offset,
                               prefixRemovalLength, circularShiftLength, numSubcar, bitsPerSubcar, symbolsPerTx, rollOff, seed=0,
                               handle=None):
