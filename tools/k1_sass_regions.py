@@ -4,9 +4,11 @@ The working warps of ber_tconv2.cuh announce their part of the split stream (bar
 noise while the MMA warp issues; the accumulator pass waits on the MMAs' mbarrier (SYNCS.PHASECHK).  Draws that ptxas hoists
 in front of the arrive delay the MMAs of the whole CTA (DESIGN section 7, constant switches), and the counters do not show
 it.  This prints, per kernel, the instructions from the barrier before the arrive to the arrive ("tx->arrive") and from the
-arrive to the first wait behind it ("arrive->wait"): production N = 256 and the HS instance have ~50-110 and ~650, a build
-whose draws were hoisted had 468 and 233.
-usage: k1_sass_regions.py <object or cubin> [kernel-name substring] [--regions]"""
+arrive to the first wait behind it ("arrive->wait"): production N = 256 and the HS instances have ~25-110 and ~550-650, a
+build whose draws were hoisted had 468 and 233.  "frame loop" is the longest backward branch's span (the working warps'
+loop over frames); --opcodes adds its instructions by opcode.
+usage: k1_sass_regions.py <object or cubin> [kernel-name substring] [--regions] [--opcodes]"""
+import collections
 import re
 import subprocess
 import sys
@@ -36,6 +38,16 @@ def counts(ins):
     return a - before, wait - a
 
 
+def frame_loop(ins):
+    """(first, last) instruction of the longest backward branch (16-byte instructions)"""
+    best = (0, 0)
+    for i, s in enumerate(ins):
+        m = re.match(r"BRA(\.\S+)?\s.*?0x([0-9a-f]+)$", s)
+        if m and int(m.group(2), 16) // 16 < i and i - int(m.group(2), 16) // 16 > best[1] - best[0]:
+            best = (int(m.group(2), 16) // 16, i)
+    return best
+
+
 def main():
     args = [a for a in sys.argv[1:] if not a.startswith("--")]
     want = args[1] if len(args) > 1 else "ber_tconv2_kernel"
@@ -43,7 +55,12 @@ def main():
         if want not in name:
             continue
         c = counts(ins)
-        print(f"{name}: {len(ins)} instructions" + (f", tx->arrive {c[0]}, arrive->wait {c[1]}" if c else ", no BAR.ARV"))
+        lo, hi = frame_loop(ins)
+        print(f"{name}: {len(ins)} instructions, frame loop {hi - lo + 1}" +
+              (f", tx->arrive {c[0]}, arrive->wait {c[1]}" if c else ", no BAR.ARV"))
+        if "--opcodes" in sys.argv:
+            ops = collections.Counter(i.split()[0].split(".")[0] for i in ins[lo:hi + 1])
+            print("    " + " ".join(f"{k} {v}" for k, v in ops.most_common()))
         if "--regions" in sys.argv:
             cuts = [0] + [i for i, s in enumerate(ins) if s.startswith(("BAR.", "SYNCS.PHASECHK"))] + [len(ins)]
             for a, b in zip(cuts, cuts[1:]):

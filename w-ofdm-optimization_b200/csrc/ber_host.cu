@@ -78,6 +78,14 @@ bool flat_tx_window(const wofdm_sys_t& s, const double* wt) {
 // gathered from the mask product's output (BerParams::tx_y, BerVariant::txy)
 enum class TxSource { drawn, stream, gather };
 
+// WOFDM_VARIANT: `want` occurs in `name`; with a trailing '$', at its end
+bool variant_name_matches(const char* name, const char* want) {
+    const size_t nw = strlen(want);
+    if (nw == 0 || want[nw - 1] != '$') return strstr(name, want) != nullptr;
+    const size_t nn = strlen(name);
+    return nw - 1 <= nn && strncmp(name + nn - (nw - 1), want, nw - 1) == 0;
+}
+
 // what a caller of choose_variant asks for
 struct KernelRequest {
     bool verify = false;              // the verify instantiations (wofdm_ber_verify)
@@ -94,6 +102,13 @@ struct KernelRequest {
 bool tconv2_fixed_shape(const wofdm_sys_t& s, const KernelRequest& rq) {
     return rq.win_tx != nullptr && rq.nvar == 1 && rq.tx == TxSource::drawn && s.tail_rx == 0 && s.guard == 0 &&
            flat_tx_window(s, rq.win_tx);
+}
+
+// ... and the geometry compiled into a fixed-shape instance (ber_tconv2.cuh: tconv2_geom(geom)), L the job's channel length
+bool tconv2_fixed_geometry(const wofdm_sys_t& s, int L, int geom) {
+    const Tconv2Geom g = tconv2_geom(geom);
+    return g.N > 0 && s.N == g.N && s.S == g.S && s.cp == g.cp && s.cs == g.cs && s.tail_tx == g.tail_tx && s.tail_rx == 0 &&
+           s.rm == g.rm && s.shift == g.shift && L == g.L && s.bits == g.bits;
 }
 
 // tensor-core kernel: windows that are one value between their tails (BerParams::flat_tx / flat_rx)
@@ -143,7 +158,8 @@ int choose_staged(wofdm_ctx* h, const wofdm_sys_t& s, int L, size_t smem_cap, bo
 
 // The kernel of request rq, among those without resolved counters (BerVariant::res): a tensor-core kernel wherever one
 // applies, else a register kernel, else the staged kernel.  WOFDM_NO_TCONV and WOFDM_NO_CIRC add no_tconv / no_circ;
-// WOFDM_VARIANT=<substring> restricts the tensor-core and register candidates (kernel tuning aid, e.g. "_b2").
+// WOFDM_VARIANT=<substring> restricts the tensor-core and register candidates (kernel tuning aid, e.g. "_b2"); a trailing
+// '$' anchors it at the end of the name ("tiles9_b2$": the generic kernel, not its fixed-shape instances).
 int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, size_t smem_cap, const KernelRequest& rq, Choice* out) {
     const int stride = s.N + s.cp + s.cs - s.tail_tx;
     const int sec = s.S * stride;
@@ -159,7 +175,7 @@ int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, size_t smem_cap, c
     if (s.precision != 1 && !rq.staged_only) {
         for (const auto& v : h->variants) {
             if (v.TC == 0 || v.fp64 || v.verify != rq.verify || v.N != s.N || v.res) continue;
-            if (want && !strstr(v.name, want)) continue;
+            if (want && !variant_name_matches(v.name, want)) continue;
             if (v.ntile > 0) {
                 // channel convolution on the tensor cores (ber_tconv2.cuh): first choice wherever it applies -- one Tx pass,
                 // L <= LB, prefix / suffix / tails inside the outer register rows, power sums and the zeros behind the
@@ -170,6 +186,7 @@ int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, size_t smem_cap, c
                 if (no_tconv || S_cta > v.NT / tpf || L > v.LB) continue;
                 if (v.txy != want_txy) continue;                     // (the mask product's consumers serve the channel-mask variant only)
                 if (v.fixed_shape && !fixed_shape) continue;
+                if (v.geom > 0 && !tconv2_fixed_geometry(s, L, v.geom)) continue;
                 if (v.CL > 1 && want_txs) continue;                  // (the masked Tx stream is a one-CTA-per-frame feature)
                 // a receiver thread holds at most N48_MAXLEV noise samples besides its 16 FFT rows
                 if ((stride - s.N + (s.noise_norm == 1 ? s.tail_tx + L - 1 : 0) + tpf - 1) / tpf > (v.LB > TCV_LB ? N48_MAXLEV : N48_MAXLEV_SHORT)) continue;
@@ -178,10 +195,12 @@ int choose_variant(wofdm_ctx* h, const wofdm_sys_t& s, int L, size_t smem_cap, c
                 if (need > 512 * v.ntile || sec_cta <= 512 * (v.ntile - 2)) continue;   // (the kernel range-checks its last two tiles only)
                 const BerSmem lay = v.layout(S_cta, stride, s.tail_tx, s.tail_rx, L, rq.nvar, 0);
                 if (lay.bytes > smem_cap) continue;
-                // fewest taps of history first (MMAs per tile), then fewest tiles, then the fixed-shape instance
-                // (same noise numbering and arithmetic, counters bit for bit: 3856 SASS instructions instead of 4976)
+                // fewest taps of history first (MMAs per tile), then fewest tiles, then the fixed-geometry instance, then the
+                // fixed-shape one (same noise numbering and arithmetic, counters bit for bit: DESIGN.md section 3)
+                auto fixed_rank = [](const BerVariant& x) { return x.geom > 0 ? 2 : x.fixed_shape ? 1 : 0; };
                 if (!best.var || best.var->ntile == 0 || v.LB < best.var->LB ||
-                    (v.LB == best.var->LB && (v.ntile < best.var->ntile || (v.ntile == best.var->ntile && v.fixed_shape)))) {
+                    (v.LB == best.var->LB && (v.ntile < best.var->ntile ||
+                                              (v.ntile == best.var->ntile && fixed_rank(v) > fixed_rank(*best.var))))) {
                     best.var = &v; best.lay = lay; best.chunk = 0;
                 }
                 continue;

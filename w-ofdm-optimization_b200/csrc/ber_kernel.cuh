@@ -158,7 +158,8 @@ __host__ __device__ __forceinline__ uint32_t gray_xor_mask(int bits, int constel
 __device__ __forceinline__ unsigned code_bit_errors(uint32_t x, uint32_t gmask) { return __popc(x ^ ((x >> 1) & gmask)); }
 
 // 16 level codes (one byte each) of OFDM symbol s for thread t: sub-carriers t + q*TPF
-template <int N, bool VERIFY>
+// (BITS > 0: the bits per sub-carrier of a kernel compiled for one geometry, else prm.bits)
+template <int N, bool VERIFY, int BITS = 0>
 __device__ __forceinline__ void load_sym_idx(const BerParams& prm, long long f, int s, int t, uint32_t (&w)[4]) {
     constexpr int TPF = N / 16;
     if constexpr (VERIFY) {
@@ -178,7 +179,7 @@ __device__ __forceinline__ void load_sym_idx(const BerParams& prm, long long f, 
     } else {
         const uint4 r = philox4x32_10_rk(make_uint4((uint32_t)f, (uint32_t)((unsigned long long)f >> 32),
                                                     (uint32_t)(s * TPF + t), STREAM_SYM), prm.rk);
-        const uint32_t mask = ((1u << prm.bits) - 1u) * 0x01010101u;
+        const uint32_t mask = ((1u << (BITS > 0 ? BITS : prm.bits)) - 1u) * 0x01010101u;
         w[0] = r.x & mask; w[1] = r.y & mask; w[2] = r.z & mask; w[3] = r.w & mask;
     }
 }

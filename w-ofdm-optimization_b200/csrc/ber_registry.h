@@ -19,6 +19,7 @@ struct BerVariant {
     bool txy = false;          // ber_tconv2.cuh: takes the Tx stream from the mask product's output (BerParams::tx_y) and nothing else
     bool res = false;          // counters resolved by sub-carrier / channel (BerParams::res_bins / res_chan) and nothing else
     bool fixed_shape = false;  // ber_tconv2.cuh HS: the switches of one shape class as constants (ber_host.cu: tconv2_fixed_shape)
+    int geom = 0;              // > 0: ... and the geometry tconv2_geom(geom) as constants (ber_host.cu: tconv2_fixed_geometry)
     bool fp64, verify;
     BerSmem (*layout)(int S, int stride, int tail_tx, int tail_rx, int L, int chunk, int use_global);
     const void* fn;

@@ -226,17 +226,29 @@ __host__ __device__ inline BerSmem tconv2_smem_layout(int S, int stride, int tai
 // taps are PUSHED into both CTAs, so every read is local.
 // RES: error counters resolved by sub-carrier and / or channel (BerParams::res_chan / res_bins, ber_kernel.cuh: res_flush);
 // in a cluster every CTA keeps and flushes the accumulators of its own symbols
-// HS: the frame loop of the common shape class compiled with its switches as constants (ber_host.cu: tconv2_fixed_shape):
+// HS != 0: the frame loop of the common shape class compiled with its switches as constants (ber_host.cu: tconv2_fixed_shape):
 // a flat Tx window with cp, cs >= tail_tx, tail_rx = 0, one window pair, no guard band, the symbols drawn in the kernel.
-// N, S, L, the Rx window's flatness and the conventions (noise_norm, constellation) stay run-time.
-template <int N, int NT, int NTILE, int MINB, bool VERIFY, int CL = 1, int LB = TCV_LB, bool TXY = false, bool RES = false,
-          bool HS = false>
+// HS = TCV2_HS_CLASS: S, L, the prefix / suffix / tail lengths and bits stay run-time.  HS = a geometry id (Tconv2Geom):
+// they are constants too, and with them every stream address, store test and power mask of the frame loop
+// (ber_host.cu: tconv2_fixed_geometry).  The Rx window's flatness and the conventions (noise_norm, constellation) stay
+// run-time in both.
+struct Tconv2Geom { int N, S, cp, cs, tail_tx, rm, shift, L, bits; };
+constexpr int TCV2_HS_CLASS = 1;
+constexpr int TCV2_HS_WTX256 = 2;        // bench.py's headline: wtx, N = 256, 16 symbols, cp = 16, tail_tx = 8, L = 21, 16-QAM
+__host__ __device__ constexpr Tconv2Geom tconv2_geom(int hs) {
+    return hs == TCV2_HS_WTX256 ? Tconv2Geom{256, 16, 16, 8, 8, 16, 0, 21, 4} : Tconv2Geom{0, 0, 0, 0, 0, 0, 0, 0, 0};
+}
+template <int N, int NT, int NTILE, int MINB, bool VERIFY, int CL = 1, int LB = TCV_LB, bool TXY = false, bool RES = false, int HS = 0>
 __global__ void __launch_bounds__(NT + tconv2_mma_warp_threads(N, NT), MINB)
 ber_tconv2_kernel(const BerParams prm) {
     using T = float;
     using C2 = float2;
     using P = FftPlan<N>;
     constexpr int TPF = P::TPF, FPP = NT / TPF, ER = 2, NW = NT / 32;
+    constexpr Tconv2Geom G = tconv2_geom(HS);
+    constexpr bool GEO = G.N > 0;                                         // the geometry is compiled in
+    static_assert(HS == 0 || HS == TCV2_HS_CLASS || GEO, "HS: 0, TCV2_HS_CLASS or a geometry id");
+    static_assert(!GEO || (G.N == N && G.S * TPF <= NT && G.L <= LB), "a geometry of this instance's class");
     static_assert(NT == 256 || NT == 512, "eight warps read a tile's accumulators");
     constexpr int TG = NT / 256, NTH = (NTILE + TG - 1) / TG;             // tile sets; tiles per thread
     constexpr uint32_t TMEM_COLS = tconv_tmem_cols(NTILE);
@@ -255,18 +267,25 @@ ber_tconv2_kernel(const BerParams prm) {
     int rank = 0;
     if constexpr (CL > 1) rank = (int)cooperative_groups::this_cluster().block_rank();
     const bool last_rank = rank == CL - 1;
-    const int S = prm.S / CL, sb = rank * S;    // this CTA's symbols: sb .. sb + S - 1 (the whole frame when CL == 1)
-    const int stride = prm.stride, n_tx = prm.n_tx, beta = prm.tail_tx, L = prm.L;
-    const int cp = prm.cp, cs = prm.cs;
+    // the geometry: constants of a geometry instance, else read from the parameters where the generic loop reads it
+    auto g_S = [&] { return GEO ? G.S : prm.S; };
+    auto g_tail_rx = [&] { return GEO ? 0 : prm.tail_rx; };
+    auto g_rm = [&] { return GEO ? G.rm : prm.rm; };
+    auto g_shift = [&] { return GEO ? G.shift : prm.shift; };
+    auto g_bits = [&] { return GEO ? G.bits : prm.bits; };
+    const int S = g_S() / CL, sb = rank * S;    // this CTA's symbols: sb .. sb + S - 1 (the whole frame when CL == 1)
+    const int stride = GEO ? G.N + G.cp + G.cs - G.tail_tx : prm.stride, n_tx = GEO ? G.N + G.cp + G.cs : prm.n_tx;
+    const int beta = GEO ? G.tail_tx : prm.tail_tx, L = GEO ? G.L : prm.L;
+    const int cp = GEO ? G.cp : prm.cp, cs = GEO ? G.cs : prm.cs;
     const int hh = HS ? 0 : prm.tail_rx >> 1;
-    const int hb = prm.bits >> 1, m = 1 << hb;
+    const int hb = g_bits() >> 1, m = 1 << hb;
     const int sec = S * stride;                 // samples kept after the channel (this CTA's)
     const int body = beta + sec;                // serialised Tx stream length
     const int npow = (prm.noise_norm == 1 && last_rank) ? body + L - 1 : sec;   // samples inside the frame-wide power sums
 
     const int nvar = (!VERIFY && !HS && prm.nvar > 1) ? prm.nvar : 1;     // window pairs evaluated on every frame's symbols
     constexpr int PAD = tconv2_pad(LB), KS = tconv2_ksteps(LB), TBL = tconv2_tbl(LB), ZERO = tconv2_zero(LB);
-    const BerSmem lay = tconv2_smem_layout<N, NT, NTILE, LB, RES>(S, stride, beta, prm.tail_rx, L, nvar, 0);
+    const BerSmem lay = tconv2_smem_layout<N, NT, NTILE, LB, RES>(S, stride, beta, g_tail_rx(), L, nvar, 0);
     uint32_t* const ahi = reinterpret_cast<uint32_t*>(smem_raw);
     uint32_t* const alo = reinterpret_cast<uint32_t*>(smem_raw + lay.off_lo);
     uint32_t* const uh = ahi + PAD;         // uh[i], ul[i]: split stream sample i
@@ -279,7 +298,7 @@ ber_tconv2_kernel(const BerParams prm) {
     unsigned char* bt = smem_raw + lay.off_bt;
     T* const wtx_all = reinterpret_cast<T*>(smem_raw + lay.off_wtx);   // [nvar][WTXL]
     T* const wrx_all = reinterpret_cast<T*>(smem_raw + lay.off_wrx);   // [nvar][WRXL]
-    const int WTXL = tconv2_wtx_len(stride, beta), WRXL = tconv2_wrx_len(N, prm.tail_rx);
+    const int WTXL = tconv2_wtx_len(stride, beta), WRXL = tconv2_wrx_len(N, g_tail_rx());
     T* red = reinterpret_cast<T*>(smem_raw + lay.off_red);
     C2* qlut = reinterpret_cast<C2*>(smem_raw + lay.off_qlut);     // level code -> lattice point
     C2* qtx = qlut + 256;                                           // ... times the flat Tx window value
@@ -306,27 +325,27 @@ ber_tconv2_kernel(const BerParams prm) {
     // (BerParams::flat_tx / flat_rx: bit v = window pair v)
     for (int vv = 0; vv < nvar; ++vv) {
         const T* gw = reinterpret_cast<const T*>(prm.win_tx) + (size_t)vv * n_tx;
-        const T* gr = reinterpret_cast<const T*>(prm.win_rx) + (size_t)vv * (N + prm.tail_rx);
+        const T* gr = reinterpret_cast<const T*>(prm.win_rx) + (size_t)vv * (N + g_tail_rx());
         const bool ft = (prm.flat_tx >> vv) & 1, fr = (prm.flat_rx >> vv) & 1;
-        const T wflat = ft ? gw[beta] : (T)1, rflat = fr ? gr[prm.tail_rx] : (T)1;
+        const T wflat = ft ? gw[beta] : (T)1, rflat = fr ? gr[g_tail_rx()] : (T)1;
         for (int i = tid; i < n_tx; i += NT) wtx_all[vv * WTXL + i] = ft ? gw[i] / wflat : gw[i] * TCV_XSCALE;
-        for (int i = tid; i < N + prm.tail_rx; i += NT) wrx_all[vv * WRXL + i] = gr[i] / rflat;
+        for (int i = tid; i < N + g_tail_rx(); i += NT) wrx_all[vv * WRXL + i] = gr[i] / rflat;
     }
     // constellation table of window pair vv for the Tx stage
     auto build_qtx = [&](int vv) {
         const bool ft = (prm.flat_tx >> vv) & 1;
         const T wflat = ft ? reinterpret_cast<const T*>(prm.win_tx)[(size_t)vv * n_tx + beta] : (T)1;
-        for (int i = tid; i < (1 << prm.bits); i += NT) {
+        for (int i = tid; i < (1 << g_bits()); i += NT) {
             const C2 q = mk2<T>((T)(2 * (i >> hb) - (m - 1)), (T)(2 * (i & (m - 1)) - (m - 1)));
             qtx[i] = ft ? cscale(wflat * TCV_XSCALE, q) : q;
         }
     };
     for (int i = tid; i < PAD; i += NT) ahi[i] = 0u;
     for (int i = tid; i < 2 * TBL / 4; i += NT) reinterpret_cast<uint32_t*>(bt + 2 * TBL)[i] = 0u;   // (B0, B1: their rows 4..7 stay zero)
-    for (int i = tid; i < (1 << prm.bits); i += NT) qlut[i] = mk2<T>((T)(2 * (i >> hb) - (m - 1)), (T)(2 * (i & (m - 1)) - (m - 1)));
+    for (int i = tid; i < (1 << g_bits()); i += NT) qlut[i] = mk2<T>((T)(2 * (i >> hb) - (m - 1)), (T)(2 * (i & (m - 1)) - (m - 1)));
     build_qtx(0);
-    if (tid == 0 && prm.bits < 8) { qlut[255] = mk2<T>(0, 0); qtx[255] = mk2<T>(0, 0); }
-    const uint32_t gxm = gray_xor_mask(prm.bits, prm.constellation);
+    if (tid == 0 && g_bits() < 8) { qlut[255] = mk2<T>(0, 0); qtx[255] = mk2<T>(0, 0); }
+    const uint32_t gxm = gray_xor_mask(g_bits(), prm.constellation);
     uint32_t* const racc = reinterpret_cast<uint32_t*>(smem_raw + lay.off_res);   // RES: [nvar][N][2] = {bit, sym}
     if constexpr (RES) { for (int i = tid; i < 2 * N * nvar; i += NT) racc[i] = 0u; }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -365,7 +384,10 @@ ber_tconv2_kernel(const BerParams prm) {
     // thread's samples i = i0 + q TPF all have the same i mod 4, i.e. the same half and chunk slot: base + immediate
     const int RCH = NTILE * 128 + 4;            // chunks per half (+4: the halves sit 64 bytes apart modulo 128)
     // extras of the noise draws (ber_kernel.cuh: noise_draw48)
-    const N48Geom ng = n48_geom(prm);
+    const N48Geom ng = [&] {
+        if constexpr (GEO) return N48Geom{TPF, 0, stride - N, prm.noise_norm == 1 ? beta + L - 1 : 0, (N - G.shift) & (TPF - 1)};
+        else return n48_geom(prm);
+    }();
     const int xt = (t - ng.base) & (TPF - 1);   // this thread's extras: x = xt + lev * TPF
 
     // distributed shared memory: the previous CTA's split stream (its last Tx tail and the convolution history)
@@ -554,7 +576,7 @@ ber_tconv2_kernel(const BerParams prm) {
             {
                 uint32_t w[4], wq[4];
                 if (var == 0) {
-                    load_sym_idx<N, VERIFY>(prm, f, sb + se, t, w);
+                    load_sym_idx<N, VERIFY, G.bits>(prm, f, sb + se, t, w);
                 } else {                           // the symbols of the frame, as stored by the first window pair
                     const uint4 ws = symw[se * TPF + t];
                     w[0] = ws.x; w[1] = ws.y; w[2] = ws.z; w[3] = ws.w;
@@ -759,7 +781,7 @@ ber_tconv2_kernel(const BerParams prm) {
         // on a frame id that passes through a shared-memory load behind the arrive (ahi[0], the operand's zero pad: always 0),
         // which ptxas does not move across the barrier.
         long long fn = f;
-        if constexpr (HS) {
+        if constexpr (HS != 0) {
             static_assert(CL == 1, "ahi[0] is zero only with one CTA per frame: a CTA of rank > 0 writes its neighbour's history there");
             uint32_t z;
             asm volatile("ld.volatile.shared.u32 %0, [%1];" : "=r"(z) : "r"(tcv_smem_u32(ahi)) : "memory");
@@ -769,7 +791,7 @@ ber_tconv2_kernel(const BerParams prm) {
             const bool act = slot < S;
             const int se = act ? TCV2_SLOT_SYMBOL(slot, S) : S - 1;
             const int sg = sb + se;                                      // symbol index in the frame
-            const int xas = ng.xa + (sg == prm.S - 1 ? ng.tailx : 0);    // extras of this symbol (uniform per transform group)
+            const int xas = ng.xa + (sg == g_S() - 1 ? ng.tailx : 0);    // extras of this symbol (uniform per transform group)
             const int nlev = (xas + TPF - 1) / TPF;
             const int pbase = sg * stride;
             if constexpr (VERIFY) {
@@ -944,8 +966,8 @@ ber_tconv2_kernel(const BerParams prm) {
             const int se = act ? s : S - 1;
             C2 v[16];
             // r of stream sample i: half (i >> 1) & 1, chunk i >> 2, element i & 1 -- constant i mod 4 for all of this thread's samples
-            const int ib = se * stride + prm.rm + hh;                    // stream position of block offset n = 0
-            const int i0 = ib + t + prm.shift;
+            const int ib = se * stride + g_rm() + hh;                    // stream position of block offset n = 0
+            const int i0 = ib + t + g_shift();
             const C2* const rsel = rb + ((i0 >> 1) & 1) * (2 * RCH) + (i0 & 1);
             const C2* const rrow = rsel + (i0 >> 2) * 2;                     // row q: sample i0 + q TPF
             auto r_at = [&](int i) -> C2 { return rsel[(i >> 2) * 2]; };     // i = i0 (mod 4)
@@ -954,13 +976,13 @@ ber_tconv2_kernel(const BerParams prm) {
             for (int q = 0; q < 16; ++q) {
                 if (q >= 1 && q <= 13) {
                     // tail_rx/2, shift <= TPF: rows 1..13 neither wrap nor touch the overlap-add margins (nor the window tails)
-                    const int n = t + q * TPF + prm.shift;
+                    const int n = t + q * TPF + g_shift();
                     const C2 y = caxpy(g, nz[q], rrow[q * (TPF / 2)]);
                     v[q] = flat_rx ? y : cscale(wr[n], y);
                     continue;
                 }
-                const int a0 = (q * TPF + prm.shift) & (N - 1);
-                const int n = (t + q * TPF + prm.shift) & (N - 1);
+                const int a0 = (q * TPF + g_shift()) & (N - 1);
+                const int n = (t + q * TPF + g_shift()) & (N - 1);
                 C2 o = cscale(wr[n], caxpy(g, nz[q], r_at(ib + n)));
                 if (hh > 0) {
                     const bool wraps = a0 + TPF > N;
