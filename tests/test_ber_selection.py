@@ -15,7 +15,7 @@ from oracle import wofdm_oracle as O
 pytestmark = pytest.mark.gpu
 
 ENV = ("WOFDM_DEBUG", "WOFDM_NO_TCONV", "WOFDM_NO_CIRC", "WOFDM_VARIANT", "WOFDM_RESOLVED_STAGED", "WOFDM_MASK_FFT",
-       "WOFDM_MASK_DUMP", "WOFDM_FORCE_CTAS_PER_SM", "WOFDM_MAX_CTAS_PER_SM")
+       "WOFDM_MASK_DUMP", "WOFDM_MAX_CTAS_PER_SM")
 
 # (system, N, cp, tail_tx, tail_rx, S, L, precision, guard, window pairs, flat Tx window, environment)
 SHAPES = {

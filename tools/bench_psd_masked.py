@@ -1,11 +1,11 @@
 """Throughput of wofdm_psd_masked at bench.py's mask_chain shape with long records (wtx, N = 256, cp 16, tail 8, guard 64,
 roll-off 10, S = 256 symbols per frame, MATLAB conventions), both estimators, 4096 frames (1.05e6 OFDM symbols) per call.
 
-  * wall time of the call with host buffers (both spectra), median of alternated rounds, for every product batch size in
-    --batch-cols (WOFDM_PSD_BATCH_COLS: symbols per product batch; 131072 is the default of the library);
-  * device time per kernel (symbol kernel, product, psd_masked_kernel) from a separate torch.profiler pass at the default
-    batch size, and the PSD kernel's rate over the bytes of Y it must read (every filtered symbol's n_tx complex fp32
-    samples once, for each of the two spectra);
+  * wall time of the call with host buffers (both spectra), median of alternated rounds, at the library's product batch
+    (131072 symbols);
+  * device time per kernel (symbol kernel, product, psd_masked_kernel) from a separate torch.profiler pass, and the PSD
+    kernel's rate over the bytes of Y it must read (every filtered symbol's n_tx complex fp32 samples once, for each of
+    the two spectra);
   * the card's name and power limit, read in the same run.
 Writes one JSON record to --out."""
 import argparse
@@ -24,7 +24,6 @@ from wofdm_b200 import capi
 ap = argparse.ArgumentParser()
 ap.add_argument("--frames", type=int, default=4096)
 ap.add_argument("--rounds", type=int, default=7)
-ap.add_argument("--batch-cols", default="131072,16384")
 ap.add_argument("--out", required=True)
 a = ap.parse_args()
 
@@ -34,24 +33,18 @@ s = W.params_from_name("wtx", 256, 16, 8, 0, bits=4, S=256, noise_norm=1, conste
 vt = capi.rc_window_tx(s)
 F = a.frames
 h = W.Handle([0])
-cols = [int(c) for c in a.batch_cols.split(",")]
 times = {}
-for c in cols:                                   # warm-up of every batch size and estimator
-    os.environ["WOFDM_PSD_BATCH_COLS"] = str(c)
+for est in ("reference", "hann"):                # warm-up of both estimators
+    h.psd_masked(s, vt, frames=F, seed=1, estimator=est)
+for r in range(a.rounds):                        # alternated estimators
     for est in ("reference", "hann"):
-        h.psd_masked(s, vt, frames=F, seed=1, estimator=est)
-for r in range(a.rounds):                        # alternated: batch size x estimator
-    for c in cols:
-        os.environ["WOFDM_PSD_BATCH_COLS"] = str(c)
-        for est in ("reference", "hann"):
-            t0 = time.perf_counter()
-            xm, xu = h.psd_masked(s, vt, frames=F, seed=2 + r, estimator=est)
-            times.setdefault(f"{c}/{est}", []).append(time.perf_counter() - t0)
-os.environ.pop("WOFDM_PSD_BATCH_COLS")
+        t0 = time.perf_counter()
+        xm, xu = h.psd_masked(s, vt, frames=F, seed=2 + r, estimator=est)
+        times.setdefault(est, []).append(time.perf_counter() - t0)
 wall = {k: {"median_ms": float(np.median(v) * 1e3), "min_ms": float(np.min(v) * 1e3), "max_ms": float(np.max(v) * 1e3),
             "ofdm_symbols_per_s": float(F * s.S / np.median(v))} for k, v in times.items()}
 
-# levels of the last call (Hann, last batch size) relative to the in-band mean
+# levels of the last call (Hann) relative to the in-band mean
 gb, P = 8 * s.guard, 8 * s.N
 deep = np.r_[0:gb - 256, P - gb + 256:P]
 levels = {}
@@ -60,7 +53,7 @@ for name, x in (("masked", xm), ("unmasked", xu)):
     levels[name] = {"obr_db": float(10 * np.log10(np.r_[x[:gb], x[-gb:]].mean() / inb)),
                     "deep_oob_db": float(10 * np.log10(x[deep].mean() / inb))}
 
-# device time per kernel: a separate profiled pass at the library's default batch size
+# device time per kernel: a separate profiled pass
 import torch
 from torch.profiler import ProfilerActivity, profile
 

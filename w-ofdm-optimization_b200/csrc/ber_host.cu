@@ -358,7 +358,6 @@ int prepare_kernel(wofdm_ctx* h, const BerVariant& v, size_t smem, int sm_count,
         const int by_tmem = 512 / (int)tconv_tmem_cols(v.ntile);
         nb = std::max(nb, std::min(by_smem, std::min(by_regs, by_tmem)));
     }
-    if (const char* f = getenv("WOFDM_FORCE_CTAS_PER_SM")) nb = std::max(1, atoi(f));    // tuning aid
     if (getenv("WOFDM_DEBUG")) fprintf(stderr, "[wofdm] %s: smem %zu B, %d CTAs/SM\n", v.name, smem, nb);
     if (nb < 1) return fail(h, WOFDM_EUNSUPPORTED, "kernel variant cannot be resident on this device");
     *blocks_per_sm = nb;

@@ -34,10 +34,6 @@ namespace wofdm {
 
 // transform group `slot` of a CTA works on its OFDM symbol S - 1 - slot: the pilot (symbol 0), whose receiver everybody waits
 // for, then sits in the warp with the highest index, which the warp schedulers serve first
-#ifndef TCV2_REVERSE_SLOTS
-#define TCV2_REVERSE_SLOTS 1
-#endif
-#define TCV2_SLOT_SYMBOL(slot, S) (TCV2_REVERSE_SLOTS ? (S) - 1 - (slot) : (slot))
 // development aid: per-warp clock() stamps at the phase boundaries of a few frames of CTA 0, printed from the device
 #ifndef TCV2_TRACE
 #define TCV2_TRACE 0
@@ -47,44 +43,17 @@ namespace wofdm {
 #else
 #define TCV2_STAMP(k) do { } while (0)
 #endif
-#ifndef TCV2_GT
-#define TCV2_GT 3
-#endif
-// Slicer folded into the equaliser product (production instantiations): the taps are stored halved, so the scale and offset
-// of slice_index (y = e / 2 + (m - 2) / 2) ride on the complex product's first packed FMA, and the upper clamp is taken in
-// floating point (FMNMX, one issue cycle) before the saturating round-up conversion instead of on the integers afterwards.
-// Same decisions as slice_index up to the rounding of the fused sum (fp32 grade either way; ties still go to the lower level).
-// Measured: 16 packed instructions and 32 two-cycle integer clamps fewer per thread and frame, 5.76 ms against 5.78 per
-// 202 500 frames -- within the noise, so the build keeps slice_index (one definition of the decision for every kernel).
-#ifndef TCV2_FOLD_SLICER
-#define TCV2_FOLD_SLICER 0
-#endif
-#ifndef TCV2_TXY_U
-#define TCV2_TXY_U 8      // stream samples per thread and round of the masked chain's loader (tconv2_load_masked)
-#endif
 #ifndef TCV2_DEBUG_BARRIERS
 #define TCV2_DEBUG_BARRIERS 0          // 1 (libwofdm_dbg.so): every relaxed synchronisation of the kernel replaced by a full barrier --
 #endif                                 // the reference the race test compares the production build with (compute-sanitizer is closed here)
-// Kernels whose working warps issue the MMAs (N = 1024): 1 = the issue is staggered over all warps -- four groups of four
-// warps issue a quarter of the tiles each, group g after g quarters of its noise draws -- so nobody sits in front of the
-// tensor core's queue for the whole convolution.  Each group has its own "stream complete" named barrier (14 - g).
-#ifndef TCV2_STAGGER
-#define TCV2_STAGGER 0     // (measured: 10.97 ms against 10.84 with the issuers skipping the accumulator pass -- the kernel is throughput bound)
-#endif
-#ifndef TCV2_REBALANCE
-#define TCV2_REBALANCE 1
-#endif
 // The frame's tiles complete in tconv2_nseg(N) segments, one mbarrier each: the accumulator pass starts on the first tiles while
 // the tensor core still works on the last ones.  Segment k is signalled once tile seg_end(k) -- the first tile of the NEXT
 // segment -- is complete too: that tile reads the last PAD samples of its predecessor's stream as convolution history, and
 // r is parked over the stream.
 // Measured (ms per launch, one against three segments): N = 512: 4.55 -> 4.41 (the MMAs outlast the noise draws there);
 // N = 256: 5.79 -> 5.88 (they do not: only the extra waits remain); N = 1024: 10.83 either way.
-#ifndef TCV2_NSEG_512
-#define TCV2_NSEG_512 3
-#endif
 constexpr int TCV2_MAXSEG = 4;
-__host__ __device__ constexpr int tconv2_nseg(int N) { return N == 512 ? TCV2_NSEG_512 : 1; }
+__host__ __device__ constexpr int tconv2_nseg(int N) { return N == 512 ? 3 : 1; }
 __host__ __device__ constexpr int tconv2_seg_end(int nseg, int ntile, int k) { return (ntile * (k + 1) + nseg - 1) / nseg; }   // tiles < seg_end(k): segments 0..k
 __host__ __device__ constexpr int tconv2_seg_of(int nseg, int ntile, int tt) {
     int k = 0;
@@ -99,28 +68,16 @@ constexpr int TCV2_BAR_RES = 15;         // named barrier of the working warps b
 // kernel with ~60 bytes of them (measured: 2.06e8 -> 2.12e8 OFDM symbols/s all the same).  N = 1024 (clusters) spills
 // 200 bytes under that cap (8.6e7 -> 6.8e7), so there four of the working warps, rotating from frame to frame, issue a
 // quarter of the frame's MMAs each before they draw their noise.
-#ifndef TCV2_MMAW_MAXN
-#define TCV2_MMAW_MAXN 512
-#endif
-// Register reallocation (setmaxnreg): the MMA warp is launched inside a whole warp group of four (setmaxnreg is a warp-group
-// instruction: with an incomplete group -- the MMA warp and one idle warp were tried -- the release never completes and the
-// working warps spin in their request); the three other warps are idle register donors.  The group shrinks to 24 registers
-// and the working warps grow from what the launch grants to tconv2_work_regs: NT = 256: 384 threads x 80 at launch ->
-// 256 x 104 + 128 x 24 (5.91 -> 5.83 ms per 202 500 frames).  The donors walk through the MMA warp's barrier
-// sequence and issue nothing.
-#ifndef TCV2_SETMAXNREG
-#define TCV2_SETMAXNREG 1
-#endif
-// (NT = 512: measured slower, 4.64 ms against 4.51 per 60 000 frames -- 20 warps of 112 registers against 17 of 96 with ~60
-//  bytes of spills; it keeps the lone MMA warp)
-#ifndef TCV2_SETMAXNREG_1024
-#define TCV2_SETMAXNREG_1024 0     // (measured: 104 bytes of spills at 112 registers, 11.85 ms against 11.22)
-#endif
-__host__ __device__ constexpr bool tconv2_setmaxnreg(int N, int NT) { return TCV2_SETMAXNREG && (NT == 256 || (TCV2_SETMAXNREG_1024 && N == 1024)); }
+// Register reallocation (setmaxnreg, NT = 256): the MMA warp is launched inside a whole warp group of four (setmaxnreg is a
+// warp-group instruction: with an incomplete group -- the MMA warp and one idle warp were tried -- the release never completes
+// and the working warps spin in their request); the three other warps are idle register donors.  The group shrinks to 24
+// registers and the working warps grow from the 80 the launch grants (384 threads) to 104: 256 x 104 + 128 x 24 (5.91 -> 5.83
+// ms per 202 500 frames).  The donors walk through the MMA warp's barrier sequence and issue nothing.  The donor scheme
+// measured slower at NT = 512 (DESIGN.md section 3), so N = 512 keeps the lone MMA warp and N = 1024 has none.
+__host__ __device__ constexpr bool tconv2_setmaxnreg(int NT) { return NT == 256; }
 __host__ __device__ constexpr int tconv2_mma_warp_threads(int N, int NT) {
-    return tconv2_setmaxnreg(N, NT) ? 128 : (N <= TCV2_MMAW_MAXN && NT <= 512) ? 32 : 0;
+    return tconv2_setmaxnreg(NT) ? 128 : (N <= 512 && NT <= 512) ? 32 : 0;
 }
-__host__ __device__ constexpr int tconv2_work_regs(int NT) { return NT == 256 ? 104 : 112; }   // (NT = 512: 640 x 96 -> 512 x 112 + 128 x 24)
 // (Registers: ptxas derives 96 per thread from __launch_bounds__(288, 2) and that is what the hardware grants -- the register
 //  file is allocated to an even number of warps per CTA: a build forced to 112 registers ran one CTA per SM, 7.9 ms instead
 //  of 6.0, and the 544-thread kernel at 117 failed to launch.)
@@ -155,12 +112,12 @@ __host__ __device__ constexpr int tconv2_wrx_len(int N, int tail_rx) { return (N
 // Channel-mask chain (TXY instantiations): the frame's serialised Tx stream gathered from the mask product's output
 // (mask_gemm.cu, BerParams::tx_y: column s of the frame = the filtered symbol f_s, n_tx samples (Re, Im) interleaved, the
 // filter tail of symbol s-1 already inside, main_channel_mask.m:413-416).  The filtered symbols are overlap-added with the
-// frame stride (tx2rx, :420-431): stream[s stride + i] = f_s[i] + f_{s-1}[stride + i].  TCV2_TXY_U stream samples per thread
+// frame stride (tx2rx, :420-431): stream[s stride + i] = f_s[i] + f_{s-1}[stride + i].  Eight stream samples per thread
 // and round, two loads each in flight (the loader is latency bound otherwise).
 template <int NT>
 static __device__ __forceinline__ void tconv2_load_masked(const float* __restrict__ y0, int yp, int S, int stride, int n_tx, int body,
                                                           uint32_t* __restrict__ uh, uint32_t* __restrict__ ul, int tid) {
-    constexpr int U = TCV2_TXY_U;
+    constexpr int U = 8;
     for (int p0 = tid; p0 < body; p0 += U * NT) {
         float2 a[U], c[U];
 #pragma unroll
@@ -315,7 +272,7 @@ ber_tconv2_kernel(const BerParams prm) {
     }
     if (tid == 0) {
         for (int k = 0; k < NSEG; ++k)       // one commit per issuing warp, segment and frame
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(tcv_smem_u32(bar + k)), "r"(tconv2_mma_warp_threads(N, NT) ? 1 : (TCV2_STAGGER && !TCV2_DEBUG_BARRIERS) ? NT / 32 : TCV2_NISSUE) : "memory");
+            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(tcv_smem_u32(bar + k)), "r"(tconv2_mma_warp_threads(N, NT) ? 1 : TCV2_NISSUE) : "memory");
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     for (int i = tid; i < P::NTW; i += NT) tw[i] = reinterpret_cast<const C2*>(prm.tw)[i];
@@ -405,7 +362,7 @@ ber_tconv2_kernel(const BerParams prm) {
     int trace_it = 0;
 #endif
     if (MMAW && warp >= NW) {
-        if constexpr (tconv2_setmaxnreg(N, NT)) asm volatile("setmaxnreg.dec.sync.aligned.u32 24;" ::: "memory");
+        if constexpr (tconv2_setmaxnreg(NT)) asm volatile("setmaxnreg.dec.sync.aligned.u32 24;" ::: "memory");
         // ===== the MMA warp: the CTA's extra warp issues every tcgen05.mma of the kernel and nothing else =====
         // An issuing thread sits in front of the tensor core's short queue for as long as the convolution takes (~40 cycles per
         // MMA, bound by the operand reads: ~2200 cycles per frame at N = 256).  Measured with the issue spread over four of
@@ -462,7 +419,7 @@ ber_tconv2_kernel(const BerParams prm) {
         frame_sync<CL>();
         return;
     }
-    if constexpr (MMAW && tconv2_setmaxnreg(N, NT)) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" :: "n"(tconv2_work_regs(NT)) : "memory");
+    if constexpr (tconv2_setmaxnreg(NT)) asm volatile("setmaxnreg.inc.sync.aligned.u32 104;" ::: "memory");
     long long f = prm.frame_begin + fslot * prm.frame_step;
     const long long df = nslots * prm.frame_step;
     long long fe = 0, de = 0;
@@ -569,7 +526,7 @@ ber_tconv2_kernel(const BerParams prm) {
             frame_sync<CL>();
         } else {
             const bool act = slot < S;
-            const int s = TCV2_SLOT_SYMBOL(slot, S);
+            const int s = S - 1 - slot;
             const int se = act ? s : S - 1;     // idle slots shadow the last symbol (identical stores)
             const bool first = sb + se == 0;    // the frame's first symbol has no predecessor
             C2 v[16];
@@ -705,46 +662,8 @@ ber_tconv2_kernel(const BerParams prm) {
         const uint32_t issuer = MMAW ? 0u : __shfl_sync(0xffffffffu, ((uint32_t)f * 0x9E3779B9u >> 28) + prm.variant + (uint32_t)(var + rank), 0);
         const int irank = (int)(((uint32_t)warp_u - issuer) & (NW - 1));   // warp-uniform: issuing warps have irank < TCV2_NISSUE
         const bool is_issuer = !MMAW && irank < TCV2_NISSUE;
-        constexpr bool STAG = !MMAW && TCV2_STAGGER && !TCV2_DEBUG_BARRIERS;
-        const int igrp = irank >> 2;                                    // staggered issue: this warp's group
-        auto issue_group = [&](auto gc) {                               // group g's quarter of the tiles, shared round-robin by its four warps
-            constexpr int g = decltype(gc)::value;
-            (void)g;
-            if constexpr (STAG) {
-                if (igrp == g) {
-                    asm volatile("bar.sync %0, %1;" :: "n"(TCV2_BAR_STREAM - g), "n"(NTB) : "memory");
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                    if (tcv_elect_one()) {
-                        constexpr int g0 = NTILE * g / 4, g1 = NTILE * (g + 1) / 4;
-#pragma unroll
-                        for (int ti = g0; ti < g1; ++ti) {
-                            if (((ti - g0) & 3) == (irank & 3)) {
-                                const uint32_t tacc = tmem + (uint32_t)(16 * ti);
-#pragma unroll
-                                for (int k = 0; k < KS; ++k) {
-                                    tcv_mma(tacc, d_ahi + (uint64_t)(ti * 128 + k * 2), d_bhl + (uint64_t)(k * 16), k != 0);
-                                    tcv_mma(tacc, d_alo + (uint64_t)(ti * 128 + k * 2), d_bh0 + (uint64_t)(k * 16), 1u);
-                                }
-                            }
-                        }
-                        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(tcv_smem_u32(bar)) : "memory");
-                    }
-                    __syncwarp();
-                }
-            }
-        };
-        if constexpr (STAG) {
-            static_assert(NW == 16 && NSEG == 1, "four groups of four warps, one commit per warp");
-            // "my part of the stream is stored" to the three groups this warp is not in
-            if (igrp != 0) asm volatile("bar.arrive %0, %1;" :: "n"(TCV2_BAR_STREAM), "n"(NTB) : "memory");
-            if (igrp != 1) asm volatile("bar.arrive %0, %1;" :: "n"(TCV2_BAR_STREAM - 1), "n"(NTB) : "memory");
-            if (igrp != 2) asm volatile("bar.arrive %0, %1;" :: "n"(TCV2_BAR_STREAM - 2), "n"(NTB) : "memory");
-            if (igrp != 3) asm volatile("bar.arrive %0, %1;" :: "n"(TCV2_BAR_STREAM - 3), "n"(NTB) : "memory");
-            issue_group(std::integral_constant<int, 0>{});
-        }
         if (TCV2_DEBUG_BARRIERS) __syncthreads();
-        if (STAG) {
-        } else if (is_issuer) {
+        if (is_issuer) {
             if (!TCV2_DEBUG_BARRIERS) asm volatile("bar.sync %0, %1;" :: "n"(TCV2_BAR_STREAM), "n"(NTB) : "memory");
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             if (tcv_elect_one()) {
@@ -789,7 +708,7 @@ ber_tconv2_kernel(const BerParams prm) {
         }
         {
             const bool act = slot < S;
-            const int se = act ? TCV2_SLOT_SYMBOL(slot, S) : S - 1;
+            const int se = act ? S - 1 - slot : S - 1;
             const int sg = sb + se;                                      // symbol index in the frame
             const int xas = ng.xa + (sg == g_S() - 1 ? ng.tailx : 0);    // extras of this symbol (uniform per transform group)
             const int nlev = (xas + TPF - 1) / TPF;
@@ -814,7 +733,6 @@ ber_tconv2_kernel(const BerParams prm) {
                     gauss_quad48(ca.z, ca.w, cc.y, nz[8 * gq + 2], nz[8 * gq + 3]);
                     gauss_quad48(cb.x, cb.y, cc.z, nz[8 * gq + 4], nz[8 * gq + 5]);
                     gauss_quad48(cb.z, cb.w, cc.w, nz[8 * gq + 6], nz[8 * gq + 7]);
-                    if (gq == 0) issue_group(std::integral_constant<int, 1>{}); else issue_group(std::integral_constant<int, 2>{});
                 }
                 nx[0] = nx[1] = mk2<T>(0, 0);
                 if (nlev > 0) {                                          // uniform per transform group
@@ -840,8 +758,6 @@ ber_tconv2_kernel(const BerParams prm) {
                     }
                 }
             }
-            if constexpr (VERIFY) { issue_group(std::integral_constant<int, 1>{}); issue_group(std::integral_constant<int, 2>{}); }
-            issue_group(std::integral_constant<int, 3>{});
             if (act) {
 #pragma unroll
                 for (int q = 0; q < 16; ++q) pn2 = csq_acc(nz[q], pn2);
@@ -861,8 +777,8 @@ ber_tconv2_kernel(const BerParams prm) {
         wait_tiles(0);
         TCV2_STAMP(6);
         if constexpr (CL > 1) asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-        constexpr int GT = TCV2_GT;                // tiles per batch of accumulator loads (one wait per batch)
-        if constexpr (!MMAW && TCV2_REBALANCE && !STAG) {
+        constexpr int GT = 3;                      // tiles per batch of accumulator loads (one wait per batch)
+        if constexpr (!MMAW) {
             // The working warps issue the MMAs (N = 1024): the four issuing warps of this frame reach this point ~2000 cycles
             // after the others (phase traces: they sat in front of the tensor core's queue), and everybody would wait for
             // them at the power barrier.  So they skip this pass: the tiles of a tensor-memory lane quarter -- which only the
@@ -962,7 +878,7 @@ ber_tconv2_kernel(const BerParams prm) {
         unsigned bit_cnt = 0, sym_cnt = 0;
         {
             const bool act = slot < S;
-            const int s = TCV2_SLOT_SYMBOL(slot, S);
+            const int s = S - 1 - slot;
             const int se = act ? s : S - 1;
             C2 v[16];
             // r of stream sample i: half (i >> 1) & 1, chunk i >> 2, element i & 1 -- constant i mod 4 for all of this thread's samples
@@ -1009,7 +925,7 @@ ber_tconv2_kernel(const BerParams prm) {
                 for (int k = tid; k < N; k += NT) {
                     const C2 y0 = geq[k];
                     const C2 x0 = qlut[pil[(k % TPF) * 16 + k / TPF]];
-                    C2 gk = cscale(((TCV2_FOLD_SLICER && !VERIFY) ? (T)0.5 : (T)1) * recip(y0.x * y0.x + y0.y * y0.y), cmulc(x0, y0));
+                    C2 gk = cscale(recip(y0.x * y0.x + y0.y * y0.y), cmulc(x0, y0));
                     if (!HS && prm.guard > 0 && !bin_active<N>(k, prm.guard)) gk = mk2<T>(0, 0);
                     geq[k] = gk;
                     if constexpr (CL > 1) {
@@ -1029,18 +945,8 @@ ber_tconv2_kernel(const BerParams prm) {
 #pragma unroll
                     for (int b = 0; b < 4; ++b) {
                         const int q = 4 * gq + b, k = t + q * TPF;
-                        uint32_t dq;
-                        C2 e;
-                        if constexpr (TCV2_FOLD_SLICER && !VERIFY) {
-                            const C2 gh = geq[k];                                          // G[k] / 2
-                            const T off = (T)0.5 * (T)(m - 2), top = (T)(m - 1);
-                            const C2 y = fma2(rotj(v[q]), mk2<T>(gh.y, gh.y), fma2(v[q], mk2<T>(gh.x, gh.x), mk2<T>(off, off)));   // :231, :233
-                            dq = (__float2uint_ru(fminf(y.x, top)) << hb) | __float2uint_ru(fminf(y.y, top));
-                            e = y;
-                        } else {
-                            e = cmul(v[q], geq[k]);                                        // :231
-                            dq = (uint32_t)slice_index(e, hb);                             // :233
-                        }
+                        const C2 e = cmul(v[q], geq[k]);                                   // :231
+                        const uint32_t dq = (uint32_t)slice_index(e, hb);                  // :233
                         d4 |= dq << (8 * b);
                         if constexpr (VERIFY) {
                             const size_t o = ((size_t)f * (prm.S - 1) + (sb + s - 1)) * N + k;

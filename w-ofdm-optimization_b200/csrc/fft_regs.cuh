@@ -18,9 +18,6 @@
 
 namespace wofdm {
 
-#ifndef FFT_TW_EARLY
-#define FFT_TW_EARLY 0
-#endif
 constexpr int TW1_PITCH = 18;     // row pitch of the first twiddle section (16 entries + 2: rows 144 B apart, 128-bit loads without bank conflicts)
 template <int N> struct FftPlan {
     static constexpr int a = (N % 4096 == 0) ? 3 : (N % 256 == 0) ? 2 : (N % 16 == 0) ? 1 : 0;
@@ -161,29 +158,19 @@ __device__ __forceinline__ void fft_regs(V2<T> (&v)[16], const int t, V2<T>* __r
         const int Ns = (p == 0) ? 1 : (p == 1) ? 16 : 256;
         const int k = t & (Ns - 1);
         if (p > 0) {
-            V2<T> w[16];
-#if FFT_TW_EARLY
-            if (p == 1) {                 // fetched before the barrier: they do not depend on the exchange
-                load16(w, tw + tw_off + k * TW1_PITCH);
-            } else {
-#pragma unroll
-                for (int m = 1; m < 16; ++m) w[m] = tw[tw_off + m * Ns + k];
-            }
-#endif
             fft_group_sync<TPF, NB>(group);
             {   // fft_pad(t + m TPF) = fft_pad(t) + m (TPF + TPF/8): one address, immediate offsets
                 const V2<T>* const xr = xb + fft_pad(t);
 #pragma unroll
                 for (int m = 0; m < 16; ++m) v[m] = xr[m * (TPF + TPF / 8)];
             }
-#if !FFT_TW_EARLY
+            V2<T> w[16];
             if (p == 1) {                 // (not held across the exchange: the kernels around this are register bound)
                 load16(w, tw + tw_off + k * TW1_PITCH);
             } else {
 #pragma unroll
                 for (int m = 1; m < 16; ++m) w[m] = tw[tw_off + m * Ns + k];
             }
-#endif
 #pragma unroll
             for (int m = 1; m < 16; ++m) v[m] = tw_apply<T, DIR>(v[m], w[m]);
             tw_off += p == 1 ? 16 * TW1_PITCH : 16 * Ns;

@@ -265,10 +265,9 @@ int interf_upload(wofdm_ctx* h, const wofdm_sys_t* sys, const double* win_tx, co
     // batch of channels whose B matrices fit the staging budget (1 GiB of the arena).  Measured and not kept: batches small
     // enough for the staging buffer to stay inside the 126 MB L2 (so that the operand never travels to HBM and back: one
     // 250-channel call moves 331 MB) -- 1.70 -> 2.31 ms (fp64) and 0.43 -> 0.74 ms (TF32) at 48 MB: the call is bound by its
-    // kernels, not by that traffic, and short batches quantise badly over 148 SMs.  WOFDM_K2_BATCH_MB repeats the experiment.
+    // kernels, not by that traffic, and short batches quantise badly over 148 SMs (DESIGN.md section 4).
     const size_t per_chan = (size_t)v.M * v.Kp * N * 8;
-    size_t budget = (size_t)1 << 30;
-    if (const char* e = getenv("WOFDM_K2_BATCH_MB")) budget = (size_t)std::max(1, atoi(e)) << 20;     // tuning aid
+    const size_t budget = (size_t)1 << 30;
     v.batch = (int)std::max<size_t>(1, std::min<size_t>((size_t)C, budget / per_chan));
     const size_t tf32_bytes = mode == 1 ? ((size_t)2 * 2 * N * v.Kp + (size_t)2 * v.batch * v.M * N * v.Kp) * 4 : 0;
     const size_t t32_bytes = mode == 1 ? (size_t)n_tx * N * 8 : 0;

@@ -16,7 +16,6 @@
 // split terms, tcgen05.commit frees the stage), two stages.  Epilogue (four warps): tcgen05.ld the accumulator
 // rows, mask the diagonal of slice 0, square, sum, one atomicAdd per row -- A itself is never written.
 #include <algorithm>
-#include <cstdlib>
 #include "interf.h"
 
 namespace wofdm {
@@ -27,7 +26,7 @@ constexpr int TM = 128, TN = TF32_TN, KB = TF32_KB, NSTAGE = 2;
 // Two CTAs that work on neighbouring row tiles of the same (channel, slice) form a thread-block cluster and share
 // the B operand: each fetches one half of a B stage and MULTICASTS it into both shared memories.  Without it the
 // persistent kernel pulls 96 KB per K block and SM out of L2 = 12.3 TB/s, which is the L2 limit, not the tensor pipe's.
-// (CLUSTER is a template parameter: 2 by default, WOFDM_TF32_CLUSTER=1 selects the non-multicast build for A/B runs)
+constexpr int CLUSTER = 2;
 constexpr int A_BYTES = TM * KB * 4, B_BYTES = TN * KB * 4;            // one hi (or lo) tile
 constexpr int STAGE_BYTES = 2 * A_BYTES + 2 * B_BYTES;                 // 96 KiB
 constexpr uint32_t IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(TN >> 3) << 17) | ((uint32_t)(TM >> 4) << 24);
@@ -78,7 +77,6 @@ __device__ __forceinline__ void cluster_sync_all() {
 // q, q + clusters, ...; pair p = (slice p / (mtiles/2), row tiles 2*(p % (mtiles/2)) + rank).  Warps 0-3 = epilogue (TMEM lanes 32w..32w+31), warp 4 = producer, warp 5 = MMA issuer.
 // Rt: [2N/TM][nk][hi|lo][TM*KB] tiles (tile_split_r below), Bt: [slices * N/TN][nk][hi|lo][TN*KB] tiles (build_b<true>, interf.cu)
 constexpr int NTHREADS = 192;
-template <int CLUSTER>
 __global__ void __launch_bounds__(NTHREADS, 1) gemm_power_tf32(const float* __restrict__ Rt, const float* __restrict__ Bt,
                                                               double* __restrict__ P, int N, int Kp, int Ms, int c0, int scalar,
                                                               int n_tiles, int nk_isi) {
@@ -88,8 +86,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_power_tf32(const float* __re
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     constexpr uint16_t CL_MASK = (1u << CLUSTER) - 1u;
     const int nk = Kp / KB, mtiles = 2 * N / TM;
-    uint32_t rank = 0;
-    if (CLUSTER > 1) asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
+    uint32_t rank;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
     const int q0 = blockIdx.x / CLUSTER, nq = gridDim.x / CLUSTER, n_pairs = n_tiles / CLUSTER, ppairs = mtiles / CLUSTER;
     const int ntile = N / TN;                                  // column tiles per slice: B tile sv = s * ntile + nt
 
@@ -110,7 +108,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_power_tf32(const float* __re
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (CLUSTER > 1) cluster_sync_all();          // the peer's barriers exist before anything is multicast onto them
+    cluster_sync_all();                           // the peer's barriers exist before anything is multicast onto them
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem = tmem_base_s;
 
@@ -130,11 +128,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_power_tf32(const float* __re
                     bulk_copy(dst, ra + (size_t)kb * (2 * TM * KB), 2 * A_BYTES, bar);                 // A hi | lo
                     // B hi | lo: this CTA's share, delivered to every CTA of the cluster (each receives all of it)
                     constexpr uint32_t QB = 2 * B_BYTES / CLUSTER;
-                    if (CLUSTER > 1)
-                        bulk_copy_multicast(dst + 2 * A_BYTES + rank * QB,
-                                            reinterpret_cast<const unsigned char*>(rb + (size_t)kb * (2 * TN * KB)) + (size_t)rank * QB, QB, bar, CL_MASK);
-                    else
-                        bulk_copy(dst + 2 * A_BYTES, rb + (size_t)kb * (2 * TN * KB), 2 * B_BYTES, bar);
+                    bulk_copy_multicast(dst + 2 * A_BYTES + rank * QB,
+                                        reinterpret_cast<const unsigned char*>(rb + (size_t)kb * (2 * TN * KB)) + (size_t)rank * QB, QB, bar, CL_MASK);
                 }
             }
         }
@@ -163,11 +158,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_power_tf32(const float* __re
                         mma_tf32(tacc, umma_desc(a_lo + off), umma_desc(b_hi + off), 1u);
                     }
                     // frees stage st in every CTA of the cluster (each of them multicasts into it)
-                    if (CLUSTER > 1)
-                        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                                     :: "r"(smem_u32(&empty_bar[st])), "h"(CL_MASK) : "memory");
-                    else
-                        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(smem_u32(&empty_bar[st])) : "memory");
+                    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+                                 :: "r"(smem_u32(&empty_bar[st])), "h"(CL_MASK) : "memory");
                 }
                 // completes once per tile, after every MMA of the tile
                 asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(smem_u32(&acc_full[buf])) : "memory");
@@ -214,7 +206,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_power_tf32(const float* __re
 
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (CLUSTER > 1) cluster_sync_all();          // nobody leaves while the peer's releases can still land on its barriers
+    cluster_sync_all();                           // nobody leaves while the peer's releases can still land on its barriers
     if (warp == 4) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"(2 * TN) : "memory");
 }
 
@@ -260,26 +252,19 @@ int interf_gemm_tf32(wofdm_ctx* h, const wofdm_sys_t* sys, const InterfDev& v, i
     WOFDM_CUDA(h, cudaGetLastError());
     const size_t smem = (size_t)NSTAGE * STAGE_BYTES;
     const int n_tiles = (2 * N / TM) * slices * (N / TN);
-    const char* env = getenv("WOFDM_TF32_CLUSTER");
-    const int cl = (env && atoi(env) == 1) ? 1 : 2;
-    auto launch = [&](auto kern, int CL) -> int {
-        WOFDM_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(CL * d.sm_count); cfg.blockDim = dim3(NTHREADS); cfg.dynamicSmemBytes = smem; cfg.stream = d.stream;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        int ncl = 0;
-        WOFDM_CUDA(h, cudaOccupancyMaxActiveClusters(&ncl, kern, &cfg));
-        if (ncl < 1) return fail(h, WOFDM_EUNSUPPORTED, "no cluster of the TF32 contraction kernel fits the device");
-        cfg.gridDim = dim3(CL * std::min(n_tiles / CL, ncl));
-        WOFDM_CUDA(h, cudaLaunchKernelEx(&cfg, kern, (const float*)Rt, (const float*)Bt, v.P, N, v.Kp, Ms, c0, scalar, n_tiles, nk_isi));
-        return WOFDM_OK;
-    };
-    static_assert((2 * TN / TM) % 2 == 0, "row tiles pair up inside a cluster");
-    const int rc = cl == 1 ? launch(gemm_power_tf32<1>, 1) : launch(gemm_power_tf32<2>, 2);
-    if (rc) return rc;
+    WOFDM_CUDA(h, cudaFuncSetAttribute(gemm_power_tf32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(CLUSTER * d.sm_count); cfg.blockDim = dim3(NTHREADS); cfg.dynamicSmemBytes = smem; cfg.stream = d.stream;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = CLUSTER; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    int ncl = 0;
+    WOFDM_CUDA(h, cudaOccupancyMaxActiveClusters(&ncl, gemm_power_tf32, &cfg));
+    if (ncl < 1) return fail(h, WOFDM_EUNSUPPORTED, "no cluster of the TF32 contraction kernel fits the device");
+    static_assert((2 * TN / TM) % CLUSTER == 0, "row tiles pair up inside a cluster");
+    cfg.gridDim = dim3(CLUSTER * std::min(n_tiles / CLUSTER, ncl));
+    WOFDM_CUDA(h, cudaLaunchKernelEx(&cfg, gemm_power_tf32, (const float*)Rt, (const float*)Bt, v.P, N, v.Kp, Ms, c0, scalar, n_tiles, nk_isi));
     WOFDM_CUDA(h, cudaGetLastError());
     h->launches += 2;
     return WOFDM_OK;

@@ -13,7 +13,6 @@
 // keeps |X|^2 in fp64 registers over all of the CTA's items; one fftshift-indexed atomicAdd(double) per bin and CTA at
 // the end, as psd_kernel (psd.cu) does.  fp32 arithmetic, fp64 accumulation.
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 
 #include "host_common.h"
@@ -147,8 +146,7 @@ extern "C" int wofdm_psd_masked(wofdm_handle h, const wofdm_sys_t* sys, const do
     WOFDM_CUDA(h, cudaSetDevice(d.dev));
     // batches of about `cols` symbols.  An L2-resident batch (16 384 symbols, 40 MB of Y at N = 256) measured slower than
     // 131 072 (DESIGN.md 4b): the product's tail wave and the launches per batch cost more than re-reading Y from HBM
-    long long cols = 131072;
-    if (const char* e = getenv("WOFDM_PSD_BATCH_COLS")) cols = std::max(1LL, atoll(e));     // tuning aid
+    const long long cols = 131072;
     const long long batch = std::min<long long>(n_frames, std::max<long long>(1, cols / sys->S));
     const std::vector<double> wd = tx_table(*sys, win_tx, false);
     const std::vector<float> wf(wd.begin(), wd.end());
