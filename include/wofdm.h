@@ -334,6 +334,26 @@ WOFDM_API int wofdm_ber_run_masked_segments(wofdm_handle h, const wofdm_sys_t* s
                          const int64_t* segments /* [n_seg][3] = {snr_idx, e_begin, e_count} */, int n_seg,
                          uint64_t seed, uint32_t variant, int roll_off, int shard_index, int shard_count, int resolve,
                          int64_t* bit_err, int64_t* sym_err, int64_t* sym_tot);
+/* wofdm_ber_run_masked_segments for n_var window pairs on the same frames (1 <= n_var <= WOFDM_MAX_VARIANTS), as
+ * wofdm_ber_run_masked_multi extends wofdm_ber_run_masked_shard: pair v = (win_tx + v*n_tx, win_rx + v*(N+tail_rx),
+ * roll_off[v]) gets exactly what wofdm_ber_run_masked_segments gives with that pair and variant + v, bit for bit -- the
+ * same segments, local indices, shard rule and device split.  A batch's symbols are drawn once and one tensor-core
+ * product covers all pairs; the resolved twin of the K1 kernel evaluates all pairs of a frame in one launch where its
+ * tables and accumulators fit, else one launch per pair on the same product output (the staged fallback of
+ * wofdm_ber_run_masked_resolved keeps its fp32 caveat).  wofdm_ber_run_masked_segments is this call with n_var = 1.
+ *   resolve = 0: bit_err / sym_err int64[n_var][n_snr], sym_tot int64[n_snr]; non-zero: bit_err / sym_err
+ *   int64[n_var][n_snr][Cr][Nr], sym_tot int64[n_snr][Cr][Nr] (the same for every pair).
+ * The resolved counters of several pairs over a whole job are this call with one segment {s, 0, ensemble} per point s.
+ * Errors: WOFDM_EINVAL for n_var outside [1, WOFDM_MAX_VARIANTS], a NULL roll_off, and what
+ * wofdm_ber_run_masked_segments rejects for any pair.  The handle stays usable after every error. */
+WOFDM_API int wofdm_ber_run_masked_segments_multi(wofdm_handle h, const wofdm_sys_t* sys,
+                         const double* win_tx /* n_var x n_tx */, const double* win_rx /* n_var x (N + tail_rx) */,
+                         const int* roll_off /* n_var */, int n_var,
+                         const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble_max,
+                         const int64_t* segments /* [n_seg][3] = {snr_idx, e_begin, e_count} */, int n_seg,
+                         uint64_t seed, uint32_t variant, int shard_index, int shard_count, int resolve,
+                         int64_t* bit_err /* [n_var][n_snr] or [n_var][n_snr][Cr][Nr] */, int64_t* sym_err,
+                         int64_t* sym_tot /* [n_snr] or [n_snr][Cr][Nr] */);
 /* run_sim_mc of matlab/main_channel_mask.m with the stopping rule of wofdm_ber_run_adaptive: the masked and the unmasked
  * chain on the same frames (one window pair, the same sys), every SNR point run until both have counted `target` errors
  * or ensemble_max ensemble indices.
@@ -352,6 +372,26 @@ WOFDM_API int wofdm_ber_run_masked_adaptive(wofdm_handle h, const wofdm_sys_t* s
                          int target_kind, int64_t target, uint64_t seed, uint32_t variant, int roll_off, int shard_index,
                          int shard_count, wofdm_reduce_fn reduce, void* reduce_user,
                          int64_t* ensemble_used, int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot, int* rounds);
+/* wofdm_ber_run_masked_adaptive for n_var window pairs / roll-offs on the same frames (1 <= n_var <= WOFDM_MAX_VARIANTS),
+ * pair v = (win_tx + v*n_tx, win_rx + v*(N+tail_rx), roll_off[v]).  2 n_var rows of counters, bit_err / sym_err
+ * int64[2][n_var][n_snr]:
+ *   block 0, row v: the masked chain of pair v (wofdm_ber_run_masked_segments_multi), noise stream variant + n_var + v;
+ *   block 1, row v: the unmasked chain of pair v (wofdm_ber_run_segments with n_var pairs), noise stream variant + v.
+ * These are the streams of ofdm_utils.run_sim_mc_multi; with n_var = 1 (masked variant + 1, unmasked variant) those of
+ * wofdm_ber_run_masked_adaptive, which is this call with n_var = 1.  The schedule is wofdm_ber_run_adaptive's over the
+ * 2 n_var rows: a point stops when every row has counted `target` errors, or at ensemble_max.  Sharding as in
+ * wofdm_ber_run_masked_adaptive; reduce receives int64[2][n_var][n_snr][2] = {bit, sym} (n = 4*n_var*n_snr).  Outputs:
+ * ensemble_used[n_snr], bit_tot / sym_tot int64[n_snr] (the same for every row), *rounds.  Errors: WOFDM_EINVAL for n_var
+ * outside [1, WOFDM_MAX_VARIANTS], a NULL roll_off, and what wofdm_ber_run_masked_adaptive rejects for any pair; the
+ * handle stays usable. */
+WOFDM_API int wofdm_ber_run_masked_adaptive_multi(wofdm_handle h, const wofdm_sys_t* sys,
+                         const double* win_tx /* n_var x n_tx */, const double* win_rx /* n_var x (N + tail_rx) */,
+                         const int* roll_off /* n_var */, int n_var,
+                         const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble_max,
+                         int64_t first_block, int target_kind, int64_t target, uint64_t seed, uint32_t variant,
+                         int shard_index, int shard_count, wofdm_reduce_fn reduce, void* reduce_user,
+                         int64_t* ensemble_used, int64_t* bit_err /* [2][n_var][n_snr] */, int64_t* bit_tot,
+                         int64_t* sym_err /* [2][n_var][n_snr] */, int64_t* sym_tot, int* rounds);
 
 /* ---- Window-optimisation Hessian (next-row 8f-2) -------------------------------------------------------------
  * The quadratic form of the interference power in the reduced window variables: OptimizerTx / OptimizerRx /
@@ -440,6 +480,17 @@ WOFDM_API int wofdm_psd_estimate(wofdm_handle h, int N, int cp, int cs, int tail
 WOFDM_API int wofdm_psd_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, int roll_off,
                        uint64_t seed, int64_t f0, int64_t n_frames, int estimator,
                        double* psd_masked /* 8N or NULL */, double* psd_unmasked /* 8N or NULL */);
+/* wofdm_psd_masked for n_var Tx windows / roll-offs on the same frames (1 <= n_var <= WOFDM_MAX_VARIANTS): spectrum v of
+ * psd_masked / psd_unmasked (row v of n_var x 8N) is wofdm_psd_masked's with win_tx + v*n_tx and roll_off[v], up to the
+ * order of fp64 additions.  Every requested spectrum is one pair of a single mask product (the unmasked ones with a unit
+ * impulse for the mask): a batch's symbols are drawn once, and one product and one PSD launch cover all spectra.  A NULL
+ * output skips that half for every configuration.  wofdm_psd_masked is this call with n_var = 1.  Errors: WOFDM_EINVAL
+ * for n_var outside [1, WOFDM_MAX_VARIANTS], a NULL roll_off, and what wofdm_psd_masked rejects for any roll_off[v]; the
+ * handle stays usable. */
+WOFDM_API int wofdm_psd_masked_multi(wofdm_handle h, const wofdm_sys_t* sys,
+                       const double* win_tx /* n_var x n_tx */, const int* roll_off /* n_var */, int n_var,
+                       uint64_t seed, int64_t f0, int64_t n_frames, int estimator,
+                       double* psd_masked /* n_var x 8N or NULL */, double* psd_unmasked /* n_var x 8N or NULL */);
 
 #ifdef __cplusplus
 }

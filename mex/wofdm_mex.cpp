@@ -20,6 +20,8 @@
 //   [berMasked, ber, ensembleUsed] = wofdm_mex('run_sim_mc_adaptive', ...)  run_sim_mc, each SNR point stopped at a bit-error target
 //   [berMasked, ber] = wofdm_mex('run_sim_mc_multi', ...)    run_sim_mc for several window pairs / roll-offs on the same symbols
 //   [psdMasked, psd] = wofdm_mex('psd_sim_mc', ...)         the Tx spectra of run_sim_mc's frames with and without the mask
+//   [berMasked, ber, ensembleUsed] = wofdm_mex('run_sim_mc_multi_adaptive', ...)  run_sim_mc_adaptive for several configurations
+//   [psdMasked, psd] = wofdm_mex('psd_sim_mc_multi', ...)   psd_sim_mc for several windows / roll-offs on the same frames
 //   H = wofdm_mex('window_hessian', ...)                     quad_objective_tx / _rx of matlab/window_optimization.m:596-680
 //   H = wofdm_mex('window_hessian_expected', ...), 'quad_objective_tx_expected', 'quad_objective_rx_expected'
 //       -- the same, averaged over a channel set (C x L, rows = realisations) instead of built from one impulse response
@@ -385,6 +387,56 @@ static void do_run_sim_mc_adaptive(int nlhs, mxArray* plhs[], int nrhs, const mx
     }
 }
 
+// [berMasked, ber, ensembleUsed] = wofdm_mex('run_sim_mc_multi_adaptive', <the 16 arguments of run_sim_mc_multi>,
+//                                            targetBitErrors, ensembleMax [, seed])
+//   -- run_sim_mc_adaptive for every configuration v = (windowTx{v}, windowRx{v}, rollOff(v)) on the same symbols in one
+//      call (wofdm_ber_run_masked_adaptive_multi): the noise streams of run_sim_mc_multi, every SNR point stopped once all
+//      2 n_var chains have counted targetBitErrors bit errors, or at ensembleMax.  The first argument is the first round's
+//      block.  berMasked and ber are n_snr x n_var, ensembleUsed n_snr x 1.
+static void do_run_sim_mc_multi_adaptive(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
+    if (nrhs < 18) mexErrMsgIdAndTxt("wofdm:nargin", "run_sim_mc_multi_adaptive needs 18 arguments");
+    wofdm_sys_t s;
+    memset(&s, 0, sizeof(s));
+    const long long first_block = (long long)mxGetScalar(prhs[0]);
+    s.cp = (int)mxGetScalar(prhs[1]); s.cs = (int)mxGetScalar(prhs[2]);
+    s.tail_tx = (int)mxGetScalar(prhs[3]); s.tail_rx = (int)mxGetScalar(prhs[4]);
+    s.guard = (int)mxGetScalar(prhs[9]); s.rm = (int)mxGetScalar(prhs[10]); s.shift = (int)mxGetScalar(prhs[11]);
+    s.N = (int)mxGetScalar(prhs[12]); s.bits = (int)mxGetScalar(prhs[13]); s.S = (int)mxGetScalar(prhs[14]);
+    s.noise_norm = 1; s.constellation = 1; s.precision = 0;
+    size_t nvt = 0, nvr = 0;
+    const std::vector<double> wtx = windows_of(prhs[5], (size_t)(s.N + s.cp + s.cs), &nvt);
+    const std::vector<double> wrx = windows_of(prhs[6], (size_t)(s.N + s.tail_rx), &nvr);
+    const size_t n_var = mxGetNumberOfElements(prhs[15]);
+    if (nvt != n_var || nvr != n_var || n_var < 1 || n_var > WOFDM_MAX_VARIANTS)
+        mexErrMsgIdAndTxt("wofdm:size", "windowTx, windowRx (cell arrays) and rollOff must all hold n_var <= %d entries", WOFDM_MAX_VARIANTS);
+    std::vector<int> roll_off(n_var);
+    for (size_t v = 0; v < n_var; ++v) roll_off[v] = (int)mxGetPr(prhs[15])[v];
+    int L = 0, C = 0;
+    const std::vector<double> chan = channel_rows(prhs[7], &L, &C);
+    const size_t n_snr = mxGetNumberOfElements(prhs[8]);
+    const long long target = (long long)mxGetScalar(prhs[16]), ensemble_max = (long long)mxGetScalar(prhs[17]);
+    const unsigned long long seed = nrhs > 18 ? (unsigned long long)mxGetScalar(prhs[18]) : 0ull;
+    std::vector<long long> be(2 * n_var * n_snr), se(2 * n_var * n_snr), bt(n_snr), st(n_snr), used(n_snr);
+    int rounds = 0;
+    check(wofdm_ber_run_masked_adaptive_multi(handle(), &s, wtx.data(), wrx.data(), roll_off.data(), (int)n_var, chan.data(), L,
+                                              C, mxGetPr(prhs[8]), (int)n_snr, ensemble_max, first_block,
+                                              WOFDM_TARGET_BIT_ERRORS, target, seed, 0, 0, 1, nullptr, nullptr,
+                                              (int64_t*)used.data(), (int64_t*)be.data(), (int64_t*)bt.data(),
+                                              (int64_t*)se.data(), (int64_t*)st.data(), &rounds),
+          "wofdm_ber_run_masked_adaptive_multi");
+    for (int row = 0; row < 3 && row < (nlhs > 0 ? nlhs : 1); ++row) {       // berMasked (block 0), ber (block 1), ensembleUsed
+        plhs[row] = mxCreateDoubleMatrix((mwSize)n_snr, row == 2 ? 1 : (mwSize)n_var, mxREAL);
+        double* out = mxGetPr(plhs[row]);
+        if (row == 2) {
+            for (size_t i = 0; i < n_snr; ++i) out[i] = (double)used[i];
+            continue;
+        }
+        for (size_t v = 0; v < n_var; ++v)
+            for (size_t i = 0; i < n_snr; ++i)
+                out[v * n_snr + i] = bt[i] ? (double)be[(row * n_var + v) * n_snr + i] / (double)bt[i] : 0.0;
+    }
+}
+
 // H = wofdm_mex('window_hessian', typeOFDM, numSubcar, cpLength, tailTx, tailRx, channel)
 //   -- the quadratic form of the interference power (ICI + ISI) in the REDUCED window variables (tail coefficients), as
 //      python's OptimizerTx/Rx/TxRx.gen_hessian builds it.  channel: ONE impulse response.  (quad_objective_tx / _rx of
@@ -552,10 +604,53 @@ static void do_psd_sim_mc(int nlhs, mxArray* plhs[], int nrhs, const mxArray* pr
     }
 }
 
+// [psdMasked, psd] = wofdm_mex('psd_sim_mc_multi', <the arguments of psd_sim_mc>) with windowTx a CELL ARRAY of n_var
+// windows and rollOff a vector of n_var (or one value for every window)
+//   -- psd_sim_mc for every configuration v = (windowTx{v}, rollOff(v)) on the same frames in one call
+//      (wofdm_psd_masked_multi: the symbols drawn once, one mask product for all spectra).  Each output is 8N x n_var.
+static void do_psd_sim_mc_multi(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
+    if (nrhs < 10) mexErrMsgIdAndTxt("wofdm:nargin", "psd_sim_mc_multi needs 10 arguments");
+    wofdm_sys_t s;
+    memset(&s, 0, sizeof(s));
+    const long long n_frames = (long long)mxGetScalar(prhs[0]);
+    s.cp = (int)mxGetScalar(prhs[1]); s.cs = (int)mxGetScalar(prhs[2]); s.tail_tx = (int)mxGetScalar(prhs[3]);
+    s.guard = (int)mxGetScalar(prhs[5]); s.N = (int)mxGetScalar(prhs[6]); s.bits = (int)mxGetScalar(prhs[7]);
+    s.S = (int)mxGetScalar(prhs[8]);
+    s.noise_norm = 1; s.constellation = 1; s.precision = 0;
+    size_t n_var = 0;
+    const std::vector<double> wtx = windows_of(prhs[4], (size_t)(s.N + s.cp + s.cs), &n_var);
+    const size_t n_ro = mxGetNumberOfElements(prhs[9]);
+    if (n_var < 1 || n_var > WOFDM_MAX_VARIANTS || (n_ro != n_var && n_ro != 1))
+        mexErrMsgIdAndTxt("wofdm:size", "windowTx (a cell array) must hold n_var <= %d windows and rollOff n_var values or one", WOFDM_MAX_VARIANTS);
+    std::vector<int> roll_off(n_var);
+    for (size_t v = 0; v < n_var; ++v) roll_off[v] = (int)mxGetPr(prhs[9])[n_ro == 1 ? 0 : v];
+    const unsigned long long seed = nrhs > 10 ? (unsigned long long)mxGetScalar(prhs[10]) : 0ull;
+    int estimator = 0;
+    if (nrhs > 11) {
+        char est[16];
+        if (mxIsChar(prhs[11])) {
+            if (mxGetString(prhs[11], est, sizeof(est))) mexErrMsgIdAndTxt("wofdm:usage", "estimator: 'reference' or 'hann'");
+            if (!strcmp(est, "hann")) estimator = 1;
+            else if (strcmp(est, "reference")) mexErrMsgIdAndTxt("wofdm:usage", "estimator: 'reference' or 'hann'");
+        } else {
+            estimator = (int)mxGetScalar(prhs[11]);
+        }
+    }
+    const size_t P = 8 * (size_t)(s.N > 0 ? s.N : 0);
+    std::vector<double> xm(P * n_var), xu(P * n_var);
+    check(wofdm_psd_masked_multi(handle(), &s, wtx.data(), roll_off.data(), (int)n_var, seed, 0, n_frames, estimator, xm.data(),
+                                 xu.data()),
+          "wofdm_psd_masked_multi");
+    for (int k = 0; k < 2 && k < (nlhs > 0 ? nlhs : 1); ++k) {       // column v = configuration v (row v of the library's output)
+        plhs[k] = mxCreateDoubleMatrix((mwSize)P, (mwSize)n_var, mxREAL);
+        memcpy(mxGetPr(plhs[k]), (k == 0 ? xm : xu).data(), P * n_var * sizeof(double));
+    }
+}
+
 extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     char cmd[32];
     if (nrhs < 1 || !mxIsChar(prhs[0]) || mxGetString(prhs[0], cmd, sizeof(cmd)))
-        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_simulation_adaptive', 'run_sim_mc', 'run_sim_mc_per_subcarrier', 'run_sim_mc_adaptive', 'run_sim_mc_multi', 'psd_sim_mc', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
+        mexErrMsgIdAndTxt("wofdm:usage", "first argument: 'run_simulation', 'run_simulation_sweep', 'run_simulation_sweep_multi', 'run_simulation_per_subcarrier', 'run_simulation_adaptive', 'run_sim_mc', 'run_sim_mc_per_subcarrier', 'run_sim_mc_adaptive', 'run_sim_mc_multi', 'run_sim_mc_multi_adaptive', 'psd_sim_mc', 'psd_sim_mc_multi', 'calculate_interference', 'window_hessian', 'quad_objective_tx', 'quad_objective_rx', 'window_hessian_expected', 'quad_objective_tx_expected', 'quad_objective_rx_expected' or 'gen_channels'");
     if (!strcmp(cmd, "run_simulation")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "run_simulation_sweep")) do_run_simulation(nlhs, plhs, nrhs - 1, prhs + 1, true);
     else if (!strcmp(cmd, "run_simulation_sweep_multi")) do_run_simulation_multi(nlhs, plhs, nrhs - 1, prhs + 1, false);
@@ -566,6 +661,8 @@ extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* 
     else if (!strcmp(cmd, "run_sim_mc_adaptive")) do_run_sim_mc_adaptive(nlhs, plhs, nrhs - 1, prhs + 1);
     else if (!strcmp(cmd, "run_sim_mc_multi")) do_run_sim_mc_multi(nlhs, plhs, nrhs - 1, prhs + 1);
     else if (!strcmp(cmd, "psd_sim_mc")) do_psd_sim_mc(nlhs, plhs, nrhs - 1, prhs + 1);
+    else if (!strcmp(cmd, "run_sim_mc_multi_adaptive")) do_run_sim_mc_multi_adaptive(nlhs, plhs, nrhs - 1, prhs + 1);
+    else if (!strcmp(cmd, "psd_sim_mc_multi")) do_psd_sim_mc_multi(nlhs, plhs, nrhs - 1, prhs + 1);
     else if (!strcmp(cmd, "window_hessian")) do_window_hessian(nlhs, plhs, nrhs - 1, prhs + 1, false);
     else if (!strcmp(cmd, "quad_objective_tx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, true, false);
     else if (!strcmp(cmd, "quad_objective_rx")) do_quad_objective(nlhs, plhs, nrhs - 1, prhs + 1, false, false);

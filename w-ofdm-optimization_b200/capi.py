@@ -120,6 +120,13 @@ SIGNATURES = {
     "wofdm_ber_run_masked_adaptive": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_int64,
                                                 C.c_int64, C.c_int, C.c_int64, C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_int,
                                                 REDUCE_FN, C.c_void_p, _i64p, _i64p, _i64p, _i64p, _i64p, _P(C.c_int)]),
+    "wofdm_ber_run_masked_segments_multi": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _P(C.c_int), C.c_int, _dp, C.c_int,
+                                                      C.c_int, _dp, C.c_int, C.c_int64, _i64p, C.c_int, C.c_uint64, C.c_uint32,
+                                                      C.c_int, C.c_int, C.c_int, _i64p, _i64p, _i64p]),
+    "wofdm_ber_run_masked_adaptive_multi": (C.c_int, [C.c_void_p, _P(SysT), _dp, _dp, _P(C.c_int), C.c_int, _dp, C.c_int,
+                                                      C.c_int, _dp, C.c_int, C.c_int64, C.c_int64, C.c_int, C.c_int64,
+                                                      C.c_uint64, C.c_uint32, C.c_int, C.c_int, REDUCE_FN, C.c_void_p, _i64p,
+                                                      _i64p, _i64p, _i64p, _i64p, _P(C.c_int)]),
     "wofdm_window_hessian": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, _dp, _P(C.c_int)]),
     "wofdm_window_hessian_parts": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, _dp, C.c_int, _dp, C.c_int, _dp, _dp]),
     "wofdm_window_hessian_set": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, C.c_int, _dp, _P(C.c_int)]),
@@ -132,6 +139,8 @@ SIGNATURES = {
     "wofdm_psd_estimate": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _dp, C.c_int, C.c_int,
                                      C.c_int64, C.c_uint64, _i32p, _dp]),
     "wofdm_psd_masked": (C.c_int, [C.c_void_p, _P(SysT), _dp, C.c_int, C.c_uint64, C.c_int64, C.c_int64, C.c_int, _dp, _dp]),
+    "wofdm_psd_masked_multi": (C.c_int, [C.c_void_p, _P(SysT), _dp, _P(C.c_int), C.c_int, C.c_uint64, C.c_int64, C.c_int64,
+                                         C.c_int, _dp, _dp]),
 }
 
 _lib = None
@@ -460,6 +469,60 @@ class Handle:
         self._check(rc, cb)
         return dict(bit_err=be, bit_tot=bt, sym_err=se, sym_tot=st, ensemble_used=used, rounds=rounds.value)
 
+    def ber_run_masked_segments_multi(self, s, wins_tx, wins_rx, chan, snr_db, ensemble_max, segments, seed=0, variant=0,
+                                      roll_offs=10, shard=(0, 1), by_subcarrier=False, by_channel=False):
+        """ber_run_masked_segments for n_var window pairs on the same frames (wofdm_ber_run_masked_segments_multi): pair v =
+        ber_run_masked_segments(..., variant=variant + v, roll_off=roll_offs[v]) with its windows, bit for bit.  roll_offs:
+        one value for every pair, or n_var values.  Unresolved: bit_err / sym_err (n_var, n_snr), sym_tot / bit_tot
+        (n_snr,); resolved: bit_err / sym_err (n_var, n_snr, Cr, Nr), sym_tot / bit_tot (n_snr, Cr, Nr).  One segment
+        (s, 0, E) per point gives the resolved counters of several pairs over a whole job of E ensemble indices."""
+        wt, wr = self._win_multi(s, wins_tx, wins_rx)
+        _, _, chf, L, Cn = self._win_chan(s, wt[0], wr[0], chan)
+        nv = wt.shape[0]
+        ro = _roll_offs(roll_offs, nv)
+        snr = _f64(np.ravel(snr_db))
+        n = snr.size
+        seg = np.ascontiguousarray(np.asarray(segments, dtype=np.int64).reshape(-1, 3))
+        resolve, shape = _resolve(s, n, Cn, by_subcarrier, by_channel)
+        be, se = np.zeros((nv,) + shape, dtype=np.int64), np.zeros((nv,) + shape, dtype=np.int64)
+        st = np.zeros(shape, dtype=np.int64)
+        rc = load().wofdm_ber_run_masked_segments_multi(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), _ptr(ro, _P(C.c_int)),
+                                                        nv, _ptr(chf, _dp), L, Cn, _ptr(snr, _dp), n, int(ensemble_max),
+                                                        _ptr(seg, _i64p), seg.shape[0], int(seed), int(variant), int(shard[0]),
+                                                        int(shard[1]), int(resolve), _ptr(be, _i64p), _ptr(se, _i64p),
+                                                        _ptr(st, _i64p))
+        self._check(rc)
+        return dict(bit_err=be, sym_err=se, sym_tot=st, bit_tot=st * int(s.bits))
+
+    def ber_run_masked_adaptive_multi(self, s, wins_tx, wins_rx, chan, snr_db, ensemble_max, target_bit_errors=None,
+                                      target_symbol_errors=None, first_block=1, seed=0, variant=0, roll_offs=10, shard=(0, 1),
+                                      reduce=None):
+        """ber_run_masked_adaptive for n_var window pairs / roll-offs on the same frames
+        (wofdm_ber_run_masked_adaptive_multi): bit_err / sym_err (2, n_var, n_snr), block 0 the masked chain of pair v
+        (noise stream variant + n_var + v), block 1 its unmasked chain (variant + v); a point stops when all 2 n_var rows
+        reach the target or at ensemble_max.  roll_offs: one value for every pair, or n_var values.  reduce: as in
+        ber_run_adaptive, on int64 counts of shape (2, n_var, n_snr, 2).  Returns also bit_tot / sym_tot (n_snr,),
+        ensemble_used (n_snr,) and rounds."""
+        kind, target = _target(target_bit_errors, target_symbol_errors)
+        wt, wr = self._win_multi(s, wins_tx, wins_rx)
+        _, _, chf, L, Cn = self._win_chan(s, wt[0], wr[0], chan)
+        nv = wt.shape[0]
+        ro = _roll_offs(roll_offs, nv)
+        snr = _f64(np.ravel(snr_db))
+        n = snr.size
+        be, se = np.zeros((2, nv, n), dtype=np.int64), np.zeros((2, nv, n), dtype=np.int64)
+        bt, st, used = (np.zeros(n, dtype=np.int64) for _ in range(3))
+        rounds = C.c_int(0)
+        cb = reduce_trampoline(reduce, (2, nv, n, 2)) if reduce is not None else REDUCE_FN()
+        rc = load().wofdm_ber_run_masked_adaptive_multi(self._h, C.byref(s), _ptr(wt, _dp), _ptr(wr, _dp), _ptr(ro, _P(C.c_int)),
+                                                        nv, _ptr(chf, _dp), L, Cn, _ptr(snr, _dp), n, int(ensemble_max),
+                                                        int(first_block), kind, int(target), int(seed), int(variant),
+                                                        int(shard[0]), int(shard[1]), cb, None, _ptr(used, _i64p),
+                                                        _ptr(be, _i64p), _ptr(bt, _i64p), _ptr(se, _i64p), _ptr(st, _i64p),
+                                                        C.byref(rounds))
+        self._check(rc, cb)
+        return dict(bit_err=be, bit_tot=bt, sym_err=se, sym_tot=st, ensemble_used=used, rounds=rounds.value)
+
     def psd_estimate(self, N, cp, cs, tail_tx, win_tx, guard_band=48, n_sym=256, records=1, seed=0, sym_idx=None,
                      bits=4, constellation=0):
         """X_est of timefreq_simulation.py:104-123 for the Tx signal of window win_tx (8N doubles, fftshifted), averaged
@@ -492,6 +555,28 @@ class Handle:
         ou = np.empty(8 * s.N, dtype=np.float64) if unmasked else None
         rc = load().wofdm_psd_masked(self._h, C.byref(s), _ptr(w, _dp), int(roll_off), int(seed), int(f0), int(frames), est,
                                      _ptr(om, _dp) if om is not None else None, _ptr(ou, _dp) if ou is not None else None)
+        self._check(rc)
+        return om, ou
+
+    def psd_masked_multi(self, s, wins_tx, roll_offs=10, frames=1, f0=0, seed=0, estimator="reference", masked=True,
+                         unmasked=True):
+        """psd_masked for n_var Tx windows / roll-offs on the same frames (wofdm_psd_masked_multi): row v = psd_masked with
+        window v and roll_offs[v], up to the order of fp64 additions; one symbol draw, one mask product and one PSD launch per
+        batch for every spectrum.  roll_offs: one value for every window, or n_var values.  Returns (masked, unmasked), each
+        (n_var, 8N) doubles (fftshifted) or None where not asked for."""
+        w = _f64(np.atleast_2d(np.asarray(wins_tx, dtype=np.float64)))
+        if w.ndim != 2 or w.shape[1] != s.n_tx:
+            raise WofdmError(EINVAL, f"psd_masked_multi: windows must be (n_var, n_tx={s.n_tx})")
+        nv = w.shape[0]
+        ro = _roll_offs(roll_offs, nv)
+        est = {"reference": 0, "hann": 1}.get(estimator)
+        if est is None:
+            raise WofdmError(EINVAL, f"psd_masked_multi: estimator must be 'reference' or 'hann', not {estimator!r}")
+        om = np.empty((nv, 8 * s.N), dtype=np.float64) if masked else None
+        ou = np.empty((nv, 8 * s.N), dtype=np.float64) if unmasked else None
+        rc = load().wofdm_psd_masked_multi(self._h, C.byref(s), _ptr(w, _dp), _ptr(ro, _P(C.c_int)), nv, int(seed), int(f0),
+                                           int(frames), est, _ptr(om, _dp) if om is not None else None,
+                                           _ptr(ou, _dp) if ou is not None else None)
         self._check(rc)
         return om, ou
 

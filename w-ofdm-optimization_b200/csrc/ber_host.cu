@@ -454,6 +454,21 @@ int check_masked(wofdm_ctx* h, const wofdm_sys_t* sys, const double* win_tx, con
     return rc ? rc : check_counters(h, *sys, C, n_snr, 1, resolve);
 }
 
+// check_masked for n_var window pairs with roll-offs roll_off[n_var] (the pairs differ only in what check_masked reads of
+// roll_off), and their counters [n_var][n_snr][Cr][Nr]
+int check_masked_multi(wofdm_ctx* h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, const double* chan,
+                       int L, int C, const double* snr_db, int n_snr, int64_t ensemble, const int* roll_off, int n_var,
+                       int shard_index, int shard_count, int resolve, bool outputs_ok) {
+    if (n_var < 1 || n_var > WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "n_var must be in [1, WOFDM_MAX_VARIANTS]");
+    if (!roll_off) return fail(h, WOFDM_EINVAL, "NULL roll_off");
+    for (int v = 0; v < n_var; ++v) {
+        const int rc = check_masked(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, roll_off[v], shard_index,
+                                    shard_count, resolve, outputs_ok);
+        if (rc) return rc;
+    }
+    return check_counters(h, *sys, C, n_snr, n_var, resolve);
+}
+
 // segments[n_seg][3] of a job: inside [0, n_snr) x [0, ensemble_max), e_count >= 1, no two segments of one point overlap
 int check_segments(wofdm_ctx* h, const int64_t* segments, int n_seg, int n_snr, int64_t ensemble_max) {
     if (!segments || n_seg < 1) return fail(h, WOFDM_EINVAL, "segments must be a non-empty list");
@@ -1200,7 +1215,7 @@ struct MaskedJob {
 // Set-up of a checked channel-mask call of n_var window pairs (win_tx / win_rx back to back, roll_off[n_var]; pair v's
 // noise stream is variant + v): the kernels, the tables, and on every device that takes part (contiguous ranges of at least
 // 64 frames out of max_frames, the most frames one masked_run covers) its buffers and the mask product's matrices.
-// resolve != 0 or seg_cap > 0 (n_var = 1 only): the resolved twin of the K1 kernel (counters [n_snr][Cr][Nr], [n_snr] with
+// resolve != 0 or seg_cap > 0: the resolved twin of the K1 kernel (counters [n_var][n_snr][Cr][Nr], [n_var][n_snr] with
 // resolve 0); seg_cap > 0 also gives every device a segment table of seg_cap entries.
 int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
                  const int* roll_off, const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
@@ -1243,23 +1258,24 @@ int masked_setup(MaskedJob& J, wofdm_handle h, const wofdm_sys_t* sys, const dou
         if (rc) return rc;
         if (prod[v].var->CL > 1) return fail(h, WOFDM_EUNSUPPORTED, "no channel-mask variant for cluster kernels");
     }
-    // several pairs: one launch of the gathering kernel for all of them where it holds all their tables (the same kernel
-    // as for one pair, so the same counters); else one launch per pair
-    int nv_launch = 1;
-    if (J.fused && n_var > 1) {
-        const BerSmem lay = ch.var->layout(sys->S, stride, sys->tail_tx, sys->tail_rx, L, n_var, 0);
-        if (lay.bytes <= d0.smem_optin) { nv_launch = n_var; ch.lay = lay; }
-    }
     // the kernel that runs: ch, or (resolved counters, segments) its twin -- the noise numbering below stays ch's either way,
-    // so a staged fallback draws ch's noise; it reads the assembled stream even where ch gathers from the product itself
+    // so a staged fallback draws ch's noise; it reads the assembled stream even where ch gathers from the product itself.
+    // Several pairs: one launch of the gathering kernel (or of its twin) for all of them where it holds all their tables
+    // and accumulators (the same kernel as for one pair, so the same counters); else one launch per pair on the shared
+    // product output.
+    int nv_launch = 1;
     J.run = ch;
     if (resolve || seg_cap > 0) {
         Choice nz = ch;
         if (ch.var->TC == 0) nz.chunk = prod[0].chunk;
         bool rfused = false;
-        rc = choose_resolved(h, *sys, L, d0.smem_optin, nz, false, 1, &J.run, &rfused);
+        rc = choose_resolved(h, *sys, L, d0.smem_optin, nz, J.fused, n_var, &J.run, &rfused);
         if (rc) return rc;
         J.fused = J.run.var->txy;
+        if (rfused) nv_launch = n_var;
+    } else if (J.fused && n_var > 1) {
+        const BerSmem lay = ch.var->layout(sys->S, stride, sys->tail_tx, sys->tail_rx, L, n_var, 0);
+        if (lay.bytes <= d0.smem_optin) { nv_launch = n_var; J.run.lay = lay; }
     }
     const Choice& run = J.run;
     int nb = 0;
@@ -1516,8 +1532,8 @@ int masked_run(MaskedJob& J, long long g_lo, long long g_hi, const Segments* seg
 
 // A checked job of the channel-mask chain for n_var window pairs: the whole job (segs == nullptr: global frame ids, the
 // unsegmented kernels) or the frames of a segment list, in either case this shard's contiguous block of the local indices.
-// resolve == 0: bit_err / sym_err [n_var][n_snr]; else [n_snr][Cr][Nr] (wofdm_ber_run_resolved's layout, one window pair),
-// counted by the resolved twin of the K1 kernel this chain picks.  Totals as in run_job; bit_tot may be NULL.
+// resolve == 0: bit_err / sym_err [n_var][n_snr]; else [n_var][n_snr][Cr][Nr] (wofdm_ber_run_resolved's layout), counted by
+// the resolved twin of the K1 kernel this chain picks.  Totals as in run_job; bit_tot may be NULL.
 int run_masked_impl(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx, int n_var,
                     const int* roll_off, const double* chan, int L, int C, const double* snr_db, int n_snr, int64_t ensemble,
                     const Segments* segs, uint64_t seed, uint32_t variant, int shard_index, int shard_count, int resolve,
@@ -1565,13 +1581,9 @@ int wofdm_ber_run_masked_multi(wofdm_handle h, const wofdm_sys_t* sys, const dou
                                int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot) {
     NvtxRange nvtx_("wofdm_ber_run_masked_multi");
     if (!h) return WOFDM_EINVAL;
-    if (n_var < 1 || n_var > WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "n_var must be in [1, WOFDM_MAX_VARIANTS]");
-    if (!roll_off) return fail(h, WOFDM_EINVAL, "NULL roll_off");
-    for (int v = 0; v < n_var; ++v) {         // (the pairs differ only in what check_masked reads of roll_off)
-        const int rc = check_masked(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, roll_off[v], shard_index,
-                                    shard_count, 0, bit_err && bit_tot && sym_err && sym_tot);
-        if (rc) return rc;
-    }
+    const int rc = check_masked_multi(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble, roll_off, n_var, shard_index,
+                                      shard_count, 0, bit_err && bit_tot && sym_err && sym_tot);
+    if (rc) return rc;
     return run_masked_impl(h, sys, win_tx, win_rx, n_var, roll_off, chan, L, C, snr_db, n_snr, ensemble, nullptr, seed, variant,
                            shard_index, shard_count, 0, bit_err, sym_err, sym_tot, bit_tot);
 }
@@ -1596,15 +1608,25 @@ int wofdm_ber_run_masked_segments(wofdm_handle h, const wofdm_sys_t* sys, const 
                                   const int64_t* segments, int n_seg, uint64_t seed, uint32_t variant, int roll_off,
                                   int shard_index, int shard_count, int resolve, int64_t* bit_err, int64_t* sym_err,
                                   int64_t* sym_tot) {
+    return wofdm_ber_run_masked_segments_multi(h, sys, win_tx, win_rx, &roll_off, 1, chan, L, C, snr_db, n_snr, ensemble_max,
+                                               segments, n_seg, seed, variant, shard_index, shard_count, resolve, bit_err,
+                                               sym_err, sym_tot);
+}
+
+int wofdm_ber_run_masked_segments_multi(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                                        const int* roll_off, int n_var, const double* chan, int L, int C, const double* snr_db,
+                                        int n_snr, int64_t ensemble_max, const int64_t* segments, int n_seg, uint64_t seed,
+                                        uint32_t variant, int shard_index, int shard_count, int resolve, int64_t* bit_err,
+                                        int64_t* sym_err, int64_t* sym_tot) {
     NvtxRange nvtx_("wofdm_ber_run_masked_segments");
     if (!h) return WOFDM_EINVAL;
     int rc = check_resolve(h, resolve, false);
-    if (!rc) rc = check_masked(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, roll_off, shard_index, shard_count,
-                               resolve, bit_err && sym_err && sym_tot);
+    if (!rc) rc = check_masked_multi(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, roll_off, n_var, shard_index,
+                                     shard_count, resolve, bit_err && sym_err && sym_tot);
     if (!rc) rc = check_segments(h, segments, n_seg, n_snr, ensemble_max);
     if (rc) return rc;
     const Segments sg = seg_table(segments, n_seg, C);
-    return run_masked_impl(h, sys, win_tx, win_rx, 1, &roll_off, chan, L, C, snr_db, n_snr, ensemble_max, &sg, seed, variant,
+    return run_masked_impl(h, sys, win_tx, win_rx, n_var, roll_off, chan, L, C, snr_db, n_snr, ensemble_max, &sg, seed, variant,
                            shard_index, shard_count, resolve, bit_err, sym_err, sym_tot, nullptr);
 }
 
@@ -1614,31 +1636,43 @@ int wofdm_ber_run_masked_adaptive(wofdm_handle h, const wofdm_sys_t* sys, const 
                                   int roll_off, int shard_index, int shard_count, wofdm_reduce_fn reduce, void* reduce_user,
                                   int64_t* ensemble_used, int64_t* bit_err, int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot,
                                   int* rounds) {
+    return wofdm_ber_run_masked_adaptive_multi(h, sys, win_tx, win_rx, &roll_off, 1, chan, L, C, snr_db, n_snr, ensemble_max,
+                                               first_block, target_kind, target, seed, variant, shard_index, shard_count, reduce,
+                                               reduce_user, ensemble_used, bit_err, bit_tot, sym_err, sym_tot, rounds);
+}
+
+int wofdm_ber_run_masked_adaptive_multi(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const double* win_rx,
+                                        const int* roll_off, int n_var, const double* chan, int L, int C, const double* snr_db,
+                                        int n_snr, int64_t ensemble_max, int64_t first_block, int target_kind, int64_t target,
+                                        uint64_t seed, uint32_t variant, int shard_index, int shard_count,
+                                        wofdm_reduce_fn reduce, void* reduce_user, int64_t* ensemble_used, int64_t* bit_err,
+                                        int64_t* bit_tot, int64_t* sym_err, int64_t* sym_tot, int* rounds) {
     NvtxRange nvtx_("wofdm_ber_run_masked_adaptive");
     if (!h) return WOFDM_EINVAL;
     const bool outputs_ok = ensemble_used && bit_err && bit_tot && sym_err && sym_tot && rounds;
-    int rc = check_masked(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, roll_off, shard_index, shard_count, 0,
-                          outputs_ok);
+    int rc = check_masked_multi(h, sys, win_tx, win_rx, chan, L, C, snr_db, n_snr, ensemble_max, roll_off, n_var, shard_index,
+                                shard_count, 0, outputs_ok);
     if (!rc) rc = check_target(h, target_kind, target, first_block, shard_count, reduce);
     if (rc) return rc;
     if (variant > 0xfffffff0u - WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "variant too large");
-    // row 0: the masked chain (noise stream variant + 1), set up once for the largest round of this shard; row 1: the
-    // unmasked chain, a plan of its own device buffers (the masked chain's live in the arena).  Each row shards by its
-    // chain's rule.
+    // rows [0, n_var): the masked chain, pair v on noise stream variant + n_var + v, set up once for the largest round of
+    // this shard; rows [n_var, 2 n_var): the unmasked chain, pair v on variant + v, a plan of its own device buffers (the
+    // masked chain's live in the arena).  Each chain shards by its own rule.
     const long long total = (long long)n_snr * C * ensemble_max;
+    const size_t half = (size_t)n_var * n_snr;
     MaskedJob J;
-    rc = masked_setup(J, h, sys, win_tx, win_rx, 1, &roll_off, chan, L, C, snr_db, n_snr, ensemble_max, seed, variant + 1, 0,
-                      (long long)(((__int128)total + shard_count - 1) / shard_count), n_snr);
+    rc = masked_setup(J, h, sys, win_tx, win_rx, n_var, roll_off, chan, L, C, snr_db, n_snr, ensemble_max, seed,
+                      variant + (uint32_t)n_var, 0, (long long)(((__int128)total + shard_count - 1) / shard_count), n_snr);
     if (rc) return rc;
     wofdm_ber_plan p = nullptr;
-    rc = plan_create_impl(h, sys, win_tx, win_rx, 1, chan, L, C, snr_db, n_snr, &p, false, 0, n_snr);
+    rc = plan_create_impl(h, sys, win_tx, win_rx, n_var, chan, L, C, snr_db, n_snr, &p, false, 0, n_snr);
     if (rc) return rc;
-    rc = run_adaptive(h, *sys, C, n_snr, 2, ensemble_max, first_block, target_kind, target, reduce, reduce_user,
+    rc = run_adaptive(h, *sys, C, n_snr, 2 * n_var, ensemble_max, first_block, target_kind, target, reduce, reduce_user,
                       [&](const Segments& sg, int64_t* be, int64_t* se) {
                           const ShardRule r = ShardRule::block(sg.n_local, shard_index, shard_count);
                           const int rc_m = masked_run(J, r.lo, r.hi, &sg, be, se);
                           if (rc_m) return rc_m;
-                          return run_plan(p, ensemble_max, seed, variant, shard_index, shard_count, &sg, be + n_snr, se + n_snr);
+                          return run_plan(p, ensemble_max, seed, variant, shard_index, shard_count, &sg, be + half, se + half);
                       },
                       ensemble_used, bit_err, bit_tot, sym_err, sym_tot, rounds);
     wofdm_ber_plan_destroy(p);

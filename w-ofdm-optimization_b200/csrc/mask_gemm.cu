@@ -385,7 +385,7 @@ size_t mask_gemm_plan(const wofdm_sys_t& sys, long long batch, int nvar, MaskGem
            (size_t)mg.M * mg.nact * 16 + (size_t)nvar * 32 + 4096;
 }
 
-int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, const int* roll_off, const float* d_wtx, bool unit_impulse) {
+int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, const int* roll_off, const float* d_wtx) {
     const size_t cols = (size_t)((mg.batch * mg.S + TN - 1) / TN) * TN;
     const size_t at_b = (size_t)mg.RT * mg.nk * 2 * A_BYTES, bt_b = cols * mg.Kp * 2, y_b = cols * mg.Yp * 4;
     mg.At = static_cast<__half*>(arena_take(d, mg.nvar * at_b));
@@ -400,6 +400,7 @@ int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, const int* roll_of
     WOFDM_CUDA(h, cudaMemsetAsync(mg.Bt, 0, bt_b, d.stream));      // K padding and the columns behind the batch stay zero
     // pair by pair on one g / Mm (the stream orders them)
     for (int v = 0; v < mg.nvar; ++v) {
+        const bool unit_impulse = roll_off[v] == 0;
         if (unit_impulse) {
             const double2 one = make_double2(1.0, 0.0);       // (pageable source: the copy returns once it is staged)
             WOFDM_CUDA(h, cudaMemsetAsync(mg.g, 0, (size_t)mg.M * 16, d.stream));

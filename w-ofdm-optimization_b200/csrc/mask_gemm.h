@@ -29,10 +29,10 @@ struct MaskGemm {
 // dimensions for `sys`, `batch` frames and nvar window pairs; returns the device bytes mask_gemm_setup takes from the arena
 size_t mask_gemm_plan(const wofdm_sys_t& sys, long long batch, int nvar, MaskGemm& mg);
 // arena buffers + the matrices: pair v's mask of roll_off[v] bins (main_channel_mask.m:404-412, 477-493) on its Tx table
-// d_wtx + v n_tx (K1's tables, back to back).  unit_impulse: g = delta instead of the mask (roll_off unused), so Mtop = the
-// windowed, CP-extended IDFT columns and Mbot = 0 -- the UNMASKED symbols through the same product (wofdm_psd_masked's
-// second spectrum)
-int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, const int* roll_off, const float* d_wtx, bool unit_impulse = false);
+// d_wtx + v n_tx (K1's tables, back to back).  roll_off[v] == 0: g = delta instead of the mask, so Mtop = the windowed,
+// CP-extended IDFT columns and Mbot = 0 -- the UNMASKED symbols through the same product (wofdm_psd_masked's unmasked
+// spectra; the BER chain's roll-offs are all >= 1)
+int mask_gemm_setup(wofdm_ctx* h, DeviceCtx& d, MaskGemm& mg, const int* roll_off, const float* d_wtx);
 // masked symbols of frames f0 .. f0 + nf - 1 (nf <= batch) of every pair into Y: the symbols are drawn once, one product
 // covers all pairs.  seg (a device segment table [n_seg][4], BerParams::seg): f0 .. f0 + nf - 1 are local indices of the
 // segment list of a job with C channels and `ensemble` ensemble indices per point

@@ -5,10 +5,12 @@
 // stride (the rule of mask_assemble_kernel and of the K1 loader tconv2_load_masked):
 //     stream[s stride + i] = f_s[i] + f_{s-1}[stride + i]   (the second term while stride + i < n_tx; zero past len)
 // psd_masked_kernel reads its slices straight from Y by that rule, so no assembled stream is written.  The unmasked
-// stream is the same product with the mask's impulse response replaced by a unit impulse (mask_gemm_setup, unit_impulse):
-// the two spectra come from one code path on identical symbols.
+// stream is the same product with the mask's impulse response replaced by a unit impulse (mask_gemm_setup, roll-off 0):
+// every requested spectrum -- masked and unmasked, of every configuration -- is one pair of a single product, so a batch's
+// symbols are drawn once and all spectra come from one code path on identical symbols.
 //
-// One CTA of 256 threads works on G = 256 / (8N/16) slices of one frame at a time (4 / 2 / 1 for N = 128 / 256 / 512):
+// Spectrum p is blockIdx.y.  One CTA of 256 threads works on G = 256 / (8N/16) slices of one frame at a time (4 / 2 / 1 for
+// N = 128 / 256 / 512):
 // each thread loads its 16 samples of its slice, applies the taper (estimator 1), runs the 8N-point register FFT and
 // keeps |X|^2 in fp64 registers over all of the CTA's items; one fftshift-indexed atomicAdd(double) per bin and CTA at
 // the end, as psd_kernel (psd.cu) does.  fp32 arithmetic, fp64 accumulation.
@@ -22,7 +24,8 @@ namespace wofdm {
 namespace {
 
 struct PsdMaskedParams {
-    const float* Y;                // [frames * S][Yp]: the filtered symbols of the batch, (Re, Im) interleaved
+    const float* Y;                // [spectra][frames * S][Yp]: the filtered symbols of the batch, (Re, Im) interleaved
+    long long ypair;               // floats between two spectra's columns (MaskGemm::ypair)
     int Yp, S, stride, n_tx;
     int len;                       // samples of a frame's stream: tail_tx + S * stride
     int n_slices;                  // slices per frame
@@ -31,7 +34,7 @@ struct PsdMaskedParams {
     int hann;                      // taper sin^2(pi n / 8N)
     long long items;               // frames of the batch * groups
     const float2* twp;             // twiddles of the 8N-point transform
-    double* psd;                   // [8N], sum over slices and frames
+    double* psd;                   // [spectra][8N], sum over slices and frames
 };
 
 template <int N>
@@ -60,7 +63,7 @@ __global__ void __launch_bounds__(256, 2) psd_masked_kernel(const PsdMaskedParam
         const int k = (int)(it - fl * p.groups) * G + slot;
         const bool live = k < p.n_slices;
         const int a0 = k * p.hop;
-        const float* yf = p.Y + (size_t)fl * p.S * p.Yp;
+        const float* yf = p.Y + (size_t)blockIdx.y * p.ypair + (size_t)fl * p.S * p.Yp;
         float2 v[16];
 #pragma unroll
         for (int q = 0; q < 16; ++q) {
@@ -82,7 +85,7 @@ __global__ void __launch_bounds__(256, 2) psd_masked_kernel(const PsdMaskedParam
     }
     // fftshift: bin k of the transform is entry (k + P/2) mod P of the estimate
 #pragma unroll
-    for (int q = 0; q < 16; ++q) atomicAdd(&p.psd[(t + q * TPF + P / 2) & (P - 1)], acc[q]);
+    for (int q = 0; q < 16; ++q) atomicAdd(&p.psd[(size_t)blockIdx.y * P + ((t + q * TPF + P / 2) & (P - 1))], acc[q]);
 }
 
 template <int N> size_t psd_masked_smem() {
@@ -90,12 +93,13 @@ template <int N> size_t psd_masked_smem() {
     return ((size_t)PP::NTW + (size_t)(256 / PP::TPF) * PP::XLEN) * sizeof(float2);
 }
 
-// one batch's frames of one half (its product already in mg.Y) into psd
-template <int N> cudaError_t psd_masked_launch(const DeviceCtx& d, PsdMaskedParams p) {
+// one batch's frames of all n_spec spectra (their product already in Y) into psd: about two CTAs per SM in all
+template <int N> cudaError_t psd_masked_launch(const DeviceCtx& d, PsdMaskedParams p, int n_spec) {
     const size_t sm = psd_masked_smem<N>();
     const cudaError_t e = cudaFuncSetAttribute(psd_masked_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
     if (e != cudaSuccess) return e;
-    psd_masked_kernel<N><<<(int)std::min<long long>(p.items, 2LL * d.sm_count), 256, sm, d.stream>>>(p);
+    const int gx = (int)std::min<long long>(p.items, std::max(1, 2 * d.sm_count / n_spec));
+    psd_masked_kernel<N><<<dim3(gx, n_spec), 256, sm, d.stream>>>(p);
     return cudaGetLastError();
 }
 
@@ -126,13 +130,22 @@ using namespace wofdm;
 
 extern "C" int wofdm_psd_masked(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, int roll_off, uint64_t seed,
                                 int64_t f0, int64_t n_frames, int estimator, double* psd_masked, double* psd_unmasked) {
+    return wofdm_psd_masked_multi(h, sys, win_tx, &roll_off, 1, seed, f0, n_frames, estimator, psd_masked, psd_unmasked);
+}
+
+extern "C" int wofdm_psd_masked_multi(wofdm_handle h, const wofdm_sys_t* sys, const double* win_tx, const int* roll_off,
+                                      int n_var, uint64_t seed, int64_t f0, int64_t n_frames, int estimator, double* psd_masked,
+                                      double* psd_unmasked) {
     NvtxRange nvtx_("wofdm_psd_masked");
     if (!h) return WOFDM_EINVAL;
     if (!win_tx) return fail(h, WOFDM_EINVAL, "win_tx is NULL");
     if (!psd_masked && !psd_unmasked) return fail(h, WOFDM_EINVAL, "both outputs are NULL");
     if (f0 < 0 || n_frames < 1 || f0 > INT64_MAX - n_frames) return fail(h, WOFDM_EINVAL, "bad frame range (f0 >= 0, n_frames >= 1, no overflow)");
     if (estimator != 0 && estimator != 1) return fail(h, WOFDM_EINVAL, "estimator must be 0 (reference) or 1 (Hann, 50 % overlap)");
-    int rc = check_masked_tx(h, sys, roll_off);
+    if (n_var < 1 || n_var > WOFDM_MAX_VARIANTS) return fail(h, WOFDM_EINVAL, "n_var must be in [1, WOFDM_MAX_VARIANTS]");
+    if (!roll_off) return fail(h, WOFDM_EINVAL, "NULL roll_off");
+    int rc = WOFDM_OK;
+    for (int v = 0; v < n_var && !rc; ++v) rc = check_masked_tx(h, sys, roll_off[v]);
     if (rc) return rc;
     const int N = sys->N, P = 8 * N, n_tx = N + sys->cp + sys->cs, stride = n_tx - sys->tail_tx;
     const long long len = (long long)sys->tail_tx + (long long)sys->S * stride;
@@ -148,51 +161,56 @@ extern "C" int wofdm_psd_masked(wofdm_handle h, const wofdm_sys_t* sys, const do
     // 131 072 (DESIGN.md 4b): the product's tail wave and the launches per batch cost more than re-reading Y from HBM
     const long long cols = 131072;
     const long long batch = std::min<long long>(n_frames, std::max<long long>(1, cols / sys->S));
-    const std::vector<double> wd = tx_table(*sys, win_tx, false);
-    const std::vector<float> wf(wd.begin(), wd.end());
+    // the spectra as pairs of one product: the masked ones (window v, roll_off[v]), then the unmasked ones (window v, a unit
+    // impulse); spectrum k goes to outs[k]
+    std::vector<float> wf;
+    std::vector<int> ro;
+    std::vector<double*> outs;
+    for (int half = 0; half < 2; ++half) {
+        double* o = half == 0 ? psd_masked : psd_unmasked;
+        if (!o) continue;
+        for (int v = 0; v < n_var; ++v) {
+            const std::vector<double> wd = tx_table(*sys, win_tx + (size_t)v * n_tx, false);
+            wf.insert(wf.end(), wd.begin(), wd.end());
+            ro.push_back(half == 0 ? roll_off[v] : 0);
+            outs.push_back(o + (size_t)v * P);
+        }
+    }
+    const int n_spec = (int)outs.size();
     const std::vector<double> twd = build_twiddles(P);
     const std::vector<float> twf(twd.begin(), twd.end());
-    double* outs[2] = {psd_masked, psd_unmasked};
-    MaskGemm mg[2];
-    size_t need = wf.size() * 4 + twf.size() * 4 + 2 * (size_t)P * 8;
-    for (int k = 0; k < 2; ++k)
-        if (outs[k]) need += mask_gemm_plan(*sys, batch, 1, mg[k]);
+    MaskGemm mg;
+    const size_t need = wf.size() * 4 + twf.size() * 4 + (size_t)n_spec * P * 8 + mask_gemm_plan(*sys, batch, n_spec, mg);
     rc = arena_reserve(h, d, need);
     if (rc) return rc;
     float* d_w = static_cast<float*>(arena_take(d, wf.size() * 4));
     float2* d_twp = static_cast<float2*>(arena_take(d, twf.size() * 4));
-    double* d_psd = static_cast<double*>(arena_take(d, 2 * (size_t)P * 8));
+    double* d_psd = static_cast<double*>(arena_take(d, (size_t)n_spec * P * 8));
     if (!d_w || !d_twp || !d_psd) return fail(h, WOFDM_ENOMEM, "arena exhausted");
     WOFDM_CUDA(h, cudaMemcpyAsync(d_w, wf.data(), wf.size() * 4, cudaMemcpyHostToDevice, d.stream));
     WOFDM_CUDA(h, cudaMemcpyAsync(d_twp, twf.data(), twf.size() * 4, cudaMemcpyHostToDevice, d.stream));
-    WOFDM_CUDA(h, cudaMemsetAsync(d_psd, 0, 2 * (size_t)P * 8, d.stream));
+    WOFDM_CUDA(h, cudaMemsetAsync(d_psd, 0, (size_t)n_spec * P * 8, d.stream));
 
     auto run = [&]() -> int {
-        for (int k = 0; k < 2; ++k) {
-            if (!outs[k]) continue;
-            const int r = mask_gemm_setup(h, d, mg[k], &roll_off, d_w, k == 1);
-            if (r) return r;
-        }
+        const int r = mask_gemm_setup(h, d, mg, ro.data(), d_w);
+        if (r) return r;
         PsdMaskedParams p;
         memset(&p, 0, sizeof(p));
-        p.Yp = mg[outs[0] ? 0 : 1].Yp; p.S = sys->S; p.stride = stride; p.n_tx = n_tx; p.len = (int)len;
-        p.n_slices = n_slices; p.groups = groups; p.hop = hop; p.hann = estimator == 1; p.twp = d_twp;
+        p.Y = mg.Y; p.ypair = mg.ypair; p.Yp = mg.Yp; p.S = sys->S; p.stride = stride; p.n_tx = n_tx; p.len = (int)len;
+        p.n_slices = n_slices; p.groups = groups; p.hop = hop; p.hann = estimator == 1; p.twp = d_twp; p.psd = d_psd;
         for (long long fb = f0; fb < f0 + n_frames; fb += batch) {
             const long long nf = std::min(batch, f0 + n_frames - fb);
-            for (int k = 0; k < 2; ++k) {
-                if (!outs[k]) continue;
-                const int r = mask_gemm_batch(h, d, mg[k], seed, fb, nf);
-                if (r) return r;
-                p.Y = mg[k].Y; p.items = nf * groups; p.psd = d_psd + (size_t)k * P;
-                cudaError_t e = cudaSuccess;
-                switch (N) {
-                    case 128: e = psd_masked_launch<128>(d, p); break;
-                    case 256: e = psd_masked_launch<256>(d, p); break;
-                    default:  e = psd_masked_launch<512>(d, p); break;
-                }
-                WOFDM_CUDA(h, e);
-                h->launches += 1;
+            const int rb = mask_gemm_batch(h, d, mg, seed, fb, nf);
+            if (rb) return rb;
+            p.items = nf * groups;
+            cudaError_t e = cudaSuccess;
+            switch (N) {
+                case 128: e = psd_masked_launch<128>(d, p, n_spec); break;
+                case 256: e = psd_masked_launch<256>(d, p, n_spec); break;
+                default:  e = psd_masked_launch<512>(d, p, n_spec); break;
             }
+            WOFDM_CUDA(h, e);
+            h->launches += 1;
         }
         return WOFDM_OK;
     };
@@ -201,13 +219,12 @@ extern "C" int wofdm_psd_masked(wofdm_handle h, const wofdm_sys_t* sys, const do
         cudaStreamSynchronize(d.stream);
         return rc;
     }
-    std::vector<double> acc(2 * (size_t)P);
+    std::vector<double> acc((size_t)n_spec * P);
     WOFDM_CUDA(h, cudaMemcpyAsync(acc.data(), d_psd, acc.size() * 8, cudaMemcpyDeviceToHost, d.stream));
     WOFDM_CUDA(h, cudaStreamSynchronize(d.stream));
     // mean periodogram; the Hann slices carry 8N / sum(w^2) = 8/3, so a white stream reads the same level under both estimators
     const double scale = (estimator == 1 ? 8.0 / 3.0 : 1.0) / ((double)n_slices * (double)n_frames);
-    for (int k = 0; k < 2; ++k)
-        if (outs[k])
-            for (int i = 0; i < P; ++i) outs[k][i] = acc[(size_t)k * P + i] * scale;
+    for (int k = 0; k < n_spec; ++k)
+        for (int i = 0; i < P; ++i) outs[k][i] = acc[(size_t)k * P + i] * scale;
     return WOFDM_OK;
 }

@@ -278,6 +278,41 @@ def run_sim_mc_adaptive(ensemble_max, cpLength, csLength, tailTx, tailRx, window
     return r["bit_err"][0] / r["bit_tot"], r["bit_err"][1] / r["bit_tot"], r["ensemble_used"]
 
 
+def _roll_off_list(rollOff, n_var):
+    """rollOff as n_var integers: one value for every configuration, or a list of n_var"""
+    ros = [int(x) for x in np.atleast_1d(rollOff)]
+    if len(ros) == 1:
+        ros = ros * n_var
+    if len(ros) != n_var:
+        raise ValueError(f"rollOff must be one value or {n_var} of them (got {len(ros)})")
+    return ros
+
+
+def run_sim_mc_multi_adaptive(ensemble_max, cpLength, csLength, tailTx, tailRx, windowTx, windowRx, channel, snr, offset,
+                              prefixRemovalLength, circularShiftLength, numSubcar, bitsPerSubcar, symbolsPerTx, rollOff,
+                              target_bit_errors, first_block=1, seed=0, handle=None):
+    """run_sim_mc_adaptive for n_var configurations on the same symbols in one call
+    (Handle.ber_run_masked_adaptive_multi): windowTx and windowRx are lists of n_var (diagonal matrices or vectors),
+    rollOff one integer or n_var of them.  Configuration v's unmasked chain has noise stream v, its masked chain n_var + v,
+    as in run_sim_mc_multi; every SNR point runs until all 2 n_var chains have counted target_bit_errors bit errors, or
+    ensemble_max ensemble indices.  Returns (berMasked, ber, ensemble_used) of shapes (n_var, n_snr), (n_var, n_snr) and
+    (n_snr,); with one configuration this is run_sim_mc_adaptive's result exactly."""
+    wts, wrs = list(windowTx), list(windowRx)
+    if len(wts) != len(wrs) or not wts:
+        raise ValueError(f"windowTx and windowRx must be lists of the same length (got {len(wts)}, {len(wrs)})")
+    ros = _roll_off_list(rollOff, len(wts))
+    h = handle or default_handle()
+    s = capi.SysT(N=int(numSubcar), cp=int(cpLength), cs=int(csLength), tail_tx=int(tailTx), tail_rx=int(tailRx),
+                  rm=int(prefixRemovalLength), shift=int(circularShiftLength), bits=int(bitsPerSubcar),
+                  S=int(symbolsPerTx), noise_norm=1, constellation=1, precision=0, guard=int(offset))
+    ch = np.atleast_2d(np.asarray(channel)).T                         # (L, C)
+    r = h.ber_run_masked_adaptive_multi(s, [_diag(w) for w in wts], [_diag(w) for w in wrs], ch,
+                                        np.atleast_1d(np.asarray(snr, dtype=np.float64)), int(ensemble_max),
+                                        target_bit_errors=int(target_bit_errors), first_block=int(first_block), seed=seed,
+                                        variant=0, roll_offs=ros)
+    return r["bit_err"][0] / r["bit_tot"], r["bit_err"][1] / r["bit_tot"], r["ensemble_used"]
+
+
 def obr_split(x, offset):
     """(obr, mf_band) of an 8N-point fftshifted PSD of a guard-band signal: the guard band is the first and the last
     8*offset bins (8x interpolation), its mean the out-of-band radiation; mf_band the bins in between."""
@@ -305,6 +340,33 @@ def psd_sim_mc(numFrames, cpLength, csLength, tailTx, windowTx, offset, numSubca
     out = {"X_est_masked": xm, "X_est": xu, "f_axis": np.linspace(-.5, .5 - 1 / (8 * N), 8 * N)}
     out["obr_masked"], out["mf_band_masked"] = obr_split(xm, offset)
     out["obr"], out["mf_band"] = obr_split(xu, offset)
+    return out
+
+
+def psd_sim_mc_multi(numFrames, cpLength, csLength, tailTx, windowTx, offset, numSubcar, bitsPerSubcar, symbolsPerTx,
+                     rollOff, seed=0, estimator="reference", handle=None):
+    """psd_sim_mc for n_var configurations on the same frames in one call (Handle.psd_masked_multi): windowTx a list of
+    n_var Tx windows (diagonal matrices or vectors), rollOff one integer or n_var of them.  The same keys as psd_sim_mc,
+    one row per configuration: X_est_masked / X_est (n_var, 8N), obr_masked / obr (n_var,), mf_band_masked / mf_band
+    (n_var, 8N - 16 offset), and f_axis.  With one configuration it equals psd_sim_mc up to the order of fp64 additions."""
+    if int(offset) < 1:
+        raise ValueError("the OBR needs offset >= 1")
+    wts = list(windowTx)
+    if not wts:
+        raise ValueError("windowTx must be a non-empty list")
+    ros = _roll_off_list(rollOff, len(wts))
+    h = handle or default_handle()
+    N = int(numSubcar)
+    s = capi.SysT(N=N, cp=int(cpLength), cs=int(csLength), tail_tx=int(tailTx), bits=int(bitsPerSubcar),
+                  S=int(symbolsPerTx), noise_norm=1, constellation=1, precision=0, guard=int(offset))
+    xm, xu = h.psd_masked_multi(s, [_diag(w) for w in wts], roll_offs=ros, frames=int(numFrames), seed=seed,
+                                estimator=estimator)
+    out = {"X_est_masked": xm, "X_est": xu, "f_axis": np.linspace(-.5, .5 - 1 / (8 * N), 8 * N)}
+    for key, x in (("masked", xm), ("", xu)):
+        parts = [obr_split(row, offset) for row in x]
+        sfx = "_" + key if key else ""
+        out["obr" + sfx] = np.array([p[0] for p in parts])
+        out["mf_band" + sfx] = np.stack([p[1] for p in parts])
     return out
 
 
